@@ -3,12 +3,18 @@
 shows/sec to top-20, TFLOP/s vs peak, at 1/2/4/8 B200, beside the host-CPU reference).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C3] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole synthetic catalogue: K0 prep kernels ->
 K1 tcgen05 candidate pass -> K5 fp64 rescore/certify -> K6 exact repair (with N GPUs > 1: candidate
 lists exchanged by all-to-all before K5, [N, k] tables all-gathered after K6).  ``value`` is timed with the raw features already resident in HBM;
 ``e2e`` adds, inside the timed region, the H2D copy of the staged (pinned) feature buffers and the
 D2H read of the result table through the public engine API.  Prints ONE JSON line on rank 0.
+
+``--dump-outputs DIR`` writes the table the last timed step of ``value`` computed (indices, counts
+and the four score columns, as float64 ``DIR/<name>.npy``, plus ``rows``: the source rows they
+cover), so that two builds can be compared output for output.  The inputs are seeded: the same
+arguments give the same inputs on every run.
 """
 
 from __future__ import annotations
@@ -30,6 +36,19 @@ sys.path.insert(0, str(ROOT))
 
 METRIC = "shows_per_sec_to_top_k"
 UNIT = "shows/s"
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def output_sample(table, limit: int = DUMP_LIMIT_BYTES, seed: int = 0) -> dict:
+    """A host result table as float64 arrays of at most ``limit`` bytes in all: every row when it
+    fits, else a fixed seeded sample of source rows (ascending).  ``rows`` names the rows kept."""
+    n, k = table.indices.shape
+    row_bytes = 8 * (5 * k + 2)                        # five [k] columns, the count and the row number
+    cap = (limit - 4096) // row_bytes                  # 4 KB for the seven .npy headers
+    rows = np.arange(n) if n <= cap else np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+    out = {"rows": rows + table.row_begin}
+    out.update({f: getattr(table, f)[rows] for f in ("indices", "counts", "hybrid", "genre", "text", "metadata")})
+    return {name: np.asarray(a, dtype=np.float64) for name, a in out.items()}
 
 
 def _peaks() -> dict:
@@ -457,7 +476,13 @@ def main() -> None:
     ap.add_argument("--splits", type=int, default=0)
     ap.add_argument("--one-sided", action="store_true", help="disable the symmetric sweep at N > 1")
     ap.add_argument("--tuning", type=lambda x: int(x, 0), default=0, help="tvbf_params.tuning bitfield")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the table of the last timed step as DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the tables of --impl b200")
 
     from tvbingefriend_recommendation_service_b200.synthetic import CONFIGS, make_config
 
@@ -575,7 +600,7 @@ def main() -> None:
     ev0.record()
     host_t0 = time.perf_counter()
     for _ in range(args.steps):
-        step_device(events)
+        last = step_device(events)
     host_enqueue_ms = 1e3 * (time.perf_counter() - host_t0) / args.steps   # host time to ISSUE a step (no sync inside)
     ev1.record()
     sync()
@@ -588,6 +613,9 @@ def main() -> None:
             print("step", i, [round(events[a][i].elapsed_time(events[b][i]), 2) for a, b in zip(order, order[1:])],
                   file=sys.stderr)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = None
+    if args.dump_outputs and rank == 0:     # read back before the e2e steps overwrite these tables
+        dumped = output_sample(eng.to_host(last))
     t_ms = torch.tensor([total_ms, ph["seed"] + ph["sweep"]] + [ph[name] for name in PHASES], device="cuda",
                         dtype=torch.float64)
     t_min = t_ms.clone()
@@ -784,6 +812,13 @@ def main() -> None:
                                               line["parity_check"]["device_gathered_table_identical_to_single_gpu"])
     if not args.no_cpu_baseline and world == 1:      # rank 0 at N=1 only
         line["cpu_baseline"] = cpu_baseline(cat, cfg, weights, budget_s=20.0)
+    if dumped is not None:
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(out_dir / f"{name}.npy", arr)
+        line["dump_outputs"] = {"dir": str(out_dir), "rows": int(len(dumped["rows"])), "of_rows": n,
+                                "arrays": sorted(dumped)}
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
