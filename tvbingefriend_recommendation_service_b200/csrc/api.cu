@@ -457,6 +457,7 @@ size_t tvbf_topk_workspace_bytes(const tvbf_features* f, const tvbf_params* p) {
 
 int tvbf_hybrid_topk(const tvbf_features* f, const tvbf_params* p, const tvbf_topk_out* out,
                      void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   rc = validate_params(f, p);
@@ -557,6 +558,7 @@ size_t tvbf_topk_sweep_workspace_bytes(const tvbf_features* f, const tvbf_params
 int tvbf_hybrid_topk_sweep(const tvbf_features* f, const tvbf_params* p, int32_t n_weights,
                            const tvbf_topk_out* out, void* workspace, size_t workspace_bytes,
                            void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(out != nullptr && workspace != nullptr, "tvbf_hybrid_topk_sweep: NULL argument");
@@ -720,8 +722,8 @@ size_t tvbf_sym_workspace_bytes(const tvbf_features* f, const tvbf_params* p, in
   return sp.total;
 }
 
-int tvbf_sym_seed(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
-                  uint32_t* theta, void* workspace, size_t workspace_bytes, void* stream) {
+static int sym_seed_impl(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
+                         uint32_t* theta, void* workspace, size_t workspace_bytes, void* stream) {
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(theta && workspace, "tvbf_sym_seed: NULL buffer");
@@ -742,10 +744,18 @@ int tvbf_sym_seed(const tvbf_features* f, const tvbf_params* p, int32_t rank, in
   return tvbf::k1_launch(f, kp, sp.pl.entries, 2, sp.pl.grid, st);
 }
 
-static int sym_sweep_impl(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
-                          uint32_t* theta, void* cand, int32_t* cand_cnt, float* cand_bound,
-                          const uint64_t* peer_ptrs, int32_t shard_rows, void* workspace, size_t workspace_bytes,
-                          void* stream) {
+int tvbf_sym_seed(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
+                  uint32_t* theta, void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  const int rc = sym_seed_impl(f, p, rank, world, theta, workspace, workspace_bytes, stream);
+  if (rc != TVBF_OK) tvbf_absorb_pending_clear(stream);   // no sweep may trust a failed seed's clear
+  return rc;
+}
+
+static int sym_sweep_phase(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
+                           uint32_t* theta, void* cand, int32_t* cand_cnt, float* cand_bound,
+                           const uint64_t* peer_ptrs, int32_t shard_rows, void* workspace, size_t workspace_bytes,
+                           void* stream) {
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(theta && workspace && (cand || peer_ptrs), "tvbf_sym_sweep: NULL buffer");
@@ -785,11 +795,23 @@ static int sym_sweep_impl(const tvbf_features* f, const tvbf_params* p, int32_t 
     rc = tvbf::k1_launch(f, kp, sp.pl.entries, 2, sp.pl.grid, st);
     if (rc != TVBF_OK) return rc;
   } else {
-    rc = tvbf::k1_join_pending_clear(kp.g_list, st);
+    rc = tvbf_absorb_pending_clear(stream);
     if (rc != TVBF_OK) return rc;
     TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, static_cast<size_t>(f->n_pad) * 4, st));
   }
   return tvbf::k4s_launch(kp, f->n_shows, st);
+}
+
+static int sym_sweep_impl(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
+                          uint32_t* theta, void* cand, int32_t* cand_cnt, float* cand_bound,
+                          const uint64_t* peer_ptrs, int32_t shard_rows, void* workspace, size_t workspace_bytes,
+                          void* stream) {
+  int rc = tvbf_enter_call(stream, 1);
+  if (rc != TVBF_OK) return rc;
+  rc = sym_sweep_phase(f, p, rank, world, theta, cand, cand_cnt, cand_bound, peer_ptrs, shard_rows, workspace,
+                       workspace_bytes, stream);
+  if (rc != TVBF_OK) tvbf_absorb_pending_clear(stream);
+  return rc;
 }
 
 int tvbf_sym_sweep(const tvbf_features* f, const tvbf_params* p, int32_t rank, int32_t world,
@@ -812,6 +834,7 @@ int tvbf_rescore_lists(const tvbf_features* f, const tvbf_params* p, const void*
                        const int32_t* cnt_all, const float* bound_all, int32_t lists,
                        int32_t table_row0, int32_t table_rows, const tvbf_topk_out* out,
                        void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   rc = validate_params(f, p);
@@ -855,6 +878,7 @@ size_t tvbf_stats_accum_bytes(void) { return sizeof(tvbf::StatsAccum); }
 
 int tvbf_similarity_stats(const tvbf_features* f, const tvbf_params* p, void* accum, void* workspace,
                           size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(p && accum && workspace, "tvbf_similarity_stats: NULL argument");
@@ -920,6 +944,7 @@ int tvbf_similarity_stats(const tvbf_features* f, const tvbf_params* p, void* ac
 
 int tvbf_score_pairs(const tvbf_features* f, const tvbf_params* p, const int32_t* pairs,
                      int32_t n_pairs, double* out4, void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(p && pairs && out4 && n_pairs > 0, "tvbf_score_pairs: bad arguments");
@@ -937,6 +962,7 @@ size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed)
 int tvbf_exact_rows(const tvbf_features* f, const tvbf_params* p, const int32_t* rows,
                     int32_t n_rows_listed, const tvbf_topk_out* out, void* workspace,
                     size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   int rc = validate_features(f);
   if (rc != TVBF_OK) return rc;
   TVBF_REQUIRE(p && p->k >= 1 && rows && n_rows_listed > 0, "tvbf_exact_rows: bad arguments");
@@ -962,6 +988,7 @@ int tvbf_matrix_rows_topk(const double* hybrid, const double* genre, const doubl
                           const double* metadata, int32_t n, const tvbf_params* p,
                           const int32_t* rows, int32_t n_rows_listed, const tvbf_topk_out* out,
                           void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(hybrid && genre && text && metadata && n > 0, "tvbf_matrix_rows_topk: bad matrices");
   TVBF_REQUIRE(p && p->k >= 1 && rows && n_rows_listed > 0, "tvbf_matrix_rows_topk: bad arguments");
   TVBF_REQUIRE(out && out->indices && out->counts && out->hybrid && out->genre && out->text &&
@@ -1097,11 +1124,13 @@ int32_t tvbf_debug_schedule(int32_t col_tiles, int32_t super_blocks, int32_t sb_
 
 int tvbf_debug_gemm_tile(const tvbf_features* f, int32_t row0, int32_t col0, float* out,
                          void* stream) {
+  TVBF_ENTER_CALL(stream);
   return debug_tile(f, row0, col0, out, 1, stream);
 }
 
 int tvbf_debug_gemm_tile_pair(const tvbf_features* f, int32_t row0, int32_t col0, float* out,
                               void* stream) {
+  TVBF_ENTER_CALL(stream);
   return debug_tile(f, row0, col0, out, 2, stream);
 }
 

@@ -17,6 +17,13 @@
 void tvbf_set_error(const char* fmt, ...);
 void tvbf_count_launch(void);  // every kernel launch of the library is counted (tvbf_kernel_launches)
 void tvbf_count_coop_fallback(void);  // K1 launches that fell back from cooperative to plain
+// Every ABI call that enqueues device work enters here first (TVBF_ENTER_CALL): it is numbered per
+// device and orders `stream` after a pending shared-list clear of the symmetric sweep (hybrid_topk.cu)
+// -- except a sweep-only call (sym_sweep = 1), which may be the one that clear was started for.
+int tvbf_enter_call(void* stream, int sym_sweep);
+// `stream` waits for every shared-list clear started on this device; the pending one is forgotten
+// (error returns of the seed / sweep calls, and a sweep call that launches no candidate pass)
+int tvbf_absorb_pending_clear(void* stream);
 
 #define TVBF_CUDA_OK(expr)                                                              \
   do {                                                                                  \
@@ -34,6 +41,12 @@ void tvbf_count_coop_fallback(void);  // K1 launches that fell back from coopera
       tvbf_set_error(__VA_ARGS__);                                                      \
       return TVBF_ERR_INVALID;                                                          \
     }                                                                                   \
+  } while (0)
+
+#define TVBF_ENTER_CALL(stream)                                                         \
+  do {                                                                                  \
+    int _rc = tvbf_enter_call((stream), 0);                                             \
+    if (_rc != TVBF_OK) return _rc;                                                     \
   } while (0)
 
 #define TVBF_LAUNCH_OK(name)                                                            \

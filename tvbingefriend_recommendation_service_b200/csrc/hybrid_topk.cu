@@ -1479,10 +1479,20 @@ void k1_executed_tiles(const K1Params& kp, int grid, long long* out) {
 // sweep, so it runs on a side stream beside it.  One side stream + event pair per device, created on
 // first use; `pending` remembers a clear started by a seed-only call (multi-GPU: the caller's
 // all-reduce sits between the two calls) for the sweep-only call that follows.
+//
+// A sweep-only call skips its own clear only when the pending clear covers exactly its lists and no
+// other libtvbf call has enqueued work on the device since the seed-only call that started it: every
+// such call is numbered per device (tvbf_enter_call), and the sweep must be the very next one.  Any
+// other call first orders its stream after the pending clear and drops it -- an abandoned seed's clear
+// can then neither be trusted by a later job nor race with the writes of one.
 struct SideStream {
   cudaStream_t stream = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
-  const void* pending = nullptr;
+  const void* pending = nullptr;          // g_list of the clear the last seed-only call started
+  const void* pending_cnt = nullptr;      // ... its g_cnt
+  size_t pending_bytes = 0;               // ... bytes of g_list cleared
+  unsigned long long pending_call = 0;    // number of that seed-only call
+  unsigned long long calls = 0;           // libtvbf calls that enqueued work on this device
 };
 static std::mutex g_side_mutex;
 static SideStream g_side[64];
@@ -1504,19 +1514,45 @@ static int side_stream(SideStream** out) {
   return TVBF_OK;
 }
 
-// a sweep-only call that launches nothing (a GPU without super blocks) still has to absorb the clear
-// its seed-only call started
-int k1_join_pending_clear(const void* g_list, cudaStream_t st) {
-  std::lock_guard<std::mutex> lock(g_side_mutex);
-  SideStream* side = nullptr;
-  int rc = side_stream(&side);
-  if (rc != TVBF_OK) return rc;
-  if (side->pending == g_list && g_list != nullptr) {
-    TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
-    side->pending = nullptr;
-  }
+// st waits for the pending clear, which is forgotten.  `always`: st waits for the side stream's last
+// clear even when none is pending -- a sweep's own clear may have been absorbed by another call, on
+// another stream.  Caller holds g_side_mutex.
+static int absorb_pending(SideStream* s, cudaStream_t st, bool always) {
+  if (s->pending == nullptr && !(always && s->join != nullptr)) return TVBF_OK;
+  s->pending = nullptr;
+  TVBF_CUDA_OK(cudaStreamWaitEvent(st, s->join, 0));
   return TVBF_OK;
 }
+
+}  // namespace tvbf
+
+// The state of the current device, or nullptr without one.  Sets no error: without a device the
+// call's own argument checks or its first CUDA call report what is wrong.
+static tvbf::SideStream* current_side() {
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) {
+    cudaGetLastError();
+    return nullptr;
+  }
+  return &tvbf::g_side[dev];
+}
+
+int tvbf_enter_call(void* stream, int sym_sweep) {
+  std::lock_guard<std::mutex> lock(tvbf::g_side_mutex);
+  tvbf::SideStream* s = current_side();
+  if (s == nullptr) return TVBF_OK;
+  ++s->calls;
+  // a sweep-only call decides in k1_launch, where it knows its lists
+  return sym_sweep ? TVBF_OK : tvbf::absorb_pending(s, static_cast<cudaStream_t>(stream), false);
+}
+
+int tvbf_absorb_pending_clear(void* stream) {
+  std::lock_guard<std::mutex> lock(tvbf::g_side_mutex);
+  tvbf::SideStream* s = current_side();
+  return s == nullptr ? TVBF_OK : tvbf::absorb_pending(s, static_cast<cudaStream_t>(stream), true);
+}
+
+namespace tvbf {
 
 int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, int cta_group,
               int grid, cudaStream_t st) {
@@ -1532,6 +1568,7 @@ int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, 
     const int n_pad = f->n_pad;
     const int nw = kp.n_weights > 1 ? kp.n_weights : 1;   // weight sweep: nw * n_pad virtual shows
     const size_t n_virtual = static_cast<size_t>(nw) * n_pad;
+    const size_t list_bytes = n_virtual * kp.sym_cap * 8;
     std::lock_guard<std::mutex> lock(g_side_mutex);
     SideStream* side = nullptr;
     int rcs = side_stream(&side);
@@ -1542,9 +1579,12 @@ int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, 
       TVBF_CUDA_OK(cudaEventRecord(side->fork, st));
       TVBF_CUDA_OK(cudaStreamWaitEvent(side->stream, side->fork, 0));
       TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, n_virtual * 4, side->stream));
-      TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, n_virtual * kp.sym_cap * 8, side->stream));
+      TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, side->stream));
       TVBF_CUDA_OK(cudaEventRecord(side->join, side->stream));
       side->pending = kp.g_list;
+      side->pending_cnt = kp.g_cnt;
+      side->pending_bytes = list_bytes;
+      side->pending_call = side->calls;
       cleared = true;
     }
     if (kp.sym_phase != 2) {
@@ -1575,13 +1615,18 @@ int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, 
       }
       if (kp.sym_phase == 1) return TVBF_OK;   // the sweep-only call joins the clear
     }
-    if (!cleared && side->pending == kp.g_list) cleared = true;   // started by the preceding seed-only call
+    // a sweep-only call right after the seed-only call that started the clear of these lists
+    if (!cleared && kp.sym_phase == 2 && side->pending == kp.g_list && side->pending_cnt == kp.g_cnt &&
+        side->pending_bytes == list_bytes && side->calls == side->pending_call + 1)
+      cleared = true;
     if (cleared) {
       TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
       side->pending = nullptr;
     } else {
+      const int rca = absorb_pending(side, st, true);
+      if (rca != TVBF_OK) return rca;
       TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, n_virtual * 4, st));
-      TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, n_virtual * kp.sym_cap * 8, st));
+      TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, st));
     }
     K1Params sweep = kp;
     sweep.tile_stride = 1;

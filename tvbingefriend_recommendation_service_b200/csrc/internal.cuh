@@ -131,7 +131,6 @@ int k1_default_candidates(int k);
 int k1_choose_splits(int rb_count, int col_tiles, int sm_count);
 int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, int cta_group,
               int grid, cudaStream_t st);
-int k1_join_pending_clear(const void* g_list, cudaStream_t st);
 void k1_executed_tiles(const K1Params& kp, int grid, long long* out2);
 int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cudaStream_t st);
 // candidate list s of shard row r lives in slot  slot_base + r * row_stride + s * list_stride;

@@ -195,6 +195,7 @@ extern "C" {
 
 int tvbf_cosine_matrix_f64(const double* x, int32_t n_rows, int32_t dim, double* out,
                            void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(x && out && n_rows >= 0 && dim > 0, "tvbf_cosine_matrix_f64: bad arguments");
   if (n_rows == 0) return TVBF_OK;
   dim3 grid((n_rows + TS - 1) / TS, (n_rows + TS - 1) / TS);
@@ -205,6 +206,7 @@ int tvbf_cosine_matrix_f64(const double* x, int32_t n_rows, int32_t dim, double*
 
 int tvbf_hybrid_combine_f64(const double* g, const double* t, const double* m, double wg,
                             double wt, double wm, int64_t count, double* out, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(g && t && m && out && count >= 0, "tvbf_hybrid_combine_f64: bad arguments");
   if (count == 0) return TVBF_OK;
   long long blocks = (count + 255) / 256;
@@ -221,6 +223,7 @@ size_t tvbf_matrix_stats_workspace_bytes(void) {
 
 int tvbf_matrix_stats_f64(const double* mat, int32_t n, double* out5_host, void* workspace,
                           size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(mat && out5_host && workspace, "tvbf_matrix_stats_f64: bad arguments");
   TVBF_REQUIRE(n >= 2, "tvbf_matrix_stats_f64: need at least 2 rows (empty upper triangle)");
   if (workspace_bytes < tvbf_matrix_stats_workspace_bytes()) {

@@ -186,6 +186,7 @@ size_t tvbf_text_moments_workspace_bytes(const tvbf_features* f, int32_t with_gr
 
 int tvbf_text_moments(const tvbf_features* f, int32_t with_gram, double* out8, void* workspace,
                       size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   // out8 has TVBF_MOMENTS (24) entries: [0..7] the text moments, [8..12] sum g, g^2, m, m^2, g*m,
   // [13..17] their diagonal terms
   TVBF_REQUIRE(f && out8 && workspace, "tvbf_text_moments: NULL argument");

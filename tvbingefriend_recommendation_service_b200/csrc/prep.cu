@@ -324,6 +324,7 @@ extern "C" {
 
 int tvbf_prep_csr_normalize(const int64_t* indptr, const double* values, int32_t n_rows,
                             double* values_out, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(indptr && values_out && n_rows >= 0, "tvbf_prep_csr_normalize: bad arguments");
   if (n_rows == 0) return TVBF_OK;
   auto st = static_cast<cudaStream_t>(stream);
@@ -336,6 +337,7 @@ int tvbf_prep_csr_normalize(const int64_t* indptr, const double* values, int32_t
 int tvbf_prep_csr_to_operand(const int64_t* indptr, const int32_t* indices, const double* values,
                              int32_t n_rows, void* operand, int32_t k_pad, int32_t col_offset,
                              double scale, int32_t dtype, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(indptr && operand && n_rows >= 0 && k_pad > 0 && col_offset >= 0,
                "tvbf_prep_csr_to_operand: bad arguments");
   TVBF_REQUIRE(dtype == TVBF_TEXT_FP16 || dtype == TVBF_TEXT_BF16,
@@ -358,6 +360,7 @@ int tvbf_prep_csr_to_operand(const int64_t* indptr, const int32_t* indices, cons
 int tvbf_prep_clear_csr_positions(const int64_t* indptr, const int32_t* indices, int32_t n_rows,
                                   void* operand, int32_t k_pad, int32_t col_offset, int32_t dtype,
                                   void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(indptr && operand && n_rows >= 0 && k_pad > 0 && col_offset >= 0,
                "tvbf_prep_clear_csr_positions: bad arguments");
   TVBF_REQUIRE(dtype == TVBF_TEXT_FP16 || dtype == TVBF_TEXT_BF16,
@@ -377,6 +380,7 @@ int tvbf_prep_clear_csr_positions(const int64_t* indptr, const int32_t* indices,
 
 int tvbf_peer_push(const uint64_t* peer_base, int32_t world, int32_t rank, const uint64_t* offsets,
                    const uint64_t* bytes, int32_t n_fields, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(peer_base && offsets && bytes && world >= 1 && world <= 16 && rank >= 0 && rank < world &&
                    n_fields >= 1 && n_fields <= 8,
                "tvbf_peer_push: bad arguments");
@@ -406,6 +410,7 @@ int tvbf_peer_push(const uint64_t* peer_base, int32_t world, int32_t rank, const
 }
 
 int tvbf_device_zero(void* ptr, size_t bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(ptr != nullptr || bytes == 0, "tvbf_device_zero: NULL pointer");
   if (bytes == 0) return TVBF_OK;
   TVBF_CUDA_OK(cudaMemsetAsync(ptr, 0, bytes, static_cast<cudaStream_t>(stream)));
@@ -414,6 +419,7 @@ int tvbf_device_zero(void* ptr, size_t bytes, void* stream) {
 
 int tvbf_prep_dense_normalize(const double* in, int32_t n_rows, int32_t dim, double* out,
                               void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(in && out && n_rows >= 0 && dim > 0, "tvbf_prep_dense_normalize: bad arguments");
   if (n_rows == 0) return TVBF_OK;
   dense_normalize_kernel<<<blocks_for(n_rows, 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -425,6 +431,7 @@ int tvbf_prep_dense_normalize(const double* in, int32_t n_rows, int32_t dim, dou
 int tvbf_prep_dense_to_operand(const double* dense, int32_t n_rows, int32_t dim, void* operand,
                                int32_t k_pad, int32_t col_offset, double scale, int32_t dtype,
                                void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(dense && operand && n_rows >= 0 && dim > 0 && col_offset >= 0 &&
                    col_offset + dim <= k_pad,
                "tvbf_prep_dense_to_operand: bad arguments");
@@ -446,6 +453,7 @@ int tvbf_prep_dense_to_operand(const double* dense, int32_t n_rows, int32_t dim,
 int tvbf_prep_fold_bits(const void* col_side, const uint64_t* genre_hi, const float* meta_scale,
                         int32_t n_rows, int32_t genre_dim, void* operand, int32_t k_pad, int32_t col0,
                         double scale_genre, double scale_meta, int32_t dtype, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(col_side && meta_scale && operand && n_rows >= 0 && genre_dim >= 1 && genre_dim <= 128 &&
                    col0 >= 0 && col0 + genre_dim + 32 <= k_pad,
                "tvbf_prep_fold_bits: bad arguments");
@@ -470,6 +478,7 @@ int tvbf_prep_fold_bits(const void* col_side, const uint64_t* genre_hi, const fl
 
 int tvbf_prep_genre_bits(const uint8_t* genre, int32_t n_rows, int32_t dim, void* col_side,
                          uint64_t* genre_hi, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(genre && col_side && n_rows >= 0, "tvbf_prep_genre_bits: bad arguments");
   TVBF_REQUIRE(dim >= 1 && dim <= 128, "tvbf_prep_genre_bits: dim %d outside 1..128", dim);
   TVBF_REQUIRE(dim <= 64 || genre_hi != nullptr, "tvbf_prep_genre_bits: dim %d needs genre_hi", dim);
@@ -483,6 +492,7 @@ int tvbf_prep_genre_bits(const uint8_t* genre, int32_t n_rows, int32_t dim, void
 int tvbf_prep_meta_ids(const uint8_t* platform, int32_t p_dim, const uint8_t* type, int32_t t_dim,
                        const uint8_t* language, int32_t l_dim, int32_t n_rows, int32_t n_pad,
                        int32_t meta_kind, void* col_side, float* meta_scale, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(col_side && meta_scale && n_rows >= 0 && n_pad >= n_rows,
                "tvbf_prep_meta_ids: bad arguments");
   TVBF_REQUIRE(p_dim >= 0 && t_dim >= 0 && l_dim >= 0 && p_dim + t_dim + l_dim <= 32,
@@ -499,6 +509,7 @@ int tvbf_prep_meta_ids(const uint8_t* platform, int32_t p_dim, const uint8_t* ty
 
 int tvbf_ingest_genre(const void* raw, int32_t dtype, int32_t n_rows, int32_t n_pad, int32_t dim, void* col_side,
                       uint64_t* genre_hi, int32_t* flags, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(raw && col_side && flags && n_rows >= 0 && n_pad >= n_rows, "tvbf_ingest_genre: bad arguments");
   TVBF_REQUIRE(dim >= 1 && dim <= 128, "tvbf_ingest_genre: dim %d outside 1..128", dim);
   TVBF_REQUIRE(dim <= 64 || genre_hi != nullptr, "tvbf_ingest_genre: dim %d needs genre_hi", dim);
@@ -515,6 +526,7 @@ int tvbf_ingest_meta(const void* platform, int32_t p_dtype, int32_t p_dim, const
                      int32_t t_dim, const void* language, int32_t l_dtype, int32_t l_dim, int32_t n_rows,
                      int32_t n_pad, int32_t meta_kind, void* col_side, float* meta_scale, int32_t* flags,
                      void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(platform && type && language && col_side && meta_scale && flags && n_rows >= 0 && n_pad >= n_rows,
                "tvbf_ingest_meta: bad arguments");
   TVBF_REQUIRE(p_dim >= 0 && t_dim >= 0 && l_dim >= 0 && p_dim + t_dim + l_dim <= 32,
@@ -531,6 +543,7 @@ int tvbf_ingest_meta(const void* platform, int32_t p_dtype, int32_t p_dim, const
 int tvbf_ingest_csr(const void* indptr_raw, int32_t indptr64, const void* indices_raw, int32_t indices64,
                     const void* values_raw, int32_t values64, int32_t n_rows, int64_t* indptr, int32_t* indices,
                     double* values, int32_t* flags, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(indptr_raw && indptr && flags && n_rows >= 0, "tvbf_ingest_csr: bad arguments");
   ingest_csr_kernel<<<blocks_for((static_cast<size_t>(n_rows) + 1) * 32, 256), 256, 0,
                       static_cast<cudaStream_t>(stream)>>>(indptr_raw, indptr64, indices_raw, indices64, values_raw,
@@ -541,6 +554,7 @@ int tvbf_ingest_csr(const void* indptr_raw, int32_t indptr64, const void* indice
 
 int tvbf_csr_to_dense_f64(const int64_t* indptr, const int32_t* indices, const double* values,
                           int32_t n_rows, int32_t dim, double* dense, void* stream) {
+  TVBF_ENTER_CALL(stream);
   TVBF_REQUIRE(indptr && dense && n_rows >= 0 && dim > 0, "tvbf_csr_to_dense_f64: bad arguments");
   if (n_rows == 0) return TVBF_OK;
   csr_to_dense_kernel<<<blocks_for(static_cast<size_t>(n_rows) * 32, 256), 256, 0,

@@ -129,6 +129,7 @@ class DeviceCatalogue:
     text_indices: torch.Tensor | None = None
     fold: dict | None = None               # second operand with the packed groups as K columns (engine._folded)
     buffers: dict = field(default_factory=dict)   # named per-catalogue device buffers a later catalogue can take over
+    h2d_set: tuple | None = None           # (h2d buffer set, its write stamp) when the CSR lives in an h2d(reuse=True) set
 
 
 @dataclass
@@ -227,6 +228,7 @@ class HybridTopKEngine:
         self._fold_buf: torch.Tensor | None = None
         self._fold_owner: dict | None = None      # the catalogue fold whose content the buffer holds
         self._theta: torch.Tensor | None = None    # seeded thresholds of the tile-sharded job (valid until the next job)
+        self._h2d_stamp = 0                         # writes into the h2d(reuse=True) sets so far
 
     @property
     def kernel_launches(self) -> int:
@@ -261,13 +263,18 @@ class HybridTopKEngine:
         """Host -> device copies of the staged buffers on the current stream (no kernels).
         ``reuse``: copy into cached device buffers (two sets used in turn, so a stream of jobs allocates
         nothing and the previous job's arrays -- which ``prepare(recycle=...)`` still reads to un-scatter
-        the operand -- stay intact); the tensors of the call before the previous one are overwritten."""
+        the operand -- stay intact); the tensors of the call before the previous one are overwritten.
+        Each write stamps its set, so ``prepare`` can tell when a recycled catalogue's CSR arrays have
+        been overwritten since (it then zeroes the whole operand instead of un-scattering it); a
+        catalogue whose set has been overwritten must not run jobs any more."""
         dev = self.device
         cache = None
         if reuse:
             gen = self._pinned.setdefault(("h2d_gen",), [0])
             gen[0] ^= 1
             cache = self._pinned.setdefault(("h2d", gen[0]), {})
+            self._h2d_stamp += 1
+            cache["stamp"] = self._h2d_stamp
 
         def up(name: str, h: torch.Tensor) -> torch.Tensor:
             if cache is None:
@@ -281,7 +288,8 @@ class HybridTopKEngine:
         with torch.cuda.device(dev):
             return {"st": st, "indptr": up("indptr", st.text_indptr), "indices": up("indices", st.text_indices),
                     "values": up("values", st.text_values), "genre": up("genre", st.genre),
-                    "meta": [up(f"meta{i}", m) for i, m in enumerate(st.meta)]}
+                    "meta": [up(f"meta{i}", m) for i, m in enumerate(st.meta)],
+                    "h2d_set": None if cache is None else (cache, cache["stamp"])}
 
     def upload(self, st: StagedCatalogue, weights: tuple[float, float, float] = (0.4, 0.5, 0.1),
                recycle: DeviceCatalogue | None = None) -> DeviceCatalogue:
@@ -299,7 +307,10 @@ class HybridTopKEngine:
 
         ``recycle``: a catalogue this engine prepared earlier and the caller no longer needs.  Its
         operand buffer is taken over -- the positions its CSR had set are zeroed (one store per old
-        non-zero) instead of clearing a fresh N x V array -- and the old catalogue becomes unusable."""
+        non-zero) instead of clearing a fresh N x V array -- and the old catalogue becomes unusable.
+        When that CSR came from an ``h2d(reuse=True)`` set that a later ``h2d`` has overwritten (the
+        call before the previous one, e.g. ``raw`` itself), its positions are no longer known and the
+        whole operand is zeroed instead."""
         lib, dev, stream = self.lib, self.device, None
         st: StagedCatalogue = raw["st"]
         gw, tw, mw = (float(w) for w in weights)
@@ -406,7 +417,8 @@ class HybridTopKEngine:
             recycle.buffers = {}
         return DeviceCatalogue(c=f, n_shows=n, folded=folded,
                                weights_baked=(gw, tw, mw) if folded else None, keep=keep,
-                               operand=operand, text_indptr=indptr, text_indices=indices, buffers=bufs)
+                               operand=operand, text_indptr=indptr, text_indices=indices, buffers=bufs,
+                               h2d_set=raw.get("h2d_set"))
 
     # ------------------------------------------------------------------------------------ device-side ingest
     _RAW_DTYPES = {np.dtype(np.bool_): 0, np.dtype(np.uint8): 0, np.dtype(np.int32): 1, np.dtype(np.int64): 2,
@@ -533,9 +545,14 @@ class HybridTopKEngine:
                 and tuple(recycle.operand.shape) == (n_pad, k_pad) and recycle.operand.dtype == tdt
                 and recycle.operand.device == dev):
             operand = recycle.operand
-            check(lib.tvbf_prep_clear_csr_positions(recycle.text_indptr.data_ptr(), recycle.text_indices.data_ptr(),
-                                                    recycle.n_shows, operand.data_ptr(), k_pad, 0, code, stream),
-                  "tvbf_prep_clear_csr_positions")
+            src = recycle.h2d_set
+            if src is None or src[0]["stamp"] == src[1]:
+                check(lib.tvbf_prep_clear_csr_positions(recycle.text_indptr.data_ptr(),
+                                                        recycle.text_indices.data_ptr(), recycle.n_shows,
+                                                        operand.data_ptr(), k_pad, 0, code, stream),
+                      "tvbf_prep_clear_csr_positions")
+            else:           # the h2d set holding its CSR has been overwritten since
+                self._zero(operand)
             recycle.operand = None          # ownership moved: the old catalogue must not be used again
             recycle.c.operand = None
             recycle.keep.clear()
