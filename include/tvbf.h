@@ -276,6 +276,22 @@ int tvbf_rescore_lists(const tvbf_features* f, const tvbf_params* p, const void*
                        int32_t table_row0, int32_t table_rows, const tvbf_topk_out* out,
                        void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- append shows to a catalogue whose table exists (instead of the whole job again).
+ *      f: the grown catalogue of n_shows = N + Q shows, rows [0, n_old = N) unchanged since `prev` was
+ *      computed, rows [N, N + Q) the new shows in the same vocabulary and widths; prev: the [N, k]
+ *      table of the old catalogue from a job with the same p (weights, k, min_similarity,
+ *      exclude_self = 1).  Writes the [N + Q, k] table of the grown catalogue to `out` -- bit-identical
+ *      to tvbf_hybrid_topk on f (indices, counts and the four scores; stats differ) -- and
+ *      changed[r] = 1 for every old row r whose indices or counts differ from prev (0 otherwise:
+ *      the row is byte-identical).  An old row that receives no new candidate above its threshold is
+ *      copied from prev without rescoring.  Only the 256 x 256 tiles that hold a new show are computed; the
+ *      old rows' thresholds start just below their previous k-th score.  Jobs tvbf_sym_eligible
+ *      rejects, and signed text, are rejected (the caller runs the whole job).  `out` must not alias `prev`. */
+size_t tvbf_append_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_old);
+int tvbf_append_topk(const tvbf_features* f, const tvbf_params* p, int32_t n_old, const tvbf_topk_out* prev,
+                     const tvbf_topk_out* out, int32_t* changed, void* workspace, size_t workspace_bytes,
+                     void* stream);
+
 /* exact fp64 scoring of explicit source rows against all columns + exact top-K
  * (replaces get_recommendations_from_matrix, content_based_service.py:161-236, for any n). */
 size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed);
@@ -354,6 +370,15 @@ int tvbf_score_pairs(const tvbf_features* f, const tvbf_params* p, const int32_t
 int32_t tvbf_debug_schedule(int32_t col_tiles, int32_t super_blocks, int32_t sb_per_group, int32_t splits,
                             int32_t world, int32_t rank, int32_t symmetric, int32_t* out,
                             int32_t max_items);
+/* host-only: tensor-core tiles tvbf_append_topk executes for this job, out2 = {tiles of its threshold
+ * seed pass over the super blocks that hold new shows, tiles of the append sweep} (256 x 256 x k_pad
+ * each).  Fails like tvbf_append_workspace_bytes for a job the append does not take. */
+int tvbf_append_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_old, int64_t* out2);
+/* host-only: the work items of the append sweep of tvbf_append_topk for n_shows shows of which the
+ * first n_old are old, on a device with sm_count SMs; out as tvbf_debug_schedule.  Returns the number
+ * of items.  Used by the CPU tests to prove that every pair with a new show is computed exactly once. */
+int32_t tvbf_debug_append_schedule(int32_t n_old, int32_t n_shows, int32_t sm_count, int32_t* out,
+                                   int32_t max_items);
 /* host-only: tensor-core tiles the candidate pass of this job executes -- out4 = {tiles of the
  * threshold seed pass, tiles of the main sweep, rows per tile (128 or 256; columns are 256 and the
  * depth is k_pad), 1 if the symmetric sweep is used}.  tile_sharded = 0: the job as tvbf_hybrid_topk

@@ -873,6 +873,203 @@ int tvbf_rescore_lists(const tvbf_features* f, const tvbf_params* p, const void*
   return tvbf::k6_launch_flagged(scp, flagged, floors, rows, p->row_begin, keys, sms, *out, st);
 }
 
+// ---- append shows to a catalogue whose table exists --------------------------------------------
+// The append sweep (K1 kMode 6) computes only the tiles that hold a new show and feeds both shows of
+// every pair with at least one new show; K4s compacts the lists; K5 merges, per show, that list with
+// the show's previous row (list 1, bound -inf) and certifies; K6 repairs over all columns.
+namespace {
+
+__global__ void append_changed_kernel(const int* prev_idx, const int* prev_cnt, const int* idx, const int* cnt,
+                                      int n_old, int k, int* changed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_old) return;
+  int c = prev_cnt[r] != cnt[r];
+  const size_t base = static_cast<size_t>(r) * k;
+  for (int e = 0; e < k && !c; ++e) c = prev_idx[base + e] != idx[base + e];
+  changed[r] = c;
+}
+
+// After K4s: an old show whose append list is empty received no new column above its threshold, which
+// lies strictly below its previous k-th score (or below min_similarity for a short row), so no new
+// column can enter and its row IS the previous row: copied, no rescoring.  Every other show (the new
+// ones and the old ones with new candidates) is listed for K5.
+__global__ void append_select_kernel(tvbf_topk_out prev, tvbf_topk_out out, const int* list0_cnt, int n_old, int n_shows,
+                                     int k, int* rows, int* n_listed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  if (r >= n_old || list0_cnt[r] != 0) {
+    rows[atomicAdd(n_listed, 1)] = r;
+    return;
+  }
+  const size_t base = static_cast<size_t>(r) * k;
+  for (int e = 0; e < k; ++e) {
+    out.indices[base + e] = prev.indices[base + e];
+    out.hybrid[base + e] = prev.hybrid[base + e];
+    out.genre[base + e] = prev.genre[base + e];
+    out.text[base + e] = prev.text[base + e];
+    out.metadata[base + e] = prev.metadata[base + e];
+  }
+  out.counts[r] = prev.counts[r];
+}
+
+struct AppendPlan {
+  Plan pl;             // a whole-catalogue symmetric job over all shows
+  tvbf::K1Params geo;  // tile schedule of the append sweep
+  int grid;
+  size_t off_cand, off_cnt, off_bound;   // two candidate lists per show: [2][n_shows]
+  size_t off_rows, off_listed, total;    // shows K5 rescores and their count
+};
+
+int make_append_plan(const tvbf_features* f, const tvbf_params* p, int n_old, AppendPlan* ap, tvbf_params* q) {
+  TVBF_REQUIRE(n_old >= 1 && n_old < f->n_shows, "append: n_old %d must lie in [1, n_shows %d)", n_old, f->n_shows);
+  TVBF_REQUIRE(!f->text_signed, "append: signed text needs the whole job");
+  *q = *p;
+  q->row_begin = 0;
+  q->row_end = f->n_shows;
+  q->tuning = (q->tuning & ~(0x3 << 20)) | (2 << 20);   // symmetric job (or fail if ineligible)
+  q->tuning = (q->tuning & ~0xF) | 2;                   // CTA pairs
+  int rc = validate_params(f, q);
+  if (rc != TVBF_OK) return rc;
+  rc = make_plan(f, q, &ap->pl);
+  if (rc != TVBF_OK) return rc;
+  int sms = 0;
+  rc = sm_count_cached(&sms);
+  if (rc != TVBF_OK) return rc;
+  memset(&ap->geo, 0, sizeof(ap->geo));
+  tvbf::k1_append_geometry(n_old, f->n_shows, sms / 2, &ap->geo);
+  const int items = (ap->geo.rb_count + ap->geo.rb_per_group - 1) / ap->geo.rb_per_group * ap->geo.rb_per_group *
+                    ap->geo.splits;
+  ap->grid = 2 * (items < sms / 2 ? items : sms / 2);
+  const size_t rows = static_cast<size_t>(f->n_shows);
+  size_t off = ap->pl.total;
+  ap->off_cand = off;  off = align_up(off + 2 * rows * ap->pl.kp * 8, 256);
+  ap->off_cnt = off;   off = align_up(off + 2 * rows * 4, 256);
+  ap->off_bound = off; off = align_up(off + 2 * rows * 4, 256);
+  ap->off_rows = off;  off = align_up(off + rows * 4, 256);
+  ap->off_listed = off; off = align_up(off + 4, 256);
+  ap->total = off;
+  return TVBF_OK;
+}
+
+// the candidate-kernel parameters of an append: a whole-catalogue symmetric job on the append geometry
+int fill_append_params(const tvbf_features* f, const tvbf_params* q, const AppendPlan& ap, uint8_t* ws,
+                       tvbf::K1Params* kp) {
+  int rc = fill_k1_params(f, q, ap.pl, ws, kp);
+  if (rc != TVBF_OK) return rc;
+  kp->sync_kb = 0;
+  kp->col_tiles = ap.geo.col_tiles;
+  kp->rb_count = ap.geo.rb_count;
+  kp->splits = ap.geo.splits;
+  kp->rb_per_group = ap.geo.rb_per_group;
+  kp->tiles_per_split = ap.geo.tiles_per_split;
+  kp->append_n_old = ap.geo.append_n_old;
+  kp->append_b0 = ap.geo.append_b0;
+  kp->cand = reinterpret_cast<uint2*>(ws + ap.off_cand);   // list 0: what the append sweep found
+  kp->cand_cnt = reinterpret_cast<int*>(ws + ap.off_cnt);
+  kp->cand_theta = reinterpret_cast<float*>(ws + ap.off_bound);
+  return TVBF_OK;
+}
+
+}  // namespace
+
+size_t tvbf_append_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_old) {
+  if (validate_features(f) != TVBF_OK || p == nullptr) return 0;
+  AppendPlan ap;
+  tvbf_params q;
+  if (make_append_plan(f, p, n_old, &ap, &q) != TVBF_OK) return 0;
+  return ap.total;
+}
+
+int tvbf_append_topk(const tvbf_features* f, const tvbf_params* p, int32_t n_old, const tvbf_topk_out* prev,
+                     const tvbf_topk_out* out, int32_t* changed, void* workspace, size_t workspace_bytes,
+                     void* stream) {
+  TVBF_ENTER_CALL(stream);
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p != nullptr, "params is NULL");
+  TVBF_REQUIRE(prev && prev->indices && prev->counts && prev->hybrid && prev->genre && prev->text && prev->metadata,
+               "previous table has NULL members");
+  TVBF_REQUIRE(out && out->indices && out->counts && out->hybrid && out->genre && out->text && out->metadata &&
+                   out->stats,
+               "output table has NULL members");
+  TVBF_REQUIRE(changed != nullptr && workspace != nullptr, "tvbf_append_topk: NULL argument");
+  AppendPlan ap;
+  tvbf_params q;
+  rc = make_append_plan(f, p, n_old, &ap, &q);
+  if (rc != TVBF_OK) return rc;
+  if (workspace_bytes < ap.total) {
+    tvbf_set_error("workspace too small: %zu < %zu", workspace_bytes, ap.total);
+    return TVBF_ERR_WORKSPACE;
+  }
+  auto st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const Plan& pl = ap.pl;
+  const int rows = f->n_shows;
+  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
+  double* floors = reinterpret_cast<double*>(ws + pl.off_floor);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+  int* listed_rows = reinterpret_cast<int*>(ws + ap.off_rows);
+  int* n_listed = reinterpret_cast<int*>(ws + ap.off_listed);
+  tvbf::K1Params kp;
+  rc = fill_append_params(f, &q, ap, ws, &kp);
+  if (rc != TVBF_OK) return rc;
+  uint2* cand = kp.cand;
+  int* cnt = kp.cand_cnt;
+  float* bound = kp.cand_theta;
+  const tvbf::AppendPrev pv{prev->indices, prev->counts, prev->hybrid, n_old, p->k,
+                            cand + static_cast<size_t>(rows) * pl.kp, cnt + rows, bound + rows};
+  TVBF_CUDA_OK(cudaMemsetAsync(out->stats, 0, 8 * sizeof(int32_t), st));
+  rc = tvbf::k1_launch_append(f, kp, ap.grid, pv, st);
+  if (rc != TVBF_OK) return rc;
+  rc = tvbf::k4s_launch(kp, rows, st);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaMemsetAsync(n_listed, 0, 4, st));
+  append_select_kernel<<<(rows + 255) / 256, 256, 0, st>>>(*prev, *out, cnt, n_old, rows, p->k, listed_rows, n_listed);
+  TVBF_LAUNCH_OK("append_select_kernel");
+  const tvbf::ScoreParams sp = score_params(f, &q);
+  const tvbf::CandLayout lay{0, 1, rows, 0};   // list s of show r: slot r + s * rows
+  rc = tvbf::k5_launch_listed(sp, cand, cnt, bound, 2, lay, pl.kp, 0, rows, listed_rows, n_listed, *out, flagged,
+                              floors, st);
+  if (rc != TVBF_OK) return rc;
+  rc = tvbf::k6_launch_flagged(sp, flagged, floors, rows, 0, keys, pl.k6_grid, *out, st);
+  if (rc != TVBF_OK) return rc;
+  append_changed_kernel<<<(n_old + 255) / 256, 256, 0, st>>>(prev->indices, prev->counts, out->indices, out->counts,
+                                                             n_old, p->k, changed);
+  TVBF_LAUNCH_OK("append_changed_kernel");
+  return TVBF_OK;
+}
+
+int tvbf_append_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_old, int64_t* out2) {
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p && out2, "tvbf_append_plan_tiles: NULL argument");
+  AppendPlan ap;
+  tvbf_params q;
+  rc = make_append_plan(f, p, n_old, &ap, &q);
+  if (rc != TVBF_OK) return rc;
+  uint8_t* fake_ws = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(4096));   // offsets only, never dereferenced
+  tvbf::K1Params kp;
+  rc = fill_append_params(f, &q, ap, fake_ws, &kp);
+  if (rc != TVBF_OK) return rc;
+  long long t[2];
+  tvbf::k1_append_executed_tiles(f, kp, ap.grid, t);
+  out2[0] = t[0];
+  out2[1] = t[1];
+  return TVBF_OK;
+}
+
+int32_t tvbf_debug_append_schedule(int32_t n_old, int32_t n_shows, int32_t sm_count, int32_t* out,
+                                   int32_t max_items) {
+  if (n_old < 1 || n_old >= n_shows || sm_count < 2 || out == nullptr || max_items < 0) {
+    tvbf_set_error("tvbf_debug_append_schedule: bad arguments");
+    return TVBF_ERR_INVALID;
+  }
+  tvbf::K1Params kp;
+  memset(&kp, 0, sizeof(kp));
+  tvbf::k1_append_geometry(n_old, n_shows, sm_count / 2, &kp);
+  return tvbf::k1_debug_append_schedule(kp, out, max_items);
+}
+
 // ---- streaming statistics of the four similarity matrices (no N x N) --------------------------
 size_t tvbf_stats_accum_bytes(void) { return sizeof(tvbf::StatsAccum); }
 

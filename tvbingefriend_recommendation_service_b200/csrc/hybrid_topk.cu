@@ -221,6 +221,9 @@ __host__ __device__ __forceinline__ int global_super_block(const K1Params& p, in
   return static_cast<int>(p.deal_gid[g]) * p.deal_r + (local - g * p.deal_r);
 }
 
+// kAppend (append sweep): every super block only needs the column tiles >= append_b0, the first one
+// holding new shows
+template <bool kAppend = false>
 __host__ __device__ __forceinline__ ItemCoord item_coord(const K1Params& p, int item) {
   const int per_group = p.rb_per_group * p.splits;
   const int g = item / per_group;
@@ -232,7 +235,8 @@ __host__ __device__ __forceinline__ ItemCoord item_coord(const K1Params& p, int 
   if (p.sym) {
     // the group's super blocks lie at or right of tile i0 on the diagonal; only columns >= i0 matter
     // (with several GPUs a wave is one dealt group: rb_per_group == deal_r)
-    const int i0 = global_super_block(p, g * p.rb_per_group);
+    int i0 = global_super_block(p, g * p.rb_per_group);
+    if constexpr (kAppend) i0 = i0 > p.append_b0 ? i0 : p.append_b0;
     const int span = p.col_tiles > i0 ? p.col_tiles - i0 : 0;
     const int tps = (span + p.splits - 1) / p.splits;
     c.tile0 = i0 + c.split * tps;
@@ -397,7 +401,9 @@ struct Pacer {
 
 // kMode: 0 one-sided top-k sweep, 1 symmetric top-k sweep, 2 symmetric statistics sweep,
 // 3 threshold seed pass (one-sided walk over sampled tiles, per-row score histograms, no lists),
-// 5 symmetric top-k sweep for p.n_weights weight triples at once (one shared list per triple and show)
+// 5 symmetric top-k sweep for p.n_weights weight triples at once (one shared list per triple and show),
+// 6 append sweep: the symmetric top-k sweep restricted to the tiles that hold a new show (column tile
+// >= p.append_b0), offering no pair of two old shows (p.append_n_old)
 // kG2: multi-hot genres with 64 < G <= 128 -- the second word of every column's mask is staged beside
 // the column-side records (in the threshold slices a single-triple sweep leaves unused) and the
 // popcount runs over both words.
@@ -416,6 +422,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
   constexpr bool kSym = kMode != 0 && !kHist;   // tiles on/above the diagonal, 8 (kWide: 16) epilogue warps
   constexpr bool kStats = kMode == 2;    // accumulate statistics instead of candidate lists
   constexpr bool kMulti = kMode == 5;    // weight sweep
+  constexpr bool kAppend = kMode == 6;   // append sweep
   static_assert(!(kG2 && (kMulti || kStats)), "two-word genre masks: single-triple top-k sweeps only");
   static_assert(!(kFold && (kMulti || kStats || kDump || kG2)), "folded groups: single-triple top-k sweeps only");
   // Seed pass: hist[bin][row of the CTA] (32-bit counters; bank = row % 32, so the 32 lanes of a warp
@@ -490,7 +497,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       Pacer pacer{p.sync_kb > 0 ? p.progress : nullptr, gridDim.x, p.sync_slack, 0u};
       const int chunks_per_tile = p.sync_kb > 0 ? (p.k_blocks + p.sync_kb - 1) / p.sync_kb : 0;
       for (int item = cluster_id; item < n_items; item += num_clusters) {
-        ItemCoord c = item_coord(p, item);
+        ItemCoord c = item_coord<kAppend>(p, item);
         if (kDump) { c.sb = 0; c.tile0 = 0; c.tile1 = 1; }
         const int row0 = p.row_begin + (kDump ? 0 : c.sb * BM * CG) + static_cast<int>(cta_rank) * BM;
         for (int jt = c.tile0; jt < c.tile1; jt += p.tile_stride) {
@@ -561,7 +568,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const uint64_t desc_a0 = umma_desc_sw128(smem_u32(smem + L::OFF_A));
       const uint64_t desc_b0 = umma_desc_sw128(smem_u32(smem + L::OFF_B));
       for (int item = cluster_id; item < n_items; item += num_clusters) {
-        ItemCoord c = item_coord(p, item);
+        ItemCoord c = item_coord<kAppend>(p, item);
         if (kDump) { c.sb = 0; c.tile0 = 0; c.tile1 = 1; }
         if (c.sb < 0) continue;
         const int tile_beg = kDump ? c.tile0 : c.real0, tile_end = kDump ? c.tile1 : c.real1;
@@ -626,7 +633,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
     uint32_t* ring = reinterpret_cast<uint32_t*>(smem + L::OFF_Q) + warp * (3 * RING);
     int ring_n = 0;
     for (int item = cluster_id; item < n_items; item += num_clusters) {
-      ItemCoord c = item_coord(p, item);
+      ItemCoord c = item_coord<kAppend>(p, item);
       if (kDump) { c.sb = 0; c.tile0 = 0; c.tile1 = 1; }
       if (c.sb < 0) continue;
       const int row_local0 = (kDump ? 0 : c.sb * BM * CG) + static_cast<int>(cta_rank) * BM;  // within shard
@@ -874,6 +881,16 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
               }
               if (kSym) {
                 if (!do_col) hit_c = 0u;
+                if constexpr (kAppend) {
+                  // a pair of two old shows is in the previous table already (or ranks below all of it):
+                  // offered to neither list.  Only the column tile append_b0 mixes old and new columns.
+                  const int old_cols = p.append_n_old - (col0 + cbase + h * GW);
+                  if (row < p.append_n_old && old_cols > 0) {
+                    const uint32_t m = old_cols >= GW ? (1u << GW) - 1u : (1u << old_cols) - 1u;
+                    hit_r &= ~m;
+                    hit_c &= ~m;
+                  }
+                }
                 push_hits(hit_r | (hit_c << GW), u, col0 + cbase + h * GW, 0);
               } else if (kHist) {
 #pragma unroll
@@ -1216,6 +1233,34 @@ __global__ void sym_init_kernel(unsigned int* theta, int n_shows, int n_pad, int
   if (i < n_virtual) theta[i] = (i % n_pad) < n_shows ? __float_as_uint(theta_init) : 0x7f800000u;
 }
 
+// Append: every old show's previous row becomes its candidate list 1 (bound -inf: an old column missing
+// from the row ranks below all k entries of it and can never enter), and an old show with a full row
+// starts the sweep with the largest float strictly BELOW its k-th previous score -- a new column that
+// does not beat that cannot enter either, and the strict certificate "theta < k-th" of K5 still passes
+// for an unchanged row.  New shows get an empty list 1 and keep their seeded thresholds.
+__global__ void append_prev_kernel(AppendPrev a, unsigned int* theta, float theta_init, int n_shows, int kp) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  int cnt = 0;
+  if (r < a.n_old) {
+    cnt = a.counts[r];
+    uint2* dst = a.list + static_cast<size_t>(r) * kp;
+    const size_t base = static_cast<size_t>(r) * a.k;
+    for (int e = 0; e < cnt; ++e)
+      dst[e] = make_uint2(__float_as_uint(__double2float_ru(a.hybrid[base + e])), static_cast<uint32_t>(a.indices[base + e]));
+    float th = theta_init;   // a short row: every new column that qualifies may enter
+    if (cnt == a.k) {
+      const double kth = a.hybrid[base + a.k - 1];
+      th = __double2float_rd(kth);
+      if (static_cast<double>(th) >= kth) th = nextafterf(th, -INFINITY);
+      th = fmaxf(th, theta_init);
+    }
+    theta[r] = __float_as_uint(th);   // (the seed pass over block append_b0 also wrote the old shows there)
+  }
+  a.cnt[r] = cnt;
+  a.bound[r] = __int_as_float(0xff800000);
+}
+
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
@@ -1288,6 +1333,45 @@ int k1_debug_schedule(const K1Params& p, int* out, int max_items) {
   const int n_items = ((p.rb_count + p.rb_per_group - 1) / p.rb_per_group) * p.rb_per_group * p.splits;
   for (int item = 0; item < n_items && item < max_items; ++item) {
     const ItemCoord c = item_coord(p, item);
+    int* o = out + 6 * item;
+    o[0] = c.sb; o[1] = c.split; o[2] = c.tile0; o[3] = c.tile1; o[4] = c.real0; o[5] = c.real1;
+  }
+  return n_items;
+}
+
+// Append sweep: old super blocks all cover the same narrow band [b0, col_tiles) (1 to ~20 tiles), new
+// ones the rest of their row.  Items = (super block, column split), dealt round-robin to the clusters;
+// the split count minimises the tiles of the busiest cluster (rounds of items x tiles per item), so
+// that a band of a few tiles still spreads over every SM.  No pacing: nothing waits for anyone.
+void k1_append_geometry(int n_old, int n_shows, int clusters, K1Params* p) {
+  p->sym = 1;
+  p->col_tiles = (n_shows + 255) / 256;
+  p->rb_count = p->col_tiles;
+  p->append_n_old = n_old;
+  p->append_b0 = n_old / 256;
+  p->deal_groups = 0;
+  p->deal_r = 1;
+  const int span = p->col_tiles - p->append_b0;
+  if (clusters < 1) clusters = 1;
+  long long best_cost = -1;
+  for (int s = 1; s <= span && s <= 16 && s <= clusters; ++s) {
+    int rb = clusters / s;
+    if (rb > p->rb_count) rb = p->rb_count;
+    const long long items = static_cast<long long>((p->rb_count + rb - 1) / rb) * rb * s;
+    const long long cost = (items + clusters - 1) / clusters * ((span + s - 1) / s);
+    if (best_cost < 0 || cost < best_cost) {
+      best_cost = cost;
+      p->splits = s;
+      p->rb_per_group = rb;
+    }
+  }
+  p->tiles_per_split = (span + p->splits - 1) / p->splits;
+}
+
+int k1_debug_append_schedule(const K1Params& p, int* out, int max_items) {
+  const int n_items = ((p.rb_count + p.rb_per_group - 1) / p.rb_per_group) * p.rb_per_group * p.splits;
+  for (int item = 0; item < n_items && item < max_items; ++item) {
+    const ItemCoord c = item_coord<true>(p, item);
     int* o = out + 6 * item;
     o[0] = c.sb; o[1] = c.split; o[2] = c.tile0; o[3] = c.tile1; o[4] = c.real0; o[5] = c.real1;
   }
@@ -1676,6 +1760,83 @@ int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, 
   }
   tvbf_set_error("unsupported candidate capacity (entries per lane %d)", entries_per_lane);
   return TVBF_ERR_INVALID;
+}
+
+// histogram seed pass of an append: over the super blocks that hold new shows (from append_b0 on; the old
+// shows among them are overwritten from the previous table afterwards)
+static K1Params append_seed_params(const tvbf_features* f, const K1Params& kp, int grid) {
+  K1Params seed = make_seed_params(kp, grid, 0);
+  seed.row_begin = kp.append_b0 * 256;
+  seed.rb_count = (f->n_shows - seed.row_begin + 255) / 256;
+  seed.rb_per_group = grid / 2 < seed.rb_count ? grid / 2 : seed.rb_count;
+  return seed;
+}
+
+void k1_append_executed_tiles(const tvbf_features* f, const K1Params& kp, int grid, long long* out) {
+  out[0] = count_tiles(append_seed_params(f, kp, grid));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  long long t = 0;
+  const int n_items = ((sweep.rb_count + sweep.rb_per_group - 1) / sweep.rb_per_group) * sweep.rb_per_group * sweep.splits;
+  for (int item = 0; item < n_items; ++item) {
+    const ItemCoord c = item_coord<true>(sweep, item);
+    if (c.sb >= 0 && c.real1 > c.real0) t += c.real1 - c.real0;
+  }
+  out[1] = t;
+}
+
+int k1_launch_append(const tvbf_features* f, const K1Params& kp, int grid, const AppendPrev& prev,
+                     cudaStream_t st) {
+  if (!kp.sym || kp.n_weights > 1 || kp.sync_kb != 0) {
+    tvbf_set_error("append sweep: bad parameters");
+    return TVBF_ERR_INVALID;
+  }
+  const int n_pad = f->n_pad;
+  const size_t list_bytes = static_cast<size_t>(n_pad) * kp.sym_cap * 8;
+  std::lock_guard<std::mutex> lock(g_side_mutex);
+  SideStream* side = nullptr;
+  int rc = side_stream(&side);
+  if (rc != TVBF_OK) return rc;
+  // the shared lists are cleared on the side stream beside the seed pass, as in a full job
+  rc = absorb_pending(side, st, true);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaEventRecord(side->fork, st));
+  TVBF_CUDA_OK(cudaStreamWaitEvent(side->stream, side->fork, 0));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, static_cast<size_t>(n_pad) * 4, side->stream));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, side->stream));
+  TVBF_CUDA_OK(cudaEventRecord(side->join, side->stream));
+  sym_init_kernel<<<static_cast<unsigned>((n_pad + 255) / 256), 256, 0, st>>>(kp.g_theta, f->n_shows, n_pad, n_pad,
+                                                                               kp.theta_init);
+  TVBF_LAUNCH_OK("sym_init_kernel");
+  {
+    const K1Params seed = append_seed_params(f, kp, grid);
+    const int sg = seed.rb_per_group * 2;
+    if (kp.wide_epilogue) {
+      if (kp.fold) rc = launch_k1<4, false, 2, 3, true, false, true>(f, seed, sg, st);
+      else if (kp.genre_hi != nullptr) rc = launch_k1<4, false, 2, 3, true, true>(f, seed, sg, st);
+      else rc = launch_k1<4, false, 2, 3, true>(f, seed, sg, st);
+    } else {
+      if (kp.fold) rc = launch_k1<4, false, 2, 3, false, false, true>(f, seed, sg, st);
+      else if (kp.genre_hi != nullptr) rc = launch_k1<4, false, 2, 3, false, true>(f, seed, sg, st);
+      else rc = launch_k1<4, false, 2, 3>(f, seed, sg, st);
+    }
+    if (rc != TVBF_OK) return rc;
+  }
+  append_prev_kernel<<<static_cast<unsigned>((f->n_shows + 255) / 256), 256, 0, st>>>(prev, kp.g_theta, kp.theta_init,
+                                                                                      f->n_shows, kp.kp);
+  TVBF_LAUNCH_OK("append_prev_kernel");
+  TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  if (kp.wide_epilogue) {
+    if (sweep.stages > Smem<2, true>::STAGES) sweep.stages = Smem<2, true>::STAGES;
+    if (kp.fold) return launch_k1<4, false, 2, 6, true, false, true>(f, sweep, grid, st);
+    return kp.genre_hi ? launch_k1<4, false, 2, 6, true, true>(f, sweep, grid, st)
+                       : launch_k1<4, false, 2, 6, true>(f, sweep, grid, st);
+  }
+  if (kp.fold) return launch_k1<4, false, 2, 6, false, false, true>(f, sweep, grid, st);
+  return kp.genre_hi ? launch_k1<4, false, 2, 6, false, true>(f, sweep, grid, st)
+                     : launch_k1<4, false, 2, 6>(f, sweep, grid, st);
 }
 
 int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cudaStream_t st) {

@@ -115,6 +115,23 @@ struct K1Params {
   float mw_text[kMaxSweep], mw_text_err[kMaxSweep], mw_genre[kMaxSweep], mw_meta[kMaxSweep], mw_eps[kMaxSweep];
   float mw_text_acc[kMaxSweep], mw_eps_term[kMaxSweep];
   float mw_score_hi[kMaxSweep];   // score_hi of each triple (histogram range of its seed pass)
+  // append sweep (kMode 6, tvbf_append_topk): shows [0, append_n_old) had a table already; only tiles
+  // with a column tile >= append_b0 = append_n_old / 256 are computed, and pairs of two old shows are
+  // offered to neither list
+  int append_n_old;
+  int append_b0;
+};
+
+// The previous table of an append and where its rows go: list 1 of the two-list candidate table K5
+// merges (list 0 is K4s' compaction of the append sweep's shared lists).
+struct AppendPrev {
+  const int* indices;   // [n_old, k]
+  const int* counts;    // [n_old]
+  const double* hybrid; // [n_old, k]
+  int n_old, k;
+  uint2* list;          // [n_shows][kp]
+  int* cnt;             // [n_shows]
+  float* bound;         // [n_shows]
 };
 
 // parameters of the exact fp64 scorers (rescore.cu)
@@ -143,11 +160,27 @@ struct CandLayout {
 int k5_launch(const ScoreParams& sp, const uint2* cand, const int* cand_cnt,
               const float* cand_theta, int splits, CandLayout lay, int kp, int row_begin, int n_rows,
               const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor, cudaStream_t st);
+// K5 over the table rows rows[0 .. *n_listed) (a device count; at most n_rows)
+int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_cnt, const float* cand_theta,
+                     int splits, CandLayout lay, int kp, int row_begin, int n_rows, const int* rows,
+                     const int* n_listed, const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
+                     cudaStream_t st);
 // deal the ceil(total / r) groups of r consecutive super blocks to `world` GPUs; fills gid[] with the
 // groups of `rank` (cost descending) and returns {groups, super blocks} of that rank, or -1 when a
 // rank would own more than kMaxDealGroups groups
 int k1_deal_groups(int total_super_blocks, int r, int world, int rank, unsigned short* gid, int* local_sb);
 int k1_debug_schedule(const K1Params& p, int* out, int max_items);
+// geometry of the append sweep over n_shows shows of which the first n_old are old, on `clusters` CTA
+// pairs: fills col_tiles, rb_count (= super blocks), splits and rb_per_group of p
+void k1_append_geometry(int n_old, int n_shows, int clusters, K1Params* p);
+// items of the append sweep, as k1_debug_schedule
+int k1_debug_append_schedule(const K1Params& p, int* out, int max_items);
+// seed pass over the new shows, thresholds of the old shows from the previous table, the previous
+// table as candidate list 1, then the append sweep (kp.sym == 1, kp.append_* set)
+int k1_launch_append(const tvbf_features* f, const K1Params& kp, int grid, const AppendPrev& prev,
+                     cudaStream_t st);
+// tiles of the append: out[0] its seed pass over the new super blocks, out[1] the append sweep
+void k1_append_executed_tiles(const tvbf_features* f, const K1Params& kp, int grid, long long* out);
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);

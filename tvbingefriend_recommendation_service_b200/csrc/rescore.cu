@@ -116,15 +116,13 @@ __device__ __forceinline__ bool ranks_before(double ha, int ja, double hb, int j
 // ---------------------------------------------------------------------------------------------
 constexpr int K5_WARPS = 4;
 
-__global__ void __launch_bounds__(K5_WARPS * 32)
-rescore_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
-               const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta, int splits,
-               const CandLayout lay, int kp, int row_begin, int n_rows, tvbf_topk_out out,
-               int* flagged_rows, double* flagged_floor, int max_cand, int keep) {
+// the work of one warp on table row r (source row row_begin + r); n_rows sizes the flagged lists
+__device__ __forceinline__ void rescore_row(const ScoreParams& sp, const uint2* __restrict__ cand,
+                                            const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta,
+                                            int splits, const CandLayout& lay, int kp, int row_begin, int n_rows,
+                                            const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
+                                            int max_cand, int keep, int warp, int lane, int r) {
   extern __shared__ __align__(16) uint8_t k5_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int r = blockIdx.x * (blockDim.x >> 5) + warp;
-  if (r >= n_rows) return;
   const int i = row_begin + r;
   uint8_t* base = k5_smem + static_cast<size_t>(warp) * max_cand * 48;
   double* sh = reinterpret_cast<double*>(base);
@@ -261,6 +259,33 @@ rescore_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
       flagged_floor[pos] = bound;
     }
   }
+}
+
+__global__ void __launch_bounds__(K5_WARPS * 32)
+rescore_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
+               const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta, int splits,
+               const CandLayout lay, int kp, int row_begin, int n_rows, tvbf_topk_out out,
+               int* flagged_rows, double* flagged_floor, int max_cand, int keep) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int r = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (r >= n_rows) return;
+  rescore_row(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin, n_rows, out, flagged_rows, flagged_floor,
+              max_cand, keep, warp, lane, r);
+}
+
+// K5 over the listed table rows only (rows[0 .. *n_listed)): an append rescores the new shows and the old
+// shows that received new candidates; the others keep their previous rows
+__global__ void __launch_bounds__(K5_WARPS * 32)
+rescore_listed_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
+                      const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta, int splits,
+                      const CandLayout lay, int kp, int row_begin, int n_rows, const int* __restrict__ rows,
+                      const int* __restrict__ n_listed, tvbf_topk_out out, int* flagged_rows, double* flagged_floor,
+                      int max_cand, int keep) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (e >= *n_listed) return;
+  rescore_row(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin, n_rows, out, flagged_rows, flagged_floor,
+              max_cand, keep, warp, lane, rows[e]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1011,6 +1036,28 @@ int k5_launch(const ScoreParams& sp, const uint2* cand, const int* cand_cnt,
                                                  row_begin, n_rows, out, flagged_rows, flagged_floor,
                                                  max_cand, 2 * kp);
   TVBF_LAUNCH_OK("rescore_kernel");
+  return TVBF_OK;
+}
+
+int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_cnt, const float* cand_theta,
+                     int splits, CandLayout lay, int kp, int row_begin, int n_rows, const int* rows,
+                     const int* n_listed, const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
+                     cudaStream_t st) {
+  const int max_cand = splits * kp;
+  int warps = K5_WARPS;
+  while (warps > 1 && static_cast<size_t>(warps) * max_cand * 48 > 200 * 1024) warps >>= 1;
+  const size_t smem = static_cast<size_t>(warps) * max_cand * 48;
+  if (smem > 200 * 1024) {
+    tvbf_set_error("rescore: lists*candidates = %d is too large", max_cand);
+    return TVBF_ERR_INVALID;
+  }
+  TVBF_CUDA_OK(cudaFuncSetAttribute(rescore_listed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    static_cast<int>(smem)));
+  const int grid = (n_rows + warps - 1) / warps;   // at most n_rows listed; the count is on the device
+  rescore_listed_kernel<<<grid, warps * 32, smem, st>>>(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin,
+                                                        n_rows, rows, n_listed, out, flagged_rows, flagged_floor,
+                                                        max_cand, 2 * kp);
+  TVBF_LAUNCH_OK("rescore_listed_kernel");
   return TVBF_OK;
 }
 

@@ -130,6 +130,7 @@ class DeviceCatalogue:
     fold: dict | None = None               # second operand with the packed groups as K columns (engine._folded)
     buffers: dict = field(default_factory=dict)   # named per-catalogue device buffers a later catalogue can take over
     h2d_set: tuple | None = None           # (h2d buffer set, its write stamp) when the CSR lives in an h2d(reuse=True) set
+    parts: dict = field(default_factory=dict)     # the tensors behind ``c`` by name and the text nnz (``extend``)
 
 
 @dataclass
@@ -146,6 +147,7 @@ class TopK:
     row_begin: int = 0
     flagged_rows: int = 0    # rows the certificate sent to the exact kernel
     rescored_pairs: int = 0
+    changed_rows: np.ndarray | None = None   # extend_top_k: sorted int32 old rows whose neighbours changed
 
     @property
     def k(self) -> int:
@@ -358,6 +360,7 @@ class HybridTopKEngine:
             f.meta_kind = _lib.META_MEAN3 if st.metadata_mode == "mean3" else _lib.META_HSTACK
             col = v
             folded = False
+            dense = {}
 
             def fold(g_raw: torch.Tensor, weight: float, what: str) -> int:
                 nonlocal col, folded
@@ -376,6 +379,7 @@ class HybridTopKEngine:
                                                      k_pad, col, scale * float(np.sqrt(ratio)), code, stream),
                       "tvbf_prep_dense_to_operand")
                 keep.append(g_norm)
+                dense.setdefault(what, []).append(g_norm)
                 col += g_norm.shape[1]
                 folded = True
                 return g_norm.data_ptr()
@@ -415,10 +419,14 @@ class HybridTopKEngine:
             bufs["genre_hi"] = genre_hi
         if recycle is not None:
             recycle.buffers = {}
+        parts = {"values": values, "col_side": col_side, "meta_scale": meta_scale,
+                 "genre_hi": genre_hi if f.genre_hi else None, "nnz": int(raw["values"].numel()),
+                 "genre_dense": dense.get("genre", [None])[0], "meta_dense": dense.get("metadata", []),
+                 "meta_widths": tuple(int(m.shape[1]) for m in st.meta)}
         return DeviceCatalogue(c=f, n_shows=n, folded=folded,
                                weights_baked=(gw, tw, mw) if folded else None, keep=keep,
                                operand=operand, text_indptr=indptr, text_indices=indices, buffers=bufs,
-                               h2d_set=raw.get("h2d_set"))
+                               h2d_set=raw.get("h2d_set"), parts=parts)
 
     # ------------------------------------------------------------------------------------ device-side ingest
     _RAW_DTYPES = {np.dtype(np.bool_): 0, np.dtype(np.uint8): 0, np.dtype(np.int32): 1, np.dtype(np.int64): 2,
@@ -530,7 +538,10 @@ class HybridTopKEngine:
             f.text_signed = int(bool(bits & 8))
         return DeviceCatalogue(c=f, n_shows=n, folded=False, weights_baked=None,
                                keep=[indptr, indices, values, operand, col_side, meta_scale, genre_hi],
-                               operand=operand, text_indptr=indptr, text_indices=indices)
+                               operand=operand, text_indptr=indptr, text_indices=indices,
+                               parts={"values": values, "col_side": col_side, "meta_scale": meta_scale,
+                                      "genre_hi": genre_hi, "nnz": nnz, "genre_dense": None, "meta_dense": [],
+                                      "meta_widths": tuple(int(a.shape[1]) for a in groups)})
 
     def _text_operand(self, indptr, indices, rawv, n: int, n_pad: int, k_pad: int,
                       recycle: DeviceCatalogue | None, folded: bool = False, values: torch.Tensor | None = None):
@@ -664,6 +675,197 @@ class HybridTopKEngine:
                                             ws.numel(), self._stream()), "tvbf_hybrid_topk")
         t["row_begin"] = row_begin
         return t
+
+    # ------------------------------------------------------------------------------------ appends
+    def extend(self, cat: DeviceCatalogue, new_features: dict) -> DeviceCatalogue:
+        """``cat`` grown by the shows of ``new_features`` (rows N .. N+Q-1 after its N shows).  Only
+        the new rows are prepared (ingest, normalisation, operand rows, CSR, column-side records);
+        the old rows are kept -- in place when the spare rows up to ``n_pad`` suffice, else copied
+        into buffers grown with headroom.  ``cat`` is consumed, as with ``prepare(recycle=...)``.
+
+        Precondition: the old shows' features are unchanged and the new shows are encoded in the
+        same vocabulary and widths (transformed by the already fitted extractor).  A different
+        vocabulary size, genre or metadata width, group encoding (binary / float) or metadata mode
+        raises ``ValueError``; a refitted extractor changes every row and needs a whole job."""
+        c = cat.c
+        if cat.operand is None or not cat.parts:
+            raise ValueError("extend: the catalogue was recycled or does not come from ingest / prepare")
+        mode = "mean3" if c.meta_kind == _lib.META_MEAN3 else "hstack"
+        new = self.ingest(new_features, mode, cat.weights_baked or (0.4, 0.5, 0.1))
+        nc = new.c
+        for what, a, b in (("vocabulary size", c.vocab, nc.vocab), ("genre encoding", c.genre_mode, nc.genre_mode),
+                           ("genre columns", c.genre_dim, nc.genre_dim),
+                           ("metadata encoding", c.meta_mode, nc.meta_mode),
+                           ("metadata groups", c.meta_groups, nc.meta_groups),
+                           ("metadata widths", cat.parts["meta_widths"], new.parts["meta_widths"]),
+                           ("operand width", c.k_pad, nc.k_pad), ("text dtype", c.text_dtype, nc.text_dtype)):
+            if a != b:
+                raise ValueError(f"extend: the new shows' {what} ({b}) differs from the catalogue's ({a})")
+        if cat.folded and (not new.folded or new.weights_baked != cat.weights_baked):
+            raise ValueError("extend: the new shows' float groups do not match the catalogue's")
+        n_old, q = cat.n_shows, new.n_shows
+        n = n_old + q
+        dev, lib, stream = self.device, self.lib, self._stream()
+        code, _ = _DTYPES[self.text_dtype]
+        p_old, p_new = cat.parts, new.parts
+        with torch.cuda.device(dev):
+            n_pad = int(c.n_pad)
+            grow = n > n_pad
+            if grow:
+                n_pad = (n + n // 8 + 255) // 256 * 256     # headroom for the next appends
+
+            def rows(old: torch.Tensor | None, fresh: torch.Tensor | None) -> torch.Tensor | None:
+                """[n_pad, ...] buffer: old rows (in place or copied), then the new rows."""
+                if old is None:
+                    return None
+                if grow:
+                    t = torch.zeros((n_pad, *old.shape[1:]), dtype=old.dtype, device=dev)
+                    t[:n_old].copy_(old[:n_old])
+                else:
+                    t = old
+                t[n_old:n].copy_(fresh[:q])
+                return t
+
+            operand = rows(cat.operand, new.operand)
+            col_side = rows(p_old["col_side"], p_new["col_side"])
+            meta_scale = rows(p_old["meta_scale"], p_new["meta_scale"])
+            genre_hi = rows(p_old["genre_hi"], p_new["genre_hi"])
+            nnz_old, nnz_new = p_old["nnz"], p_new["nnz"]
+            indptr = torch.cat([cat.text_indptr[:n_old + 1], new.text_indptr[1:] + cat.text_indptr[n_old]])
+            indices = torch.cat([cat.text_indices[:nnz_old], new.text_indices[:nnz_new]])
+            values = torch.cat([p_old["values"][:nnz_old], p_new["values"][:nnz_new]])
+            if nnz_old + nnz_new == 0:     # the C ABI wants non-NULL arrays, which are never read
+                indices = torch.zeros((1,), dtype=torch.int32, device=dev)
+                values = torch.zeros((1,), dtype=torch.float64, device=dev)
+            genre_dense = None if p_old["genre_dense"] is None else \
+                torch.cat([p_old["genre_dense"][:n_old], p_new["genre_dense"][:q]])
+            meta_dense = [torch.cat([a[:n_old], b[:q]]) for a, b in zip(p_old["meta_dense"], p_new["meta_dense"])]
+            f = Features.from_buffer_copy(c)
+            f.n_shows, f.n_pad = n, n_pad
+            f.operand = operand.data_ptr()
+            f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.col_side, f.meta_scale = col_side.data_ptr(), meta_scale.data_ptr()
+            f.genre_hi = None if genre_hi is None else genre_hi.data_ptr()
+            f.text_signed = int(bool(c.text_signed) or bool(nc.text_signed))
+            if genre_dense is not None:
+                f.genre_dense = genre_dense.data_ptr()
+            for gi, m in enumerate(meta_dense):
+                f.meta_dense[gi] = m.data_ptr()
+            grown = DeviceCatalogue(
+                c=f, n_shows=n, folded=cat.folded, weights_baked=cat.weights_baked,
+                keep=[indptr, indices, values, operand, col_side, meta_scale, genre_hi, genre_dense, *meta_dense],
+                operand=operand, text_indptr=indptr, text_indices=indices,
+                parts={"values": values, "col_side": col_side, "meta_scale": meta_scale, "genre_hi": genre_hi,
+                       "nnz": nnz_old + nnz_new, "genre_dense": genre_dense, "meta_dense": meta_dense,
+                       "meta_widths": p_old["meta_widths"]})
+            fc = cat.fold
+            if fc is not None and self._fold_owner is fc and not grow and not f.text_signed:
+                # the second operand (small vocabularies): write the new rows' text and group columns
+                ff = Features.from_buffer_copy(fc["c"])
+                k_fold, buf = int(ff.k_pad), fc["operand"]
+                row0 = buf[n_old:].data_ptr()
+                scale = float(2 ** TEXT_SCALE_LOG2)
+                check(lib.tvbf_prep_csr_to_operand(new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
+                                                   p_new["values"].data_ptr(), q, row0, k_fold, 0, scale, code, stream),
+                      "tvbf_prep_csr_to_operand")
+                if fc["weights"] is not None:
+                    gw, tw, mw = fc["weights"]
+                    check(lib.tvbf_prep_fold_bits(col_side[n_old:].data_ptr(),
+                                                  None if genre_hi is None else genre_hi[n_old:].data_ptr(),
+                                                  meta_scale[n_old:].data_ptr(), q, int(c.genre_dim), row0, k_fold,
+                                                  int(c.vocab), scale * float(np.sqrt(gw / tw)),
+                                                  scale * float(np.sqrt(mw / tw)), code, stream),
+                          "tvbf_prep_fold_bits")
+                for name in ("n_shows", "text_indptr", "text_indices", "text_values", "col_side", "meta_scale",
+                             "genre_hi"):
+                    setattr(ff, name, getattr(f, name))
+                grown.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+            grown.keep.append(new)          # the new rows' tensors stay alive while the grown catalogue uses them
+        cat.operand = None                  # consumed: its buffers now belong to the grown catalogue
+        cat.c.operand = None
+        cat.keep.clear()
+        cat.parts = {}
+        cat.fold = None
+        cat.buffers = {}                    # prepare(recycle=cat) must not take the grown catalogue's buffers
+        cat.h2d_set = None
+        return grown
+
+    def top_k_append_device(self, cat: DeviceCatalogue, n_old: int, previous: dict, weights=(0.4, 0.5, 0.1),
+                            k: int = 20, min_similarity: float = 0.1, out: dict | None = None) -> dict:
+        """Table of the grown catalogue ``cat`` (from ``extend``) from ``previous``, the device table
+        (``top_k_device``) of its first ``n_old`` shows for the same weights, ``k`` and
+        ``min_similarity`` (``exclude_self=True``).  Bit-identical to ``top_k_device(cat, ...)``
+        (indices, counts and the four scores); ``changed_rows`` of the result holds the sorted int32
+        old rows whose indices or counts differ from ``previous`` (every other old row is
+        byte-identical to its previous row).
+
+        The incremental path (``tvbf_append_topk``) computes only the 256 x 256 tiles that hold a new
+        show and copies the previous row of every old show that received no new candidate.  Jobs the
+        symmetric sweep does not take (float-valued groups, negative weights, k > 100, ...) and
+        catalogues with signed text run the whole job and compare.  ``incremental`` of the result
+        says which of the two ran."""
+        n_old, k = int(n_old), int(k)
+        if previous["indices"].dim() != 2 or tuple(previous["indices"].shape) != (n_old, k) \
+                or tuple(previous["counts"].shape) != (n_old,):
+            raise ValueError(f"previous table has shape {tuple(previous['indices'].shape)}, expected ({n_old}, {k})")
+        if not 0 <= n_old <= cat.n_shows:
+            raise ValueError(f"n_old {n_old} outside [0, {cat.n_shows}]")
+        gw, tw, mw = (float(w) for w in weights)
+        if n_old == cat.n_shows:
+            return {**previous, "changed_rows": torch.zeros((0,), dtype=torch.int32, device=self.device),
+                    "incremental": True}
+        p = self._params(cat, weights, k, min_similarity)
+        with torch.cuda.device(self.device):
+            feats = self._append_features(cat, n_old, weights, k, min_similarity)
+            if feats is None:
+                # whole job on the grown catalogue, changed rows by comparison
+                t = self.top_k_device(cat, weights, k, min_similarity, out=out)
+                diff = (t["counts"][:n_old] != previous["counts"]) | \
+                    (t["indices"][:n_old] != previous["indices"]).any(dim=1)
+                t["changed_rows"] = torch.nonzero(diff).flatten().to(torch.int32)
+                t["incremental"] = False
+                return t
+            nbytes = self.lib.tvbf_append_workspace_bytes(C.byref(feats), C.byref(p), n_old)
+            if nbytes == 0:
+                check(-1, "tvbf_append_workspace_bytes")
+            ws = self._workspace(nbytes)
+            t = out if out is not None else self._alloc_tables(cat.n_shows, k)
+            changed = torch.empty((n_old,), dtype=torch.int32, device=self.device)
+            prev = self._c_tables({**previous, "stats": t["stats"]})
+            check(self.lib.tvbf_append_topk(C.byref(feats), C.byref(p), n_old, C.byref(prev), C.byref(self._c_tables(t)),
+                                            changed.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()),
+                  "tvbf_append_topk")
+            t["changed_rows"] = torch.nonzero(changed).flatten().to(torch.int32)
+            t["incremental"] = True
+        t["row_begin"] = 0
+        return t
+
+    def _append_features(self, cat: DeviceCatalogue, n_old: int, weights, k: int, min_similarity: float):
+        """``tvbf_features`` the incremental append runs on (the folded second operand when the job
+        qualifies), or None when the job needs the whole job: signed text, or not eligible for the
+        symmetric sweep."""
+        gw, tw, mw = (float(w) for w in weights)
+        if n_old <= 0 or cat.c.text_signed:
+            return None
+        p = self._params(cat, weights, k, min_similarity)
+        if not self.lib.tvbf_sym_eligible(C.byref(cat.c), C.byref(p)):
+            return None
+        feats = self._folded(cat, gw, tw, mw, int(k))
+        return cat.c if feats is None else feats
+
+    def append_tiles(self, cat: DeviceCatalogue, n_old: int, weights=(0.4, 0.5, 0.1), k: int = 20,
+                     min_similarity: float = 0.1) -> dict | None:
+        """Tensor-core tiles (256 x 256 x k_pad) the incremental append of ``top_k_append_device``
+        executes on ``cat`` (host only): its threshold seed pass over the super blocks that hold new
+        shows and the append sweep.  None when the job runs the whole job instead."""
+        with torch.cuda.device(self.device):
+            feats = self._append_features(cat, int(n_old), weights, int(k), float(min_similarity))
+            if feats is None or int(n_old) >= cat.n_shows:
+                return None
+            out = (C.c_int64 * 2)()
+            check(self.lib.tvbf_append_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
+                                                  int(n_old), out), "tvbf_append_plan_tiles")
+        return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
 
     def top_k_sweep_device(self, cat: DeviceCatalogue, weight_list, k: int = 20, min_similarity: float = 0.1,
                            exclude_self: bool = True, shared: bool | None = None, tuning: int = 0,

@@ -18,6 +18,16 @@ from ..engine import HybridTopKEngine, TopK, default_engine
 logger = logging.getLogger(__name__)
 
 
+def _split_rows(features: dict, n: int) -> tuple[dict, dict]:
+    """(rows [0, n), rows [n, ...)) of the five feature matrices of a features dict."""
+    keys = ("genre_features", "text_features", "platform_features", "type_features", "language_features")
+    old, new = dict(features), dict(features)
+    for key in keys:
+        a = features[key]
+        old[key], new[key] = a[:n], a[n:]
+    return old, new
+
+
 # noinspection PyMethodMayBeStatic
 class SimilarityComputer:
     """Compute similarity matrices (and top-K tables) from feature arrays."""
@@ -133,6 +143,61 @@ class SimilarityComputer:
                                            exclude_self, list(device_ids), **kw)
         eng = self.engine if device_ids is None else HybridTopKEngine(device_ids[0])
         return eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self, **kw)
+
+    def extend_top_k(self, features: dict, previous: TopK, k: int = 20, min_similarity: float = 0.1,
+                     exclude_self: bool = True, metadata_mode: str = "mean3",
+                     normalize_weights: bool = False) -> TopK:
+        """Top-K table after appending shows to a catalogue whose table exists.
+
+        ``features`` covers all N + Q shows: the N shows of ``previous`` (the ``compute_top_k``
+        table of the first N rows with the same arguments) followed by the Q new ones.  The result
+        equals ``compute_top_k(features, ...)`` bit for bit; its ``changed_rows`` lists the old rows
+        (sorted int32) whose neighbours or their count changed -- every other old row is identical
+        to its row in ``previous``, so a caller only has to store the listed rows and the new ones.
+        Only the pairs with a new show are scored on the tensor cores.
+
+        Precondition: the first N shows' features are those ``previous`` was computed from, and the
+        new shows are encoded in the same vocabulary and widths (the already fitted extractor); a
+        refitted extractor changes every row and needs ``compute_top_k``.  Jobs the incremental path
+        does not take (signed text, float-valued groups, k > 100, ``exclude_self=False``, ...) run the
+        whole job and compare."""
+        weights = self._normalized_weights() if normalize_weights else \
+            (self.genre_weight, self.text_weight, self.metadata_weight)
+        n_all = int(np.asarray(features["genre_features"]).shape[0])
+        n_old = int(previous.counts.shape[0])
+        if previous.indices.ndim != 2 or previous.indices.shape != (n_old, k) or previous.row_begin != 0:
+            raise ValueError(f"previous table has shape {previous.indices.shape}, expected ({n_old}, {k}) from row 0")
+        if n_old > n_all:
+            raise ValueError(f"previous table has {n_old} rows, features only {n_all}")
+        eng = self.engine
+
+        def full() -> TopK:
+            top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
+            diff = (top.counts[:n_old] != previous.counts) | (top.indices[:n_old] != previous.indices).any(axis=1)
+            top.changed_rows = np.nonzero(diff)[0].astype(np.int32)
+            return top
+
+        if n_old == n_all:
+            return TopK(previous.indices, previous.counts, previous.hybrid, previous.genre, previous.text,
+                        previous.metadata, changed_rows=np.zeros(0, dtype=np.int32))
+        if not exclude_self or n_old == 0:
+            return full()
+        old, new = _split_rows(features, n_old)
+        try:
+            cat = eng.extend(eng.ingest(old, metadata_mode, weights), new)
+        except ValueError:
+            # the two parts classify differently (e.g. binary genres before, fractional ones among the
+            # new shows): one catalogue encoding for all rows needs the whole job
+            return full()
+        with torch.cuda.device(eng.device):
+            dev = eng.device
+            prev = {name: torch.from_numpy(np.ascontiguousarray(getattr(previous, name))).to(dev)
+                    for name in ("indices", "counts", "hybrid", "genre", "text", "metadata")}
+            t = eng.top_k_append_device(cat, n_old, prev, weights, k, min_similarity)
+            changed = t["changed_rows"].cpu().numpy()
+        top = eng.to_host(t)
+        top.changed_rows = changed
+        return top
 
     def compute_top_k_sweep(self, features: dict, weight_list, k: int = 20, min_similarity: float = 0.1,
                             exclude_self: bool = True, metadata_mode: str = "mean3",
