@@ -292,6 +292,23 @@ int tvbf_append_topk(const tvbf_features* f, const tvbf_params* p, int32_t n_old
                      const tvbf_topk_out* out, int32_t* changed, void* workspace, size_t workspace_bytes,
                      void* stream);
 
+/* ---- update the features of shows in a catalogue whose table exists (instead of the whole job again).
+ *      f: the catalogue of n_shows shows AFTER the update, the rows rows[0 .. n_rows) (device array,
+ *      sorted, distinct, in [0, n_shows)) with their new features, every other row unchanged since
+ *      `prev` was computed, all in the same vocabulary and widths; prev: the [n_shows, k] table of the
+ *      catalogue before the update from a job with the same p (weights, k, min_similarity,
+ *      exclude_self = 1).  Writes the [n_shows, k] table of the updated catalogue to `out` --
+ *      bit-identical to tvbf_hybrid_topk on f (indices, counts and the four scores; stats differ) --
+ *      and changed[r] = 1 for every row r, updated or not, that differs from prev in any of the six
+ *      fields (0 otherwise: the row is byte-identical).  Only the updated shows' rows are swept against
+ *      all columns; a row that names no updated show and receives no candidate from one above its
+ *      threshold is copied from prev without rescoring.  Jobs tvbf_sym_eligible rejects, and signed
+ *      text, are rejected (the caller runs the whole job).  `out` must not alias `prev`. */
+size_t tvbf_update_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_rows);
+int tvbf_update_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* rows, int32_t n_rows,
+                     const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
+                     size_t workspace_bytes, void* stream);
+
 /* exact fp64 scoring of explicit source rows against all columns + exact top-K
  * (replaces get_recommendations_from_matrix, content_based_service.py:161-236, for any n). */
 size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed);
@@ -379,6 +396,15 @@ int tvbf_append_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t
  * of items.  Used by the CPU tests to prove that every pair with a new show is computed exactly once. */
 int32_t tvbf_debug_append_schedule(int32_t n_old, int32_t n_shows, int32_t sm_count, int32_t* out,
                                    int32_t max_items);
+/* host-only: tensor-core tiles tvbf_update_topk executes for this job with n_rows updated shows,
+ * out2 = {tiles of its threshold seed pass over the gathered rows, tiles of the update sweep}
+ * (256 x 256 x k_pad each).  Fails like tvbf_update_workspace_bytes for a job the update does not take. */
+int tvbf_update_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2);
+/* host-only: the work items of the update sweep of tvbf_update_topk for q updated shows in a catalogue
+ * of n_shows on a device with sm_count SMs; out as tvbf_debug_schedule (super block = block of 256
+ * gathered rows).  Returns the number of items.  Used by the CPU tests to prove that every (gathered
+ * row block, column tile) is computed exactly once. */
+int32_t tvbf_debug_update_schedule(int32_t q, int32_t n_shows, int32_t sm_count, int32_t* out, int32_t max_items);
 /* host-only: tensor-core tiles the candidate pass of this job executes -- out4 = {tiles of the
  * threshold seed pass, tiles of the main sweep, rows per tile (128 or 256; columns are 256 and the
  * depth is k_pad), 1 if the symmetric sweep is used}.  tile_sharded = 0: the job as tvbf_hybrid_topk

@@ -1070,6 +1070,253 @@ int32_t tvbf_debug_append_schedule(int32_t n_old, int32_t n_shows, int32_t sm_co
   return tvbf::k1_debug_append_schedule(kp, out, max_items);
 }
 
+// ---- update the features of shows in a catalogue whose table exists ----------------------------
+// The updated shows' operand rows are gathered into a [q_pad, k_pad] operand.  The update sweep (K1
+// kMode 7) runs those rows against every column tile and offers each score to the row's show and to
+// the column's show unless that one was updated too (it has a gathered row of its own): every ordered
+// pair with an updated show reaches its list once.  K4s compacts the lists; K5 merges them with the
+// previous rows minus the updated shows (list 1) under the rank cut; K6 repairs over all columns.
+namespace {
+
+__global__ void update_bits_kernel(const int* rows, int q, unsigned int* bits) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < q) atomicOr(bits + (rows[r] >> 5), 1u << (rows[r] & 31));
+}
+
+// dst row r = operand row rows[r] (r < q), zero for the padding rows up to q_pad
+__global__ void update_gather_kernel(const uint4* operand, const int* rows, int q, int q_pad, int row_vec,
+                                     uint4* dst) {
+  const size_t n = static_cast<size_t>(q_pad) * row_vec;
+  for (size_t e = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; e < n;
+       e += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const int r = static_cast<int>(e / row_vec), c = static_cast<int>(e % row_vec);
+    dst[e] = r < q ? operand[static_cast<size_t>(rows[r]) * row_vec + c] : make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+
+// After K4s: a show that was not updated, received no candidate from an updated one above its threshold
+// (strictly below its previous k-th score, or below min_similarity for a short row) and names no
+// updated show in its previous row keeps that row: the scores of all its other columns are unchanged.
+// It is copied, no rescoring.  Every other show is listed for K5.
+__global__ void update_select_kernel(tvbf_topk_out prev, tvbf_topk_out out, const int* list0_cnt,
+                                     const unsigned int* bits, int n_shows, int k, int* rows, int* n_listed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  const size_t base = static_cast<size_t>(r) * k;
+  bool listed = ((bits[r >> 5] >> (r & 31)) & 1u) != 0u || list0_cnt[r] != 0;
+  for (int e = 0; e < prev.counts[r] && !listed; ++e) {
+    const int j = prev.indices[base + e];
+    listed = ((bits[j >> 5] >> (j & 31)) & 1u) != 0u;
+  }
+  if (listed) {
+    rows[atomicAdd(n_listed, 1)] = r;
+    return;
+  }
+  for (int e = 0; e < k; ++e) {
+    out.indices[base + e] = prev.indices[base + e];
+    out.hybrid[base + e] = prev.hybrid[base + e];
+    out.genre[base + e] = prev.genre[base + e];
+    out.text[base + e] = prev.text[base + e];
+    out.metadata[base + e] = prev.metadata[base + e];
+  }
+  out.counts[r] = prev.counts[r];
+}
+
+__device__ __forceinline__ bool same_bits(double a, double b) { return __double_as_longlong(a) == __double_as_longlong(b); }
+
+// changed[r] = 1 when row r differs from the previous row in any of the six fields (bit for bit)
+__global__ void update_changed_kernel(tvbf_topk_out prev, tvbf_topk_out out, int n_shows, int k, int* changed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  int c = prev.counts[r] != out.counts[r];
+  const size_t base = static_cast<size_t>(r) * k;
+  for (int e = 0; e < k && !c; ++e)
+    c = prev.indices[base + e] != out.indices[base + e] || !same_bits(prev.hybrid[base + e], out.hybrid[base + e]) ||
+        !same_bits(prev.genre[base + e], out.genre[base + e]) || !same_bits(prev.text[base + e], out.text[base + e]) ||
+        !same_bits(prev.metadata[base + e], out.metadata[base + e]);
+  changed[r] = c;
+}
+
+struct UpdatePlan {
+  Plan pl;             // a whole-catalogue symmetric job over all shows
+  tvbf::K1Params geo;  // tile schedule of the update sweep
+  int grid, q_pad;
+  size_t off_cand, off_cnt, off_bound;   // two candidate lists per show: [2][n_shows]
+  size_t off_rows, off_listed;           // shows K5 rescores and their count
+  size_t off_gather, off_bits, off_cut_s, off_cut_j, total;
+};
+
+int make_update_plan(const tvbf_features* f, const tvbf_params* p, int n_rows, UpdatePlan* up, tvbf_params* q) {
+  TVBF_REQUIRE(n_rows >= 1 && n_rows <= f->n_shows, "update: %d rows outside [1, n_shows %d]", n_rows, f->n_shows);
+  TVBF_REQUIRE(!f->text_signed, "update: signed text needs the whole job");
+  *q = *p;
+  q->row_begin = 0;
+  q->row_end = f->n_shows;
+  q->tuning = (q->tuning & ~(0x3 << 20)) | (2 << 20);   // symmetric job (or fail if ineligible)
+  q->tuning = (q->tuning & ~0xF) | 2;                   // CTA pairs
+  int rc = validate_params(f, q);
+  if (rc != TVBF_OK) return rc;
+  rc = make_plan(f, q, &up->pl);
+  if (rc != TVBF_OK) return rc;
+  int sms = 0;
+  rc = sm_count_cached(&sms);
+  if (rc != TVBF_OK) return rc;
+  memset(&up->geo, 0, sizeof(up->geo));
+  tvbf::k1_update_geometry(n_rows, f->n_shows, sms / 2, &up->geo);
+  const int items = (up->geo.rb_count + up->geo.rb_per_group - 1) / up->geo.rb_per_group * up->geo.rb_per_group *
+                    up->geo.splits;
+  up->grid = 2 * (items < sms / 2 ? items : sms / 2);
+  up->q_pad = up->geo.rb_count * 256;
+  const size_t rows = static_cast<size_t>(f->n_shows);
+  size_t off = up->pl.total;
+  up->off_cand = off;   off = align_up(off + 2 * rows * up->pl.kp * 8, 256);
+  up->off_cnt = off;    off = align_up(off + 2 * rows * 4, 256);
+  up->off_bound = off;  off = align_up(off + 2 * rows * 4, 256);
+  up->off_rows = off;   off = align_up(off + rows * 4, 256);
+  up->off_listed = off; off = align_up(off + 4, 256);
+  up->off_gather = off; off = align_up(off + static_cast<size_t>(up->q_pad) * f->k_pad * 2, 256);
+  up->off_bits = off;   off = align_up(off + static_cast<size_t>(f->n_pad) / 32 * 4, 256);
+  up->off_cut_s = off;  off = align_up(off + rows * 8, 256);
+  up->off_cut_j = off;  off = align_up(off + rows * 4, 256);
+  up->total = off;
+  return TVBF_OK;
+}
+
+// the candidate-kernel parameters of an update: a whole-catalogue symmetric job on the update geometry
+int fill_update_params(const tvbf_features* f, const tvbf_params* q, const UpdatePlan& up, uint8_t* ws,
+                       const int* rows, int n_rows, tvbf::K1Params* kp) {
+  int rc = fill_k1_params(f, q, up.pl, ws, kp);
+  if (rc != TVBF_OK) return rc;
+  kp->sync_kb = 0;
+  kp->sym = 0;   // the one-sided schedule: a rectangle (the epilogue of kMode 7 still feeds both lists)
+  // 8 epilogue warps whatever the vocabulary: the 16-warp epilogue spills under its register cap, and
+  // the sweep covers few tiles
+  kp->wide_epilogue = 0;
+  kp->col_tiles = up.geo.col_tiles;
+  kp->rb_count = up.geo.rb_count;
+  kp->splits = up.geo.splits;
+  kp->rb_per_group = up.geo.rb_per_group;
+  kp->tiles_per_split = up.geo.tiles_per_split;
+  kp->upd_rows = rows;
+  kp->upd_q = n_rows;
+  kp->upd_bits = reinterpret_cast<const unsigned int*>(ws + up.off_bits);
+  kp->cand = reinterpret_cast<uint2*>(ws + up.off_cand);   // list 0: what the update sweep found
+  kp->cand_cnt = reinterpret_cast<int*>(ws + up.off_cnt);
+  kp->cand_theta = reinterpret_cast<float*>(ws + up.off_bound);
+  return TVBF_OK;
+}
+
+}  // namespace
+
+size_t tvbf_update_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_rows) {
+  if (validate_features(f) != TVBF_OK || p == nullptr) return 0;
+  UpdatePlan up;
+  tvbf_params q;
+  if (make_update_plan(f, p, n_rows, &up, &q) != TVBF_OK) return 0;
+  return up.total;
+}
+
+int tvbf_update_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* rows, int32_t n_rows,
+                     const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p != nullptr, "params is NULL");
+  TVBF_REQUIRE(prev && prev->indices && prev->counts && prev->hybrid && prev->genre && prev->text && prev->metadata,
+               "previous table has NULL members");
+  TVBF_REQUIRE(out && out->indices && out->counts && out->hybrid && out->genre && out->text && out->metadata &&
+                   out->stats,
+               "output table has NULL members");
+  TVBF_REQUIRE(rows != nullptr && changed != nullptr && workspace != nullptr, "tvbf_update_topk: NULL argument");
+  UpdatePlan up;
+  tvbf_params q;
+  rc = make_update_plan(f, p, n_rows, &up, &q);
+  if (rc != TVBF_OK) return rc;
+  if (workspace_bytes < up.total) {
+    tvbf_set_error("workspace too small: %zu < %zu", workspace_bytes, up.total);
+    return TVBF_ERR_WORKSPACE;
+  }
+  auto st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const Plan& pl = up.pl;
+  const int n = f->n_shows;
+  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
+  double* floors = reinterpret_cast<double*>(ws + pl.off_floor);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+  int* listed_rows = reinterpret_cast<int*>(ws + up.off_rows);
+  int* n_listed = reinterpret_cast<int*>(ws + up.off_listed);
+  unsigned int* bits = reinterpret_cast<unsigned int*>(ws + up.off_bits);
+  double* cut_s = reinterpret_cast<double*>(ws + up.off_cut_s);
+  int* cut_j = reinterpret_cast<int*>(ws + up.off_cut_j);
+  tvbf::K1Params kp;
+  rc = fill_update_params(f, &q, up, ws, rows, n_rows, &kp);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaMemsetAsync(bits, 0, static_cast<size_t>(f->n_pad) / 32 * 4, st));
+  update_bits_kernel<<<(n_rows + 255) / 256, 256, 0, st>>>(rows, n_rows, bits);
+  TVBF_LAUNCH_OK("update_bits_kernel");
+  const int row_vec = f->k_pad / 8;   // 16-byte vectors per operand row
+  update_gather_kernel<<<1024, 256, 0, st>>>(static_cast<const uint4*>(f->operand), rows, n_rows, up.q_pad, row_vec,
+                                             reinterpret_cast<uint4*>(ws + up.off_gather));
+  TVBF_LAUNCH_OK("update_gather_kernel");
+  tvbf_features g = *f;   // the gathered rows as the A operand
+  g.operand = ws + up.off_gather;
+  g.n_pad = up.q_pad;
+  uint2* cand = kp.cand;
+  int* cnt = kp.cand_cnt;
+  float* bound = kp.cand_theta;
+  const tvbf::UpdatePrev pv{prev->indices, prev->counts, prev->hybrid, p->k, bits,
+                            cand + static_cast<size_t>(n) * pl.kp, cnt + n, bound + n, cut_s, cut_j};
+  TVBF_CUDA_OK(cudaMemsetAsync(out->stats, 0, 8 * sizeof(int32_t), st));
+  rc = tvbf::k1_launch_update(f, &g, kp, up.grid, pv, st);
+  if (rc != TVBF_OK) return rc;
+  rc = tvbf::k4s_launch(kp, n, st);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaMemsetAsync(n_listed, 0, 4, st));
+  update_select_kernel<<<(n + 255) / 256, 256, 0, st>>>(*prev, *out, cnt, bits, n, p->k, listed_rows, n_listed);
+  TVBF_LAUNCH_OK("update_select_kernel");
+  const tvbf::ScoreParams sp = score_params(f, &q);
+  const tvbf::CandLayout lay{0, 1, n, 0};   // list s of show r: slot r + s * n
+  rc = tvbf::k5_launch_listed(sp, cand, cnt, bound, 2, lay, pl.kp, 0, n, listed_rows, n_listed, *out, flagged, floors,
+                              st, cut_s, cut_j);
+  if (rc != TVBF_OK) return rc;
+  rc = tvbf::k6_launch_flagged(sp, flagged, floors, n, 0, keys, pl.k6_grid, *out, st);
+  if (rc != TVBF_OK) return rc;
+  update_changed_kernel<<<(n + 255) / 256, 256, 0, st>>>(*prev, *out, n, p->k, changed);
+  TVBF_LAUNCH_OK("update_changed_kernel");
+  return TVBF_OK;
+}
+
+int tvbf_update_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2) {
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p && out2, "tvbf_update_plan_tiles: NULL argument");
+  UpdatePlan up;
+  tvbf_params q;
+  rc = make_update_plan(f, p, n_rows, &up, &q);
+  if (rc != TVBF_OK) return rc;
+  uint8_t* fake_ws = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(4096));   // offsets only, never dereferenced
+  tvbf::K1Params kp;
+  rc = fill_update_params(f, &q, up, fake_ws, nullptr, n_rows, &kp);
+  if (rc != TVBF_OK) return rc;
+  long long t[2];
+  tvbf::k1_update_executed_tiles(kp, up.grid, t);
+  out2[0] = t[0];
+  out2[1] = t[1];
+  return TVBF_OK;
+}
+
+int32_t tvbf_debug_update_schedule(int32_t q, int32_t n_shows, int32_t sm_count, int32_t* out, int32_t max_items) {
+  if (q < 1 || q > n_shows || sm_count < 2 || out == nullptr || max_items < 0) {
+    tvbf_set_error("tvbf_debug_update_schedule: bad arguments");
+    return TVBF_ERR_INVALID;
+  }
+  tvbf::K1Params kp;
+  memset(&kp, 0, sizeof(kp));
+  tvbf::k1_update_geometry(q, n_shows, sm_count / 2, &kp);
+  return tvbf::k1_debug_schedule(kp, out, max_items);
+}
+
 // ---- streaming statistics of the four similarity matrices (no N x N) --------------------------
 size_t tvbf_stats_accum_bytes(void) { return sizeof(tvbf::StatsAccum); }
 

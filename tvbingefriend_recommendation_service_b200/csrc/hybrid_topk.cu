@@ -403,7 +403,10 @@ struct Pacer {
 // 3 threshold seed pass (one-sided walk over sampled tiles, per-row score histograms, no lists),
 // 5 symmetric top-k sweep for p.n_weights weight triples at once (one shared list per triple and show),
 // 6 append sweep: the symmetric top-k sweep restricted to the tiles that hold a new show (column tile
-// >= p.append_b0), offering no pair of two old shows (p.append_n_old)
+// >= p.append_b0), offering no pair of two old shows (p.append_n_old),
+// 7 update sweep: the gathered rows of the updated shows (p.upd_rows) against every column tile, a
+// rectangle without a diagonal; offered to the row's show and to every column show not updated itself,
+// 8 the threshold seed pass (as 3) over the gathered rows of an update
 // kG2: multi-hot genres with 64 < G <= 128 -- the second word of every column's mask is staged beside
 // the column-side records (in the threshold slices a single-triple sweep leaves unused) and the
 // popcount runs over both words.
@@ -418,11 +421,13 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
                    const __grid_constant__ CUtensorMap tmap_b, const K1Params p,
                    const uint32_t idesc) {
   using L = Smem<CG, kWide>;
-  constexpr bool kHist = kMode == 3;     // threshold seed pass: per-row histograms of the sampled scores
+  constexpr bool kHist = kMode == 3 || kMode == 8;   // threshold seed pass: per-row histograms of the sampled scores
   constexpr bool kSym = kMode != 0 && !kHist;   // tiles on/above the diagonal, 8 (kWide: 16) epilogue warps
   constexpr bool kStats = kMode == 2;    // accumulate statistics instead of candidate lists
   constexpr bool kMulti = kMode == 5;    // weight sweep
   constexpr bool kAppend = kMode == 6;   // append sweep
+  constexpr bool kUpdate = kMode == 7;   // update sweep
+  constexpr bool kGather = kMode == 7 || kMode == 8;   // rows are the gathered rows of an update
   static_assert(!(kG2 && (kMulti || kStats)), "two-word genre masks: single-triple top-k sweeps only");
   static_assert(!(kFold && (kMulti || kStats || kDump || kG2)), "folded groups: single-triple top-k sweeps only");
   // Seed pass: hist[bin][row of the CTA] (32-bit counters; bank = row % 32, so the 32 lanes of a warp
@@ -637,8 +642,9 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       if (kDump) { c.sb = 0; c.tile0 = 0; c.tile1 = 1; }
       if (c.sb < 0) continue;
       const int row_local0 = (kDump ? 0 : c.sb * BM * CG) + static_cast<int>(cta_rank) * BM;  // within shard
-      const int row = p.row_begin + row_local0 + row_in_tile;
-      const bool row_valid = row < p.row_end;
+      const int grow = p.row_begin + row_local0 + row_in_tile;
+      const bool row_valid = kGather ? grow < p.upd_q : grow < p.row_end;
+      const int row = kGather ? (row_valid ? p.upd_rows[grow] : -1) : grow;   // the show of this row
       // row-side operands of the fused scores
       unsigned long long g_bits = 0ull, g_hi = 0ull;
       uint32_t m_bits = 0u;
@@ -743,8 +749,9 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
         const unsigned long long* sgh =
             reinterpret_cast<const unsigned long long*>(smem + L::OFF_TH + (b * kMaxSweep + 1) * MS_BYTES);
         const uint32_t taddr = tmem_base + tmem_lane + b * BN;
-        // off-diagonal tiles also feed the column shows (their mirror tile is never computed)
-        const bool do_col = kSym && row_valid && jt != c.sb;
+        // off-diagonal tiles also feed the column shows (their mirror tile is never computed); the
+        // update sweep's rectangle has no mirror tiles
+        const bool do_col = kSym && row_valid && (kUpdate || jt != c.sb);
 
         float tile_sum[4] = {0.f, 0.f, 0.f, 0.f}, tile_sq[4] = {0.f, 0.f, 0.f, 0.f}, tile_gm = 0.f;
         float stat_scale[4];
@@ -889,6 +896,13 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
                     const uint32_t m = old_cols >= GW ? (1u << GW) - 1u : (1u << old_cols) - 1u;
                     hit_r &= ~m;
                     hit_c &= ~m;
+                  }
+                }
+                if constexpr (kUpdate) {
+                  // an updated column has a gathered row of its own, which offers it this pair
+                  if (hit_c != 0u) {
+                    const int c0 = col0 + cbase + h * GW;   // GW-aligned: one word of the bit set
+                    hit_c &= ~((p.upd_bits[c0 >> 5] >> (c0 & 31)) & ((1u << GW) - 1u));
                   }
                 }
                 push_hits(hit_r | (hit_c << GW), u, col0 + cbase + h * GW, 0);
@@ -1261,6 +1275,42 @@ __global__ void append_prev_kernel(AppendPrev a, unsigned int* theta, float thet
   a.bound[r] = __int_as_float(0xff800000);
 }
 
+// Update: a show that was not updated gets its previous row without the updated shows as list 1 (bound
+// -inf) and, when that row was full, the threshold of append_prev_kernel and a rank cut at its previous
+// k-th entry e_k: a column missing from the row that was not updated ranks below e_k, and K5 accepts the
+// merged row only if its k-th entry ranks at or above e_k.  An updated show gets an empty list 1, no
+// cut, and keeps the threshold its seed pass writes.
+__global__ void update_prev_kernel(UpdatePrev a, unsigned int* theta, float theta_init, int n_shows, int kp) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  int cnt = 0, cut_j = -1;
+  double cut_h = 0.0;
+  if (((a.upd_bits[r >> 5] >> (r & 31)) & 1u) == 0u) {
+    const int n = a.counts[r];
+    uint2* dst = a.list + static_cast<size_t>(r) * kp;
+    const size_t base = static_cast<size_t>(r) * a.k;
+    for (int e = 0; e < n; ++e) {
+      const int j = a.indices[base + e];
+      if ((a.upd_bits[j >> 5] >> (j & 31)) & 1u) continue;
+      dst[cnt++] = make_uint2(__float_as_uint(__double2float_ru(a.hybrid[base + e])), static_cast<uint32_t>(j));
+    }
+    float th = theta_init;
+    if (n == a.k) {
+      const double kth = a.hybrid[base + a.k - 1];
+      th = __double2float_rd(kth);
+      if (static_cast<double>(th) >= kth) th = nextafterf(th, -INFINITY);
+      th = fmaxf(th, theta_init);
+      cut_h = kth;
+      cut_j = a.indices[base + a.k - 1];
+    }
+    theta[r] = __float_as_uint(th);
+  }
+  a.cnt[r] = cnt;
+  a.bound[r] = __int_as_float(0xff800000);
+  a.cut_score[r] = cut_h;
+  a.cut_index[r] = cut_j;
+}
+
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
@@ -1378,6 +1428,33 @@ int k1_debug_append_schedule(const K1Params& p, int* out, int max_items) {
   return n_items;
 }
 
+// Update sweep: a rectangle of ceil(q / 256) gathered super blocks x every column tile, on the one-sided
+// schedule (p->sym = 0: no diagonal, split s of a super block walks tiles [s * tps, (s + 1) * tps)).
+// Items = (super block, column split) dealt round-robin to the clusters; as for the append, the split
+// count minimises the tiles of the busiest cluster, so that one or a few super blocks still spread
+// over every SM.
+void k1_update_geometry(int q, int n_shows, int clusters, K1Params* p) {
+  p->sym = 0;
+  p->col_tiles = (n_shows + 255) / 256;
+  p->rb_count = (q + 255) / 256;
+  p->deal_groups = 0;
+  p->deal_r = 1;
+  if (clusters < 1) clusters = 1;
+  long long best_cost = -1;
+  for (int s = 1; s <= p->col_tiles && s <= clusters; ++s) {
+    int rb = clusters / s;
+    if (rb > p->rb_count) rb = p->rb_count;
+    const long long items = static_cast<long long>((p->rb_count + rb - 1) / rb) * rb * s;
+    const long long cost = (items + clusters - 1) / clusters * ((p->col_tiles + s - 1) / s);
+    if (best_cost < 0 || cost < best_cost) {
+      best_cost = cost;
+      p->splits = s;
+      p->rb_per_group = rb;
+    }
+  }
+  p->tiles_per_split = (p->col_tiles + p->splits - 1) / p->splits;
+}
+
 int k1_entries_per_lane(int k) {
   if (k <= 48) return 4;
   if (k <= 160) return 8;
@@ -1442,11 +1519,13 @@ static bool profiler_attached() {
   return cached != 0;
 }
 
+// fa: the features whose operand feeds the A (row) side, when not f's (the gathered rows of an update)
 template <int E, bool kDump, int CG, int kMode, bool kWide = false, bool kG2 = false, bool kFold = false>
-static int launch_k1(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st) {
+static int launch_k1(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st,
+                     const tvbf_features* fa = nullptr) {
   using L = Smem<CG, kWide>;
   CUtensorMap ta, tb;
-  int rc = make_operand_map(f, BM, &ta);
+  int rc = make_operand_map(fa != nullptr ? fa : f, BM, &ta);
   if (rc != TVBF_OK) return rc;
   rc = make_operand_map(f, static_cast<int>(L::B_ROWS), &tb);
   if (rc != TVBF_OK) return rc;
@@ -1837,6 +1916,63 @@ int k1_launch_append(const tvbf_features* f, const K1Params& kp, int grid, const
   if (kp.fold) return launch_k1<4, false, 2, 6, false, false, true>(f, sweep, grid, st);
   return kp.genre_hi ? launch_k1<4, false, 2, 6, false, true>(f, sweep, grid, st)
                      : launch_k1<4, false, 2, 6>(f, sweep, grid, st);
+}
+
+// histogram seed pass of an update: the gathered rows against every tile_stride-th column tile
+static K1Params update_seed_params(const K1Params& kp, int grid) {
+  K1Params seed = make_seed_params(kp, grid, 0);
+  seed.row_begin = 0;
+  return seed;
+}
+
+void k1_update_executed_tiles(const K1Params& kp, int grid, long long* out) {
+  out[0] = count_tiles(update_seed_params(kp, grid));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  out[1] = count_tiles(sweep);
+}
+
+int k1_launch_update(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                     const UpdatePrev& prev, cudaStream_t st) {
+  if (kp.sym || kp.n_weights > 1 || kp.sync_kb != 0 || kp.wide_epilogue || kp.upd_q < 1 || kp.upd_rows == nullptr ||
+      kp.upd_bits == nullptr) {
+    tvbf_set_error("update sweep: bad parameters");
+    return TVBF_ERR_INVALID;
+  }
+  const int n_pad = f->n_pad;
+  const size_t list_bytes = static_cast<size_t>(n_pad) * kp.sym_cap * 8;
+  std::lock_guard<std::mutex> lock(g_side_mutex);
+  SideStream* side = nullptr;
+  int rc = side_stream(&side);
+  if (rc != TVBF_OK) return rc;
+  // the shared lists are cleared on the side stream beside the seed pass, as in a full job
+  rc = absorb_pending(side, st, true);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaEventRecord(side->fork, st));
+  TVBF_CUDA_OK(cudaStreamWaitEvent(side->stream, side->fork, 0));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, static_cast<size_t>(n_pad) * 4, side->stream));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, side->stream));
+  TVBF_CUDA_OK(cudaEventRecord(side->join, side->stream));
+  sym_init_kernel<<<static_cast<unsigned>((n_pad + 255) / 256), 256, 0, st>>>(kp.g_theta, f->n_shows, n_pad, n_pad,
+                                                                               kp.theta_init);
+  TVBF_LAUNCH_OK("sym_init_kernel");
+  update_prev_kernel<<<static_cast<unsigned>((f->n_shows + 255) / 256), 256, 0, st>>>(prev, kp.g_theta, kp.theta_init,
+                                                                                      f->n_shows, kp.kp);
+  TVBF_LAUNCH_OK("update_prev_kernel");
+  {
+    const K1Params seed = update_seed_params(kp, grid);
+    const int sg = seed.rb_per_group * 2;
+    if (kp.fold) rc = launch_k1<4, false, 2, 8, false, false, true>(f, seed, sg, st, g);
+    else if (kp.genre_hi != nullptr) rc = launch_k1<4, false, 2, 8, false, true>(f, seed, sg, st, g);
+    else rc = launch_k1<4, false, 2, 8>(f, seed, sg, st, g);
+    if (rc != TVBF_OK) return rc;
+  }
+  TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  if (kp.fold) return launch_k1<4, false, 2, 7, false, false, true>(f, sweep, grid, st, g);
+  return kp.genre_hi ? launch_k1<4, false, 2, 7, false, true>(f, sweep, grid, st, g)
+                     : launch_k1<4, false, 2, 7>(f, sweep, grid, st, g);
 }
 
 int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cudaStream_t st) {

@@ -120,6 +120,29 @@ struct K1Params {
   // offered to neither list
   int append_n_old;
   int append_b0;
+  // update sweep (kMode 7) and its threshold seed pass (kMode 8), tvbf_update_topk: the A operand is
+  // the gather of the updated shows' operand rows, and gathered row r < upd_q is show upd_rows[r],
+  // whose records, slack terms, threshold and list are read through that map.  A column whose bit is
+  // set in upd_bits (bit j % 32 of word j / 32) was updated itself: it is offered nothing from the
+  // column side, its own gathered row feeds its list.
+  const int* upd_rows;
+  int upd_q;
+  const unsigned int* upd_bits;
+};
+
+// The previous table of an update and where its rows go (list 1 of the two-list candidate table, as
+// AppendPrev), plus the rank cut K5 checks for every show whose previous row was full.
+struct UpdatePrev {
+  const int* indices;   // [n_shows, k]
+  const int* counts;    // [n_shows]
+  const double* hybrid; // [n_shows, k]
+  int k;
+  const unsigned int* upd_bits;
+  uint2* list;          // [n_shows][kp]
+  int* cnt;             // [n_shows]
+  float* bound;         // [n_shows]
+  double* cut_score;    // [n_shows] previous k-th entry (score, index); index -1: no cut
+  int* cut_index;
 };
 
 // The previous table of an append and where its rows go: list 1 of the two-list candidate table K5
@@ -160,11 +183,13 @@ struct CandLayout {
 int k5_launch(const ScoreParams& sp, const uint2* cand, const int* cand_cnt,
               const float* cand_theta, int splits, CandLayout lay, int kp, int row_begin, int n_rows,
               const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor, cudaStream_t st);
-// K5 over the table rows rows[0 .. *n_listed) (a device count; at most n_rows)
+// K5 over the table rows rows[0 .. *n_listed) (a device count; at most n_rows).  With cut_index
+// (update): a row r with cut_index[r] >= 0 is final only if its k-th entry also ranks at or above
+// (cut_score[r], cut_index[r]).
 int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_cnt, const float* cand_theta,
                      int splits, CandLayout lay, int kp, int row_begin, int n_rows, const int* rows,
                      const int* n_listed, const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
-                     cudaStream_t st);
+                     cudaStream_t st, const double* cut_score = nullptr, const int* cut_index = nullptr);
 // deal the ceil(total / r) groups of r consecutive super blocks to `world` GPUs; fills gid[] with the
 // groups of `rank` (cost descending) and returns {groups, super blocks} of that rank, or -1 when a
 // rank would own more than kMaxDealGroups groups
@@ -181,6 +206,15 @@ int k1_launch_append(const tvbf_features* f, const K1Params& kp, int grid, const
                      cudaStream_t st);
 // tiles of the append: out[0] its seed pass over the new super blocks, out[1] the append sweep
 void k1_append_executed_tiles(const tvbf_features* f, const K1Params& kp, int grid, long long* out);
+// geometry of the update sweep of q gathered rows against n_shows columns on `clusters` CTA pairs:
+// a rectangle of ceil(q / 256) super blocks x ceil(n_shows / 256) column tiles (p->sym = 0 schedule)
+void k1_update_geometry(int q, int n_shows, int clusters, K1Params* p);
+// thresholds and list 1 from the previous table, seed pass over the gathered rows, then the update
+// sweep; g: f with the gathered operand ([kp.upd_q rounded up to 256, k_pad]) as its operand
+int k1_launch_update(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                     const UpdatePrev& prev, cudaStream_t st);
+// tiles of the update: out[0] its seed pass over the gathered rows, out[1] the update sweep
+void k1_update_executed_tiles(const K1Params& kp, int grid, long long* out);
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);

@@ -116,12 +116,16 @@ __device__ __forceinline__ bool ranks_before(double ha, int ja, double hb, int j
 // ---------------------------------------------------------------------------------------------
 constexpr int K5_WARPS = 4;
 
-// the work of one warp on table row r (source row row_begin + r); n_rows sizes the flagged lists
+// the work of one warp on table row r (source row row_begin + r); n_rows sizes the flagged lists.
+// kCut (update): a row with cut_index[r] >= 0 must also rank its k-th entry at or above
+// (cut_score[r], cut_index[r]) to be final.
+template <bool kCut = false>
 __device__ __forceinline__ void rescore_row(const ScoreParams& sp, const uint2* __restrict__ cand,
                                             const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta,
                                             int splits, const CandLayout& lay, int kp, int row_begin, int n_rows,
                                             const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
-                                            int max_cand, int keep, int warp, int lane, int r) {
+                                            int max_cand, int keep, int warp, int lane, int r,
+                                            const double* cut_score = nullptr, const int* cut_index = nullptr) {
   extern __shared__ __align__(16) uint8_t k5_smem[];
   const int i = row_begin + r;
   uint8_t* base = k5_smem + static_cast<size_t>(warp) * max_cand * 48;
@@ -246,7 +250,17 @@ __device__ __forceinline__ void rescore_row(const ScoreParams& sp, const uint2* 
     atomicAdd(&out.stats[1], total);
     // certificate: all dropped columns have exact score <= U <= theta
     const double bound = s_kth[warp];  // k-th exact score, or min_similarity if fewer than k
-    const bool safe = static_cast<double>(theta) < bound;
+    bool safe = static_cast<double>(theta) < bound;
+    if constexpr (kCut) {
+      // the columns list 1 left out rank below the previous k-th entry: the row is final only if its
+      // k-th entry ranks at or above that (a short row does not)
+      const int cj = cut_index[r];
+      if (cj >= 0) {
+        const double cs = cut_score[r];
+        const int jk = out.indices[obase + k - 1];
+        safe = safe && count == k && (bound > cs || (bound == cs && jk <= cj));
+      }
+    }
     if (!safe) {
       atomicAdd(&out.stats[0], 1);
       // shows with text are listed from the front, shows without (the usual tie plateaus, which
@@ -286,6 +300,20 @@ rescore_listed_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
   if (e >= *n_listed) return;
   rescore_row(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin, n_rows, out, flagged_rows, flagged_floor,
               max_cand, keep, warp, lane, rows[e]);
+}
+
+// ... with the rank cut of an update (rescore_row<true>)
+__global__ void __launch_bounds__(K5_WARPS * 32)
+rescore_cut_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
+                   const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta, int splits,
+                   const CandLayout lay, int kp, int row_begin, int n_rows, const int* __restrict__ rows,
+                   const int* __restrict__ n_listed, tvbf_topk_out out, int* flagged_rows, double* flagged_floor,
+                   int max_cand, int keep, const double* __restrict__ cut_score, const int* __restrict__ cut_index) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (e >= *n_listed) return;
+  rescore_row<true>(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin, n_rows, out, flagged_rows,
+                    flagged_floor, max_cand, keep, warp, lane, rows[e], cut_score, cut_index);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1042,7 +1070,7 @@ int k5_launch(const ScoreParams& sp, const uint2* cand, const int* cand_cnt,
 int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_cnt, const float* cand_theta,
                      int splits, CandLayout lay, int kp, int row_begin, int n_rows, const int* rows,
                      const int* n_listed, const tvbf_topk_out& out, int* flagged_rows, double* flagged_floor,
-                     cudaStream_t st) {
+                     cudaStream_t st, const double* cut_score, const int* cut_index) {
   const int max_cand = splits * kp;
   int warps = K5_WARPS;
   while (warps > 1 && static_cast<size_t>(warps) * max_cand * 48 > 200 * 1024) warps >>= 1;
@@ -1051,9 +1079,18 @@ int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_c
     tvbf_set_error("rescore: lists*candidates = %d is too large", max_cand);
     return TVBF_ERR_INVALID;
   }
+  const int grid = (n_rows + warps - 1) / warps;   // at most n_rows listed; the count is on the device
+  if (cut_index != nullptr) {
+    TVBF_CUDA_OK(cudaFuncSetAttribute(rescore_cut_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      static_cast<int>(smem)));
+    rescore_cut_kernel<<<grid, warps * 32, smem, st>>>(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin,
+                                                       n_rows, rows, n_listed, out, flagged_rows, flagged_floor,
+                                                       max_cand, 2 * kp, cut_score, cut_index);
+    TVBF_LAUNCH_OK("rescore_cut_kernel");
+    return TVBF_OK;
+  }
   TVBF_CUDA_OK(cudaFuncSetAttribute(rescore_listed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     static_cast<int>(smem)));
-  const int grid = (n_rows + warps - 1) / warps;   // at most n_rows listed; the count is on the device
   rescore_listed_kernel<<<grid, warps * 32, smem, st>>>(sp, cand, cand_cnt, cand_theta, splits, lay, kp, row_begin,
                                                         n_rows, rows, n_listed, out, flagged_rows, flagged_floor,
                                                         max_cand, 2 * kp);

@@ -147,7 +147,7 @@ class TopK:
     row_begin: int = 0
     flagged_rows: int = 0    # rows the certificate sent to the exact kernel
     rescored_pairs: int = 0
-    changed_rows: np.ndarray | None = None   # extend_top_k: sorted int32 old rows whose neighbours changed
+    changed_rows: np.ndarray | None = None   # extend_top_k / update_top_k: sorted int32 rows that changed
 
     @property
     def k(self) -> int:
@@ -677,6 +677,28 @@ class HybridTopKEngine:
         return t
 
     # ------------------------------------------------------------------------------------ appends
+    def _ingest_like(self, cat: DeviceCatalogue, features: dict, caller: str) -> DeviceCatalogue:
+        """``features`` ingested as rows of ``cat``: same metadata mode and baked weights.  Raises
+        ``ValueError`` when ``cat`` was consumed, or when the rows differ from it in vocabulary size,
+        genre or metadata width, group encoding (binary / float) or operand width."""
+        c = cat.c
+        if cat.operand is None or not cat.parts:
+            raise ValueError(f"{caller}: the catalogue was recycled or does not come from ingest / prepare")
+        mode = "mean3" if c.meta_kind == _lib.META_MEAN3 else "hstack"
+        new = self.ingest(features, mode, cat.weights_baked or (0.4, 0.5, 0.1))
+        nc = new.c
+        for what, a, b in (("vocabulary size", c.vocab, nc.vocab), ("genre encoding", c.genre_mode, nc.genre_mode),
+                           ("genre columns", c.genre_dim, nc.genre_dim),
+                           ("metadata encoding", c.meta_mode, nc.meta_mode),
+                           ("metadata groups", c.meta_groups, nc.meta_groups),
+                           ("metadata widths", cat.parts["meta_widths"], new.parts["meta_widths"]),
+                           ("operand width", c.k_pad, nc.k_pad), ("text dtype", c.text_dtype, nc.text_dtype)):
+            if a != b:
+                raise ValueError(f"{caller}: the new shows' {what} ({b}) differs from the catalogue's ({a})")
+        if cat.folded and (not new.folded or new.weights_baked != cat.weights_baked):
+            raise ValueError(f"{caller}: the new shows' float groups do not match the catalogue's")
+        return new
+
     def extend(self, cat: DeviceCatalogue, new_features: dict) -> DeviceCatalogue:
         """``cat`` grown by the shows of ``new_features`` (rows N .. N+Q-1 after its N shows).  Only
         the new rows are prepared (ingest, normalisation, operand rows, CSR, column-side records);
@@ -688,21 +710,8 @@ class HybridTopKEngine:
         vocabulary size, genre or metadata width, group encoding (binary / float) or metadata mode
         raises ``ValueError``; a refitted extractor changes every row and needs a whole job."""
         c = cat.c
-        if cat.operand is None or not cat.parts:
-            raise ValueError("extend: the catalogue was recycled or does not come from ingest / prepare")
-        mode = "mean3" if c.meta_kind == _lib.META_MEAN3 else "hstack"
-        new = self.ingest(new_features, mode, cat.weights_baked or (0.4, 0.5, 0.1))
+        new = self._ingest_like(cat, new_features, "extend")
         nc = new.c
-        for what, a, b in (("vocabulary size", c.vocab, nc.vocab), ("genre encoding", c.genre_mode, nc.genre_mode),
-                           ("genre columns", c.genre_dim, nc.genre_dim),
-                           ("metadata encoding", c.meta_mode, nc.meta_mode),
-                           ("metadata groups", c.meta_groups, nc.meta_groups),
-                           ("metadata widths", cat.parts["meta_widths"], new.parts["meta_widths"]),
-                           ("operand width", c.k_pad, nc.k_pad), ("text dtype", c.text_dtype, nc.text_dtype)):
-            if a != b:
-                raise ValueError(f"extend: the new shows' {what} ({b}) differs from the catalogue's ({a})")
-        if cat.folded and (not new.folded or new.weights_baked != cat.weights_baked):
-            raise ValueError("extend: the new shows' float groups do not match the catalogue's")
         n_old, q = cat.n_shows, new.n_shows
         n = n_old + q
         dev, lib, stream = self.device, self.lib, self._stream()
@@ -844,8 +853,14 @@ class HybridTopKEngine:
         """``tvbf_features`` the incremental append runs on (the folded second operand when the job
         qualifies), or None when the job needs the whole job: signed text, or not eligible for the
         symmetric sweep."""
+        return None if n_old <= 0 else self._incremental_features(cat, weights, k, min_similarity)
+
+    def _incremental_features(self, cat: DeviceCatalogue, weights, k: int, min_similarity: float):
+        """``tvbf_features`` an incremental append or update of ``cat`` runs on (the folded second
+        operand when the job qualifies), or None when it needs the whole job: signed text, or not
+        eligible for the symmetric sweep."""
         gw, tw, mw = (float(w) for w in weights)
-        if n_old <= 0 or cat.c.text_signed:
+        if cat.c.text_signed:
             return None
         p = self._params(cat, weights, k, min_similarity)
         if not self.lib.tvbf_sym_eligible(C.byref(cat.c), C.byref(p)):
@@ -865,6 +880,186 @@ class HybridTopKEngine:
             out = (C.c_int64 * 2)()
             check(self.lib.tvbf_append_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
                                                   int(n_old), out), "tvbf_append_plan_tiles")
+        return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
+
+    # ------------------------------------------------------------------------------------ updates
+    @staticmethod
+    def _update_rows(rows, n: int) -> np.ndarray:
+        """``rows`` as a sorted int64 array; ``ValueError`` unless they are distinct integers in [0, n)."""
+        r = np.asarray(rows)
+        if r.ndim != 1 or (r.size and not np.issubdtype(r.dtype, np.integer)):
+            raise ValueError(f"rows must be a 1-D array of integers, got shape {r.shape} and dtype {r.dtype}")
+        r = np.sort(r.astype(np.int64))
+        if r.size and (r[0] < 0 or r[-1] >= n):
+            raise ValueError(f"rows must lie in [0, {n}), got [{r[0]}, {r[-1]}]")
+        if r.size > 1 and (r[1:] == r[:-1]).any():
+            raise ValueError("rows must be distinct")
+        return r
+
+    def update(self, cat: DeviceCatalogue, rows, new_features: dict) -> DeviceCatalogue:
+        """``cat`` with the shows ``rows`` (distinct, any order) given the features of
+        ``new_features`` (row e of it for the e-th smallest of ``rows``).  Only the Q new rows are
+        prepared; they are written over the old ones in place (operand rows, column-side records,
+        metadata scales, second genre words, dense float groups, the rows of the engine's second
+        operand when this catalogue owns it) and the text CSR is spliced on the device.  The result
+        equals a fresh ``ingest`` of the updated features.  ``cat`` is consumed, as with ``extend``.
+
+        Precondition: the new features are encoded in the catalogue's vocabulary and widths (the
+        already fitted extractor); a different vocabulary size, genre or metadata width, group
+        encoding (binary / float) or metadata mode raises ``ValueError``."""
+        r = self._update_rows(rows, cat.n_shows)
+        q = int(r.size)
+        n_feat = int(np.asarray(new_features["genre_features"]).shape[0])
+        if n_feat != q:
+            raise ValueError(f"update: {q} rows but new features for {n_feat} shows")
+        if q == 0:
+            if cat.operand is None or not cat.parts:
+                raise ValueError("update: the catalogue was recycled or does not come from ingest / prepare")
+            return cat
+        c = cat.c
+        new = self._ingest_like(cat, new_features, "update")
+        nc = new.c
+        n = cat.n_shows
+        dev, lib, stream = self.device, self.lib, self._stream()
+        code, _ = _DTYPES[self.text_dtype]
+        p_old, p_new = cat.parts, new.parts
+        with torch.cuda.device(dev):
+            idx = torch.from_numpy(r).to(dev)
+            operand = cat.operand
+            operand.index_copy_(0, idx, new.operand[:q])
+            col_side, meta_scale, genre_hi = p_old["col_side"], p_old["meta_scale"], p_old["genre_hi"]
+            col_side.index_copy_(0, idx, p_new["col_side"][:q])
+            meta_scale.index_copy_(0, idx, p_new["meta_scale"][:q])
+            if genre_hi is not None:
+                genre_hi.index_copy_(0, idx, p_new["genre_hi"][:q])
+            genre_dense = p_old["genre_dense"]
+            if genre_dense is not None:
+                genre_dense.index_copy_(0, idx, p_new["genre_dense"][:q])
+            meta_dense = p_old["meta_dense"]
+            for a, b in zip(meta_dense, p_new["meta_dense"]):
+                a.index_copy_(0, idx, b[:q])
+            # CSR splice: row lengths -> indptr, then every output entry gathered from [old nnz | new nnz]
+            nnz_old, nnz_new = p_old["nnz"], p_new["nnz"]
+            ip_old = cat.text_indptr[:n + 1].to(torch.int64)
+            ip_new = new.text_indptr[:q + 1].to(torch.int64)
+            lens = ip_old[1:] - ip_old[:-1]
+            lens[idx] = ip_new[1:] - ip_new[:-1]
+            indptr = torch.zeros((n + 1,), dtype=torch.int64, device=dev)
+            indptr[1:] = torch.cumsum(lens, 0)
+            start = ip_old[:-1].clone()
+            start[idx] = ip_new[:-1] + nnz_old
+            nnz = int(indptr[-1].item())
+            if nnz == 0:               # the C ABI wants non-NULL arrays, which are never read
+                indices = torch.zeros((1,), dtype=torch.int32, device=dev)
+                values = torch.zeros((1,), dtype=torch.float64, device=dev)
+            else:
+                row_of = torch.repeat_interleave(torch.arange(n, device=dev), lens, output_size=nnz)
+                pos = torch.arange(nnz, device=dev) - indptr[row_of] + start[row_of]
+                indices = torch.cat([cat.text_indices[:nnz_old], new.text_indices[:nnz_new]])[pos]
+                values = torch.cat([p_old["values"][:nnz_old], p_new["values"][:nnz_new]])[pos]
+            f = Features.from_buffer_copy(c)
+            f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            signed = bool(c.text_signed) or bool(nc.text_signed)
+            f.text_signed = int(signed and nnz > 0 and bool((values < 0).any()))
+            parts = {**p_old, "values": values, "nnz": nnz}
+            buffers = {**cat.buffers, "values": values} if "values" in cat.buffers else dict(cat.buffers)
+            upd = DeviceCatalogue(c=f, n_shows=n, folded=cat.folded, weights_baked=cat.weights_baked,
+                                  keep=[indptr, indices, values, operand, col_side, meta_scale, genre_hi, genre_dense,
+                                        *meta_dense], operand=operand,
+                                  text_indptr=indptr, text_indices=indices, buffers=buffers, parts=parts)
+            fc = cat.fold
+            if fc is not None and self._fold_owner is fc and not f.text_signed:
+                # the second operand (small vocabularies): rebuild the updated rows and write them over
+                ff = Features.from_buffer_copy(fc["c"])
+                k_fold, buf = int(ff.k_pad), fc["operand"]
+                rows_fold = torch.zeros((q, k_fold), dtype=buf.dtype, device=dev)
+                scale = float(2 ** TEXT_SCALE_LOG2)
+                check(lib.tvbf_prep_csr_to_operand(new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
+                                                   p_new["values"].data_ptr(), q, rows_fold.data_ptr(), k_fold, 0,
+                                                   scale, code, stream), "tvbf_prep_csr_to_operand")
+                if fc["weights"] is not None:
+                    gw, tw, mw = fc["weights"]
+                    check(lib.tvbf_prep_fold_bits(p_new["col_side"].data_ptr(),
+                                                  None if p_new["genre_hi"] is None else p_new["genre_hi"].data_ptr(),
+                                                  p_new["meta_scale"].data_ptr(), q, int(c.genre_dim),
+                                                  rows_fold.data_ptr(), k_fold, int(c.vocab),
+                                                  scale * float(np.sqrt(gw / tw)), scale * float(np.sqrt(mw / tw)),
+                                                  code, stream), "tvbf_prep_fold_bits")
+                buf.index_copy_(0, idx, rows_fold)
+                for name in ("text_indptr", "text_indices", "text_values"):
+                    setattr(ff, name, getattr(f, name))
+                upd.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+        cat.operand = None                  # consumed: its buffers now belong to the updated catalogue
+        cat.c.operand = None
+        cat.keep.clear()
+        cat.parts = {}
+        cat.fold = None
+        cat.buffers = {}
+        cat.h2d_set = None
+        return upd
+
+    def top_k_update_device(self, cat: DeviceCatalogue, rows, previous: dict, weights=(0.4, 0.5, 0.1),
+                            k: int = 20, min_similarity: float = 0.1, out: dict | None = None) -> dict:
+        """Table of ``cat`` after the shows ``rows`` got new features (``update``) from
+        ``previous``, the device table (``top_k_device``) of the catalogue before the update for the
+        same weights, ``k`` and ``min_similarity`` (``exclude_self=True``).  Bit-identical to
+        ``top_k_device(cat, ...)`` (indices, counts and the four scores); ``changed_rows`` of the
+        result holds the sorted int32 rows, updated or not, that differ from ``previous`` in any
+        field (every other row is byte-identical to its previous row).
+
+        The incremental path (``tvbf_update_topk``) sweeps only the updated shows' rows against all
+        columns and copies the previous row of every show that names no updated show and received
+        no candidate from one.  Jobs the symmetric sweep does not take (float-valued groups,
+        negative weights, k > 100, ...) and catalogues with signed text run the whole job and
+        compare.  ``incremental`` of the result says which of the two ran."""
+        n, k = cat.n_shows, int(k)
+        r = self._update_rows(rows, n)
+        if previous["indices"].dim() != 2 or tuple(previous["indices"].shape) != (n, k) \
+                or tuple(previous["counts"].shape) != (n,):
+            raise ValueError(f"previous table has shape {tuple(previous['indices'].shape)}, expected ({n}, {k})")
+        if r.size == 0:
+            return {**previous, "changed_rows": torch.zeros((0,), dtype=torch.int32, device=self.device),
+                    "incremental": True}
+        p = self._params(cat, weights, k, min_similarity)
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, k, min_similarity)
+            if feats is None:
+                # whole job on the updated catalogue, changed rows by comparison of all six fields
+                t = self.top_k_device(cat, weights, k, min_similarity, out=out)
+                diff = (t["counts"] != previous["counts"]) | (t["indices"] != previous["indices"]).any(dim=1)
+                for name in ("hybrid", "genre", "text", "metadata"):
+                    diff |= (t[name].view(torch.int64) != previous[name].view(torch.int64)).any(dim=1)
+                t["changed_rows"] = torch.nonzero(diff).flatten().to(torch.int32)
+                t["incremental"] = False
+                return t
+            nbytes = self.lib.tvbf_update_workspace_bytes(C.byref(feats), C.byref(p), int(r.size))
+            if nbytes == 0:
+                check(-1, "tvbf_update_workspace_bytes")
+            ws = self._workspace(nbytes)
+            t = out if out is not None else self._alloc_tables(n, k)
+            rows_d = torch.from_numpy(r.astype(np.int32)).to(self.device)
+            changed = torch.empty((n,), dtype=torch.int32, device=self.device)
+            prev = self._c_tables({**previous, "stats": t["stats"]})
+            check(self.lib.tvbf_update_topk(C.byref(feats), C.byref(p), rows_d.data_ptr(), int(r.size), C.byref(prev),
+                                            C.byref(self._c_tables(t)), changed.data_ptr(), ws.data_ptr(), ws.numel(),
+                                            self._stream()), "tvbf_update_topk")
+            t["changed_rows"] = torch.nonzero(changed).flatten().to(torch.int32)
+            t["incremental"] = True
+        t["row_begin"] = 0
+        return t
+
+    def update_tiles(self, cat: DeviceCatalogue, n_rows: int, weights=(0.4, 0.5, 0.1), k: int = 20,
+                     min_similarity: float = 0.1) -> dict | None:
+        """Tensor-core tiles (256 x 256 x k_pad) the incremental update of ``top_k_update_device``
+        executes on ``cat`` with ``n_rows`` updated shows (host only): its threshold seed pass over
+        the gathered rows and the update sweep.  None when the job runs the whole job instead."""
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, int(k), float(min_similarity))
+            if feats is None or not 1 <= int(n_rows) <= cat.n_shows:
+                return None
+            out = (C.c_int64 * 2)()
+            check(self.lib.tvbf_update_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
+                                                  int(n_rows), out), "tvbf_update_plan_tiles")
         return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
 
     def top_k_sweep_device(self, cat: DeviceCatalogue, weight_list, k: int = 20, min_similarity: float = 0.1,

@@ -199,6 +199,54 @@ class SimilarityComputer:
         top.changed_rows = changed
         return top
 
+    def update_top_k(self, features: dict, previous: TopK, rows, k: int = 20, min_similarity: float = 0.1,
+                     exclude_self: bool = True, metadata_mode: str = "mean3",
+                     normalize_weights: bool = False) -> TopK:
+        """Top-K table after the shows ``rows`` of a catalogue whose table exists got new features.
+
+        ``features`` is the whole catalogue after the update; ``previous`` is the ``compute_top_k``
+        table of the catalogue before it, with the same arguments.  The result equals
+        ``compute_top_k(features, ...)`` bit for bit; its ``changed_rows`` lists the rows (sorted
+        int32, updated or not) that differ from ``previous`` in any field -- every other row is
+        identical to its row in ``previous``, so a caller only has to store the listed rows.  Only
+        the updated shows' rows are scored against the catalogue on the tensor cores.
+
+        Precondition, which the library cannot check: every row not in ``rows`` has the features
+        ``previous`` was computed from, and all rows are encoded in the same vocabulary and widths
+        (the already fitted extractor); a refitted extractor changes every row and needs
+        ``compute_top_k``.  Jobs the incremental path does not take (signed text, float-valued
+        groups, k > 100, ``exclude_self=False``, ...) run the whole job and compare."""
+        weights = self._normalized_weights() if normalize_weights else \
+            (self.genre_weight, self.text_weight, self.metadata_weight)
+        n_all = int(np.asarray(features["genre_features"]).shape[0])
+        if previous.indices.ndim != 2 or previous.indices.shape != (n_all, k) or previous.counts.shape != (n_all,) \
+                or previous.row_begin != 0:
+            raise ValueError(f"previous table has shape {previous.indices.shape}, expected ({n_all}, {k}) from row 0")
+        eng = self.engine
+        r = eng._update_rows(rows, n_all)
+        fields = ("indices", "counts", "hybrid", "genre", "text", "metadata")
+
+        if r.size == 0:
+            return TopK(*(getattr(previous, name) for name in fields), changed_rows=np.zeros(0, dtype=np.int32))
+        if not exclude_self:
+            top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
+            diff = (top.counts != previous.counts) | (top.indices != previous.indices).any(axis=1)
+            for name in ("hybrid", "genre", "text", "metadata"):
+                diff |= (getattr(top, name).view(np.int64) != getattr(previous, name).view(np.int64)).any(axis=1)
+            top.changed_rows = np.nonzero(diff)[0].astype(np.int32)
+            return top
+        # one catalogue encoding for all rows: when the updated rows make a group float-valued (or the
+        # others are), the whole catalogue is ingested that way and the whole job runs
+        cat = eng.ingest(features, metadata_mode, weights)
+        with torch.cuda.device(eng.device):
+            prev = {name: torch.from_numpy(np.ascontiguousarray(getattr(previous, name))).to(eng.device)
+                    for name in fields}
+            t = eng.top_k_update_device(cat, r, prev, weights, k, min_similarity)
+            changed = t["changed_rows"].cpu().numpy()
+        top = eng.to_host(t)
+        top.changed_rows = changed
+        return top
+
     def compute_top_k_sweep(self, features: dict, weight_list, k: int = 20, min_similarity: float = 0.1,
                             exclude_self: bool = True, metadata_mode: str = "mean3",
                             normalize_weights: bool = False, **kw) -> list[TopK]:
