@@ -827,11 +827,10 @@ class HybridTopKEngine:
         with torch.cuda.device(self.device):
             feats = self._append_features(cat, n_old, weights, k, min_similarity)
             if feats is None:
-                # whole job on the grown catalogue, changed rows by comparison
+                # whole job on the grown catalogue, changed rows by comparison (for old rows, a score
+                # changes only with the indices: the score of two old shows is the same)
                 t = self.top_k_device(cat, weights, k, min_similarity, out=out)
-                diff = (t["counts"][:n_old] != previous["counts"]) | \
-                    (t["indices"][:n_old] != previous["indices"]).any(dim=1)
-                t["changed_rows"] = torch.nonzero(diff).flatten().to(torch.int32)
+                t["changed_rows"] = self._changed_rows(t, previous)
                 t["incremental"] = False
                 return t
             nbytes = self.lib.tvbf_append_workspace_bytes(C.byref(feats), C.byref(p), n_old)
@@ -848,6 +847,16 @@ class HybridTopKEngine:
             t["incremental"] = True
         t["row_begin"] = 0
         return t
+
+    @staticmethod
+    def _changed_rows(t: dict, previous: dict) -> torch.Tensor:
+        """Sorted int32 rows of ``previous`` that differ from the same rows of ``t`` in any of the six
+        fields (the scores bit for bit)."""
+        n = previous["counts"].shape[0]
+        diff = (t["counts"][:n] != previous["counts"]) | (t["indices"][:n] != previous["indices"]).any(dim=1)
+        for name in ("hybrid", "genre", "text", "metadata"):
+            diff |= (t[name][:n].view(torch.int64) != previous[name].view(torch.int64)).any(dim=1)
+        return torch.nonzero(diff).flatten().to(torch.int32)
 
     def _append_features(self, cat: DeviceCatalogue, n_old: int, weights, k: int, min_similarity: float):
         """``tvbf_features`` the incremental append runs on (the folded second operand when the job
@@ -1024,12 +1033,9 @@ class HybridTopKEngine:
         with torch.cuda.device(self.device):
             feats = self._incremental_features(cat, weights, k, min_similarity)
             if feats is None:
-                # whole job on the updated catalogue, changed rows by comparison of all six fields
+                # whole job on the updated catalogue, changed rows by comparison
                 t = self.top_k_device(cat, weights, k, min_similarity, out=out)
-                diff = (t["counts"] != previous["counts"]) | (t["indices"] != previous["indices"]).any(dim=1)
-                for name in ("hybrid", "genre", "text", "metadata"):
-                    diff |= (t[name].view(torch.int64) != previous[name].view(torch.int64)).any(dim=1)
-                t["changed_rows"] = torch.nonzero(diff).flatten().to(torch.int32)
+                t["changed_rows"] = self._changed_rows(t, previous)
                 t["incremental"] = False
                 return t
             nbytes = self.lib.tvbf_update_workspace_bytes(C.byref(feats), C.byref(p), int(r.size))

@@ -28,6 +28,16 @@ def _split_rows(features: dict, n: int) -> tuple[dict, dict]:
     return old, new
 
 
+def _changed_rows(top: TopK, previous: TopK) -> np.ndarray:
+    """Sorted int32 rows of ``previous`` that differ from the same rows of ``top`` in any of the six
+    fields (the scores bit for bit)."""
+    n = previous.counts.shape[0]
+    diff = (top.counts[:n] != previous.counts) | (top.indices[:n] != previous.indices).any(axis=1)
+    for name in ("hybrid", "genre", "text", "metadata"):
+        diff |= (getattr(top, name)[:n].view(np.int64) != getattr(previous, name).view(np.int64)).any(axis=1)
+    return np.nonzero(diff)[0].astype(np.int32)
+
+
 # noinspection PyMethodMayBeStatic
 class SimilarityComputer:
     """Compute similarity matrices (and top-K tables) from feature arrays."""
@@ -173,8 +183,7 @@ class SimilarityComputer:
 
         def full() -> TopK:
             top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
-            diff = (top.counts[:n_old] != previous.counts) | (top.indices[:n_old] != previous.indices).any(axis=1)
-            top.changed_rows = np.nonzero(diff)[0].astype(np.int32)
+            top.changed_rows = _changed_rows(top, previous)
             return top
 
         if n_old == n_all:
@@ -230,10 +239,7 @@ class SimilarityComputer:
             return TopK(*(getattr(previous, name) for name in fields), changed_rows=np.zeros(0, dtype=np.int32))
         if not exclude_self:
             top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
-            diff = (top.counts != previous.counts) | (top.indices != previous.indices).any(axis=1)
-            for name in ("hybrid", "genre", "text", "metadata"):
-                diff |= (getattr(top, name).view(np.int64) != getattr(previous, name).view(np.int64)).any(axis=1)
-            top.changed_rows = np.nonzero(diff)[0].astype(np.int32)
+            top.changed_rows = _changed_rows(top, previous)
             return top
         # one catalogue encoding for all rows: when the updated rows make a group float-valued (or the
         # others are), the whole catalogue is ingested that way and the whole job runs
