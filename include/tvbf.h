@@ -309,6 +309,23 @@ int tvbf_update_topk(const tvbf_features* f, const tvbf_params* p, const int32_t
                      const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
                      size_t workspace_bytes, void* stream);
 
+/* ---- remove shows from a catalogue whose table exists (instead of the whole job again).
+ *      f: the catalogue of n_shows shows AFTER the removal (the remaining shows in their old order, the
+ *      same features as before); removed: the n_removed removed rows in the OLD numbering (device array,
+ *      sorted, distinct, in [0, n_shows + n_removed)); prev: the [n_shows + n_removed, k] table of the
+ *      catalogue before the removal from a job with the same p (weights, k, min_similarity,
+ *      exclude_self = 1).  Writes the [n_shows, k] table of the remaining catalogue to `out` (new
+ *      numbering) -- bit-identical to tvbf_hybrid_topk on f (indices, counts and the four scores; stats
+ *      differ) -- and changed[r] = 1 for every new row r whose previous row names a removed show (0
+ *      otherwise: the row is byte-identical to its previous row with the indices renumbered).  Only
+ *      those rows are swept against all columns; every other row is copied without rescoring.  The call
+ *      waits for the stream once, to size the sweep by their number.  Jobs tvbf_sym_eligible rejects,
+ *      and signed text, are rejected (the caller runs the whole job).  `out` must not alias `prev`. */
+size_t tvbf_remove_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_removed);
+int tvbf_remove_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* removed, int32_t n_removed,
+                     const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
+                     size_t workspace_bytes, void* stream);
+
 /* exact fp64 scoring of explicit source rows against all columns + exact top-K
  * (replaces get_recommendations_from_matrix, content_based_service.py:161-236, for any n). */
 size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed);
@@ -400,6 +417,11 @@ int32_t tvbf_debug_append_schedule(int32_t n_old, int32_t n_shows, int32_t sm_co
  * out2 = {tiles of its threshold seed pass over the gathered rows, tiles of the update sweep}
  * (256 x 256 x k_pad each).  Fails like tvbf_update_workspace_bytes for a job the update does not take. */
 int tvbf_update_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2);
+/* host-only: tensor-core tiles tvbf_remove_topk executes for this job (f after the removal) when
+ * n_rows remaining shows named a removed one, out2 = {tiles of its threshold seed pass over their
+ * gathered rows, tiles of the repair sweep} (256 x 256 x k_pad each); the schedule is the update
+ * sweep's for n_rows rows.  Fails like tvbf_remove_workspace_bytes for a job the removal does not take. */
+int tvbf_remove_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2);
 /* host-only: the work items of the update sweep of tvbf_update_topk for q updated shows in a catalogue
  * of n_shows on a device with sm_count SMs; out as tvbf_debug_schedule (super block = block of 256
  * gathered rows).  Returns the number of items.  Used by the CPU tests to prove that every (gathered

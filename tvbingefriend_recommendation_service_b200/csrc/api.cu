@@ -1317,6 +1317,247 @@ int32_t tvbf_debug_update_schedule(int32_t q, int32_t n_shows, int32_t sm_count,
   return tvbf::k1_debug_schedule(kp, out, max_items);
 }
 
+// ---- remove shows from a catalogue whose table exists -------------------------------------------
+// No pair score changes.  A remaining show whose previous row names no removed show keeps that row with
+// its indices renumbered: removing columns cannot bring a new one in.  The other remaining shows (A)
+// are swept against every column as gathered rows (K1 kMode 9: each score goes to the gathered row's
+// own list only), compacted (K4s over |A| lists), rescored (K5 on those lists alone, plain
+// certificate) and repaired (K6).
+namespace {
+
+// map[o] = new row of old row o, or -1 when o is removed (removed: sorted, distinct)
+__global__ void remove_map_kernel(const int* removed, int q, int n_old, int* map) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  if (o >= n_old) return;
+  int lo = 0, hi = q;   // removed rows below o
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (removed[mid] < o) lo = mid + 1;
+    else hi = mid;
+  }
+  map[o] = lo < q && removed[lo] == o ? -1 : o - lo;
+}
+
+// Remaining old row o becomes new row r = map[o].  in_a[r] = 1 when its previous row names a removed
+// show (row r is in A, K5 and K6 write it); otherwise the previous row is copied with its indices
+// renumbered, the -1 padding and the scores as they are.
+__global__ void remove_rows_kernel(tvbf_topk_out prev, tvbf_topk_out out, const int* map, int n_old, int k,
+                                   int* in_a) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  if (o >= n_old) return;
+  const int r = map[o];
+  if (r < 0) return;
+  const int n = prev.counts[o];
+  const size_t src = static_cast<size_t>(o) * k, dst = static_cast<size_t>(r) * k;
+  bool named = false;
+  for (int e = 0; e < n && !named; ++e) named = map[prev.indices[src + e]] < 0;
+  in_a[r] = named;
+  if (named) return;
+  for (int e = 0; e < k; ++e) {
+    const int j = prev.indices[src + e];
+    out.indices[dst + e] = e < n ? map[j] : j;
+    out.hybrid[dst + e] = prev.hybrid[src + e];
+    out.genre[dst + e] = prev.genre[src + e];
+    out.text[dst + e] = prev.text[src + e];
+    out.metadata[dst + e] = prev.metadata[src + e];
+  }
+  out.counts[r] = n;
+}
+
+// rows[0 .. *n_rows) = the rows r with in_a[r] = 1, ascending (one block: a chunk per thread, then a
+// scan of the chunk counts)
+constexpr int kCompactThreads = 1024;
+__global__ void __launch_bounds__(kCompactThreads) remove_compact_kernel(const int* in_a, int n, int* rows,
+                                                                          int* n_rows) {
+  __shared__ int sums[kCompactThreads];
+  const int t = threadIdx.x;
+  const int chunk = (n + kCompactThreads - 1) / kCompactThreads;
+  const int b = min(n, t * chunk), e = min(n, b + chunk);
+  int c = 0;
+  for (int r = b; r < e; ++r) c += in_a[r] != 0;
+  sums[t] = c;
+  __syncthreads();
+  for (int off = 1; off < kCompactThreads; off <<= 1) {   // inclusive scan
+    const int v = t >= off ? sums[t - off] : 0;
+    __syncthreads();
+    sums[t] += v;
+    __syncthreads();
+  }
+  int pos = sums[t] - c;
+  for (int r = b; r < e; ++r)
+    if (in_a[r] != 0) rows[pos++] = r;
+  if (t == kCompactThreads - 1) *n_rows = sums[t];
+}
+
+struct RemovePlan {
+  Plan pl;             // a whole-catalogue symmetric job over the remaining shows
+  tvbf::K1Params geo;  // tile schedule of the repair sweep (the update geometry over |A| gathered rows)
+  int grid, q_pad;
+  size_t off_map, off_in_a, off_rows, off_count, off_gather, off_gtheta, total;
+};
+
+// n_a: rows of A (the geometry of the sweep; 0 sizes the workspace only, which holds |A| up to every
+// remaining show)
+int make_remove_plan(const tvbf_features* f, const tvbf_params* p, int n_removed, int n_a, RemovePlan* rp,
+                     tvbf_params* q) {
+  TVBF_REQUIRE(n_removed >= 1 && n_removed <= INT32_MAX - f->n_shows, "remove: %d removed shows", n_removed);
+  TVBF_REQUIRE(n_a >= 0 && n_a <= f->n_shows, "remove: %d repaired rows outside [0, n_shows %d]", n_a, f->n_shows);
+  TVBF_REQUIRE(!f->text_signed, "remove: signed text needs the whole job");
+  *q = *p;
+  q->row_begin = 0;
+  q->row_end = f->n_shows;
+  q->tuning = (q->tuning & ~(0x3 << 20)) | (2 << 20);   // symmetric job (or fail if ineligible)
+  q->tuning = (q->tuning & ~0xF) | 2;                   // CTA pairs
+  int rc = validate_params(f, q);
+  if (rc != TVBF_OK) return rc;
+  rc = make_plan(f, q, &rp->pl);
+  if (rc != TVBF_OK) return rc;
+  int sms = 0;
+  rc = sm_count_cached(&sms);
+  if (rc != TVBF_OK) return rc;
+  memset(&rp->geo, 0, sizeof(rp->geo));
+  rp->grid = 0;
+  rp->q_pad = 0;
+  if (n_a > 0) {
+    tvbf::k1_update_geometry(n_a, f->n_shows, sms / 2, &rp->geo);
+    const int items = (rp->geo.rb_count + rp->geo.rb_per_group - 1) / rp->geo.rb_per_group * rp->geo.rb_per_group *
+                      rp->geo.splits;
+    rp->grid = 2 * (items < sms / 2 ? items : sms / 2);
+    rp->q_pad = rp->geo.rb_count * 256;
+  }
+  const size_t rows = static_cast<size_t>(f->n_shows);
+  size_t off = rp->pl.total;
+  rp->off_map = off;    off = align_up(off + (rows + n_removed) * 4, 256);
+  rp->off_in_a = off;   off = align_up(off + rows * 4, 256);
+  rp->off_rows = off;   off = align_up(off + rows * 4, 256);
+  rp->off_count = off;  off = align_up(off + 4, 256);
+  rp->off_gather = off; off = align_up(off + static_cast<size_t>(f->n_pad) * f->k_pad * 2, 256);
+  rp->off_gtheta = off; off = align_up(off + static_cast<size_t>(f->n_pad) * 4, 256);
+  rp->total = off;
+  return TVBF_OK;
+}
+
+// the candidate-kernel parameters of the repair sweep: a whole-catalogue symmetric job on the update
+// geometry, one list per gathered row (the plan's lists and candidate table, indexed by gathered row)
+int fill_remove_params(const tvbf_features* f, const tvbf_params* q, const RemovePlan& rp, uint8_t* ws,
+                       const int* rows, int n_a, tvbf::K1Params* kp) {
+  int rc = fill_k1_params(f, q, rp.pl, ws, kp);
+  if (rc != TVBF_OK) return rc;
+  kp->sync_kb = 0;
+  kp->sym = 0;   // the one-sided schedule: a rectangle
+  kp->wide_epilogue = 0;   // 8 epilogue warps, as the update sweep
+  kp->col_tiles = rp.geo.col_tiles;
+  kp->rb_count = rp.geo.rb_count;
+  kp->splits = rp.geo.splits;
+  kp->rb_per_group = rp.geo.rb_per_group;
+  kp->tiles_per_split = rp.geo.tiles_per_split;
+  kp->upd_rows = rows;
+  kp->upd_q = n_a;
+  kp->upd_bits = nullptr;
+  return TVBF_OK;
+}
+
+}  // namespace
+
+size_t tvbf_remove_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_removed) {
+  if (validate_features(f) != TVBF_OK || p == nullptr) return 0;
+  RemovePlan rp;
+  tvbf_params q;
+  if (make_remove_plan(f, p, n_removed, 0, &rp, &q) != TVBF_OK) return 0;
+  return rp.total;
+}
+
+int tvbf_remove_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* removed, int32_t n_removed,
+                     const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p != nullptr, "params is NULL");
+  TVBF_REQUIRE(prev && prev->indices && prev->counts && prev->hybrid && prev->genre && prev->text && prev->metadata,
+               "previous table has NULL members");
+  TVBF_REQUIRE(out && out->indices && out->counts && out->hybrid && out->genre && out->text && out->metadata &&
+                   out->stats,
+               "output table has NULL members");
+  TVBF_REQUIRE(removed != nullptr && changed != nullptr && workspace != nullptr, "tvbf_remove_topk: NULL argument");
+  RemovePlan rp;
+  tvbf_params q;
+  rc = make_remove_plan(f, p, n_removed, 0, &rp, &q);
+  if (rc != TVBF_OK) return rc;
+  if (workspace_bytes < rp.total) {
+    tvbf_set_error("workspace too small: %zu < %zu", workspace_bytes, rp.total);
+    return TVBF_ERR_WORKSPACE;
+  }
+  auto st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const int n = f->n_shows, n_old = n + n_removed;
+  int* map = reinterpret_cast<int*>(ws + rp.off_map);
+  int* in_a = reinterpret_cast<int*>(ws + rp.off_in_a);
+  int* a_rows = reinterpret_cast<int*>(ws + rp.off_rows);
+  int* a_count = reinterpret_cast<int*>(ws + rp.off_count);
+  TVBF_CUDA_OK(cudaMemsetAsync(out->stats, 0, 8 * sizeof(int32_t), st));
+  remove_map_kernel<<<(n_old + 255) / 256, 256, 0, st>>>(removed, n_removed, n_old, map);
+  TVBF_LAUNCH_OK("remove_map_kernel");
+  remove_rows_kernel<<<(n_old + 255) / 256, 256, 0, st>>>(*prev, *out, map, n_old, p->k, in_a);
+  TVBF_LAUNCH_OK("remove_rows_kernel");
+  remove_compact_kernel<<<1, kCompactThreads, 0, st>>>(in_a, n, a_rows, a_count);
+  TVBF_LAUNCH_OK("remove_compact_kernel");
+  TVBF_CUDA_OK(cudaMemcpyAsync(changed, in_a, static_cast<size_t>(n) * 4, cudaMemcpyDeviceToDevice, st));
+  // the sweep's geometry depends on |A|
+  int n_a = 0;
+  TVBF_CUDA_OK(cudaMemcpyAsync(&n_a, a_count, 4, cudaMemcpyDeviceToHost, st));
+  TVBF_CUDA_OK(cudaStreamSynchronize(st));
+  if (n_a == 0) return TVBF_OK;
+  rc = make_remove_plan(f, p, n_removed, n_a, &rp, &q);
+  if (rc != TVBF_OK) return rc;
+  const Plan& pl = rp.pl;
+  tvbf::K1Params kp;
+  rc = fill_remove_params(f, &q, rp, ws, a_rows, n_a, &kp);
+  if (rc != TVBF_OK) return rc;
+  const int row_vec = f->k_pad / 8;   // 16-byte vectors per operand row
+  update_gather_kernel<<<1024, 256, 0, st>>>(static_cast<const uint4*>(f->operand), a_rows, n_a, rp.q_pad, row_vec,
+                                             reinterpret_cast<uint4*>(ws + rp.off_gather));
+  TVBF_LAUNCH_OK("update_gather_kernel");
+  tvbf_features g = *f;   // the gathered rows as the A operand
+  g.operand = ws + rp.off_gather;
+  g.n_pad = rp.q_pad;
+  unsigned int* gtheta = reinterpret_cast<unsigned int*>(ws + rp.off_gtheta);
+  rc = tvbf::k1_launch_remove(f, &g, kp, rp.grid, gtheta, st);
+  if (rc != TVBF_OK) return rc;
+  kp.g_theta = gtheta;   // K4s: the gathered rows' lists under their thresholds
+  rc = tvbf::k4s_launch(kp, n_a, st);
+  if (rc != TVBF_OK) return rc;
+  const tvbf::ScoreParams sp = score_params(f, &q);
+  const tvbf::CandLayout lay{0, 1, 0, 0, 1};   // the list of rows[e] is slot e
+  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
+  double* floors = reinterpret_cast<double*>(ws + pl.off_floor);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+  rc = tvbf::k5_launch_listed(sp, kp.cand, kp.cand_cnt, kp.cand_theta, 1, lay, pl.kp, 0, n, a_rows, a_count, *out,
+                              flagged, floors, st);
+  if (rc != TVBF_OK) return rc;
+  return tvbf::k6_launch_flagged(sp, flagged, floors, n, 0, keys, pl.k6_grid, *out, st);
+}
+
+int tvbf_remove_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2) {
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p && out2, "tvbf_remove_plan_tiles: NULL argument");
+  TVBF_REQUIRE(n_rows >= 1, "tvbf_remove_plan_tiles: %d repaired rows", n_rows);
+  RemovePlan rp;
+  tvbf_params q;
+  rc = make_remove_plan(f, p, 1, n_rows, &rp, &q);
+  if (rc != TVBF_OK) return rc;
+  uint8_t* fake_ws = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(4096));   // offsets only, never dereferenced
+  tvbf::K1Params kp;
+  rc = fill_remove_params(f, &q, rp, fake_ws, nullptr, n_rows, &kp);
+  if (rc != TVBF_OK) return rc;
+  long long t[2];
+  tvbf::k1_update_executed_tiles(kp, rp.grid, t);
+  out2[0] = t[0];
+  out2[1] = t[1];
+  return TVBF_OK;
+}
+
 // ---- streaming statistics of the four similarity matrices (no N x N) --------------------------
 size_t tvbf_stats_accum_bytes(void) { return sizeof(tvbf::StatsAccum); }
 

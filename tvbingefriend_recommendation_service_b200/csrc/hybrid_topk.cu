@@ -406,7 +406,9 @@ struct Pacer {
 // >= p.append_b0), offering no pair of two old shows (p.append_n_old),
 // 7 update sweep: the gathered rows of the updated shows (p.upd_rows) against every column tile, a
 // rectangle without a diagonal; offered to the row's show and to every column show not updated itself,
-// 8 the threshold seed pass (as 3) over the gathered rows of an update
+// 8 the threshold seed pass (as 3) over the gathered rows of an update,
+// 9 repair sweep of a removal: the update sweep without the column side -- every score goes to the
+// gathered row's list only, and that list, its count and its threshold are indexed by the gathered row
 // kG2: multi-hot genres with 64 < G <= 128 -- the second word of every column's mask is staged beside
 // the column-side records (in the threshold slices a single-triple sweep leaves unused) and the
 // popcount runs over both words.
@@ -427,7 +429,8 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
   constexpr bool kMulti = kMode == 5;    // weight sweep
   constexpr bool kAppend = kMode == 6;   // append sweep
   constexpr bool kUpdate = kMode == 7;   // update sweep
-  constexpr bool kGather = kMode == 7 || kMode == 8;   // rows are the gathered rows of an update
+  constexpr bool kRepair = kMode == 9;   // repair sweep of a removal
+  constexpr bool kGather = kMode == 7 || kMode == 8 || kRepair;   // rows are gathered rows
   static_assert(!(kG2 && (kMulti || kStats)), "two-word genre masks: single-triple top-k sweeps only");
   static_assert(!(kFold && (kMulti || kStats || kDump || kG2)), "folded groups: single-triple top-k sweeps only");
   // Seed pass: hist[bin][row of the CTA] (32-bit counters; bank = row % 32, so the 32 lanes of a warp
@@ -521,13 +524,14 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
             if (elect_one()) {
               const uint32_t n_th = kMulti ? static_cast<uint32_t>(p.n_weights) : 1u;
               mbar_arrive_expect_tx(&col_full[b], (kFold ? 0u : COL_BYTES + MS_BYTES) +
-                                                      ((kSym && !kStats) ? n_th * MS_BYTES : 0u) + (kG2 ? GH_BYTES : 0u));
+                                                      ((kSym && !kStats && !kRepair) ? n_th * MS_BYTES : 0u) +
+                                                      (kG2 ? GH_BYTES : 0u));
               if (!kFold) bulk_load_1d(smem + L::OFF_COL + b * COL_BYTES, p.col_side + col0, COL_BYTES, &col_full[b]);
               if (kG2)   // threshold slices 1-2 of this buffer (slice 0 holds the thresholds)
                 bulk_load_1d(smem + L::OFF_TH + (b * kMaxSweep + 1) * MS_BYTES, p.genre_hi + col0, GH_BYTES,
                              &col_full[b]);
               if (!kFold) bulk_load_1d(smem + L::OFF_MS + b * MS_BYTES, p.meta_scale + col0, MS_BYTES, &col_full[b]);
-              if (kSym && !kStats)  // snapshot of the column shows' thresholds (stale = lower = conservative)
+              if (kSym && !kStats && !kRepair)  // snapshot of the column shows' thresholds (stale = lower = conservative)
                 for (uint32_t w = 0; w < n_th; ++w)
                   bulk_load_1d(smem + L::OFF_TH + (b * kMaxSweep + w) * MS_BYTES,
                                p.g_theta + static_cast<size_t>(w) * (kMulti ? p.n_pad : 0) + col0, MS_BYTES,
@@ -645,6 +649,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const int grow = p.row_begin + row_local0 + row_in_tile;
       const bool row_valid = kGather ? grow < p.upd_q : grow < p.row_end;
       const int row = kGather ? (row_valid ? p.upd_rows[grow] : -1) : grow;   // the show of this row
+      const int lrow = kRepair ? grow : row;   // the list (and threshold) of this row
       // row-side operands of the fused scores
       unsigned long long g_bits = 0ull, g_hi = 0ull;
       uint32_t m_bits = 0u;
@@ -718,7 +723,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
           const unsigned m = __ballot_sync(kFullMask, act);
           const int slot = ring_n + __popc(m & ((1u << lane) - 1u));
           if (act) {
-            ring[slot] = static_cast<uint32_t>(voff + (to_row ? row : col));
+            ring[slot] = static_cast<uint32_t>(voff + (to_row ? lrow : col));
             ring[RING + slot] = __float_as_uint(ue);
             ring[2 * RING + slot] = static_cast<uint32_t>(to_row ? col : row);
           }
@@ -737,7 +742,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
           // current shared threshold of this thread's show (raised by any CTA working on it)
           unsigned int tb = 0x7f800000u;
           if (row_valid)
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(tb) : "l"(p.g_theta + row) : "memory");
+            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(tb) : "l"(p.g_theta + lrow) : "memory");
           theta = __uint_as_float(tb);
         }
         if (!kDump) mbar_wait_backoff(&col_full[b], ph, 32, 32);
@@ -750,8 +755,8 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
             reinterpret_cast<const unsigned long long*>(smem + L::OFF_TH + (b * kMaxSweep + 1) * MS_BYTES);
         const uint32_t taddr = tmem_base + tmem_lane + b * BN;
         // off-diagonal tiles also feed the column shows (their mirror tile is never computed); the
-        // update sweep's rectangle has no mirror tiles
-        const bool do_col = kSym && row_valid && (kUpdate || jt != c.sb);
+        // update sweep's rectangle has no mirror tiles; the repair sweep feeds its rows only
+        const bool do_col = kSym && !kRepair && row_valid && (kUpdate || jt != c.sb);
 
         float tile_sum[4] = {0.f, 0.f, 0.f, 0.f}, tile_sq[4] = {0.f, 0.f, 0.f, 0.f}, tile_gm = 0.f;
         float stat_scale[4];
@@ -978,7 +983,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
                 load_thw();
               } else if (row_valid) {
                 unsigned int tb;
-                asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(tb) : "l"(p.g_theta + row) : "memory");
+                asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(tb) : "l"(p.g_theta + lrow) : "memory");
                 theta = __uint_as_float(tb);
               }
             }
@@ -1973,6 +1978,60 @@ int k1_launch_update(const tvbf_features* f, const tvbf_features* g, const K1Par
   if (kp.fold) return launch_k1<4, false, 2, 7, false, false, true>(f, sweep, grid, st, g);
   return kp.genre_hi ? launch_k1<4, false, 2, 7, false, true>(f, sweep, grid, st, g)
                      : launch_k1<4, false, 2, 7>(f, sweep, grid, st, g);
+}
+
+// Removal: the gathered rows' thresholds move from their shows' slots (where the seed pass over the
+// gathered rows wrote them) to the gathered-row slots the repair sweep and K4s index; +inf for the
+// padding rows
+__global__ void remove_theta_kernel(const unsigned int* theta, const int* rows, int q, int q_pad,
+                                    unsigned int* gtheta) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < q_pad) gtheta[e] = e < q ? theta[rows[e]] : 0x7f800000u;
+}
+
+int k1_launch_remove(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                     unsigned int* gtheta, cudaStream_t st) {
+  if (kp.sym || kp.n_weights > 1 || kp.sync_kb != 0 || kp.wide_epilogue || kp.upd_q < 1 || kp.upd_rows == nullptr ||
+      gtheta == nullptr) {
+    tvbf_set_error("repair sweep: bad parameters");
+    return TVBF_ERR_INVALID;
+  }
+  const int q_pad = kp.rb_count * 256;   // gathered rows, each with a list of its own
+  const size_t list_bytes = static_cast<size_t>(q_pad) * kp.sym_cap * 8;
+  std::lock_guard<std::mutex> lock(g_side_mutex);
+  SideStream* side = nullptr;
+  int rc = side_stream(&side);
+  if (rc != TVBF_OK) return rc;
+  // only the gathered rows' lists are cleared, on the side stream beside the seed pass
+  rc = absorb_pending(side, st, true);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaEventRecord(side->fork, st));
+  TVBF_CUDA_OK(cudaStreamWaitEvent(side->stream, side->fork, 0));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, static_cast<size_t>(q_pad) * 4, side->stream));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, side->stream));
+  TVBF_CUDA_OK(cudaEventRecord(side->join, side->stream));
+  const int n_pad = f->n_pad;
+  sym_init_kernel<<<static_cast<unsigned>((n_pad + 255) / 256), 256, 0, st>>>(kp.g_theta, f->n_shows, n_pad, n_pad,
+                                                                               kp.theta_init);
+  TVBF_LAUNCH_OK("sym_init_kernel");
+  {
+    const K1Params seed = update_seed_params(kp, grid);
+    const int sg = seed.rb_per_group * 2;
+    if (kp.fold) rc = launch_k1<4, false, 2, 8, false, false, true>(f, seed, sg, st, g);
+    else if (kp.genre_hi != nullptr) rc = launch_k1<4, false, 2, 8, false, true>(f, seed, sg, st, g);
+    else rc = launch_k1<4, false, 2, 8>(f, seed, sg, st, g);
+    if (rc != TVBF_OK) return rc;
+  }
+  remove_theta_kernel<<<static_cast<unsigned>((q_pad + 255) / 256), 256, 0, st>>>(kp.g_theta, kp.upd_rows, kp.upd_q,
+                                                                                   q_pad, gtheta);
+  TVBF_LAUNCH_OK("remove_theta_kernel");
+  TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  sweep.g_theta = gtheta;
+  if (kp.fold) return launch_k1<4, false, 2, 9, false, false, true>(f, sweep, grid, st, g);
+  return kp.genre_hi ? launch_k1<4, false, 2, 9, false, true>(f, sweep, grid, st, g)
+                     : launch_k1<4, false, 2, 9>(f, sweep, grid, st, g);
 }
 
 int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cudaStream_t st) {

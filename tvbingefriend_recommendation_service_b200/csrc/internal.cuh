@@ -120,7 +120,8 @@ struct K1Params {
   // offered to neither list
   int append_n_old;
   int append_b0;
-  // update sweep (kMode 7) and its threshold seed pass (kMode 8), tvbf_update_topk: the A operand is
+  // update sweep (kMode 7), its threshold seed pass (kMode 8) and the repair sweep of a removal
+  // (kMode 9, tvbf_remove_topk, which indexes the lists by gathered row), tvbf_update_topk: the A operand is
   // the gather of the updated shows' operand rows, and gathered row r < upd_q is show upd_rows[r],
   // whose records, slack terms, threshold and list are read through that map.  A column whose bit is
   // set in upd_bits (bit j % 32 of word j / 32) was updated itself: it is offered nothing from the
@@ -179,6 +180,7 @@ int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cu
 struct CandLayout {
   long long slot_base, row_stride, list_stride;
   int packed;
+  int gathered;   // k5_launch_listed only: the lists of rows[e] are at row position e instead of rows[e]
 };
 int k5_launch(const ScoreParams& sp, const uint2* cand, const int* cand_cnt,
               const float* cand_theta, int splits, CandLayout lay, int kp, int row_begin, int n_rows,
@@ -215,6 +217,11 @@ int k1_launch_update(const tvbf_features* f, const tvbf_features* g, const K1Par
                      const UpdatePrev& prev, cudaStream_t st);
 // tiles of the update: out[0] its seed pass over the gathered rows, out[1] the update sweep
 void k1_update_executed_tiles(const K1Params& kp, int grid, long long* out);
+// seed pass over the gathered rows of a removal (kp.upd_rows, thresholds in kp.g_theta by show), then
+// the repair sweep (kMode 9) on the update geometry: the lists kp.g_cnt / kp.g_list and the thresholds
+// gtheta ([rb_count * 256]) are indexed by the gathered row; only those lists are cleared
+int k1_launch_remove(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                     unsigned int* gtheta, cudaStream_t st);
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);

@@ -302,6 +302,23 @@ rescore_listed_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
               max_cand, keep, warp, lane, rows[e]);
 }
 
+// ... where the lists of rows[e] are at row position e (the gathered rows of a removal)
+__global__ void __launch_bounds__(K5_WARPS * 32)
+rescore_gathered_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
+                        const int* __restrict__ cand_cnt, const float* __restrict__ cand_theta, int splits,
+                        const CandLayout lay, int kp, int row_begin, int n_rows, const int* __restrict__ rows,
+                        const int* __restrict__ n_listed, tvbf_topk_out out, int* flagged_rows, double* flagged_floor,
+                        int max_cand, int keep) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (e >= *n_listed) return;
+  const int r = rows[e];
+  CandLayout at = lay;
+  at.slot_base += static_cast<long long>(e) - static_cast<long long>(r) * lay.row_stride;   // slot of row r: e
+  rescore_row(sp, cand, cand_cnt, cand_theta, splits, at, kp, row_begin, n_rows, out, flagged_rows, flagged_floor,
+              max_cand, keep, warp, lane, r);
+}
+
 // ... with the rank cut of an update (rescore_row<true>)
 __global__ void __launch_bounds__(K5_WARPS * 32)
 rescore_cut_kernel(const ScoreParams sp, const uint2* __restrict__ cand,
@@ -1080,6 +1097,19 @@ int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_c
     return TVBF_ERR_INVALID;
   }
   const int grid = (n_rows + warps - 1) / warps;   // at most n_rows listed; the count is on the device
+  if (lay.gathered) {
+    if (cut_index != nullptr) {
+      tvbf_set_error("rescore: gathered lists take no rank cut");
+      return TVBF_ERR_INVALID;
+    }
+    TVBF_CUDA_OK(cudaFuncSetAttribute(rescore_gathered_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      static_cast<int>(smem)));
+    rescore_gathered_kernel<<<grid, warps * 32, smem, st>>>(sp, cand, cand_cnt, cand_theta, splits, lay, kp,
+                                                            row_begin, n_rows, rows, n_listed, out, flagged_rows,
+                                                            flagged_floor, max_cand, 2 * kp);
+    TVBF_LAUNCH_OK("rescore_gathered_kernel");
+    return TVBF_OK;
+  }
   if (cut_index != nullptr) {
     TVBF_CUDA_OK(cudaFuncSetAttribute(rescore_cut_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       static_cast<int>(smem)));

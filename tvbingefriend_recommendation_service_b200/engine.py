@@ -849,9 +849,17 @@ class HybridTopKEngine:
         return t
 
     @staticmethod
-    def _changed_rows(t: dict, previous: dict) -> torch.Tensor:
+    def _changed_rows(t: dict, previous: dict, row_map: torch.Tensor | None = None) -> torch.Tensor:
         """Sorted int32 rows of ``previous`` that differ from the same rows of ``t`` in any of the six
-        fields (the scores bit for bit)."""
+        fields (the scores bit for bit).  With ``row_map`` (a removal: previous row o is row
+        ``row_map[o]`` of ``t``, -1 when it was removed) the rows of ``t`` are compared with their
+        previous rows, whose indices are renumbered by ``row_map`` (a removed show becomes -1)."""
+        if row_map is not None:
+            keep = torch.nonzero(row_map >= 0).flatten()
+            previous = {name: previous[name].index_select(0, keep)
+                        for name in ("indices", "counts", "hybrid", "genre", "text", "metadata")}
+            idx = previous["indices"]
+            previous["indices"] = torch.where(idx >= 0, row_map[idx.clamp(min=0).long()].to(idx.dtype), idx)
         n = previous["counts"].shape[0]
         diff = (t["counts"][:n] != previous["counts"]) | (t["indices"][:n] != previous["indices"]).any(dim=1)
         for name in ("hybrid", "genre", "text", "metadata"):
@@ -1066,6 +1074,168 @@ class HybridTopKEngine:
             out = (C.c_int64 * 2)()
             check(self.lib.tvbf_update_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
                                                   int(n_rows), out), "tvbf_update_plan_tiles")
+        return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
+
+    # ------------------------------------------------------------------------------------ removals
+    def remove(self, cat: DeviceCatalogue, rows) -> DeviceCatalogue:
+        """``cat`` without the shows ``rows`` (distinct, any order): the remaining shows keep their
+        order and become rows 0 .. N - Q - 1.  Compacted on the device (operand rows, column-side
+        records, metadata scales, second genre words, dense float groups, the text CSR and the rows of
+        the engine's second operand when this catalogue owns it); the freed rows are zeroed and
+        ``n_pad`` shrinks to that of N - Q shows.  The result equals a fresh ``ingest`` of the
+        remaining features.  ``cat`` is consumed, as with ``extend``.  Removing every show raises
+        ``ValueError``."""
+        n = cat.n_shows
+        r = self._update_rows(rows, n)
+        if cat.operand is None or not cat.parts:
+            raise ValueError("remove: the catalogue was recycled or does not come from ingest / prepare")
+        q = int(r.size)
+        if q == 0:
+            return cat
+        if q == n:
+            raise ValueError("remove: removing every show leaves no catalogue")
+        m = n - q
+        c = cat.c
+        dev = self.device
+        p_old = cat.parts
+        keep_np = np.delete(np.arange(n, dtype=np.int64), r)
+        with torch.cuda.device(dev):
+            keep = torch.from_numpy(keep_np).to(dev)
+            n_pad = (m + 255) // 256 * 256
+
+            def compact(t: torch.Tensor | None) -> torch.Tensor | None:
+                """rows ``keep`` of a padded buffer moved to the front, the freed rows zeroed; the first
+                ``n_pad`` rows (a view)"""
+                if t is None:
+                    return None
+                t[:m].copy_(t.index_select(0, keep))
+                t[m:n].zero_()
+                return t[:n_pad]
+
+            operand = compact(cat.operand)
+            col_side = compact(p_old["col_side"])
+            meta_scale = compact(p_old["meta_scale"])
+            genre_hi = compact(p_old["genre_hi"])
+            genre_dense = None if p_old["genre_dense"] is None else p_old["genre_dense"].index_select(0, keep)
+            meta_dense = [a.index_select(0, keep) for a in p_old["meta_dense"]]
+            # CSR: the kept rows' lengths -> indptr, every output entry gathered from its old position
+            ip_old = cat.text_indptr[:n + 1].to(torch.int64)
+            lens = (ip_old[1:] - ip_old[:-1]).index_select(0, keep)
+            indptr = torch.zeros((m + 1,), dtype=torch.int64, device=dev)
+            indptr[1:] = torch.cumsum(lens, 0)
+            nnz = int(indptr[-1].item())
+            if nnz == 0:               # the C ABI wants non-NULL arrays, which are never read
+                indices = torch.zeros((1,), dtype=torch.int32, device=dev)
+                values = torch.zeros((1,), dtype=torch.float64, device=dev)
+            else:
+                row_of = torch.repeat_interleave(torch.arange(m, device=dev), lens, output_size=nnz)
+                pos = torch.arange(nnz, device=dev) - indptr[row_of] + ip_old[:-1].index_select(0, keep)[row_of]
+                indices = cat.text_indices[pos]
+                values = p_old["values"][pos]
+            f = Features.from_buffer_copy(c)
+            f.n_shows, f.n_pad = m, n_pad
+            f.operand = operand.data_ptr()
+            f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_signed = int(bool(c.text_signed) and nnz > 0 and bool((values < 0).any()))
+            if genre_dense is not None:
+                f.genre_dense = genre_dense.data_ptr()
+            for gi, a in enumerate(meta_dense):
+                f.meta_dense[gi] = a.data_ptr()
+            parts = {**p_old, "values": values, "nnz": nnz, "col_side": col_side, "meta_scale": meta_scale,
+                     "genre_hi": genre_hi, "genre_dense": genre_dense, "meta_dense": meta_dense}
+            buffers = {"values": values, "col_side": col_side, "meta_scale": meta_scale}
+            if genre_hi is not None:
+                buffers["genre_hi"] = genre_hi
+            rem = DeviceCatalogue(c=f, n_shows=m, folded=cat.folded, weights_baked=cat.weights_baked,
+                                  keep=[indptr, indices, values, operand, col_side, meta_scale, genre_hi, genre_dense,
+                                        *meta_dense], operand=operand,
+                                  text_indptr=indptr, text_indices=indices,
+                                  buffers=buffers if cat.buffers else {}, parts=parts)
+            fc = cat.fold
+            if fc is not None and self._fold_owner is fc and not f.text_signed:
+                # the second operand (small vocabularies): its rows move with the shows
+                buf = compact(fc["operand"])
+                ff = Features.from_buffer_copy(fc["c"])
+                ff.n_shows, ff.n_pad, ff.operand = m, n_pad, buf.data_ptr()
+                for name in ("text_indptr", "text_indices", "text_values", "col_side", "meta_scale", "genre_hi"):
+                    setattr(ff, name, getattr(f, name))
+                rem.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+        cat.operand = None                  # consumed: its buffers now belong to the compacted catalogue
+        cat.c.operand = None
+        cat.keep.clear()
+        cat.parts = {}
+        cat.fold = None
+        cat.buffers = {}
+        cat.h2d_set = None
+        return rem
+
+    def top_k_remove_device(self, cat: DeviceCatalogue, rows, previous: dict, weights=(0.4, 0.5, 0.1),
+                            k: int = 20, min_similarity: float = 0.1, out: dict | None = None) -> dict:
+        """Table of ``cat`` after the shows ``rows`` (old numbering) were removed (``remove``) from
+        ``previous``, the device table (``top_k_device``) of the catalogue before the removal for the
+        same weights, ``k`` and ``min_similarity`` (``exclude_self=True``).  Row r of the result is
+        the r-th remaining show, with indices in the new numbering.  Bit-identical to
+        ``top_k_device(cat, ...)`` (indices, counts and the four scores); ``changed_rows`` of the
+        result holds the sorted int32 new rows that differ in any field from their previous row with
+        its indices renumbered (every other row is byte-identical to it).  These are exactly the rows
+        whose previous row names a removed show.
+
+        The incremental path (``tvbf_remove_topk``) copies every other row and sweeps only those rows
+        against all columns.  Jobs the symmetric sweep does not take (float-valued groups, negative
+        weights, k > 100, ...) and catalogues with signed text run the whole job and compare.
+        ``incremental`` of the result says which of the two ran."""
+        m, k = cat.n_shows, int(k)
+        n = int(previous["counts"].shape[0])
+        r = self._update_rows(rows, n)
+        q = int(r.size)
+        if previous["indices"].dim() != 2 or tuple(previous["indices"].shape) != (m + q, k) \
+                or tuple(previous["counts"].shape) != (m + q,):
+            raise ValueError(f"previous table has shape {tuple(previous['indices'].shape)}, expected ({m + q}, {k})")
+        if q == 0:
+            return {**previous, "changed_rows": torch.zeros((0,), dtype=torch.int32, device=self.device),
+                    "incremental": True}
+        p = self._params(cat, weights, k, min_similarity)
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, k, min_similarity)
+            if feats is None:
+                # whole job on the remaining catalogue, changed rows by comparison with the renumbered rows
+                t = self.top_k_device(cat, weights, k, min_similarity, out=out)
+                row_map = torch.full((n,), -1, dtype=torch.int64)
+                row_map[np.delete(np.arange(n), r)] = torch.arange(m)
+                t["changed_rows"] = self._changed_rows(t, previous, row_map.to(self.device))
+                t["incremental"] = False
+                return t
+            nbytes = self.lib.tvbf_remove_workspace_bytes(C.byref(feats), C.byref(p), q)
+            if nbytes == 0:
+                check(-1, "tvbf_remove_workspace_bytes")
+            ws = self._workspace(nbytes)
+            t = out if out is not None else self._alloc_tables(m, k)
+            rows_d = torch.from_numpy(r.astype(np.int32)).to(self.device)
+            changed = torch.empty((m,), dtype=torch.int32, device=self.device)
+            prev = self._c_tables({**previous, "stats": t["stats"]})
+            check(self.lib.tvbf_remove_topk(C.byref(feats), C.byref(p), rows_d.data_ptr(), q, C.byref(prev),
+                                            C.byref(self._c_tables(t)), changed.data_ptr(), ws.data_ptr(), ws.numel(),
+                                            self._stream()), "tvbf_remove_topk")
+            t["changed_rows"] = torch.nonzero(changed).flatten().to(torch.int32)
+            t["incremental"] = True
+        t["row_begin"] = 0
+        return t
+
+    def remove_tiles(self, cat: DeviceCatalogue, n_rows: int, weights=(0.4, 0.5, 0.1), k: int = 20,
+                     min_similarity: float = 0.1) -> dict | None:
+        """Tensor-core tiles (256 x 256 x k_pad) the incremental removal of ``top_k_remove_device``
+        executes on the remaining catalogue ``cat`` when ``n_rows`` of its rows named a removed show
+        (the length of ``changed_rows``; host only): its threshold seed pass over their gathered rows
+        and the repair sweep.  {0, 0} for no such row; None when the job runs the whole job instead."""
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, int(k), float(min_similarity))
+            if feats is None or not 0 <= int(n_rows) <= cat.n_shows:
+                return None
+            if int(n_rows) == 0:
+                return {"seed_tiles": 0, "sweep_tiles": 0}
+            out = (C.c_int64 * 2)()
+            check(self.lib.tvbf_remove_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
+                                                  int(n_rows), out), "tvbf_remove_plan_tiles")
         return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
 
     def top_k_sweep_device(self, cat: DeviceCatalogue, weight_list, k: int = 20, min_similarity: float = 0.1,

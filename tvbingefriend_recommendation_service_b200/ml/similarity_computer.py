@@ -28,13 +28,21 @@ def _split_rows(features: dict, n: int) -> tuple[dict, dict]:
     return old, new
 
 
-def _changed_rows(top: TopK, previous: TopK) -> np.ndarray:
+def _changed_rows(top: TopK, previous: TopK, row_map: np.ndarray | None = None) -> np.ndarray:
     """Sorted int32 rows of ``previous`` that differ from the same rows of ``top`` in any of the six
-    fields (the scores bit for bit)."""
-    n = previous.counts.shape[0]
-    diff = (top.counts[:n] != previous.counts) | (top.indices[:n] != previous.indices).any(axis=1)
+    fields (the scores bit for bit).  With ``row_map`` (a removal: previous row o is row
+    ``row_map[o]`` of ``top``, -1 when it was removed) the rows of ``top`` are compared with their
+    previous rows, whose indices are renumbered by ``row_map`` (a removed show becomes -1)."""
+    prev = {name: getattr(previous, name) for name in ("indices", "counts", "hybrid", "genre", "text", "metadata")}
+    if row_map is not None:
+        keep = np.nonzero(row_map >= 0)[0]
+        prev = {name: a[keep] for name, a in prev.items()}
+        idx = prev["indices"]
+        prev["indices"] = np.where(idx >= 0, row_map[np.maximum(idx, 0)], idx).astype(idx.dtype)
+    n = prev["counts"].shape[0]
+    diff = (top.counts[:n] != prev["counts"]) | (top.indices[:n] != prev["indices"]).any(axis=1)
     for name in ("hybrid", "genre", "text", "metadata"):
-        diff |= (getattr(top, name)[:n].view(np.int64) != getattr(previous, name).view(np.int64)).any(axis=1)
+        diff |= (getattr(top, name)[:n].view(np.int64) != prev[name].view(np.int64)).any(axis=1)
     return np.nonzero(diff)[0].astype(np.int32)
 
 
@@ -248,6 +256,56 @@ class SimilarityComputer:
             prev = {name: torch.from_numpy(np.ascontiguousarray(getattr(previous, name))).to(eng.device)
                     for name in fields}
             t = eng.top_k_update_device(cat, r, prev, weights, k, min_similarity)
+            changed = t["changed_rows"].cpu().numpy()
+        top = eng.to_host(t)
+        top.changed_rows = changed
+        return top
+
+    def remove_top_k(self, features: dict, previous: TopK, rows, k: int = 20, min_similarity: float = 0.1,
+                     exclude_self: bool = True, metadata_mode: str = "mean3",
+                     normalize_weights: bool = False) -> TopK:
+        """Top-K table after the shows ``rows`` left a catalogue whose table exists.
+
+        ``features`` is the catalogue after the removal (the remaining shows in their old order);
+        ``previous`` is the ``compute_top_k`` table of the catalogue before it, with the same
+        arguments, and ``rows`` are the removed shows' rows in it.  Row r of the result is the r-th
+        remaining show, and its indices are rows of ``features``.  The result equals
+        ``compute_top_k(features, ...)`` bit for bit; its ``changed_rows`` lists the rows (sorted
+        int32) that differ in any field from their previous row with its indices renumbered -- every
+        other row is identical to that, so a caller only has to store the listed rows.  Only the
+        shows whose previous row names a removed show are scored against the catalogue on the
+        tensor cores.  Removing every show raises ``ValueError``.
+
+        Precondition, which the library cannot check: the remaining shows have the features
+        ``previous`` was computed from.  Jobs the incremental path does not take (signed text,
+        float-valued groups, k > 100, ``exclude_self=False``, ...) run the whole job and compare."""
+        weights = self._normalized_weights() if normalize_weights else \
+            (self.genre_weight, self.text_weight, self.metadata_weight)
+        n_all = int(np.asarray(features["genre_features"]).shape[0])
+        n_old = int(previous.counts.shape[0])
+        eng = self.engine
+        r = eng._update_rows(rows, n_old)
+        if previous.indices.ndim != 2 or previous.indices.shape != (n_all + r.size, k) \
+                or previous.counts.shape != (n_all + r.size,) or previous.row_begin != 0:
+            raise ValueError(f"previous table has shape {previous.indices.shape}, expected "
+                             f"({n_all + r.size}, {k}) from row 0")
+        if n_all == 0:
+            raise ValueError("remove_top_k: removing every show leaves no catalogue")
+        fields = ("indices", "counts", "hybrid", "genre", "text", "metadata")
+
+        if r.size == 0:
+            return TopK(*(getattr(previous, name) for name in fields), changed_rows=np.zeros(0, dtype=np.int32))
+        if not exclude_self:
+            row_map = np.full(n_old, -1, dtype=np.int64)
+            row_map[np.delete(np.arange(n_old), r)] = np.arange(n_all)
+            top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
+            top.changed_rows = _changed_rows(top, previous, row_map)
+            return top
+        cat = eng.ingest(features, metadata_mode, weights)
+        with torch.cuda.device(eng.device):
+            prev = {name: torch.from_numpy(np.ascontiguousarray(getattr(previous, name))).to(eng.device)
+                    for name in fields}
+            t = eng.top_k_remove_device(cat, r, prev, weights, k, min_similarity)
             changed = t["changed_rows"].cpu().numpy()
         top = eng.to_host(t)
         top.changed_rows = changed
