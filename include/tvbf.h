@@ -134,6 +134,7 @@ typedef struct tvbf_topk_out {
   double* metadata;  /* [rows, k] metadata_score                                              */
   int32_t* stats;    /* [8] device ints: 0 flagged rows repaired by the exact kernel,         */
                      /*     1 candidate pairs rescored, 2 / 3 flagged rows with / without text,*/
+                     /*     5 rows repaired by the second sweep of tvbf_refresh_topk,         */
                      /*     rest reserved                                                     */
 } tvbf_topk_out;
 
@@ -326,6 +327,32 @@ int tvbf_remove_topk(const tvbf_features* f, const tvbf_params* p, const int32_t
                      const tvbf_topk_out* prev, const tvbf_topk_out* out, int32_t* changed, void* workspace,
                      size_t workspace_bytes, void* stream);
 
+/* ---- refresh a catalogue whose table exists: remove, update and append shows in one call (instead of
+ *      the whole job again).  f: the catalogue of n_shows = N - n_removed + n_appended shows AFTER the
+ *      refresh -- the N - n_removed remaining shows in their old order, the updated ones with their new
+ *      features, then the n_appended new shows, all in the same vocabulary and widths; removed: the
+ *      removed rows, updated: the updated rows, both in the OLD numbering (device arrays, sorted,
+ *      distinct, in [0, N), disjoint; NULL when empty); prev: the [N, k] table of the catalogue before the
+ *      refresh from a job with the same p (weights, k, min_similarity, exclude_self = 1).  Writes the
+ *      [n_shows, k] table of f to `out` (new numbering) -- bit-identical to tvbf_hybrid_topk on f
+ *      (indices, counts and the four scores; stats differ) -- and changed[r] = 1 for every appended row
+ *      and for every remaining row that differs in any of the six fields from its previous row with the
+ *      indices renumbered (0 otherwise: the row is byte-identical to it).  Unlike tvbf_append_topk,
+ *      whose changed flags cover the old rows only, the appended rows are flagged too.
+ *      The updated and appended shows (S), and the remaining shows whose previous row names a removed show
+ *      (A), are swept against all columns; a row outside those that names no show of S and receives no
+ *      candidate from one above its threshold is copied without rescoring.  Rows outside S and A that fail
+ *      the certificate are swept against all columns a second time (stats[5] counts them) instead of
+ *      going to the exact kernel.  The call waits for the stream twice, to size the two sweeps.  Jobs
+ *      tvbf_sym_eligible rejects, signed text, and an `out` aliasing `prev` are rejected (the caller runs
+ *      the whole job); at least one show must remain. */
+size_t tvbf_refresh_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_removed,
+                                    int32_t n_updated, int32_t n_appended);
+int tvbf_refresh_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* removed, int32_t n_removed,
+                      const int32_t* updated, int32_t n_updated, int32_t n_appended, const tvbf_topk_out* prev,
+                      const tvbf_topk_out* out, int32_t* changed, void* workspace, size_t workspace_bytes,
+                      void* stream);
+
 /* exact fp64 scoring of explicit source rows against all columns + exact top-K
  * (replaces get_recommendations_from_matrix, content_based_service.py:161-236, for any n). */
 size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed);
@@ -422,6 +449,13 @@ int tvbf_update_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t
  * gathered rows, tiles of the repair sweep} (256 x 256 x k_pad each); the schedule is the update
  * sweep's for n_rows rows.  Fails like tvbf_remove_workspace_bytes for a job the removal does not take. */
 int tvbf_remove_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_rows, int64_t* out2);
+/* host-only: tensor-core tiles tvbf_refresh_topk executes for this job (f after the refresh) when
+ * n_gathered rows are in S or A and n_repaired rows go to the second sweep, out4 = {seed pass tiles,
+ * sweep tiles} of the refresh sweep, then of the second sweep (256 x 256 x k_pad each; 0 for a stage
+ * without rows).  Both are the update sweep's schedule for their row counts.  Fails like
+ * tvbf_refresh_workspace_bytes for a job the refresh does not take. */
+int tvbf_refresh_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_gathered, int32_t n_repaired,
+                            int64_t* out4);
 /* host-only: the work items of the update sweep of tvbf_update_topk for q updated shows in a catalogue
  * of n_shows on a device with sm_count SMs; out as tvbf_debug_schedule (super block = block of 256
  * gathered rows).  Returns the number of items.  Used by the CPU tests to prove that every (gathered

@@ -114,6 +114,10 @@ SIGNATURES = {
     "tvbf_remove_workspace_bytes": (c_size_t, [C.POINTER(Features), C.POINTER(Params), c_int32]),
     "tvbf_remove_topk": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int32, C.POINTER(TopKOut),
                                    C.POINTER(TopKOut), c_void_p, c_void_p, c_size_t, c_void_p]),
+    "tvbf_refresh_workspace_bytes": (c_size_t, [C.POINTER(Features), C.POINTER(Params), c_int32, c_int32, c_int32]),
+    "tvbf_refresh_topk": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int32, c_void_p, c_int32,
+                                    c_int32, C.POINTER(TopKOut), C.POINTER(TopKOut), c_void_p, c_void_p, c_size_t,
+                                    c_void_p]),
     "tvbf_exact_workspace_bytes": (c_size_t, [C.POINTER(Features), c_int32]),
     "tvbf_exact_rows": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int32,
                                   C.POINTER(TopKOut), c_void_p, c_size_t, c_void_p]),
@@ -140,6 +144,8 @@ SIGNATURES = {
     "tvbf_update_plan_tiles": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_int32, C.POINTER(c_int64)]),
     "tvbf_debug_update_schedule": (c_int32, [c_int32, c_int32, c_int32, C.POINTER(c_int32), c_int32]),
     "tvbf_remove_plan_tiles": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_int32, C.POINTER(c_int64)]),
+    "tvbf_refresh_plan_tiles": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_int32, c_int32,
+                                          C.POINTER(c_int64)]),
     "tvbf_plan_tiles": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_int32, c_int32, c_int32,
                                   C.POINTER(c_int64)]),
     "tvbf_debug_slack": (C.c_int, [C.POINTER(Features), C.POINTER(Params), C.POINTER(C.c_float)]),

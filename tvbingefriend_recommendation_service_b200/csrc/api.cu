@@ -1558,6 +1558,444 @@ int tvbf_remove_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t
   return TVBF_OK;
 }
 
+// ---- refresh a catalogue whose table exists: removed, updated and appended shows in one call ------
+// New numbering: the remaining shows in their old order, then the appended ones.  S = updated and
+// appended shows (their pair scores changed or are new); A = the other remaining shows whose previous
+// row names a removed show; G = S + A.  Stage 1 sweeps the gathered rows of G against every column (K1
+// kMode 10): a row of G scores its whole row into its own list, and a row of S also offers each score to
+// the column's list unless that column is in G.  A show outside G merges the renumbered previous row T'
+// without S (list 1, with the rank cut at its previous k-th entry) with what S offered it (list 0); one
+// that was offered nothing and names no show of S in T' keeps T'.  K5 rescores the rest.  Stage 2
+// repairs the rows outside G that K5 rejects -- mostly rows that lost a neighbour of S below their
+// previous k-th entry, which no list can refill -- on the tensor cores as the removal repairs A (kMode 8
+// seed, kMode 9 sweep, K5 on the gathered lists).  K6 takes the rows of G that K5 rejects (tie plateaus,
+// overflowed lists: a second sweep would reject them again) and what stage 2 rejects.
+namespace {
+
+// S bits: the new rows of the updated shows (old rows updated[0 .. n_upd)) and of the n_app appended ones
+__global__ void refresh_sbits_kernel(const int* updated, int n_upd, const int* map, int n, int n_app,
+                                     unsigned int* s_bits) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_upd + n_app) return;
+  const int r = t < n_upd ? map[updated[t]] : n - n_app + (t - n_upd);
+  atomicOr(s_bits + (r >> 5), 1u << (r & 31));
+}
+
+// Thread t < n_old: old row t, remaining as new row r = map[t]; thread n_old + a: appended new row
+// n - n_app + a.  old_row[r] = its old row (-1 appended); in_g[r] = 1 and the G bit for S and for a
+// remaining show whose previous row names a removed show (A).
+__global__ void refresh_rows_kernel(tvbf_topk_out prev, const int* map, int n_old, int n, int n_app, int k,
+                                    const unsigned int* s_bits, int* old_row, int* in_g, unsigned int* g_bits) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_old + n_app) return;
+  int r = n - n_app + (t - n_old), o = -1;
+  bool g = true;
+  if (t < n_old) {
+    o = t;
+    r = map[o];
+    if (r < 0) return;
+    g = ((s_bits[r >> 5] >> (r & 31)) & 1u) != 0u;
+    const int c = prev.counts[o];
+    const size_t src = static_cast<size_t>(o) * k;
+    for (int e = 0; e < c && !g; ++e) g = map[prev.indices[src + e]] < 0;
+  }
+  old_row[r] = o;
+  in_g[r] = g;
+  if (g) atomicOr(g_bits + (r >> 5), 1u << (r & 31));
+}
+
+__device__ __forceinline__ bool refresh_bit(const unsigned int* bits, int j) { return ((bits[j >> 5] >> (j & 31)) & 1u) != 0u; }
+
+// After K4s: a show outside G that received no candidate from S above its threshold and whose T' names no
+// show of S keeps T' (the scores of all its columns are unchanged): copied with the indices renumbered,
+// no rescoring.  Every other show is listed for K5.
+__global__ void refresh_select_kernel(tvbf_topk_out prev, tvbf_topk_out out, const int* list0_cnt, const int* map,
+                                      const int* old_row, const unsigned int* s_bits, const unsigned int* g_bits,
+                                      int n, int k, int* rows, int* n_listed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  bool listed = refresh_bit(g_bits, r) || list0_cnt[r] != 0;
+  const int o = old_row[r];
+  const size_t src = static_cast<size_t>(o) * k, dst = static_cast<size_t>(r) * k;
+  const int c = listed ? 0 : prev.counts[o];
+  for (int e = 0; e < c && !listed; ++e) listed = refresh_bit(s_bits, map[prev.indices[src + e]]);
+  if (listed) {
+    rows[atomicAdd(n_listed, 1)] = r;
+    return;
+  }
+  for (int e = 0; e < k; ++e) {
+    const int j = prev.indices[src + e];
+    out.indices[dst + e] = e < c ? map[j] : j;
+    out.hybrid[dst + e] = prev.hybrid[src + e];
+    out.genre[dst + e] = prev.genre[src + e];
+    out.text[dst + e] = prev.text[src + e];
+    out.metadata[dst + e] = prev.metadata[src + e];
+  }
+  out.counts[r] = c;
+}
+
+// After K5 (one block): of the rows K5 flagged, those in G move to the second flagged arrays (flag2 /
+// floor2, counts c2[2] / c2[3], with text at the front as K5 lays them out) for K6; the others are marked
+// in in2 for the second sweep, leave stats[0] (they are not the exact kernel's) and are counted in
+// stats[5].  The first flagged arrays are then empty for the K5 of the second stage.
+constexpr int kSplitThreads = 1024;
+__global__ void __launch_bounds__(kSplitThreads) refresh_split_kernel(const int* flagged, const double* floors,
+                                                                       const unsigned int* g_bits, int n, int* stats,
+                                                                       int* in2, int* flag2, double* floor2, int* c2) {
+  __shared__ int front, back, moved;
+  if (threadIdx.x == 0) front = back = moved = 0;
+  const int n_front = stats[2], n_back = stats[3];
+  __syncthreads();
+  for (int i = threadIdx.x; i < n_front + n_back; i += kSplitThreads) {
+    const int pos = i < n_front ? i : n - 1 - (i - n_front);
+    const int r = flagged[pos];
+    if (refresh_bit(g_bits, r)) {
+      const int at = i < n_front ? atomicAdd(&front, 1) : n - 1 - atomicAdd(&back, 1);
+      flag2[at] = r;
+      floor2[at] = floors[pos];
+    } else {
+      in2[r] = 1;
+      atomicAdd(&moved, 1);
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    c2[2] = front;
+    c2[3] = back;
+    stats[0] -= moved;
+    stats[2] = 0;
+    stats[3] = 0;
+    stats[5] = moved;
+  }
+}
+
+// changed[r] = 1 for an appended row and for a row that differs from T'_r in any of the six fields (bit
+// for bit)
+__global__ void refresh_changed_kernel(tvbf_topk_out prev, tvbf_topk_out out, const int* map, const int* old_row,
+                                       int n, int k, int* changed) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int o = old_row[r];
+  if (o < 0) {
+    changed[r] = 1;
+    return;
+  }
+  const int cnt = prev.counts[o];
+  int c = cnt != out.counts[r];
+  const size_t src = static_cast<size_t>(o) * k, dst = static_cast<size_t>(r) * k;
+  for (int e = 0; e < k && !c; ++e) {
+    const int j = prev.indices[src + e];
+    c = (e < cnt ? map[j] : j) != out.indices[dst + e] || !same_bits(prev.hybrid[src + e], out.hybrid[dst + e]) ||
+        !same_bits(prev.genre[src + e], out.genre[dst + e]) || !same_bits(prev.text[src + e], out.text[dst + e]) ||
+        !same_bits(prev.metadata[src + e], out.metadata[dst + e]);
+  }
+  changed[r] = c;
+}
+
+struct RefreshPlan {
+  Plan pl;                // a whole-catalogue symmetric job over the shows after the refresh
+  tvbf::K1Params geo[2];  // tile schedules of the refresh sweep (|G| rows) and the repair sweep (stage 2)
+  int grid[2], q_pad[2];
+  size_t off_cand, off_cnt, off_bound;   // stage 1: two candidate lists per show, [2][n_shows]
+  size_t off_rows, off_listed;           // shows K5 rescores and their count
+  size_t off_gather;                     // gathered operand rows of either stage: [n_pad, k_pad]
+  size_t off_sbits, off_gbits, off_cut_s, off_cut_j, off_map, off_old_row, off_in_g, off_grows, off_gcount;
+  size_t off_in2, off_rows2, off_count2, off_flag2, off_floor2, off_c2, off_gtheta2, total;
+};
+
+int refresh_counts_ok(const tvbf_features* f, int n_removed, int n_updated, int n_appended) {
+  TVBF_REQUIRE(n_removed >= 0 && n_updated >= 0 && n_appended >= 0, "refresh: negative count (%d, %d, %d)",
+               n_removed, n_updated, n_appended);
+  TVBF_REQUIRE(n_appended < f->n_shows && n_updated <= f->n_shows - n_appended,
+               "refresh: %d updated and %d appended shows in a catalogue of %d (at least one show must remain)",
+               n_updated, n_appended, f->n_shows);
+  TVBF_REQUIRE(n_removed <= INT32_MAX - f->n_shows, "refresh: %d removed shows", n_removed);
+  return TVBF_OK;
+}
+
+// n_rows[0] = |G|, n_rows[1] = rows of the second stage (the sweep geometries; 0 sizes the workspace
+// only, which holds either up to every show)
+int make_refresh_plan(const tvbf_features* f, const tvbf_params* p, int n_removed, int n_updated, int n_appended,
+                      const int* n_rows, RefreshPlan* rp, tvbf_params* q) {
+  int rc = refresh_counts_ok(f, n_removed, n_updated, n_appended);
+  if (rc != TVBF_OK) return rc;
+  for (int s = 0; s < 2; ++s)
+    TVBF_REQUIRE(n_rows[s] >= 0 && n_rows[s] <= f->n_shows, "refresh: %d swept rows outside [0, n_shows %d]",
+                 n_rows[s], f->n_shows);
+  TVBF_REQUIRE(!f->text_signed, "refresh: signed text needs the whole job");
+  *q = *p;
+  q->row_begin = 0;
+  q->row_end = f->n_shows;
+  q->tuning = (q->tuning & ~(0x3 << 20)) | (2 << 20);   // symmetric job (or fail if ineligible)
+  q->tuning = (q->tuning & ~0xF) | 2;                   // CTA pairs
+  rc = validate_params(f, q);
+  if (rc != TVBF_OK) return rc;
+  rc = make_plan(f, q, &rp->pl);
+  if (rc != TVBF_OK) return rc;
+  int sms = 0;
+  rc = sm_count_cached(&sms);
+  if (rc != TVBF_OK) return rc;
+  for (int s = 0; s < 2; ++s) {
+    memset(&rp->geo[s], 0, sizeof(rp->geo[s]));
+    rp->grid[s] = 0;
+    rp->q_pad[s] = 0;
+    if (n_rows[s] == 0) continue;
+    tvbf::k1_update_geometry(n_rows[s], f->n_shows, sms / 2, &rp->geo[s]);
+    const tvbf::K1Params& g = rp->geo[s];
+    const int items = (g.rb_count + g.rb_per_group - 1) / g.rb_per_group * g.rb_per_group * g.splits;
+    rp->grid[s] = 2 * (items < sms / 2 ? items : sms / 2);
+    rp->q_pad[s] = g.rb_count * 256;
+  }
+  const size_t rows = static_cast<size_t>(f->n_shows);
+  const size_t words = static_cast<size_t>(f->n_pad) / 32 * 4;
+  size_t off = rp->pl.total;
+  rp->off_cand = off;    off = align_up(off + 2 * rows * rp->pl.kp * 8, 256);
+  rp->off_cnt = off;     off = align_up(off + 2 * rows * 4, 256);
+  rp->off_bound = off;   off = align_up(off + 2 * rows * 4, 256);
+  rp->off_rows = off;    off = align_up(off + rows * 4, 256);
+  rp->off_listed = off;  off = align_up(off + 4, 256);
+  rp->off_gather = off;  off = align_up(off + static_cast<size_t>(f->n_pad) * f->k_pad * 2, 256);
+  rp->off_sbits = off;   off = align_up(off + words, 256);
+  rp->off_gbits = off;   off = align_up(off + words, 256);
+  rp->off_cut_s = off;   off = align_up(off + rows * 8, 256);
+  rp->off_cut_j = off;   off = align_up(off + rows * 4, 256);
+  rp->off_map = off;     off = align_up(off + (rows - n_appended + n_removed) * 4, 256);
+  rp->off_old_row = off; off = align_up(off + rows * 4, 256);
+  rp->off_in_g = off;    off = align_up(off + rows * 4, 256);
+  rp->off_grows = off;   off = align_up(off + rows * 4, 256);
+  rp->off_gcount = off;  off = align_up(off + 4, 256);
+  rp->off_in2 = off;     off = align_up(off + rows * 4, 256);
+  rp->off_rows2 = off;   off = align_up(off + rows * 4, 256);
+  rp->off_count2 = off;  off = align_up(off + 4, 256);
+  rp->off_flag2 = off;   off = align_up(off + rows * 4, 256);
+  rp->off_floor2 = off;  off = align_up(off + rows * 8, 256);
+  rp->off_c2 = off;      off = align_up(off + 8 * 4, 256);
+  rp->off_gtheta2 = off; off = align_up(off + static_cast<size_t>(f->n_pad) * 4, 256);
+  rp->total = off;
+  return TVBF_OK;
+}
+
+// the candidate-kernel parameters of stage s: a whole-catalogue symmetric job on the sweep geometry.
+// Stage 0, the refresh sweep: lists by show, list 0 of the two-list table.  Stage 1, the repair sweep:
+// lists by gathered row (the plan's lists and candidate table), as the removal.
+int fill_refresh_params(const tvbf_features* f, const tvbf_params* q, const RefreshPlan& rp, uint8_t* ws, int s,
+                        const int* rows, int n_rows, tvbf::K1Params* kp) {
+  int rc = fill_k1_params(f, q, rp.pl, ws, kp);
+  if (rc != TVBF_OK) return rc;
+  kp->sync_kb = 0;
+  kp->sym = 0;              // the one-sided schedule: a rectangle
+  kp->wide_epilogue = 0;    // 8 epilogue warps, as the update sweep
+  kp->col_tiles = rp.geo[s].col_tiles;
+  kp->rb_count = rp.geo[s].rb_count;
+  kp->splits = rp.geo[s].splits;
+  kp->rb_per_group = rp.geo[s].rb_per_group;
+  kp->tiles_per_split = rp.geo[s].tiles_per_split;
+  kp->upd_rows = rows;
+  kp->upd_q = n_rows;
+  kp->upd_bits = nullptr;
+  kp->upd_sbits = nullptr;
+  if (s == 0) {
+    kp->upd_bits = reinterpret_cast<const unsigned int*>(ws + rp.off_gbits);
+    kp->upd_sbits = reinterpret_cast<const unsigned int*>(ws + rp.off_sbits);
+    kp->cand = reinterpret_cast<uint2*>(ws + rp.off_cand);
+    kp->cand_cnt = reinterpret_cast<int*>(ws + rp.off_cnt);
+    kp->cand_theta = reinterpret_cast<float*>(ws + rp.off_bound);
+  }
+  return TVBF_OK;
+}
+
+}  // namespace
+
+size_t tvbf_refresh_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int32_t n_removed,
+                                    int32_t n_updated, int32_t n_appended) {
+  if (validate_features(f) != TVBF_OK || p == nullptr) return 0;
+  RefreshPlan rp;
+  tvbf_params q;
+  const int none[2] = {0, 0};
+  if (make_refresh_plan(f, p, n_removed, n_updated, n_appended, none, &rp, &q) != TVBF_OK) return 0;
+  return rp.total;
+}
+
+int tvbf_refresh_topk(const tvbf_features* f, const tvbf_params* p, const int32_t* removed, int32_t n_removed,
+                      const int32_t* updated, int32_t n_updated, int32_t n_appended, const tvbf_topk_out* prev,
+                      const tvbf_topk_out* out, int32_t* changed, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  // the arguments first: these checks need no device
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p != nullptr, "params is NULL");
+  TVBF_REQUIRE(prev && prev->indices && prev->counts && prev->hybrid && prev->genre && prev->text && prev->metadata,
+               "previous table has NULL members");
+  TVBF_REQUIRE(out && out->indices && out->counts && out->hybrid && out->genre && out->text && out->metadata &&
+                   out->stats,
+               "output table has NULL members");
+  {
+    const void* po[6] = {prev->indices, prev->counts, prev->hybrid, prev->genre, prev->text, prev->metadata};
+    const void* oo[6] = {out->indices, out->counts, out->hybrid, out->genre, out->text, out->metadata};
+    for (int a = 0; a < 6; ++a)
+      for (int b = 0; b < 6; ++b) TVBF_REQUIRE(po[a] != oo[b], "tvbf_refresh_topk: the output table aliases the previous one");
+  }
+  TVBF_REQUIRE(changed != nullptr && workspace != nullptr, "tvbf_refresh_topk: NULL argument");
+  TVBF_REQUIRE((removed != nullptr || n_removed == 0) && (updated != nullptr || n_updated == 0),
+               "tvbf_refresh_topk: NULL row list");
+  rc = refresh_counts_ok(f, n_removed, n_updated, n_appended);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(!f->text_signed, "refresh: signed text needs the whole job");
+  TVBF_ENTER_CALL(stream);
+  RefreshPlan rp;
+  tvbf_params q;
+  int n_rows[2] = {0, 0};
+  rc = make_refresh_plan(f, p, n_removed, n_updated, n_appended, n_rows, &rp, &q);
+  if (rc != TVBF_OK) return rc;
+  if (workspace_bytes < rp.total) {
+    tvbf_set_error("workspace too small: %zu < %zu", workspace_bytes, rp.total);
+    return TVBF_ERR_WORKSPACE;
+  }
+  auto st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const Plan& pl = rp.pl;
+  const int n = f->n_shows, k = p->k, n_old = n - n_appended + n_removed;
+  const size_t words = static_cast<size_t>(f->n_pad) / 32 * 4;
+  auto at = [&](size_t off) { return reinterpret_cast<int*>(ws + off); };
+  int *map = at(rp.off_map), *old_row = at(rp.off_old_row), *in_g = at(rp.off_in_g), *g_rows = at(rp.off_grows);
+  int *g_count = at(rp.off_gcount), *listed_rows = at(rp.off_rows), *n_listed = at(rp.off_listed);
+  int *in2 = at(rp.off_in2), *rows2 = at(rp.off_rows2), *count2 = at(rp.off_count2), *flag2 = at(rp.off_flag2);
+  int *c2 = at(rp.off_c2), *cut_j = at(rp.off_cut_j), *flagged = at(pl.off_flag);
+  unsigned int* s_bits = reinterpret_cast<unsigned int*>(ws + rp.off_sbits);
+  unsigned int* g_bits = reinterpret_cast<unsigned int*>(ws + rp.off_gbits);
+  double* cut_s = reinterpret_cast<double*>(ws + rp.off_cut_s);
+  double* floors = reinterpret_cast<double*>(ws + pl.off_floor);
+  double* floor2 = reinterpret_cast<double*>(ws + rp.off_floor2);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+  int* cnt = reinterpret_cast<int*>(ws + rp.off_cnt);
+  // 1. map and classify
+  TVBF_CUDA_OK(cudaMemsetAsync(out->stats, 0, 8 * sizeof(int32_t), st));
+  TVBF_CUDA_OK(cudaMemsetAsync(s_bits, 0, words, st));
+  TVBF_CUDA_OK(cudaMemsetAsync(g_bits, 0, words, st));
+  remove_map_kernel<<<(n_old + 255) / 256, 256, 0, st>>>(removed, n_removed, n_old, map);
+  TVBF_LAUNCH_OK("remove_map_kernel");
+  if (n_updated + n_appended > 0) {
+    refresh_sbits_kernel<<<(n_updated + n_appended + 255) / 256, 256, 0, st>>>(updated, n_updated, map, n, n_appended,
+                                                                              s_bits);
+    TVBF_LAUNCH_OK("refresh_sbits_kernel");
+  }
+  refresh_rows_kernel<<<(n_old + n_appended + 255) / 256, 256, 0, st>>>(*prev, map, n_old, n, n_appended, k, s_bits,
+                                                                         old_row, in_g, g_bits);
+  TVBF_LAUNCH_OK("refresh_rows_kernel");
+  remove_compact_kernel<<<1, kCompactThreads, 0, st>>>(in_g, n, g_rows, g_count);
+  TVBF_LAUNCH_OK("remove_compact_kernel");
+  // the sweep's geometry depends on |G|
+  TVBF_CUDA_OK(cudaMemcpyAsync(&n_rows[0], g_count, 4, cudaMemcpyDeviceToHost, st));
+  TVBF_CUDA_OK(cudaStreamSynchronize(st));
+  const tvbf::ScoreParams sp = score_params(f, &q);
+  if (n_rows[0] == 0) {   // nothing was swept: every row keeps T'
+    TVBF_CUDA_OK(cudaMemsetAsync(cnt, 0, static_cast<size_t>(n) * 4, st));
+  } else {
+    // 2.-4. the refresh sweep over G, K4s, select, K5 with the rank cut
+    rc = make_refresh_plan(f, p, n_removed, n_updated, n_appended, n_rows, &rp, &q);
+    if (rc != TVBF_OK) return rc;
+    tvbf::K1Params kp;
+    rc = fill_refresh_params(f, &q, rp, ws, 0, g_rows, n_rows[0], &kp);
+    if (rc != TVBF_OK) return rc;
+    const int row_vec = f->k_pad / 8;   // 16-byte vectors per operand row
+    update_gather_kernel<<<1024, 256, 0, st>>>(static_cast<const uint4*>(f->operand), g_rows, n_rows[0], rp.q_pad[0],
+                                               row_vec, reinterpret_cast<uint4*>(ws + rp.off_gather));
+    TVBF_LAUNCH_OK("update_gather_kernel");
+    tvbf_features g = *f;   // the gathered rows as the A operand
+    g.operand = ws + rp.off_gather;
+    g.n_pad = rp.q_pad[0];
+    const tvbf::RefreshPrev pv{prev->indices, prev->counts, prev->hybrid, k, old_row, map, s_bits, g_bits,
+                               kp.cand + static_cast<size_t>(n) * pl.kp, cnt + n, kp.cand_theta + n, cut_s, cut_j};
+    rc = tvbf::k1_launch_refresh(f, &g, kp, rp.grid[0], pv, st);
+    if (rc != TVBF_OK) return rc;
+    rc = tvbf::k4s_launch(kp, n, st);
+    if (rc != TVBF_OK) return rc;
+  }
+  TVBF_CUDA_OK(cudaMemsetAsync(n_listed, 0, 4, st));
+  refresh_select_kernel<<<(n + 255) / 256, 256, 0, st>>>(*prev, *out, cnt, map, old_row, s_bits, g_bits, n, k,
+                                                          listed_rows, n_listed);
+  TVBF_LAUNCH_OK("refresh_select_kernel");
+  if (n_rows[0] > 0) {
+    const tvbf::CandLayout lay{0, 1, n, 0};   // list s of show r: slot r + s * n
+    rc = tvbf::k5_launch_listed(sp, reinterpret_cast<uint2*>(ws + rp.off_cand), cnt,
+                                reinterpret_cast<float*>(ws + rp.off_bound), 2, lay, pl.kp, 0, n, listed_rows, n_listed,
+                                *out, flagged, floors, st, cut_s, cut_j);
+    if (rc != TVBF_OK) return rc;
+    // 5. rejected rows of G to K6 now, the others to the second stage
+    TVBF_CUDA_OK(cudaMemsetAsync(in2, 0, static_cast<size_t>(n) * 4, st));
+    refresh_split_kernel<<<1, kSplitThreads, 0, st>>>(flagged, floors, g_bits, n, out->stats, in2, flag2, floor2, c2);
+    TVBF_LAUNCH_OK("refresh_split_kernel");
+    tvbf_topk_out o2 = *out;
+    o2.stats = c2;   // the counts of the second flagged arrays, at the slots K6 reads
+    rc = tvbf::k6_launch_flagged(sp, flag2, floor2, n, 0, keys, pl.k6_grid, o2, st);
+    if (rc != TVBF_OK) return rc;
+    remove_compact_kernel<<<1, kCompactThreads, 0, st>>>(in2, n, rows2, count2);
+    TVBF_LAUNCH_OK("remove_compact_kernel");
+    TVBF_CUDA_OK(cudaMemcpyAsync(&n_rows[1], count2, 4, cudaMemcpyDeviceToHost, st));
+    TVBF_CUDA_OK(cudaStreamSynchronize(st));
+  }
+  if (n_rows[1] > 0) {
+    // the second stage: the rejected rows outside G against every column, lists by gathered row
+    rc = make_refresh_plan(f, p, n_removed, n_updated, n_appended, n_rows, &rp, &q);
+    if (rc != TVBF_OK) return rc;
+    tvbf::K1Params kp;
+    rc = fill_refresh_params(f, &q, rp, ws, 1, rows2, n_rows[1], &kp);
+    if (rc != TVBF_OK) return rc;
+    const int row_vec = f->k_pad / 8;
+    update_gather_kernel<<<1024, 256, 0, st>>>(static_cast<const uint4*>(f->operand), rows2, n_rows[1], rp.q_pad[1],
+                                               row_vec, reinterpret_cast<uint4*>(ws + rp.off_gather));
+    TVBF_LAUNCH_OK("update_gather_kernel");
+    tvbf_features g = *f;
+    g.operand = ws + rp.off_gather;
+    g.n_pad = rp.q_pad[1];
+    unsigned int* gtheta = reinterpret_cast<unsigned int*>(ws + rp.off_gtheta2);
+    rc = tvbf::k1_launch_remove(f, &g, kp, rp.grid[1], gtheta, st);
+    if (rc != TVBF_OK) return rc;
+    kp.g_theta = gtheta;   // K4s: the gathered rows' lists under their thresholds
+    rc = tvbf::k4s_launch(kp, n_rows[1], st);
+    if (rc != TVBF_OK) return rc;
+    const tvbf::CandLayout lay{0, 1, 0, 0, 1};   // the list of rows2[e] is slot e
+    rc = tvbf::k5_launch_listed(sp, kp.cand, kp.cand_cnt, kp.cand_theta, 1, lay, pl.kp, 0, n, rows2, count2, *out,
+                                flagged, floors, st);
+    if (rc != TVBF_OK) return rc;
+  }
+  if (n_rows[0] > 0) {
+    rc = tvbf::k6_launch_flagged(sp, flagged, floors, n, 0, keys, pl.k6_grid, *out, st);
+    if (rc != TVBF_OK) return rc;
+  }
+  // 6. changed flags against T'
+  refresh_changed_kernel<<<(n + 255) / 256, 256, 0, st>>>(*prev, *out, map, old_row, n, k, changed);
+  TVBF_LAUNCH_OK("refresh_changed_kernel");
+  return TVBF_OK;
+}
+
+int tvbf_refresh_plan_tiles(const tvbf_features* f, const tvbf_params* p, int32_t n_gathered, int32_t n_repaired,
+                            int64_t* out4) {
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(p && out4, "tvbf_refresh_plan_tiles: NULL argument");
+  TVBF_REQUIRE(n_gathered >= 1 || n_repaired == 0, "tvbf_refresh_plan_tiles: %d gathered and %d repaired rows",
+               n_gathered, n_repaired);
+  RefreshPlan rp;
+  tvbf_params q;
+  const int n_rows[2] = {n_gathered, n_repaired};
+  rc = make_refresh_plan(f, p, 0, 0, 0, n_rows, &rp, &q);
+  if (rc != TVBF_OK) return rc;
+  uint8_t* fake_ws = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(4096));   // offsets only, never dereferenced
+  for (int s = 0; s < 2; ++s) {
+    out4[2 * s] = out4[2 * s + 1] = 0;
+    if (n_rows[s] == 0) continue;
+    tvbf::K1Params kp;
+    rc = fill_refresh_params(f, &q, rp, fake_ws, s, nullptr, n_rows[s], &kp);
+    if (rc != TVBF_OK) return rc;
+    long long t[2];
+    tvbf::k1_update_executed_tiles(kp, rp.grid[s], t);
+    out4[2 * s] = t[0];
+    out4[2 * s + 1] = t[1];
+  }
+  return TVBF_OK;
+}
+
 // ---- streaming statistics of the four similarity matrices (no N x N) --------------------------
 size_t tvbf_stats_accum_bytes(void) { return sizeof(tvbf::StatsAccum); }
 

@@ -408,7 +408,9 @@ struct Pacer {
 // rectangle without a diagonal; offered to the row's show and to every column show not updated itself,
 // 8 the threshold seed pass (as 3) over the gathered rows of an update,
 // 9 repair sweep of a removal: the update sweep without the column side -- every score goes to the
-// gathered row's list only, and that list, its count and its threshold are indexed by the gathered row
+// gathered row's list only, and that list, its count and its threshold are indexed by the gathered row,
+// 10 refresh sweep: the update sweep over the gathered rows of the shows in G = S + A (p.upd_bits), where
+// only a row whose show is in S (p.upd_sbits: updated or appended) feeds the column side
 // kG2: multi-hot genres with 64 < G <= 128 -- the second word of every column's mask is staged beside
 // the column-side records (in the threshold slices a single-triple sweep leaves unused) and the
 // popcount runs over both words.
@@ -428,9 +430,10 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
   constexpr bool kStats = kMode == 2;    // accumulate statistics instead of candidate lists
   constexpr bool kMulti = kMode == 5;    // weight sweep
   constexpr bool kAppend = kMode == 6;   // append sweep
-  constexpr bool kUpdate = kMode == 7;   // update sweep
+  constexpr bool kRefresh = kMode == 10;   // refresh sweep
+  constexpr bool kUpdate = kMode == 7 || kRefresh;   // update sweep (or its refresh variant)
   constexpr bool kRepair = kMode == 9;   // repair sweep of a removal
-  constexpr bool kGather = kMode == 7 || kMode == 8 || kRepair;   // rows are gathered rows
+  constexpr bool kGather = kMode == 7 || kMode == 8 || kRepair || kRefresh;   // rows are gathered rows
   static_assert(!(kG2 && (kMulti || kStats)), "two-word genre masks: single-triple top-k sweeps only");
   static_assert(!(kFold && (kMulti || kStats || kDump || kG2)), "folded groups: single-triple top-k sweeps only");
   // Seed pass: hist[bin][row of the CTA] (32-bit counters; bank = row % 32, so the 32 lanes of a warp
@@ -650,6 +653,8 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const bool row_valid = kGather ? grow < p.upd_q : grow < p.row_end;
       const int row = kGather ? (row_valid ? p.upd_rows[grow] : -1) : grow;   // the show of this row
       const int lrow = kRepair ? grow : row;   // the list (and threshold) of this row
+      // refresh: a row of A (its scores are unchanged) feeds its own list only
+      const bool feeds_cols = !kRefresh || (row_valid && ((p.upd_sbits[row >> 5] >> (row & 31)) & 1u) != 0u);
       // row-side operands of the fused scores
       unsigned long long g_bits = 0ull, g_hi = 0ull;
       uint32_t m_bits = 0u;
@@ -756,7 +761,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
         const uint32_t taddr = tmem_base + tmem_lane + b * BN;
         // off-diagonal tiles also feed the column shows (their mirror tile is never computed); the
         // update sweep's rectangle has no mirror tiles; the repair sweep feeds its rows only
-        const bool do_col = kSym && !kRepair && row_valid && (kUpdate || jt != c.sb);
+        const bool do_col = kSym && !kRepair && row_valid && (kUpdate || jt != c.sb) && feeds_cols;
 
         float tile_sum[4] = {0.f, 0.f, 0.f, 0.f}, tile_sq[4] = {0.f, 0.f, 0.f, 0.f}, tile_gm = 0.f;
         float stat_scale[4];
@@ -1307,6 +1312,42 @@ __global__ void update_prev_kernel(UpdatePrev a, unsigned int* theta, float thet
       th = fmaxf(th, theta_init);
       cut_h = kth;
       cut_j = a.indices[base + a.k - 1];
+    }
+    theta[r] = __float_as_uint(th);
+  }
+  a.cnt[r] = cnt;
+  a.bound[r] = __int_as_float(0xff800000);
+  a.cut_score[r] = cut_h;
+  a.cut_index[r] = cut_j;
+}
+
+// Refresh: update_prev_kernel on the renumbered previous table T' with two bit sets.  A show outside G
+// (remaining, not updated, its previous row names no removed show) gets T'_r without the shows of S as
+// list 1, the threshold of its previous k-th entry and the rank cut there when the row was full.  A show
+// in G gets an empty list 1 and no cut: the rows of A in T' name removed shows and are not read.
+__global__ void refresh_prev_kernel(RefreshPrev a, unsigned int* theta, float theta_init, int n_shows, int kp) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_shows) return;
+  int cnt = 0, cut_j = -1;
+  double cut_h = 0.0;
+  if (((a.g_bits[r >> 5] >> (r & 31)) & 1u) == 0u) {
+    const int o = a.old_row[r];
+    const int n = a.counts[o];
+    uint2* dst = a.list + static_cast<size_t>(r) * kp;
+    const size_t base = static_cast<size_t>(o) * a.k;
+    for (int e = 0; e < n; ++e) {
+      const int j = a.map[a.indices[base + e]];
+      if ((a.s_bits[j >> 5] >> (j & 31)) & 1u) continue;
+      dst[cnt++] = make_uint2(__float_as_uint(__double2float_ru(a.hybrid[base + e])), static_cast<uint32_t>(j));
+    }
+    float th = theta_init;
+    if (n == a.k) {
+      const double kth = a.hybrid[base + a.k - 1];
+      th = __double2float_rd(kth);
+      if (static_cast<double>(th) >= kth) th = nextafterf(th, -INFINITY);
+      th = fmaxf(th, theta_init);
+      cut_h = kth;
+      cut_j = a.map[a.indices[base + a.k - 1]];
     }
     theta[r] = __float_as_uint(th);
   }
@@ -2032,6 +2073,50 @@ int k1_launch_remove(const tvbf_features* f, const tvbf_features* g, const K1Par
   if (kp.fold) return launch_k1<4, false, 2, 9, false, false, true>(f, sweep, grid, st, g);
   return kp.genre_hi ? launch_k1<4, false, 2, 9, false, true>(f, sweep, grid, st, g)
                      : launch_k1<4, false, 2, 9>(f, sweep, grid, st, g);
+}
+
+// Refresh: as k1_launch_update, with the lists of the renumbered previous table and the refresh sweep
+int k1_launch_refresh(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                      const RefreshPrev& prev, cudaStream_t st) {
+  if (kp.sym || kp.n_weights > 1 || kp.sync_kb != 0 || kp.wide_epilogue || kp.upd_q < 1 || kp.upd_rows == nullptr ||
+      kp.upd_bits == nullptr || kp.upd_sbits == nullptr) {
+    tvbf_set_error("refresh sweep: bad parameters");
+    return TVBF_ERR_INVALID;
+  }
+  const int n_pad = f->n_pad;
+  const size_t list_bytes = static_cast<size_t>(n_pad) * kp.sym_cap * 8;
+  std::lock_guard<std::mutex> lock(g_side_mutex);
+  SideStream* side = nullptr;
+  int rc = side_stream(&side);
+  if (rc != TVBF_OK) return rc;
+  // the shared lists are cleared on the side stream beside the seed pass, as in an update
+  rc = absorb_pending(side, st, true);
+  if (rc != TVBF_OK) return rc;
+  TVBF_CUDA_OK(cudaEventRecord(side->fork, st));
+  TVBF_CUDA_OK(cudaStreamWaitEvent(side->stream, side->fork, 0));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_cnt, 0, static_cast<size_t>(n_pad) * 4, side->stream));
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.g_list, 0, list_bytes, side->stream));
+  TVBF_CUDA_OK(cudaEventRecord(side->join, side->stream));
+  sym_init_kernel<<<static_cast<unsigned>((n_pad + 255) / 256), 256, 0, st>>>(kp.g_theta, f->n_shows, n_pad, n_pad,
+                                                                               kp.theta_init);
+  TVBF_LAUNCH_OK("sym_init_kernel");
+  refresh_prev_kernel<<<static_cast<unsigned>((f->n_shows + 255) / 256), 256, 0, st>>>(prev, kp.g_theta,
+                                                                                       kp.theta_init, f->n_shows, kp.kp);
+  TVBF_LAUNCH_OK("refresh_prev_kernel");
+  {
+    const K1Params seed = update_seed_params(kp, grid);
+    const int sg = seed.rb_per_group * 2;
+    if (kp.fold) rc = launch_k1<4, false, 2, 8, false, false, true>(f, seed, sg, st, g);
+    else if (kp.genre_hi != nullptr) rc = launch_k1<4, false, 2, 8, false, true>(f, seed, sg, st, g);
+    else rc = launch_k1<4, false, 2, 8>(f, seed, sg, st, g);
+    if (rc != TVBF_OK) return rc;
+  }
+  TVBF_CUDA_OK(cudaStreamWaitEvent(st, side->join, 0));
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  if (kp.fold) return launch_k1<4, false, 2, 10, false, false, true>(f, sweep, grid, st, g);
+  return kp.genre_hi ? launch_k1<4, false, 2, 10, false, true>(f, sweep, grid, st, g)
+                     : launch_k1<4, false, 2, 10>(f, sweep, grid, st, g);
 }
 
 int k1_launch_dump(const tvbf_features* f, const K1Params& kp, int cta_group, cudaStream_t st) {

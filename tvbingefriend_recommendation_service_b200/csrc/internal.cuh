@@ -129,6 +129,9 @@ struct K1Params {
   const int* upd_rows;
   int upd_q;
   const unsigned int* upd_bits;
+  // refresh sweep (kMode 10, tvbf_refresh_topk): upd_bits marks G (every gathered show), upd_sbits the
+  // shows of S (updated or appended); only a gathered row whose show is in S feeds the column side
+  const unsigned int* upd_sbits;
 };
 
 // The previous table of an update and where its rows go (list 1 of the two-list candidate table, as
@@ -143,6 +146,24 @@ struct UpdatePrev {
   int* cnt;             // [n_shows]
   float* bound;         // [n_shows]
   double* cut_score;    // [n_shows] previous k-th entry (score, index); index -1: no cut
+  int* cut_index;
+};
+
+// The previous table of a refresh (old numbering) read as the renumbered table T': new row r is old row
+// old_row[r] (-1: appended) with every index j renumbered to map[j].  Lists and cut as UpdatePrev.
+struct RefreshPrev {
+  const int* indices;   // [n_old, k]
+  const int* counts;    // [n_old]
+  const double* hybrid; // [n_old, k]
+  int k;
+  const int* old_row;   // [n_shows]
+  const int* map;       // [n_old] (-1: removed)
+  const unsigned int* s_bits;   // S: updated or appended shows
+  const unsigned int* g_bits;   // G: S and the remaining shows whose previous row names a removed show
+  uint2* list;          // [n_shows][kp]
+  int* cnt;             // [n_shows]
+  float* bound;         // [n_shows]
+  double* cut_score;    // [n_shows]
   int* cut_index;
 };
 
@@ -222,6 +243,10 @@ void k1_update_executed_tiles(const K1Params& kp, int grid, long long* out);
 // gtheta ([rb_count * 256]) are indexed by the gathered row; only those lists are cleared
 int k1_launch_remove(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
                      unsigned int* gtheta, cudaStream_t st);
+// thresholds and list 1 from the renumbered previous table, seed pass over the gathered rows of G, then
+// the refresh sweep (kMode 10); kp.upd_bits holds G, kp.upd_sbits S
+int k1_launch_refresh(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
+                      const RefreshPrev& prev, cudaStream_t st);
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);

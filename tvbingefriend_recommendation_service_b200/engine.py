@@ -1238,6 +1238,102 @@ class HybridTopKEngine:
                                                   int(n_rows), out), "tvbf_remove_plan_tiles")
         return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1])}
 
+    # ------------------------------------------------------------------------------------ refreshes
+    def top_k_refresh_device(self, cat: DeviceCatalogue, previous: dict, removed=(), updated=(), n_appended: int = 0,
+                             weights=(0.4, 0.5, 0.1), k: int = 20, min_similarity: float = 0.1,
+                             exclude_self: bool = True, out: dict | None = None) -> dict:
+        """Table of ``cat`` after a refresh that removed the shows ``removed``, gave the shows
+        ``updated`` new features (both rows of ``previous``, distinct and disjoint, any order) and
+        appended ``n_appended`` shows, from ``previous``, the device table (``top_k_device``) of the
+        catalogue before it for the same weights, ``k``, ``min_similarity`` and ``exclude_self``.
+        ``cat`` holds the remaining shows in their old order, the updated ones with their new
+        features, then the appended shows: the chain ``update(cat, updated, new_features)``,
+        ``remove(cat, removed)``, ``extend(cat, appended_features)`` builds it (no other catalogue
+        operation is needed), and so does a fresh ``ingest`` of the features after the refresh.
+
+        Row r of the result is row r of ``cat``, with indices in that numbering.  Bit-identical to
+        ``top_k_device(cat, ...)`` (indices, counts and the four scores); ``changed_rows`` of the
+        result holds the sorted int32 rows to rewrite: every appended row, and every remaining row
+        that differs in any field from its previous row with the indices renumbered (every other row
+        is byte-identical to that).  Unlike ``top_k_append_device``, whose ``changed_rows`` holds old
+        rows only, the appended rows are listed too.
+
+        The incremental path (``tvbf_refresh_topk``) sweeps the updated and appended shows, and the
+        remaining shows whose previous row names a removed show, against all columns; it copies
+        every row no changed score can reach, and sweeps the rows whose lost neighbours it cannot
+        refill a second time on the tensor cores (``stats[5]`` counts them; ``stats[0]`` counts the
+        rows left to the exact kernel).  Jobs the symmetric sweep does not take (float-valued
+        groups, negative weights, k > 100, ...), catalogues with signed text and
+        ``exclude_self=False`` run the whole job and compare.  ``incremental`` of the result says
+        which of the two ran.  Rows out of range, duplicates, ``removed`` and ``updated``
+        overlapping, a ``previous`` of the wrong shape, an ``n_appended`` that does not match
+        ``cat.n_shows`` and removing every old show raise ``ValueError``."""
+        k, qa = int(k), int(n_appended)
+        if previous["indices"].dim() != 2 or previous["indices"].shape[1] != k \
+                or tuple(previous["counts"].shape) != (previous["indices"].shape[0],):
+            raise ValueError(f"previous table has shape {tuple(previous['indices'].shape)}, expected (N, {k})")
+        n_old, n = int(previous["counts"].shape[0]), cat.n_shows
+        rem = self._update_rows(removed, n_old)
+        upd = self._update_rows(updated, n_old)
+        if np.intersect1d(rem, upd).size:
+            raise ValueError("removed and updated rows overlap")
+        if rem.size == n_old:
+            raise ValueError("refresh: removing every old show leaves no catalogue to refresh")
+        if qa < 0 or n_old - rem.size + qa != n:
+            raise ValueError(f"n_appended {qa}: {n_old} previous rows - {rem.size} removed + {qa} appended "
+                             f"!= {n} shows in the catalogue")
+        if rem.size == 0 and upd.size == 0 and qa == 0:
+            return {**previous, "changed_rows": torch.zeros((0,), dtype=torch.int32, device=self.device),
+                    "incremental": True}
+        p = self._params(cat, weights, k, min_similarity)
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, k, min_similarity) if exclude_self else None
+            if feats is None:
+                # whole job, changed rows by comparison with the renumbered rows, plus the appended ones
+                t = self.top_k_device(cat, weights, k, min_similarity, exclude_self=exclude_self, out=out)
+                row_map = torch.full((n_old,), -1, dtype=torch.int64)
+                row_map[np.delete(np.arange(n_old), rem)] = torch.arange(n_old - rem.size)
+                ch = self._changed_rows(t, previous, row_map.to(self.device))
+                t["changed_rows"] = torch.cat([ch, torch.arange(n - qa, n, dtype=torch.int32, device=self.device)])
+                t["incremental"] = False
+                return t
+            nbytes = self.lib.tvbf_refresh_workspace_bytes(C.byref(feats), C.byref(p), int(rem.size), int(upd.size), qa)
+            if nbytes == 0:
+                check(-1, "tvbf_refresh_workspace_bytes")
+            ws = self._workspace(nbytes)
+            t = out if out is not None else self._alloc_tables(n, k)
+            rem_d = torch.from_numpy(rem.astype(np.int32)).to(self.device)
+            upd_d = torch.from_numpy(upd.astype(np.int32)).to(self.device)
+            changed = torch.empty((n,), dtype=torch.int32, device=self.device)
+            prev = self._c_tables({**previous, "stats": t["stats"]})
+            check(self.lib.tvbf_refresh_topk(C.byref(feats), C.byref(p), rem_d.data_ptr() if rem.size else None,
+                                             int(rem.size), upd_d.data_ptr() if upd.size else None, int(upd.size), qa,
+                                             C.byref(prev), C.byref(self._c_tables(t)), changed.data_ptr(),
+                                             ws.data_ptr(), ws.numel(), self._stream()), "tvbf_refresh_topk")
+            t["changed_rows"] = torch.nonzero(changed).flatten().to(torch.int32)
+            t["incremental"] = True
+        t["row_begin"] = 0
+        return t
+
+    def refresh_tiles(self, cat: DeviceCatalogue, n_gathered: int, n_repaired: int = 0, weights=(0.4, 0.5, 0.1),
+                      k: int = 20, min_similarity: float = 0.1) -> dict | None:
+        """Tensor-core tiles (256 x 256 x k_pad) the incremental refresh of ``top_k_refresh_device``
+        executes on the catalogue after the refresh ``cat`` (host only) when ``n_gathered`` rows are
+        updated, appended or named a removed show, and ``n_repaired`` rows go to the second sweep
+        (``stats[5]`` of the result): the threshold seed pass and the sweep of each stage, 0 for a
+        stage without rows.  None when the job runs the whole job instead."""
+        with torch.cuda.device(self.device):
+            feats = self._incremental_features(cat, weights, int(k), float(min_similarity))
+            if feats is None or not 0 <= int(n_repaired) <= cat.n_shows or not 0 <= int(n_gathered) <= cat.n_shows:
+                return None
+            if int(n_gathered) == 0:
+                return {"seed_tiles": 0, "sweep_tiles": 0, "repair_seed_tiles": 0, "repair_sweep_tiles": 0}
+            out = (C.c_int64 * 4)()
+            check(self.lib.tvbf_refresh_plan_tiles(C.byref(feats), C.byref(self._params(cat, weights, k, min_similarity)),
+                                                   int(n_gathered), int(n_repaired), out), "tvbf_refresh_plan_tiles")
+        return {"seed_tiles": int(out[0]), "sweep_tiles": int(out[1]), "repair_seed_tiles": int(out[2]),
+                "repair_sweep_tiles": int(out[3])}
+
     def top_k_sweep_device(self, cat: DeviceCatalogue, weight_list, k: int = 20, min_similarity: float = 0.1,
                            exclude_self: bool = True, shared: bool | None = None, tuning: int = 0,
                            out: list | None = None, **kw) -> list[dict]:

@@ -311,6 +311,67 @@ class SimilarityComputer:
         top.changed_rows = changed
         return top
 
+    def refresh_top_k(self, features: dict, previous: TopK, removed=(), updated=(), k: int = 20,
+                      min_similarity: float = 0.1, exclude_self: bool = True, metadata_mode: str = "mean3",
+                      normalize_weights: bool = False) -> TopK:
+        """Top-K table after a refresh of a catalogue whose table exists: the shows ``removed`` left,
+        the shows ``updated`` got new features and new shows were appended, all at once.
+
+        ``features`` is the catalogue after the refresh: the remaining shows in their old order (the
+        updated ones with their new features), then the appended shows.  ``previous`` is the
+        ``compute_top_k`` table of the catalogue before it, with the same arguments; ``removed`` and
+        ``updated`` are rows of it (distinct, disjoint).  The number of appended shows follows from
+        the shapes.  Row r of the result is row r of ``features``.  The result equals
+        ``compute_top_k(features, ...)`` bit for bit; its ``changed_rows`` lists the rows to store
+        (sorted int32): every appended row, and every remaining row that differs in any field from
+        its previous row with the indices renumbered -- every other row is identical to that.
+        Unlike ``extend_top_k``, whose ``changed_rows`` holds old rows only, the appended rows are
+        listed too.  Only the updated and appended shows, the shows whose previous row names a
+        removed show, and rows that lost a neighbour they cannot refill otherwise are scored against
+        the catalogue on the tensor cores.  Removing every old show raises ``ValueError``.
+
+        Precondition, which the library cannot check: every remaining show not in ``updated`` has
+        the features ``previous`` was computed from, and all rows are encoded in the same vocabulary
+        and widths (the already fitted extractor).  Jobs the incremental path does not take (signed
+        text, float-valued groups, k > 100, ``exclude_self=False``, ...) run the whole job and
+        compare."""
+        weights = self._normalized_weights() if normalize_weights else \
+            (self.genre_weight, self.text_weight, self.metadata_weight)
+        n_all = int(np.asarray(features["genre_features"]).shape[0])
+        n_old = int(previous.counts.shape[0])
+        if previous.indices.ndim != 2 or previous.indices.shape != (n_old, k) or previous.row_begin != 0:
+            raise ValueError(f"previous table has shape {previous.indices.shape}, expected ({n_old}, {k}) from row 0")
+        eng = self.engine
+        rem = eng._update_rows(removed, n_old)
+        upd = eng._update_rows(updated, n_old)
+        if np.intersect1d(rem, upd).size:
+            raise ValueError("removed and updated rows overlap")
+        if rem.size == n_old:
+            raise ValueError("refresh_top_k: removing every old show leaves no catalogue to refresh")
+        n_app = n_all - (n_old - int(rem.size))
+        if n_app < 0:
+            raise ValueError(f"features hold {n_all} shows, fewer than the {n_old - rem.size} remaining ones")
+        fields = ("indices", "counts", "hybrid", "genre", "text", "metadata")
+
+        if rem.size == 0 and upd.size == 0 and n_app == 0:
+            return TopK(*(getattr(previous, name) for name in fields), changed_rows=np.zeros(0, dtype=np.int32))
+        if not exclude_self:
+            row_map = np.full(n_old, -1, dtype=np.int64)
+            row_map[np.delete(np.arange(n_old), rem)] = np.arange(n_old - rem.size)
+            top = eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self)
+            top.changed_rows = np.concatenate([_changed_rows(top, previous, row_map),
+                                               np.arange(n_all - n_app, n_all, dtype=np.int32)])
+            return top
+        cat = eng.ingest(features, metadata_mode, weights)
+        with torch.cuda.device(eng.device):
+            prev = {name: torch.from_numpy(np.ascontiguousarray(getattr(previous, name))).to(eng.device)
+                    for name in fields}
+            t = eng.top_k_refresh_device(cat, prev, rem, upd, n_app, weights, k, min_similarity)
+            changed = t["changed_rows"].cpu().numpy()
+        top = eng.to_host(t)
+        top.changed_rows = changed
+        return top
+
     def compute_top_k_sweep(self, features: dict, weight_list, k: int = 20, min_similarity: float = 0.1,
                             exclude_self: bool = True, metadata_mode: str = "mean3",
                             normalize_weights: bool = False, **kw) -> list[TopK]:
