@@ -91,6 +91,11 @@ typedef struct tvbf_features {
                              /* rescoring still uses the packed records                              */
   int32_t fold_col0;
   double fold_weights[3];    /* genre / text / metadata weights baked by tvbf_prep_fold_bits         */
+  int32_t text_cols;         /* 0: text column c of the operand is vocabulary column c.  > 0: the  */
+                             /* operand carries MERGED text (tvbf_prep_csr_to_operand_mapped) in   */
+                             /* columns [0, text_cols): for non-negative text the tensor-core dot  */
+                             /* is an upper bound of the text cosine, not the cosine; only the      */
+                             /* candidate pass takes such an operand (needs text_signed == 0)       */
 } tvbf_features;
 
 /* Parameters of one top-K job: populate_database.py:85-91 (weights, top_n_per_show,
@@ -158,6 +163,25 @@ int tvbf_prep_csr_normalize(const int64_t* indptr, const double* values, int32_t
 int tvbf_prep_csr_to_operand(const int64_t* indptr, const int32_t* indices, const double* values,
                              int32_t n_rows, void* operand, int32_t k_pad, int32_t col_offset,
                              double scale, int32_t dtype, void* stream);
+/* ---- merged text operand (large vocabularies, non-negative text) ----------------------------------
+ * A merge plan maps the V vocabulary columns onto text_cols < V operand columns: the text_cols / 2
+ * columns with the most non-zeros (document frequency; ties by ascending column) keep a column of
+ * their own, the others are dealt round-robin by that rank over the remaining columns.
+ * col_map[V]: operand column of every vocabulary column; slot_ptr[text_cols + 1] / slot_cols[V]:
+ * the vocabulary columns of every operand column (CSR, in rank order).  Deterministic: the same CSR
+ * gives the same plan on every GPU.  Fails unless every operand column takes at most 4096 vocabulary
+ * columns (a merged entry of a unit row stays <= 64 before the 2^s scale, far below fp16's range). */
+size_t tvbf_merge_plan_workspace_bytes(int32_t vocab);
+int tvbf_merge_plan(const int64_t* indptr, const int32_t* indices, int32_t n_rows, int32_t vocab,
+                    int32_t text_cols, int32_t* col_map, int32_t* slot_ptr, int32_t* slot_cols,
+                    void* workspace, size_t workspace_bytes, void* stream);
+/* tvbf_prep_csr_to_operand through a merge plan: operand[r, col_offset + col_map[c]] = sum of x * scale
+ * over the row's entries that share that column, summed in fp64 in slot_cols order and rounded once
+ * (fp16 / bf16).  operand must be zero-initialised. */
+int tvbf_prep_csr_to_operand_mapped(const int64_t* indptr, const int32_t* indices, const double* values,
+                                    int32_t n_rows, const int32_t* col_map, const int32_t* slot_ptr,
+                                    const int32_t* slot_cols, void* operand, int32_t k_pad, int32_t col_offset,
+                                    double scale, int32_t dtype, void* stream);
 /* Recycling an operand buffer: store 0 at every position the CSR of the catalogue it held had set
  * (one 2-byte store per old non-zero instead of a memset of the whole n_pad x k_pad array). */
 int tvbf_prep_clear_csr_positions(const int64_t* indptr, const int32_t* indices, int32_t n_rows,

@@ -38,6 +38,7 @@ class Features(C.Structure):
         ("genre_hi", c_void_p),
         ("text_signed", c_int32),
         ("bits_folded", c_int32), ("fold_col0", c_int32), ("fold_weights", c_double * 3),
+        ("text_cols", c_int32),
     ]
 
 
@@ -72,6 +73,11 @@ SIGNATURES = {
                                            c_int32, c_double, c_int32, c_void_p]),
     "tvbf_prep_fold_bits": (C.c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32, c_int32,
                                       c_double, c_double, c_int32, c_void_p]),
+    "tvbf_merge_plan_workspace_bytes": (c_size_t, [c_int32]),
+    "tvbf_merge_plan": (C.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_size_t, c_void_p]),
+    "tvbf_prep_csr_to_operand_mapped": (C.c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
+                                                  c_void_p, c_void_p, c_int32, c_int32, c_double, c_int32, c_void_p]),
     "tvbf_prep_clear_csr_positions": (C.c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32,
                                                 c_void_p]),
     "tvbf_device_zero": (C.c_int, [c_void_p, c_size_t, c_void_p]),

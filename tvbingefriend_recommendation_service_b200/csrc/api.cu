@@ -71,10 +71,15 @@ int validate_features(const tvbf_features* f) {
                  "packed genre: genre_hi must be given exactly when there are more than 64 columns");
     if (f->genre_hi) TVBF_REQUIRE((reinterpret_cast<uintptr_t>(f->genre_hi) & 15) == 0, "genre_hi must be 16-byte aligned");
   }
+  TVBF_REQUIRE(f->text_cols >= 0 && f->text_cols <= f->vocab && f->text_cols <= f->k_pad,
+               "text_cols %d outside [0, min(vocab %d, k_pad %d)]", f->text_cols, f->vocab, f->k_pad);
+  if (f->text_cols > 0)
+    TVBF_REQUIRE(!f->text_signed, "a merged text operand (text_cols > 0) needs non-negative text");
   if (f->bits_folded) {
     TVBF_REQUIRE(f->genre_mode == TVBF_GROUP_PACKED && f->meta_mode == TVBF_GROUP_PACKED && !f->text_signed,
                  "bits_folded needs packed genre and metadata groups and non-negative text");
-    TVBF_REQUIRE(f->fold_col0 >= f->vocab && f->fold_col0 + f->genre_dim + 32 <= f->k_pad,
+    const int text_end = f->text_cols > 0 ? f->text_cols : f->vocab;
+    TVBF_REQUIRE(f->fold_col0 >= text_end && f->fold_col0 + f->genre_dim + 32 <= f->k_pad,
                  "bits_folded: columns [%d, %d) do not fit k_pad %d", f->fold_col0, f->fold_col0 + f->genre_dim + 32,
                  f->k_pad);
     TVBF_REQUIRE(f->fold_weights[1] > 0.0 && f->fold_weights[0] >= 0.0 && f->fold_weights[2] >= 0.0,
@@ -252,6 +257,11 @@ Slack make_slack(const tvbf_features* f, double wg, double wt, double wm, double
     // the whole accumulator): largest operand magnitude relative to a text entry (<= 1)
     op_max = std::fmax(op_max, std::sqrt(std::fabs(wg) / wt));
     op_max = std::fmax(op_max, std::sqrt(std::fabs(wm) / wt));
+  }
+  if (f->text_cols > 0) {
+    // merged text: an entry sums at most vocab - text_cols + 1 entries of a unit row, so it is at most
+    // the square root of that (Cauchy-Schwarz); only the subnormal term needs the largest operand
+    op_max = std::fmax(op_max, std::sqrt(static_cast<double>(f->vocab - f->text_cols + 1)));
   }
   const double wsum = std::fabs(wg) + std::fabs(wt) + std::fabs(wm);
   const double eps0 = 4e-6 * (wsum + 1.0);   // fp32 rounding of the epilogue's four FMAs
@@ -2008,6 +2018,7 @@ int tvbf_similarity_stats(const tvbf_features* f, const tvbf_params* p, void* ac
   TVBF_REQUIRE(f->genre_mode != TVBF_GROUP_FOLDED && f->meta_mode != TVBF_GROUP_FOLDED && f->genre_hi == nullptr,
                "streaming statistics need binary genre (at most 64 columns) / one-hot metadata features");
   TVBF_REQUIRE(!f->bits_folded, "streaming statistics need the plain text operand (bits_folded is set)");
+  TVBF_REQUIRE(f->text_cols == 0, "streaming statistics need the plain text operand (text_cols is set)");
   TVBF_REQUIRE(p->genre_weight >= 0.0 && p->text_weight >= 0.0 && p->metadata_weight >= 0.0,
                "streaming statistics need non-negative weights");
   tvbf_params q = *p;

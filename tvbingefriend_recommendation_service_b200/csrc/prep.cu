@@ -6,6 +6,8 @@
 // instead of five times per source show, plus the packing of the binary groups.
 #include "common.cuh"
 
+#include <cub/device/device_radix_sort.cuh>
+
 namespace {
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -53,6 +55,91 @@ __global__ void csr_to_operand_kernel(const int64_t* __restrict__ indptr,
   int64_t b = indptr[row], e = indptr[row + 1];
   T* dst = operand + static_cast<size_t>(row) * k_pad + col_offset;
   for (int64_t i = b + lane; i < e; i += 32) dst[indices[i]] = cvt_operand<T>(values[i] * scale);
+}
+
+// Merged text (tvbf_prep_csr_to_operand_mapped): one warp per row, one lane per entry.  An entry
+// finds the row's other entries of its operand column by binary search for every vocabulary column of
+// that slot (a handful, in slot_cols order); the lane of the first one present stores the fp64 sum,
+// rounded once, and the others store nothing -- no atomics, the same bits on every run.
+template <typename T>
+__global__ void csr_to_operand_mapped_kernel(const int64_t* __restrict__ indptr,
+                                             const int32_t* __restrict__ indices,
+                                             const double* __restrict__ values, int n_rows,
+                                             const int32_t* __restrict__ col_map,
+                                             const int32_t* __restrict__ slot_ptr,
+                                             const int32_t* __restrict__ slot_cols,
+                                             T* __restrict__ operand, int k_pad, int col_offset, double scale) {
+  int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;
+  const int64_t b = indptr[row], e = indptr[row + 1];
+  T* dst = operand + static_cast<size_t>(row) * k_pad + col_offset;
+  for (int64_t i = b + lane; i < e; i += 32) {
+    const int c = indices[i];
+    const int s = col_map[c];
+    const int p0 = slot_ptr[s], p1 = slot_ptr[s + 1];
+    if (p1 - p0 == 1) {
+      dst[s] = cvt_operand<T>(values[i] * scale);
+      continue;
+    }
+    double sum = 0.0;
+    int owner = -1;
+    for (int p = p0; p < p1; ++p) {
+      const int c2 = slot_cols[p];
+      int64_t lo = b, hi = e;          // first position in [b, e) whose column is >= c2
+      while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (indices[mid] < c2) lo = mid + 1; else hi = mid;
+      }
+      if (lo < e && indices[lo] == c2) {
+        if (owner < 0) owner = c2;
+        sum += values[lo];
+      }
+    }
+    if (owner == c) dst[s] = cvt_operand<T>(sum * scale);
+  }
+}
+
+// document frequency of every vocabulary column: an integer histogram of the CSR's column indices
+__global__ void column_df_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
+                                 int n_rows, int vocab, int32_t* __restrict__ df) {
+  const int64_t nnz = indptr[n_rows];
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < nnz;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int c = indices[i];
+    if (c >= 0 && c < vocab) atomicAdd(df + c, 1);
+  }
+}
+
+__global__ void iota_kernel(int32_t* __restrict__ out, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = i;
+}
+
+// order[r] = vocabulary column of rank r (descending frequency).  Ranks below head keep their own
+// operand column r; rank r >= head goes to head + (r - head) % tail, so slot head + t holds the ranks
+// head + t + j * tail, j = 0, 1, ...: q + 1 of them for t < rem, q for the others.
+__global__ void merge_plan_fill_kernel(const int32_t* __restrict__ order, int vocab, int text_cols,
+                                       int32_t* __restrict__ col_map, int32_t* __restrict__ slot_ptr,
+                                       int32_t* __restrict__ slot_cols) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int head = text_cols / 2, tail = text_cols - head;
+  const int q = (vocab - head) / tail, rem = (vocab - head) % tail;
+  if (i < vocab) {
+    const int c = order[i];
+    if (i < head) {
+      col_map[c] = i;
+      slot_cols[i] = c;
+    } else {
+      const int t = (i - head) % tail, j = (i - head) / tail;
+      col_map[c] = head + t;
+      slot_cols[head + t * q + min(t, rem) + j] = c;
+    }
+  }
+  if (i <= text_cols) {
+    const int t = i - head;
+    slot_ptr[i] = i <= head ? i : (i == text_cols ? vocab : head + t * q + min(t, rem));
+  }
 }
 
 // un-scatter: zero the operand entries a previous catalogue's CSR had set (recycling an operand
@@ -354,6 +441,90 @@ int tvbf_prep_csr_to_operand(const int64_t* indptr, const int32_t* indices, cons
         indptr, indices, values, n_rows, static_cast<__nv_bfloat16*>(operand), k_pad, col_offset,
         scale);
   TVBF_LAUNCH_OK("csr_to_operand_kernel");
+  return TVBF_OK;
+}
+
+namespace {
+struct MergeWs {
+  size_t df, keys, iota, order, cub, cub_bytes, total;
+};
+MergeWs merge_ws(int vocab) {
+  MergeWs w;
+  const size_t v = static_cast<size_t>(vocab) * 4, a = (v + 255) / 256 * 256;
+  w.df = 0;
+  w.keys = a;
+  w.iota = 2 * a;
+  w.order = 3 * a;
+  w.cub = 4 * a;
+  w.cub_bytes = 0;
+  cub::DeviceRadixSort::SortPairsDescending(nullptr, w.cub_bytes, static_cast<const int32_t*>(nullptr),
+                                            static_cast<int32_t*>(nullptr), static_cast<const int32_t*>(nullptr),
+                                            static_cast<int32_t*>(nullptr), vocab);
+  w.total = w.cub + w.cub_bytes;
+  return w;
+}
+}  // namespace
+
+size_t tvbf_merge_plan_workspace_bytes(int32_t vocab) { return vocab > 0 ? merge_ws(vocab).total : 0; }
+
+int tvbf_merge_plan(const int64_t* indptr, const int32_t* indices, int32_t n_rows, int32_t vocab,
+                    int32_t text_cols, int32_t* col_map, int32_t* slot_ptr, int32_t* slot_cols,
+                    void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_REQUIRE(indptr && indices && col_map && slot_ptr && slot_cols && workspace && n_rows >= 0 && vocab > 0,
+               "tvbf_merge_plan: bad arguments");
+  TVBF_REQUIRE(text_cols >= 2 && text_cols <= vocab, "tvbf_merge_plan: text_cols %d outside [2, %d]", text_cols, vocab);
+  {
+    const int head = text_cols / 2, tail = text_cols - head;
+    const int most = (vocab - head + tail - 1) / tail;
+    TVBF_REQUIRE(most <= 4096, "tvbf_merge_plan: %d vocabulary columns per operand column (at most 4096)", most);
+  }
+  TVBF_ENTER_CALL(stream);   // after the argument checks, which touch no device
+  const MergeWs w = merge_ws(vocab);
+  TVBF_REQUIRE(workspace_bytes >= w.total, "tvbf_merge_plan: workspace of %zu bytes, needs %zu", workspace_bytes,
+               w.total);
+  auto st = static_cast<cudaStream_t>(stream);
+  auto* ws = static_cast<uint8_t*>(workspace);
+  auto* df = reinterpret_cast<int32_t*>(ws + w.df);
+  auto* keys = reinterpret_cast<int32_t*>(ws + w.keys);
+  auto* iota = reinterpret_cast<int32_t*>(ws + w.iota);
+  auto* order = reinterpret_cast<int32_t*>(ws + w.order);
+  TVBF_CUDA_OK(cudaMemsetAsync(df, 0, static_cast<size_t>(vocab) * 4, st));
+  column_df_kernel<<<296, 512, 0, st>>>(indptr, indices, n_rows, vocab, df);
+  TVBF_LAUNCH_OK("column_df_kernel");
+  iota_kernel<<<blocks_for(vocab, 256), 256, 0, st>>>(iota, vocab);
+  TVBF_LAUNCH_OK("iota_kernel");
+  // stable: equal frequencies keep the ascending column order of iota
+  size_t cub_bytes = w.cub_bytes;
+  TVBF_CUDA_OK(cub::DeviceRadixSort::SortPairsDescending(ws + w.cub, cub_bytes, df, keys, iota, order, vocab, 0, 32,
+                                                         st));
+  tvbf_count_launch();   // the sort's kernels count as one launch
+  merge_plan_fill_kernel<<<blocks_for(static_cast<size_t>(vocab) + 1, 256), 256, 0, st>>>(
+      order, vocab, text_cols, col_map, slot_ptr, slot_cols);
+  TVBF_LAUNCH_OK("merge_plan_fill_kernel");
+  return TVBF_OK;
+}
+
+int tvbf_prep_csr_to_operand_mapped(const int64_t* indptr, const int32_t* indices, const double* values,
+                                    int32_t n_rows, const int32_t* col_map, const int32_t* slot_ptr,
+                                    const int32_t* slot_cols, void* operand, int32_t k_pad, int32_t col_offset,
+                                    double scale, int32_t dtype, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  TVBF_REQUIRE(indptr && operand && col_map && slot_ptr && slot_cols && n_rows >= 0 && k_pad > 0 && col_offset >= 0,
+               "tvbf_prep_csr_to_operand_mapped: bad arguments");
+  TVBF_REQUIRE(dtype == TVBF_TEXT_FP16 || dtype == TVBF_TEXT_BF16,
+               "tvbf_prep_csr_to_operand_mapped: dtype must be TVBF_TEXT_FP16 or TVBF_TEXT_BF16");
+  if (n_rows == 0) return TVBF_OK;
+  auto st = static_cast<cudaStream_t>(stream);
+  unsigned grid = blocks_for(static_cast<size_t>(n_rows) * 32, 256);
+  if (dtype == TVBF_TEXT_FP16)
+    csr_to_operand_mapped_kernel<__half><<<grid, 256, 0, st>>>(indptr, indices, values, n_rows, col_map, slot_ptr,
+                                                               slot_cols, static_cast<__half*>(operand), k_pad,
+                                                               col_offset, scale);
+  else
+    csr_to_operand_mapped_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(
+        indptr, indices, values, n_rows, col_map, slot_ptr, slot_cols, static_cast<__nv_bfloat16*>(operand), k_pad,
+        col_offset, scale);
+  TVBF_LAUNCH_OK("csr_to_operand_mapped_kernel");
   return TVBF_OK;
 }
 

@@ -115,6 +115,25 @@ def stage(features: dict, metadata_mode: str = "mean3", pin: bool = True) -> Sta
         text_signed=bool(text.nnz and text.data.min() < 0.0))
 
 
+def merge_text_cols(vocab: int, genre_dim: int, fold_max_k: int = 4096, ratio: float = 0.4) -> int:
+    """Text columns of the candidate pass' second operand for a vocabulary of ``vocab`` columns and
+    ``genre_dim`` packed genre columns (``HybridTopKEngine.fold_max_k`` / ``merge_ratio``).  ``vocab``
+    -- no merge -- while the text and the packed groups fit the fold limit (``vocab + genre_dim + 32
+    <= fold_max_k``), when ``ratio`` or ``fold_max_k`` is 0, or when merging would not narrow the
+    64-column padded operand; else ``max(fold_max_k - genre_dim - 32, ceil(ratio * vocab))``, so that
+    the merged text and the packed groups still fit the fold limit.  Depends on shapes only, so the
+    host never waits for the device to choose it."""
+    v, lim = int(vocab), int(fold_max_k)
+    if ratio <= 0.0 or lim <= 0 or v + genre_dim + 32 <= lim:
+        return v
+    kt = max(lim - genre_dim - 32, int(np.ceil(ratio * v)), 2)
+    head = kt // 2
+    # tvbf_merge_plan takes at most 4096 vocabulary columns per operand column
+    if (kt + 63) // 64 >= (v + 63) // 64 or -(-(v - head) // (kt - head)) > 4096:
+        return v
+    return kt
+
+
 @dataclass
 class DeviceCatalogue:
     """Prepared, device-resident features (``tvbf_features``) and the tensors that back it."""
@@ -127,7 +146,7 @@ class DeviceCatalogue:
     operand: torch.Tensor | None = None    # [n_pad, k_pad] fp16 / bf16
     text_indptr: torch.Tensor | None = None
     text_indices: torch.Tensor | None = None
-    fold: dict | None = None               # second operand with the packed groups as K columns (engine._folded)
+    fold: dict | None = None               # second operand of the candidate pass: merged text and / or the packed groups (engine._folded)
     buffers: dict = field(default_factory=dict)   # named per-catalogue device buffers a later catalogue can take over
     h2d_set: tuple | None = None           # (h2d buffer set, its write stamp) when the CSR lives in an h2d(reuse=True) set
     parts: dict = field(default_factory=dict)     # the tensors behind ``c`` by name and the text nnz (``extend``)
@@ -227,6 +246,12 @@ class HybridTopKEngine:
         # 1 000 7.9 / 6.0, 1 900 9.4 / 7.9, 3 000 12.2 / 11.5, 4 500 17.2 / 16.9 -- the gain fades as the
         # MMAs take over; the folded bound is slightly looser (3-5 % more rows go to the exact kernel).
         self.fold_max_k = int(os.environ.get("TVBF_FOLD_MAX_K", "4096"))
+        # Large vocabularies: the candidate pass is bound by its MMAs over an operand that is 99.5 %
+        # zeros.  For non-negative text it only needs an upper bound of the text cosine, and summing
+        # vocabulary columns gives one (x_i . x_j <= merged x_i . merged x_j), so the second operand
+        # carries the text merged into merge_text_cols(V, G, ...) columns (DESIGN.md section 14).  0 disables
+        # (TVBF_MERGE_RATIO overrides); fold_max_k = 0 disables it too.
+        self.merge_ratio = float(os.environ.get("TVBF_MERGE_RATIO", "0.4"))
         self._fold_buf: torch.Tensor | None = None
         self._fold_owner: dict | None = None      # the catalogue fold whose content the buffer holds
         self._theta: torch.Tensor | None = None    # seeded thresholds of the tile-sharded job (valid until the next job)
@@ -577,51 +602,107 @@ class HybridTopKEngine:
               "tvbf_prep_csr_to_operand")
         return values, operand
 
+    def _second_layout(self, cat: DeviceCatalogue, gw: float, tw: float, mw: float, k: int, tuning: int = 0,
+                       candidates: int = 0) -> tuple[int, bool] | None:
+        """(text columns, packed groups folded) of the operand the candidate pass of this job runs on
+        instead of the catalogue's, or None for the catalogue's own operand (host only)."""
+        c = cat.c
+        if cat.folded or c.text_signed or self.text_dtype != "fp16" or cat.operand is None:
+            return None
+        g_dim = int(c.genre_dim)
+        kt = merge_text_cols(int(c.vocab), g_dim, self.fold_max_k, self.merge_ratio)
+        # the folded kernels exist for CTA pairs and up to 64 candidates per list
+        bits = ((kt + g_dim + 32 + 63) // 64 * 64 <= self.fold_max_k and k <= 48
+                and (tuning & 0xF) != 1 and candidates <= 64
+                and c.genre_mode == _lib.GROUP_PACKED and c.meta_mode == _lib.GROUP_PACKED
+                and tw > 0.0 and gw >= 0.0 and mw >= 0.0
+                and all(w == 0.0 or 1e-8 <= w / tw <= 1e4 for w in (gw, mw)))   # columns stay normal fp16 numbers
+        if bits:
+            return kt, True
+        if kt < int(c.vocab) and tw >= 0.0:
+            return kt, False
+        return None
+
+    def _merge_plan(self, cat: DeviceCatalogue, text_cols: int) -> dict:
+        """``tvbf_merge_plan`` of ``cat``'s text CSR onto ``text_cols`` columns (device tensors)."""
+        lib, dev, c = self.lib, self.device, cat.c
+        v = int(c.vocab)
+        plan = {"col_map": torch.empty((v,), dtype=torch.int32, device=dev),
+                "slot_ptr": torch.empty((text_cols + 1,), dtype=torch.int32, device=dev),
+                "slot_cols": torch.empty((v,), dtype=torch.int32, device=dev)}
+        ws = torch.empty((int(lib.tvbf_merge_plan_workspace_bytes(v)),), dtype=torch.uint8, device=dev)
+        check(lib.tvbf_merge_plan(c.text_indptr, c.text_indices, cat.n_shows, v, text_cols,
+                                  plan["col_map"].data_ptr(), plan["slot_ptr"].data_ptr(), plan["slot_cols"].data_ptr(),
+                                  ws.data_ptr(), ws.numel(), self._stream()), "tvbf_merge_plan")
+        return plan
+
+    def _second_rows(self, fc: dict, indptr: int, indices: int, values: int, n_rows: int, dst: int,
+                     col_side: int, genre_hi: int | None, meta_scale: int) -> None:
+        """Write ``n_rows`` shows into the zeroed rows at ``dst`` of the second operand ``fc``: their
+        text (through the merge plan when it has one) and, once the weights are set, their packed
+        groups."""
+        lib, stream = self.lib, self._stream()
+        f = fc["c"]
+        code, _ = _DTYPES[self.text_dtype]
+        k2, scale = int(f.k_pad), float(2 ** TEXT_SCALE_LOG2)
+        plan = fc["plan"]
+        if plan is None:
+            check(lib.tvbf_prep_csr_to_operand(indptr, indices, values, n_rows, dst, k2, 0, scale, code, stream),
+                  "tvbf_prep_csr_to_operand")
+        else:
+            check(lib.tvbf_prep_csr_to_operand_mapped(indptr, indices, values, n_rows, plan["col_map"].data_ptr(),
+                                                      plan["slot_ptr"].data_ptr(), plan["slot_cols"].data_ptr(), dst,
+                                                      k2, 0, scale, code, stream), "tvbf_prep_csr_to_operand_mapped")
+        if fc["weights"] is not None:
+            gw, tw, mw = fc["weights"]
+            check(lib.tvbf_prep_fold_bits(col_side, genre_hi, meta_scale, n_rows, int(f.genre_dim), dst, k2,
+                                          int(f.fold_col0), scale * float(np.sqrt(gw / tw)),
+                                          scale * float(np.sqrt(mw / tw)), code, stream), "tvbf_prep_fold_bits")
+
     def _folded(self, cat: DeviceCatalogue, gw: float, tw: float, mw: float, k: int, tuning: int = 0,
                 candidates: int = 0) -> Features | None:
-        """``tvbf_features`` of ``cat`` over a second operand that carries the packed genre / metadata
-        groups as K columns for these weights, or None when the job does not qualify (the folded
-        kernels exist for CTA pairs and up to 64 candidates per list)."""
-        c = cat.c
-        g_dim = int(c.genre_dim)
-        k_fold = (int(c.vocab) + g_dim + 32 + 63) // 64 * 64
-        ok = (self.fold_max_k > 0 and k_fold <= self.fold_max_k and k <= 48 and not cat.folded
-              and (tuning & 0xF) != 1 and candidates <= 64
-              and c.genre_mode == _lib.GROUP_PACKED and c.meta_mode == _lib.GROUP_PACKED and not c.text_signed
-              and self.text_dtype == "fp16" and tw > 0.0 and gw >= 0.0 and mw >= 0.0
-              and all(w == 0.0 or 1e-8 <= w / tw <= 1e4 for w in (gw, mw)))   # columns stay normal fp16 numbers
-        if not ok or cat.operand is None:
+        """``tvbf_features`` of ``cat`` over the engine's second operand, or None when the job runs on
+        the catalogue's own operand.  The second operand carries the text -- merged into fewer
+        columns for large vocabularies (``merge_text_cols``) -- and, when the job qualifies, the
+        packed genre / metadata groups as K columns for these weights (``_second_layout``)."""
+        layout = self._second_layout(cat, gw, tw, mw, k, tuning, candidates)
+        if layout is None:
             return None
-        lib, stream = self.lib, self._stream()
-        code, tdt = _DTYPES[self.text_dtype]
-        scale = float(2 ** TEXT_SCALE_LOG2)
+        text_cols, bits = layout
+        c = cat.c
         fc = cat.fold
+        if fc is not None and (self._fold_owner is not fc or fc["layout"] != layout):
+            fc = cat.fold = None                # the engine's buffer went to another catalogue or layout since
         if fc is None:
             n_pad = int(c.n_pad)
+            k2 = (text_cols + (int(c.genre_dim) + 32 if bits else 0) + 63) // 64 * 64
+            _, tdt = _DTYPES[self.text_dtype]
             buf = self._fold_buf
-            if buf is None or tuple(buf.shape) != (n_pad, k_fold) or buf.dtype != tdt:
+            if buf is None or tuple(buf.shape) != (n_pad, k2) or buf.dtype != tdt:
                 self._fold_buf = None
-                buf = torch.empty((n_pad, k_fold), dtype=tdt, device=self.device)
+                buf = torch.empty((n_pad, k2), dtype=tdt, device=self.device)
                 self._fold_buf = buf            # one buffer per engine, reused by the next catalogue of this shape
             self._zero(buf)
-            check(lib.tvbf_prep_csr_to_operand(c.text_indptr, c.text_indices, c.text_values, cat.n_shows,
-                                               buf.data_ptr(), k_fold, 0, scale, code, stream),
-                  "tvbf_prep_csr_to_operand")
+            merged = text_cols < int(c.vocab)
             f = Features.from_buffer_copy(c)
-            f.operand, f.k_pad = buf.data_ptr(), k_fold
-            f.bits_folded, f.fold_col0 = 1, int(c.vocab)
-            fc = cat.fold = {"c": f, "operand": buf, "weights": None}
+            f.operand, f.k_pad = buf.data_ptr(), k2
+            f.text_cols = text_cols if merged else 0
+            f.bits_folded, f.fold_col0 = int(bits), text_cols if bits else 0
+            fc = cat.fold = {"c": f, "operand": buf, "weights": None, "layout": layout,
+                             "plan": self._merge_plan(cat, text_cols) if merged else None}
             self._fold_owner = fc
-        elif self._fold_owner is not fc:
-            cat.fold = None                     # the engine's buffer went to another catalogue since
-            return self._folded(cat, gw, tw, mw, k, tuning, candidates)
-        if fc["weights"] != (gw, tw, mw):
+            self._second_rows(fc, c.text_indptr, c.text_indices, c.text_values, cat.n_shows, buf.data_ptr(),
+                              c.col_side, c.genre_hi, c.meta_scale)
+        if bits and fc["weights"] != (gw, tw, mw):
             f = fc["c"]
-            check(lib.tvbf_prep_fold_bits(c.col_side, c.genre_hi, c.meta_scale, cat.n_shows, g_dim, f.operand, k_fold,
-                                          int(c.vocab), scale * float(np.sqrt(gw / tw)), scale * float(np.sqrt(mw / tw)),
-                                          code, stream), "tvbf_prep_fold_bits")
-            f.fold_weights[0], f.fold_weights[1], f.fold_weights[2] = gw, tw, mw
             fc["weights"] = (gw, tw, mw)
+            f.fold_weights[0], f.fold_weights[1], f.fold_weights[2] = gw, tw, mw
+            code, _ = _DTYPES[self.text_dtype]
+            scale = float(2 ** TEXT_SCALE_LOG2)
+            check(self.lib.tvbf_prep_fold_bits(c.col_side, c.genre_hi, c.meta_scale, cat.n_shows, int(c.genre_dim),
+                                               f.operand, int(f.k_pad), int(f.fold_col0),
+                                               scale * float(np.sqrt(gw / tw)), scale * float(np.sqrt(mw / tw)),
+                                               code, self._stream()), "tvbf_prep_fold_bits")
         return fc["c"]
 
     # ------------------------------------------------------------------------------------ top-k
@@ -714,8 +795,7 @@ class HybridTopKEngine:
         nc = new.c
         n_old, q = cat.n_shows, new.n_shows
         n = n_old + q
-        dev, lib, stream = self.device, self.lib, self._stream()
-        code, _ = _DTYPES[self.text_dtype]
+        dev = self.device
         p_old, p_new = cat.parts, new.parts
         with torch.cuda.device(dev):
             n_pad = int(c.n_pad)
@@ -769,26 +849,18 @@ class HybridTopKEngine:
                        "meta_widths": p_old["meta_widths"]})
             fc = cat.fold
             if fc is not None and self._fold_owner is fc and not grow and not f.text_signed:
-                # the second operand (small vocabularies): write the new rows' text and group columns
+                # the second operand: write the new rows' text (through the catalogue's merge plan)
+                # and group columns
                 ff = Features.from_buffer_copy(fc["c"])
-                k_fold, buf = int(ff.k_pad), fc["operand"]
-                row0 = buf[n_old:].data_ptr()
-                scale = float(2 ** TEXT_SCALE_LOG2)
-                check(lib.tvbf_prep_csr_to_operand(new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
-                                                   p_new["values"].data_ptr(), q, row0, k_fold, 0, scale, code, stream),
-                      "tvbf_prep_csr_to_operand")
-                if fc["weights"] is not None:
-                    gw, tw, mw = fc["weights"]
-                    check(lib.tvbf_prep_fold_bits(col_side[n_old:].data_ptr(),
-                                                  None if genre_hi is None else genre_hi[n_old:].data_ptr(),
-                                                  meta_scale[n_old:].data_ptr(), q, int(c.genre_dim), row0, k_fold,
-                                                  int(c.vocab), scale * float(np.sqrt(gw / tw)),
-                                                  scale * float(np.sqrt(mw / tw)), code, stream),
-                          "tvbf_prep_fold_bits")
+                buf = fc["operand"]
+                self._second_rows(fc, new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
+                                  p_new["values"].data_ptr(), q, buf[n_old:].data_ptr(), col_side[n_old:].data_ptr(),
+                                  None if genre_hi is None else genre_hi[n_old:].data_ptr(),
+                                  meta_scale[n_old:].data_ptr())
                 for name in ("n_shows", "text_indptr", "text_indices", "text_values", "col_side", "meta_scale",
                              "genre_hi"):
                     setattr(ff, name, getattr(f, name))
-                grown.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+                grown.fold = self._fold_owner = {**fc, "c": ff}
             grown.keep.append(new)          # the new rows' tensors stay alive while the grown catalogue uses them
         cat.operand = None                  # consumed: its buffers now belong to the grown catalogue
         cat.c.operand = None
@@ -937,8 +1009,7 @@ class HybridTopKEngine:
         new = self._ingest_like(cat, new_features, "update")
         nc = new.c
         n = cat.n_shows
-        dev, lib, stream = self.device, self.lib, self._stream()
-        code, _ = _DTYPES[self.text_dtype]
+        dev = self.device
         p_old, p_new = cat.parts, new.parts
         with torch.cuda.device(dev):
             idx = torch.from_numpy(r).to(dev)
@@ -986,26 +1057,19 @@ class HybridTopKEngine:
                                   text_indptr=indptr, text_indices=indices, buffers=buffers, parts=parts)
             fc = cat.fold
             if fc is not None and self._fold_owner is fc and not f.text_signed:
-                # the second operand (small vocabularies): rebuild the updated rows and write them over
+                # the second operand: rebuild the updated rows (through the catalogue's merge plan) and
+                # write them over
                 ff = Features.from_buffer_copy(fc["c"])
-                k_fold, buf = int(ff.k_pad), fc["operand"]
-                rows_fold = torch.zeros((q, k_fold), dtype=buf.dtype, device=dev)
-                scale = float(2 ** TEXT_SCALE_LOG2)
-                check(lib.tvbf_prep_csr_to_operand(new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
-                                                   p_new["values"].data_ptr(), q, rows_fold.data_ptr(), k_fold, 0,
-                                                   scale, code, stream), "tvbf_prep_csr_to_operand")
-                if fc["weights"] is not None:
-                    gw, tw, mw = fc["weights"]
-                    check(lib.tvbf_prep_fold_bits(p_new["col_side"].data_ptr(),
-                                                  None if p_new["genre_hi"] is None else p_new["genre_hi"].data_ptr(),
-                                                  p_new["meta_scale"].data_ptr(), q, int(c.genre_dim),
-                                                  rows_fold.data_ptr(), k_fold, int(c.vocab),
-                                                  scale * float(np.sqrt(gw / tw)), scale * float(np.sqrt(mw / tw)),
-                                                  code, stream), "tvbf_prep_fold_bits")
+                buf = fc["operand"]
+                rows_fold = torch.zeros((q, int(ff.k_pad)), dtype=buf.dtype, device=dev)
+                self._second_rows(fc, new.text_indptr.data_ptr(), new.text_indices.data_ptr(),
+                                  p_new["values"].data_ptr(), q, rows_fold.data_ptr(), p_new["col_side"].data_ptr(),
+                                  None if p_new["genre_hi"] is None else p_new["genre_hi"].data_ptr(),
+                                  p_new["meta_scale"].data_ptr())
                 buf.index_copy_(0, idx, rows_fold)
                 for name in ("text_indptr", "text_indices", "text_values"):
                     setattr(ff, name, getattr(f, name))
-                upd.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+                upd.fold = self._fold_owner = {**fc, "c": ff}
         cat.operand = None                  # consumed: its buffers now belong to the updated catalogue
         cat.c.operand = None
         cat.keep.clear()
@@ -1153,13 +1217,13 @@ class HybridTopKEngine:
                                   buffers=buffers if cat.buffers else {}, parts=parts)
             fc = cat.fold
             if fc is not None and self._fold_owner is fc and not f.text_signed:
-                # the second operand (small vocabularies): its rows move with the shows
+                # the second operand: its rows move with the shows
                 buf = compact(fc["operand"])
                 ff = Features.from_buffer_copy(fc["c"])
                 ff.n_shows, ff.n_pad, ff.operand = m, n_pad, buf.data_ptr()
                 for name in ("text_indptr", "text_indices", "text_values", "col_side", "meta_scale", "genre_hi"):
                     setattr(ff, name, getattr(f, name))
-                rem.fold = self._fold_owner = {"c": ff, "operand": buf, "weights": fc["weights"]}
+                rem.fold = self._fold_owner = {**fc, "c": ff, "operand": buf}
         cat.operand = None                  # consumed: its buffers now belong to the compacted catalogue
         cat.c.operand = None
         cat.keep.clear()
@@ -1783,20 +1847,23 @@ class HybridTopKEngine:
                    tile_sharded: bool = False, row_begin: int = 0, row_end: int | None = None, splits: int = 0,
                    tuning: int = 0) -> dict:
         """Tensor-core tiles the candidate pass of this job executes (``tvbf_plan_tiles``, host only).
-        A job that runs over the folded operand is planned over it (k_pad)."""
+        A job that runs over the second operand (``_folded``) is planned over it (k_pad)."""
         p = self._params(cat, weights, k, min_similarity, row_begin=row_begin, row_end=row_end, splits=splits,
                          tuning=tuning)
         out = (C.c_int64 * 4)()
         feats = cat.c
-        if cat.fold is not None and cat.fold["weights"] == tuple(float(w) for w in weights) \
-                and self._fold_owner is cat.fold and (int(tuning) & 0xF) != 1 and int(k) <= 48:
-            feats = cat.fold["c"]
+        w = tuple(float(x) for x in weights)
+        layout = self._second_layout(cat, *w, int(k), int(tuning))
+        fc = cat.fold
+        if layout is not None and fc is not None and self._fold_owner is fc and fc["layout"] == layout \
+                and (not layout[1] or fc["weights"] == w):
+            feats = fc["c"]
         with torch.cuda.device(self.device):
             check(self.lib.tvbf_plan_tiles(C.byref(feats), C.byref(p), int(rank), int(world), int(bool(tile_sharded)),
                                            out), "tvbf_plan_tiles")
         seed, sweep, rows, sym = (int(x) for x in out)
         return {"seed_tiles": seed, "sweep_tiles": sweep, "tile_rows": rows, "symmetric": bool(sym),
-                "k_pad": int(feats.k_pad), "folded_bits": bool(feats.bits_folded),
+                "k_pad": int(feats.k_pad), "folded_bits": bool(feats.bits_folded), "text_cols": int(feats.text_cols),
                 "flops": 2.0 * (seed + sweep) * rows * 256 * int(feats.k_pad)}
 
     def debug_slack(self, cat: DeviceCatalogue, weights, feats: Features | None = None) -> dict:
