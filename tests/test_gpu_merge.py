@@ -52,18 +52,88 @@ def _merged_cols(engine):
     return None if fc is None else int(fc["c"].text_cols)
 
 
-@pytest.mark.parametrize("vocab", [6000, 10_000])
-def test_device_plan_is_the_numpy_model(engine, vocab):
+def _plan_of_csr(engine, text, kt):
+    """tvbf_merge_plan called directly on the C ABI over a host CSR"""
+    import torch
+
+    dev, vocab = engine.device, text.shape[1]
+    indptr = torch.from_numpy(text.indptr.astype(np.int64)).to(dev)
+    indices = torch.from_numpy(np.r_[text.indices, 0].astype(np.int32)).to(dev)   # non-NULL when empty
+    plan = {"col_map": torch.empty((vocab,), dtype=torch.int32, device=dev),
+            "slot_ptr": torch.empty((kt + 1,), dtype=torch.int32, device=dev),
+            "slot_cols": torch.empty((vocab,), dtype=torch.int32, device=dev)}
+    lib = engine.lib
+    ws = torch.empty((int(lib.tvbf_merge_plan_workspace_bytes(vocab)),), dtype=torch.uint8, device=dev)
+    rc = lib.tvbf_merge_plan(indptr.data_ptr(), indices.data_ptr(), text.shape[0], vocab, kt,
+                             plan["col_map"].data_ptr(), plan["slot_ptr"].data_ptr(), plan["slot_cols"].data_ptr(),
+                             ws.data_ptr(), ws.numel(), engine._stream())
+    assert rc == 0, lib.tvbf_last_error().decode()
+    return plan
+
+
+# (vocab, text_cols, text): text "catalogue" is the synthetic one, "first_3000" uses only the first
+# 3 000 columns (the others have no document: ascending index), "each_once" every column exactly once
+# (all frequencies equal: the stable sort keeps index order), "empty" no entries at all
+PLAN_CASES = [
+    pytest.param(6000, None, "catalogue", id="6000"),
+    pytest.param(10_000, None, "catalogue", id="10000"),
+    pytest.param(50_000, 20_000, "catalogue", id="50000_rem0"),          # head 10 000, 4 columns per tail slot
+    pytest.param(8000, 4000, "catalogue", id="8000_rem0"),
+    pytest.param(10_000, 3001, "catalogue", id="odd_3001"),              # head 1 500, tail 1 501
+    pytest.param(4097, 2, "catalogue", id="4097_one_slot_of_4096"),
+    pytest.param(10_000, 4024, "first_3000", id="first_3000_of_10000"),
+    pytest.param(10_000, 4024, "each_once", id="every_column_once"),
+    pytest.param(10_000, 4024, "empty", id="no_text"),
+]
+
+
+@pytest.mark.parametrize("vocab,text_cols,text", PLAN_CASES)
+def test_device_plan_is_the_numpy_model(engine, vocab, text_cols, text):
     from tvbingefriend_recommendation_service_b200.engine import merge_text_cols
 
-    f = _catalogue(3000, vocab, seed=vocab)
-    cat = engine.ingest(f)
-    kt = merge_text_cols(vocab, 40)
-    plan = engine._merge_plan(cat, kt)
-    col_map, slot_ptr, slot_cols = model_plan(f["text_features"].indices, vocab, kt)
-    assert np.array_equal(plan["col_map"].cpu().numpy(), col_map)
-    assert np.array_equal(plan["slot_ptr"].cpu().numpy(), slot_ptr)
-    assert np.array_equal(plan["slot_cols"].cpu().numpy(), slot_cols)
+    kt = merge_text_cols(vocab, 40) if text_cols is None else text_cols
+    rng = np.random.default_rng(vocab + kt)
+    if text == "catalogue":
+        f = _catalogue(3000, vocab, seed=vocab)
+        plan = engine._merge_plan(engine.ingest(f), kt)
+        indices = f["text_features"].indices
+    else:
+        if text == "first_3000":
+            x = _catalogue(3000, 3000, seed=61)["text_features"].tocsr()
+            csr = sp.csr_matrix((x.data, x.indices, x.indptr), shape=(3000, vocab))
+            f = _catalogue(3000, vocab, seed=62)
+            f["text_features"] = csr
+            plan = engine._merge_plan(engine.ingest(f), kt)
+        elif text == "each_once":
+            cols = np.sort(rng.permutation(vocab).reshape(2000, 5), axis=1)
+            csr = sp.csr_matrix((rng.random(vocab) + 0.05, cols.reshape(-1), np.arange(0, vocab + 1, 5)),
+                                shape=(2000, vocab))
+            f = _catalogue(2000, vocab, seed=63)
+            f["text_features"] = csr
+            plan = engine._merge_plan(engine.ingest(f), kt)
+        else:
+            csr = sp.csr_matrix((100, vocab))
+            plan = _plan_of_csr(engine, csr, kt)
+        indices = csr.indices
+    col_map, slot_ptr, slot_cols = model_plan(indices, vocab, kt)
+    got = {key: plan[key].cpu().numpy() for key in ("col_map", "slot_ptr", "slot_cols")}
+    assert np.array_equal(got["col_map"], col_map)
+    assert np.array_equal(got["slot_ptr"], slot_ptr)
+    assert np.array_equal(got["slot_cols"], slot_cols)
+    head, tail = kt // 2, kt - kt // 2
+    if (vocab - head) % tail == 0:
+        assert np.all(np.diff(slot_ptr)[head:] == (vocab - head) // tail)
+    # the ranking read back from the device plan: rank r >= head is entry (r - head) // tail of slot
+    # head + (r - head) % tail; by descending frequency, equal frequencies by ascending column
+    r = np.arange(vocab)
+    pos = np.where(r < head, r, got["slot_ptr"][head + (r - head) % tail] + (r - head) // tail)
+    ranking = got["slot_cols"][pos]
+    df = np.bincount(indices, minlength=vocab)
+    assert np.array_equal(ranking, np.argsort(-df, kind="stable"))
+    if text in ("each_once", "empty"):
+        assert np.array_equal(ranking, np.arange(vocab))
+    elif text == "first_3000":
+        assert np.array_equal(ranking[3000:], np.arange(3000, vocab))
 
 
 @pytest.mark.parametrize("vocab", [6000, 10_000, 50_000])

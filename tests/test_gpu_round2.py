@@ -526,29 +526,48 @@ def test_folded_operand_follows_the_weights_and_the_catalogue(engine):
 
 
 # ---- the threshold seed pass (per-row score histograms) ------------------------------------------------------
-@pytest.mark.parametrize("vocab", [400, 6000], ids=["folded_wide", "popcount"])
-def test_seeded_thresholds_are_lower_bounds_of_the_final_ones(engine, vocab):
+@pytest.mark.parametrize("vocab,mode", [(400, "folded_wide"), (6000, "popcount"), (6000, "merged")],
+                         ids=["folded_wide", "popcount", "merged"])
+def test_seeded_thresholds_are_lower_bounds_of_the_final_ones(engine, vocab, mode):
     """A seeded threshold must not exceed the K'-th best UPPER BOUND of the show over all columns (then
-    nothing that belongs in the candidate list is ever dropped).  Checked against the exact scores: the
-    K'-th best exact hybrid, inflated by the slack of the bound, is at least the seed; and the seed is
-    useful (above min_similarity for almost every show)."""
+    nothing that belongs in the candidate list is ever dropped).  On the catalogue's own operand the
+    bound is the exact hybrid inflated by the slack, so the K'-th best exact hybrid, inflated, is at
+    least the seed.  Over the merged text operand the bound uses the merged text dot, which may exceed
+    the exact cosine: the seed may then exceed the K'-th exact hybrid, never the K'-th merged bound.
+    And the seed is useful (above min_similarity for almost every show)."""
     import torch
 
+    from test_merge_plan import merged_dense
     from tvbingefriend_recommendation_service_b200.engine import stage
     from tvbingefriend_recommendation_service_b200.synthetic import make_catalogue
 
     n, w, k, ms = 9000, (0.4, 0.5, 0.1), 20, 0.1
     cat = make_catalogue(n, vocab, nnz=15, seed=61)
     f = cat.features()
-    dc = engine.upload(stage(f), w)
-    theta = engine.sym_seed(dc, w, k, ms, 0, 1)
-    torch.cuda.synchronize()
+    old = engine.merge_ratio
+    if mode == "popcount":
+        engine.merge_ratio = 0.0           # at V = 6 000 the default merges the text and folds the groups
+    try:
+        dc = engine.upload(stage(f), w)
+        theta = engine.sym_seed(dc, w, k, ms, 0, 1)
+        torch.cuda.synchronize()
+        plan = engine.plan_tiles(dc, w, k, ms)
+        col_map = None if mode != "merged" else engine._fold_owner["plan"]["col_map"].cpu().numpy()
+    finally:
+        engine.merge_ratio = old
+    assert plan["folded_bits"] == (mode != "popcount")
+    assert plan["text_cols"] == (4024 if mode == "merged" else 0)
     th = theta.view(torch.float32)[:n].cpu().numpy().astype(np.float64)
     assert np.isfinite(th).all() and (th > ms * 0.99).mean() > 0.9
     kp = 32                                   # candidates kept for k = 20
     pr = ProductionRows(f, *w)
     rows = np.arange(0, n, 150)
-    h = pr.rows_block(rows)[0]
+    h, g, _, md = pr.rows_block(rows)
+    if mode == "merged":
+        x = pr.T
+        xm = merged_dense(x[rows], col_map, 4024)
+        slot = sp.csr_matrix((np.ones(vocab), (np.arange(vocab), col_map)), shape=(vocab, 4024))
+        h = w[0] * g + w[1] * np.asarray((x @ slot) @ xm.T).T + w[2] * md
     h[np.arange(len(rows)), rows] = -1.0      # a show is not its own candidate
     kth = -np.sort(-h, axis=1)[:, kp - 1]
     assert np.all(th[rows] <= kth * (1 + 3e-3) + 1e-4), float((th[rows] - kth).max())

@@ -36,6 +36,44 @@ def merged_dense(x, col_map: np.ndarray, text_cols: int) -> np.ndarray:
     return out
 
 
+def bf16_bits(x) -> np.ndarray:
+    """float64 -> bfloat16 bits, rounded once to nearest with ties to even (``cvt.rn.bf16.f64``,
+    which ``__double2bfloat16`` is on sm_100).  A float32 step would round twice."""
+    x = np.asarray(x, dtype=np.float64)
+    _, e = np.frexp(x)                                  # |x| in [2^(e-1), 2^e)
+    q = np.ldexp(1.0, np.maximum(e - 8, -133))          # bf16 spacing there: 8 significant bits, subnormals 2^-133
+    r = np.rint(x / q) * q                              # x / q is exact (q is a power of two); rint: ties to even
+    with np.errstate(over="ignore"):
+        return (r.astype(np.float32).view(np.uint32) >> 16).astype(np.uint16)
+
+
+def model_operand(indptr, indices, values, plan, k_pad: int, col_offset: int, scale: float,
+                  dtype: str = "fp16") -> np.ndarray:
+    """uint16 [n_rows, k_pad]: the bits tvbf_prep_csr_to_operand_mapped writes into a zeroed
+    buffer.  Operand column s of a row is the float64 sum of the row's entries in the vocabulary
+    columns of slot s, added one by one in ``slot_cols`` order (the kernel's order), times ``scale``,
+    rounded once to fp16 / bf16; every other position stays zero.  ``plan``: (col_map, slot_ptr,
+    slot_cols) as ``model_plan`` returns them."""
+    col_map, slot_ptr, slot_cols = (np.asarray(a) for a in plan)
+    indptr, indices = np.asarray(indptr, dtype=np.int64), np.asarray(indices, dtype=np.int64)
+    values = np.asarray(values, dtype=np.float64)
+    n = indptr.size - 1
+    text_cols = slot_ptr.size - 1
+    rank = np.empty(slot_cols.size, dtype=np.int64)
+    rank[slot_cols] = np.arange(slot_cols.size)         # position of a vocabulary column in slot_cols
+    row = np.repeat(np.arange(n), np.diff(indptr))
+    order = np.lexsort((rank[indices], row))            # per row, in slot_cols order
+    acc = np.zeros(n * text_cols)
+    np.add.at(acc, row[order] * text_cols + col_map[indices[order]], values[order])   # sequential, in order
+    touched = np.zeros(n * text_cols, dtype=bool)
+    touched[row * text_cols + col_map[indices]] = True
+    out = np.zeros((n, k_pad), dtype=np.uint16)
+    scaled = acc.reshape(n, text_cols) * scale
+    bits = scaled.astype(np.float16).view(np.uint16) if dtype == "fp16" else bf16_bits(scaled)
+    out[:, col_offset:col_offset + text_cols] = np.where(touched.reshape(n, text_cols), bits, 0)
+    return out
+
+
 # ---------------------------------------------------------------------------------------------- rule
 @pytest.mark.parametrize("vocab,genres,want", [
     (500, 21, 500),               # P80k: the plain fold fits, no merge
@@ -102,6 +140,8 @@ def test_merge_plan_rejects_bad_widths_before_any_device_work():
         assert rc != 0 and "text_cols" in msg
     rc, msg = call(20_000_000, 4000)
     assert rc != 0 and "at most 4096" in msg
+    rc, msg = call(4098, 2)                     # one tail slot of 4 097 columns; 4 097 / 2 is the largest accepted
+    assert rc != 0 and "4097 vocabulary columns per operand column" in msg
 
 
 def test_merged_features_need_non_negative_text():
@@ -156,3 +196,109 @@ def test_merged_dot_of_adversarial_rows_still_bounds():
     exact = (x @ x.T).toarray()
     xm = merged_dense(x, col_map, text_cols)
     assert np.all(xm @ xm.T >= exact * (1 - 1e-12))
+
+
+# ---------------------------------------------------------------------------------------------- operand model
+def test_bf16_rounder_rounds_once_to_nearest_even():
+    cases = [(1.0, 0x3F80), (-1.5, 0xBFC0), (0.0, 0x0000),
+             (1 + 2.0 ** -8, 0x3F80),                   # halfway, down to the even neighbour
+             (1 + 3 * 2.0 ** -8, 0x3F82),               # halfway, up to the even neighbour
+             (1 + 2.0 ** -8 + 2.0 ** -40, 0x3F81),      # just above halfway: a float32 step would make it a tie
+             (1 + 2.0 ** -8 - 2.0 ** -40, 0x3F80),
+             (2 - 2.0 ** -9, 0x4000),                   # carries into the exponent
+             (256 * (1 + 2.0 ** -8), 0x4380), (-(1 + 3 * 2.0 ** -8), 0xBF82),
+             (2.0 ** -133, 0x0001), (1.5 * 2.0 ** -133, 0x0002), (0.5 * 2.0 ** -133, 0x0000),   # subnormals
+             (2.0 ** -126 * (1 - 2.0 ** -9), 0x0080),   # the largest subnormal rounds up to the smallest normal
+             (2.0 ** 128 - 2.0 ** 119, 0x7F80), (2.0 ** 128 - 2.0 ** 119 - 2.0 ** 90, 0x7F7F)]   # overflow edge
+    got = bf16_bits([x for x, _ in cases])
+    for (x, want), g in zip(cases, got):
+        assert int(g) == want, (x, hex(int(g)), hex(want))
+    # the double rounding the model avoids
+    x = np.float64(1 + 2.0 ** -8 + 2.0 ** -40)
+    assert int(np.float32(x).view(np.uint32) >> 16) == 0x3F80
+    # float32 inputs round once either way: compare with torch's float32 -> bfloat16
+    import torch
+
+    rng = np.random.default_rng(1)
+    f32 = (rng.standard_normal(200_000) * np.exp2(rng.integers(-130, 120, 200_000))).astype(np.float32)
+    f32 = np.r_[f32, (np.arange(1 << 16, dtype=np.uint32) << 16 | 0x8000).view(np.float32)]   # every tie
+    f32 = f32[np.isfinite(f32)]
+    ref = torch.from_numpy(f32).to(torch.bfloat16).view(torch.int16).numpy().view(np.uint16)
+    assert np.array_equal(bf16_bits(f32.astype(np.float64)), ref)
+
+
+def _csr_rows(rows, values, vocab):
+    import scipy.sparse as sp
+
+    indptr = np.r_[0, np.cumsum([len(r) for r in rows])]
+    return sp.csr_matrix((np.asarray(values, dtype=np.float64), np.concatenate(rows).astype(np.int64), indptr),
+                         shape=(len(rows), vocab))
+
+
+@pytest.mark.parametrize("dtype", ["fp16", "bf16"])
+def test_operand_model_is_the_rounded_merged_rows(dtype):
+    """On ordinary rows the model is merged_dense times the scale, rounded once, at the layout's
+    offset, zero elsewhere"""
+    import torch
+    from sklearn.preprocessing import normalize
+
+    from tvbingefriend_recommendation_service_b200.synthetic import make_catalogue
+
+    x = normalize(make_catalogue(300, 10_000, nnz=60, n_genres=20, seed=4).features()["text_features"].tocsr())
+    x.sort_indices()
+    plan = model_plan(x.indices, 10_000, 4024)
+    got = model_operand(x.indptr, x.indices, x.data, plan, 4160, 64, 256.0, dtype)
+    m = merged_dense(x, plan[0], 4024) * 256.0
+    want = m.astype(np.float16).view(np.uint16) if dtype == "fp16" else bf16_bits(m)
+    assert np.array_equal(got[:, 64:64 + 4024], want)
+    assert not got[:, :64].any() and not got[:, 64 + 4024:].any()
+    assert np.array_equal(got[:, 64:64 + 4024] != 0, m > 0)
+    if dtype == "bf16":      # merged sums are not float32 numbers in general; where they are, torch agrees
+        sub = m.astype(np.float32).astype(np.float64) == m
+        ref = torch.from_numpy(m.astype(np.float32)).to(torch.bfloat16).view(torch.int16).numpy().view(np.uint16)
+        assert np.array_equal(want[sub], ref[sub])
+
+
+def test_operand_model_adds_in_slot_order():
+    """Entries of one slot are added in slot_cols order, not in column order: a value on an fp16 tie
+    and two tiny ones, whose float64 sum lands on either side of the tie depending on the order."""
+    vocab, text_cols = 6, 2                     # head: rank 0; the tail slot takes the five others
+    plan = model_plan(np.r_[np.repeat(5, 4), np.repeat(1, 3), np.repeat(3, 2), 0, 2, 4], vocab, text_cols)
+    assert list(plan[2]) == [5, 1, 3, 0, 2, 4]
+    a, b = 1 + 2.0 ** -11, 2.0 ** -53           # a: halfway between the fp16 numbers 1 and 1 + 2^-10
+    x = _csr_rows([[1, 3, 4]], [a, b, b], vocab)
+    got = model_operand(x.indptr, x.indices, x.data, plan, 2, 0, 1.0, "fp16")
+    assert (a + b) + b == a and got[0, 1] == 0x3C00              # column 1 first: the tiny ones vanish
+    plan2 = (plan[0], plan[1], np.array([5, 3, 4, 1, 0, 2]))     # columns 3 and 4 first: they add up to 2^-52
+    got2 = model_operand(x.indptr, x.indices, x.data, plan2, 2, 0, 1.0, "fp16")
+    assert (b + b) + a > a and got2[0, 1] == 0x3C01
+
+
+def test_merged_slack_grows_the_subnormal_term_only():
+    """tvbf_debug_slack (host only): a merged operand entry sums at most V - text_cols + 1 entries of
+    a unit row, so the fp16 subnormal allowance eps_term grows by sqrt(V - text_cols + 1); the
+    relative terms stay as they are"""
+    from tvbingefriend_recommendation_service_b200 import _lib
+
+    lib = _lib.load()
+    for vocab, text_cols in ((10_000, 4024), (50_000, 20_000), (4097, 2), (6000, 4024)):
+        f = _lib.Features(n_shows=10, n_pad=256, k_pad=(text_cols + 63) // 64 * 64, text_dtype=_lib.TEXT_FP16,
+                          text_scale_log2=8, vocab=vocab, operand=1 << 20, text_indptr=1 << 21,
+                          text_indices=1 << 22, text_values=1 << 23, col_side=1 << 24, meta_scale=1 << 25,
+                          genre_mode=_lib.GROUP_PACKED, genre_dim=40, meta_mode=_lib.GROUP_PACKED)
+        p = _lib.Params(genre_weight=0.4, text_weight=0.5, metadata_weight=0.1, min_similarity=0.1, k=60,
+                        exclude_self=1, row_begin=0, row_end=10)
+        out = {}
+        for cols in (0, text_cols):
+            f.text_cols = cols
+            o = (C.c_float * 5)()
+            assert lib.tvbf_debug_slack(C.byref(f), C.byref(p), o) == 0
+            out[cols] = list(o)
+        plain, merged = out[0], out[text_cols]
+        assert merged[:4] == plain[:4], (vocab, text_cols)
+        assert plain[4] > 0.0
+        assert merged[4] / plain[4] == pytest.approx(np.sqrt(vocab - text_cols + 1), rel=2 ** -22), (vocab, text_cols)
+        f.text_dtype = _lib.TEXT_BF16                 # bf16 has no subnormal range that matters here
+        f.text_cols = text_cols
+        o = (C.c_float * 5)()
+        assert lib.tvbf_debug_slack(C.byref(f), C.byref(p), o) == 0 and o[4] == 0.0
