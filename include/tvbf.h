@@ -96,6 +96,8 @@ typedef struct tvbf_features {
                              /* columns [0, text_cols): for non-negative text the tensor-core dot  */
                              /* is an upper bound of the text cosine, not the cosine; only the      */
                              /* candidate pass takes such an operand (needs text_signed == 0)       */
+  int64_t text_nnz;          /* entries of the text CSR (text_indptr[N]): sizes the column-major    */
+                             /* copy the exact row kernel builds in its workspace                   */
 } tvbf_features;
 
 /* Parameters of one top-K job: populate_database.py:85-91 (weights, top_n_per_show,

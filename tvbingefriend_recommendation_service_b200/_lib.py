@@ -39,6 +39,7 @@ class Features(C.Structure):
         ("text_signed", c_int32),
         ("bits_folded", c_int32), ("fold_col0", c_int32), ("fold_weights", c_double * 3),
         ("text_cols", c_int32),
+        ("text_nnz", C.c_int64),
     ]
 
 

@@ -75,6 +75,8 @@ int validate_features(const tvbf_features* f) {
                "text_cols %d outside [0, min(vocab %d, k_pad %d)]", f->text_cols, f->vocab, f->k_pad);
   if (f->text_cols > 0)
     TVBF_REQUIRE(!f->text_signed, "a merged text operand (text_cols > 0) needs non-negative text");
+  TVBF_REQUIRE(f->text_nnz >= 0 && f->text_nnz < INT32_MAX, "text_nnz %lld outside [0, 2^31 - 1)",
+               static_cast<long long>(f->text_nnz));
   if (f->bits_folded) {
     TVBF_REQUIRE(f->genre_mode == TVBF_GROUP_PACKED && f->meta_mode == TVBF_GROUP_PACKED && !f->text_signed,
                  "bits_folded needs packed genre and metadata groups and non-negative text");
@@ -195,7 +197,7 @@ int make_plan(const tvbf_features* f, const tvbf_params* p, Plan* pl, int sweep 
   pl->off_flag = off;    off = align_up(off + static_cast<size_t>(pl->rows) * 4, 256);
   pl->off_floor = off;   off = align_up(off + static_cast<size_t>(pl->rows) * 8, 256);
   pl->off_count = off;   off = align_up(off + 256, 256);
-  pl->off_keys = off;    off = align_up(off + tvbf::k6_scratch_bytes(f->n_shows, sms), 256);
+  pl->off_keys = off;    off = align_up(off + tvbf::k6_scratch_bytes(*f, sms), 256);
   pl->total = off;
   return TVBF_OK;
 }
@@ -673,7 +675,7 @@ int make_sym_plan(const tvbf_features* f, const tvbf_params* p, int rank, int wo
   sp->off_glist = off;   off = align_up(off + static_cast<size_t>(f->n_pad) * pl.sym_cap * 8, 256);
   sp->off_flag = off;    off = align_up(off + static_cast<size_t>(f->n_shows) * 4, 256);
   sp->off_floor = off;   off = align_up(off + static_cast<size_t>(f->n_shows) * 8, 256);
-  sp->off_keys = off;    off = align_up(off + tvbf::k6_scratch_bytes(f->n_shows, sms), 256);
+  sp->off_keys = off;    off = align_up(off + tvbf::k6_scratch_bytes(*f, sms), 256);
   sp->total = off;
   return TVBF_OK;
 }
@@ -2090,7 +2092,7 @@ size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed)
   if (f == nullptr || n_rows_listed <= 0) return 0;
   int sms = 0;
   if (sm_count_cached(&sms) != TVBF_OK) return 0;
-  return align_up(tvbf::k6_scratch_bytes(f->n_shows, sms), 256);
+  return align_up(tvbf::k6_scratch_bytes(*f, sms), 256);
 }
 
 int tvbf_exact_rows(const tvbf_features* f, const tvbf_params* p, const int32_t* rows,

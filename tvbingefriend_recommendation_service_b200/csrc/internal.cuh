@@ -250,7 +250,8 @@ int k1_launch_refresh(const tvbf_features* f, const tvbf_features* g, const K1Pa
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);
-size_t k6_scratch_bytes(int n_shows, int sm_count);
+// exact row kernels' scratch: survivor lists, dense keys, and the column-major copy of the text
+size_t k6_scratch_bytes(const tvbf_features& f, int sm_count);
 int k6_launch(const ScoreParams& sp, const int* rows, int n_listed, const int* count_ptr,
               const double* floors, int row_begin, int rows_are_local, unsigned long long* key_scratch,
               int grid, const tvbf_topk_out& out, cudaStream_t st, int no_text = 0, int list_cap = 0);

@@ -13,6 +13,10 @@
 // K6 (exact_rows_kernel): scores ONE source row against all N columns in fp64 and selects the
 // exact top-k with a radix select over order-preserving 64-bit keys; also the engine behind the
 // single-show query of services/content_based_service.py:161-236 for arbitrary n.
+#include <algorithm>
+
+#include <cub/device/device_radix_sort.cuh>
+
 #include "internal.cuh"
 
 namespace tvbf {
@@ -599,31 +603,29 @@ exact_rows_kernel(const Scorer scorer, const SelectParams sel, const int* __rest
 // K6, feature form.  Two kernels:
 //   exact_rows_notext_kernel  rows known to have no text (the tie plateaus K5 flags): genre /
 //                             metadata only, up to 8 rows per CTA, no CSR traffic at all
-//   exact_rows_text_kernel    rows that may have text: the catalogue CSR (~12 B per text nnz, 56 MB
-//                             at C3) is streamed warp-cooperatively against a shared-memory mask
-//                             of the batch rows' vocabulary; when only a few rows are listed (the
-//                             usual case: near-ties under the fp16 bound are rare, and the online
-//                             single-show query) each row's COLUMNS are split over the CTAs and
-//                             the last CTA of a row selects from the shared survivor list
+//   exact_rows_text_kernel    rows that may have text: a column-major copy of the text (the
+//                             postings of every vocabulary column, built by k6_launch) lets each
+//                             row's text scores follow the row's own terms.  The column shows are
+//                             cut into slices that fit fp64 accumulators in shared memory; when
+//                             only a few rows are listed (the usual case: near-ties under the
+//                             bound are rare, and the online single-show query) a row's slices go
+//                             to different CTAs and the last one selects from the shared survivor
+//                             list
 // ---------------------------------------------------------------------------------------------
 constexpr int K6B_THREADS = 1024;
-constexpr int K6B_MAXB = 8;       // no-text kernel: batch rows per CTA (scratch is sized for this)
-constexpr int K6B_TEXTB = 4;      // text kernel: batch rows
+constexpr int K6B_MAXB = 8;       // batch rows per CTA (scratch is sized for this)
 constexpr int K6B_SMALL = 4096;   // survivors that are selected from shared memory
 constexpr int K6B_LIST = 16384;   // survivors listed per row (global scratch); more -> dense keys
-constexpr int K6B_ROWNNZ = 192;   // text entries of a batch row staged in shared memory
 constexpr size_t K6T_COUNTER_BYTES = 65536;   // text kernel: survivor counters + batch tickets
+constexpr size_t K6T_ACC_BYTES = 128 * 1024;  // text kernel: fp64 text accumulators of a slice
 
-__device__ __forceinline__ double csr_lookup(const tvbf_features& f, int64_t b, int64_t e, int c) {
-  // value of column c in the sorted row segment [b, e); the caller knows it is present
-  while (b < e) {
-    const int64_t mid = (b + e) >> 1;
-    const int cm = f.text_indices[mid];
-    if (cm == c) return f.text_values[mid];
-    if (cm < c) b = mid + 1; else e = mid;
-  }
-  return 0.0;
-}
+// The text matrix column by column: the shows that hold vocabulary column c are
+// row[col_ptr[c] .. col_ptr[c + 1]) in ascending order, val[...] their values.
+struct Postings {
+  const long long* col_ptr;   // [V + 1]; null when the catalogue has no text
+  const int* row;
+  const double* val;
+};
 
 // column-independent pieces of the genre / metadata scores of the batch rows (shared memory)
 template <int MAXB>
@@ -820,24 +822,19 @@ exact_rows_notext_kernel(const ScoreParams sp, const int* __restrict__ rows, int
 // [surv_j: cap_rows x K6B_LIST int][dense keys: cap_rows x n u64].  Row slots: the listed position
 // when listed <= cap_rows (column-split mode, counters zeroed by the launcher), else per-CTA slots.
 __global__ void __launch_bounds__(K6B_THREADS, 1)
-exact_rows_text_kernel(const ScoreParams sp, const int* __restrict__ rows, int n_listed,
+exact_rows_text_kernel(const ScoreParams sp, const Postings pt, const int* __restrict__ rows, int n_listed,
                        const int* __restrict__ count_ptr, int list_cap,
                        const double* __restrict__ floors, int row_begin, int rows_are_local,
-                       int mask_bytes, unsigned long long* __restrict__ key_scratch, int cap_rows,
-                       tvbf_topk_out out) {
-  constexpr int MAXB = K6B_TEXTB;
-  // dynamic smem: [mask: vocab bytes][small_key: K6B_SMALL u64][small_j: K6B_SMALL int]
-  extern __shared__ __align__(16) unsigned int mask_words[];
+                       unsigned long long* __restrict__ key_scratch, int cap_rows, tvbf_topk_out out) {
+  constexpr int MAXB = K6B_MAXB;
+  constexpr int NWARPS = K6B_THREADS / 32;
+  // dynamic smem: [acc: K6T_ACC_BYTES][small_key: K6B_SMALL u64][small_j: K6B_SMALL int]
+  extern __shared__ __align__(16) double acc[];
   __shared__ SelectSmem sm;
   __shared__ BatchRows<MAXB> br;
   __shared__ long long s_b[MAXB], s_e[MAXB];
   __shared__ int s_last;
-  // the batch rows' own (column, value) lists, staged so that a mask hit is resolved by a binary
-  // search in shared memory (rows with more than K6B_ROWNNZ entries are searched in global memory)
-  __shared__ int s_cols[MAXB][K6B_ROWNNZ];
-  __shared__ double s_vals[MAXB][K6B_ROWNNZ];
-  unsigned long long* small_key =
-      reinterpret_cast<unsigned long long*>(reinterpret_cast<unsigned char*>(mask_words) + mask_bytes);
+  unsigned long long* small_key = reinterpret_cast<unsigned long long*>(acc + K6T_ACC_BYTES / 8);
   int* small_j = reinterpret_cast<int*>(small_key + K6B_SMALL);
   const tvbf_features& f = sp.f;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -849,12 +846,15 @@ exact_rows_text_kernel(const ScoreParams sp, const int* __restrict__ rows, int n
   int B = (listed + G - 1) / G;
   B = B < 1 ? 1 : (B > MAXB ? MAXB : B);
   const int n_batches = (listed + B - 1) / B;
+  // slices of at most W column shows (B accumulator rows of W doubles); in column-split mode a batch
+  // takes enough slices to occupy the grid, one item each, else one CTA runs all slices of a batch
+  const int W = static_cast<int>(K6T_ACC_BYTES / 8) / B;
   const bool split = listed <= cap_rows;          // one scratch slot per listed row
-  const int S = split && n_batches < G ? G / n_batches : 1;   // column slices per batch
-  const int items = n_batches * S;
-  const int chunks = (n + 31) / 32;
-  const int words = (f.vocab + 3) / 4;
-  const unsigned char* mask = reinterpret_cast<const unsigned char*>(mask_words);
+  int S = (n + W - 1) / W;
+  if (split && n_batches < G && G / n_batches > S) S = G / n_batches;
+  if (S > n) S = n;
+  const int per_item = split ? 1 : S;
+  const int items = n_batches * (S / per_item);
   int* cnt = reinterpret_cast<int*>(key_scratch);
   int* ticket = cnt + 8192;
   unsigned long long* surv_key = key_scratch + K6T_COUNTER_BYTES / 8;
@@ -867,18 +867,18 @@ exact_rows_text_kernel(const ScoreParams sp, const int* __restrict__ rows, int n
   batch_rows_init(br, tid);
 
   for (int item = blockIdx.x; item < items; item += G) {
-    const int batch = item / S, slice = item % S;
+    const int batch = split ? item / S : item;
+    const int s_first = split ? item % S : 0;
     const int nb = (listed - batch * B) < B ? (listed - batch * B) : B;
     const int slot0 = split ? batch * B : static_cast<int>(blockIdx.x) * MAXB;
     __syncthreads();
-    for (int w = tid; w < words; w += K6B_THREADS) mask_words[w] = 0u;
     if (tid < MAXB) {
       if (tid < nb) {
         const int r = rows[list0 + batch * B + tid];
         const int i = rows_are_local ? row_begin + r : r;
         batch_rows_load(br, tid, i, floors ? floors[list0 + batch * B + tid] : -INFINITY, packed, cs, ghi);
-        s_b[tid] = f.text_indptr[i];
-        s_e[tid] = f.text_indptr[i + 1];
+        s_b[tid] = pt.col_ptr ? f.text_indptr[i] : 0;
+        s_e[tid] = pt.col_ptr ? f.text_indptr[i + 1] : 0;
         if (!split) cnt[slot0 + tid] = 0;   // per-CTA slots are reused from batch to batch
       } else {
         batch_rows_load(br, tid, -1, INFINITY, packed, cs, ghi);
@@ -886,142 +886,99 @@ exact_rows_text_kernel(const ScoreParams sp, const int* __restrict__ rows, int n
       }
     }
     __syncthreads();
-    bool any_text = false;
-    for (int r = 0; r < nb; ++r) {
-      any_text |= s_e[r] > s_b[r];
-      const bool staged = (s_e[r] - s_b[r]) <= K6B_ROWNNZ;
-      for (long long e = s_b[r] + tid; e < s_e[r]; e += K6B_THREADS) {
-        const int c = f.text_indices[e];
-        atomicOr(&mask_words[c >> 2], (1u << r) << (8 * (c & 3)));
-        if (staged) {
-          s_cols[r][e - s_b[r]] = c;
-          s_vals[r][e - s_b[r]] = f.text_values[e];
-        }
-      }
-    }
-    __syncthreads();
-
-    // Each warp takes 32 consecutive column shows per step (lane = column).  Their CSR segments
-    // are one contiguous span, streamed with coalesced loads (lane = entry) and tested against
-    // the mask.  Every hit lane looks its product up in parallel; the products then go to the
-    // lane that owns the entry's column one by one in ascending entry order, so each pair's sum
-    // runs over ascending column index with one rounding per product and per add, like text_dot.
-    const int ch0 = static_cast<int>(static_cast<long long>(chunks) * slice / S);
-    const int ch1 = static_cast<int>(static_cast<long long>(chunks) * (slice + 1) / S);
-    for (int ch = ch0 + warp; ch < ch1; ch += K6B_THREADS / 32) {
-      const int j0 = ch * 32;
-      const int j = j0 + lane;
-      double acc[MAXB];
-#pragma unroll
-      for (int r = 0; r < MAXB; ++r) acc[r] = 0.0;
-      if (any_text) {
-        const long long ip = f.text_indptr[j < n ? j : n];   // first entry of this lane's column
-        const long long span_b = __shfl_sync(kFullMask, ip, 0);
-        const long long span_e = f.text_indptr[j0 + 32 < n ? j0 + 32 : n];
-        // four 32-entry groups (8 loads) are always in flight: a slot is refilled with the group
-        // 128 entries ahead as soon as it has been consumed
-        int c[4];
-        double v[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const long long e = span_b + u * 32 + lane;
-          c[u] = e < span_e ? f.text_indices[e] : -1;
-          v[u] = e < span_e ? f.text_values[e] : 0.0;
-        }
-        for (long long off = span_b; off < span_e; off += 128) {
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const long long e = off + u * 32 + lane;
-            const int cu = c[u];
-            const double vu = v[u];
-            {
-              const long long en = e + 128;
-              c[u] = en < span_e ? f.text_indices[en] : -1;
-              v[u] = en < span_e ? f.text_values[en] : 0.0;
+    for (int s = s_first; s < s_first + per_item; ++s) {
+      const int j0 = static_cast<int>(static_cast<long long>(n) * s / S);
+      const int j1 = static_cast<int>(static_cast<long long>(n) * (s + 1) / S);
+      for (int e = tid; e < nb * W; e += K6B_THREADS) acc[e] = 0.0;
+      __syncthreads();
+      // Text: warp u takes batch row u % nb over the sub-slice u / nb of [j0, j1).  For each of the
+      // row's terms c in ascending order, the lanes look up where the sub-slice starts and ends in
+      // the postings of c (32 terms at a time), then add x_ic * x_jc into the accumulators of the
+      // shows j listed there: each pair's sum runs over ascending column index with one rounding
+      // per product and per add, like text_dot.
+      const int Q = NWARPS / nb;
+      if (warp < nb * Q) {
+        const int r = warp % nb, q = warp / nb;
+        const int js = j0 + static_cast<int>(static_cast<long long>(j1 - j0) * q / Q);
+        const int je = j0 + static_cast<int>(static_cast<long long>(j1 - j0) * (q + 1) / Q);
+        double* acc_r = acc + r * W;
+        for (long long t0 = s_b[r]; t0 < s_e[r]; t0 += 32) {
+          long long lo = 0, hi = 0;
+          double x = 0.0;
+          if (t0 + lane < s_e[r]) {
+            const int c = f.text_indices[t0 + lane];
+            x = f.text_values[t0 + lane];
+            long long a = pt.col_ptr[c], b = pt.col_ptr[c + 1];
+            while (a < b) {   // first posting at or after js
+              const long long mid = (a + b) >> 1;
+              if (pt.row[mid] < js) a = mid + 1; else b = mid;
             }
-            const unsigned mu = cu >= 0 ? mask[cu] : 0u;
-            if (__ballot_sync(kFullMask, mu != 0u) == 0u) continue;
-            // lane that owns this lane's entry: the last one whose column starts at or before it
-            int owner = 0;
-#pragma unroll
-            for (int step = 16; step > 0; step >>= 1) {
-              const long long ipc = __shfl_sync(kFullMask, ip, (owner + step) & 31);
-              if (ipc <= e) owner += step;
+            lo = a;
+            b = pt.col_ptr[c + 1];
+            while (a < b) {   // first posting at or after je
+              const long long mid = (a + b) >> 1;
+              if (pt.row[mid] < je) a = mid + 1; else b = mid;
             }
-#pragma unroll
-            for (int r = 0; r < MAXB; ++r) {
-              const bool mine = (mu >> r) & 1u;
-              unsigned hits = __ballot_sync(kFullMask, mine);
-              if (hits == 0u) continue;
-              double prod = 0.0;
-              if (mine) {
-                const int len = static_cast<int>(s_e[r] - s_b[r]);
-                double xv = 0.0;
-                if (len <= K6B_ROWNNZ) {
-                  int lo = 0, hi = len;
-                  while (lo < hi) {
-                    const int mid = (lo + hi) >> 1;
-                    const int cm = s_cols[r][mid];
-                    if (cm == cu) { xv = s_vals[r][mid]; break; }
-                    if (cm < cu) lo = mid + 1; else hi = mid;
-                  }
-                } else {
-                  xv = csr_lookup(f, s_b[r], s_e[r], cu);
-                }
-                prod = __dmul_rn(xv, vu);
-              }
-              while (hits) {
-                const int hl = __ffs(hits) - 1;
-                hits &= hits - 1;
-                const int o = __shfl_sync(kFullMask, owner, hl);
-                const double pp = __shfl_sync(kFullMask, prod, hl);
-                if (lane == o) acc[r] = __dadd_rn(acc[r], pp);
-              }
+            hi = a;
+          }
+          const int nt = s_e[r] - t0 < 32 ? static_cast<int>(s_e[r] - t0) : 32;
+          for (int t = 0; t < nt; ++t) {
+            const long long lo_t = __shfl_sync(kFullMask, lo, t), hi_t = __shfl_sync(kFullMask, hi, t);
+            const double x_t = __shfl_sync(kFullMask, x, t);
+            for (long long p = lo_t + lane; p < hi_t; p += 32) {
+              double* a = acc_r + (pt.row[p] - j0);
+              *a = __dadd_rn(*a, __dmul_rn(x_t, pt.val[p]));
             }
+            __syncwarp();
           }
         }
       }
+      __syncthreads();
       // genre / metadata parts and the survivor test (all lanes stay in: ballots below)
-      const bool in = j < n;
-      TvbfColSide cj{0ull, 0.0f, 0u};
-      unsigned long long hj = 0ull;
-      double g_rj = 0.0, m_rj = 0.0;
-      if (packed && in) {
-        cj = cs[j];
-        if (ghi) hj = ghi[j];
-        g_rj = br.rs[__popcll(cj.genre_bits) + __popcll(hj)];
-        m_rj = br.rs[__popc(cj.meta_bits)];
-      }
+      for (int jb = j0 + warp * 32; jb < j1; jb += K6B_THREADS) {
+        const int j = jb + lane;
+        const bool in = j < j1;
+        TvbfColSide cj{0ull, 0.0f, 0u};
+        unsigned long long hj = 0ull;
+        double g_rj = 0.0, m_rj = 0.0;
+        if (packed && in) {
+          cj = cs[j];
+          if (ghi) hj = ghi[j];
+          g_rj = br.rs[__popcll(cj.genre_bits) + __popcll(hj)];
+          m_rj = br.rs[__popc(cj.meta_bits)];
+        }
 #pragma unroll
-      for (int r = 0; r < MAXB; ++r) {
-        if (r < nb) {
-          bool ok = false;
-          unsigned long long key = 0ull;
-          if (in) {
-            const double h = batch_hybrid(sp, br, r, j, packed, cj, hj, g_rj, m_rj, acc[r]);
-            ok = (h >= sp.min_similarity) && (h >= br.floor[r]) && !(sp.exclude_self && j == br.row[r]);
-            key = ok ? f64_orderable(h) : 0ull;
-            if (dense) dense_keys[static_cast<size_t>(slot0 + r) * n + j] = key;
-          }
-          const unsigned okb = __ballot_sync(kFullMask, ok);
-          if (okb) {   // one counter update per warp: the row's survivor list may be shared by many CTAs
-            const int leader = __ffs(okb) - 1;
-            int base = 0;
-            if (lane == leader) base = atomicAdd(&cnt[slot0 + r], __popc(okb));
-            base = __shfl_sync(kFullMask, base, leader);
-            const int pos = base + __popc(okb & ((1u << lane) - 1u));
-            if (ok && pos < K6B_LIST) {
-              surv_key[static_cast<size_t>(slot0 + r) * K6B_LIST + pos] = key;
-              surv_j[static_cast<size_t>(slot0 + r) * K6B_LIST + pos] = j;
+        for (int r = 0; r < MAXB; ++r) {
+          if (r < nb) {
+            bool ok = false;
+            unsigned long long key = 0ull;
+            if (in) {
+              const double h = batch_hybrid(sp, br, r, j, packed, cj, hj, g_rj, m_rj, acc[r * W + j - j0]);
+              ok = (h >= sp.min_similarity) && (h >= br.floor[r]) && !(sp.exclude_self && j == br.row[r]);
+              key = ok ? f64_orderable(h) : 0ull;
+              if (dense) dense_keys[static_cast<size_t>(slot0 + r) * n + j] = key;
+            }
+            const unsigned okb = __ballot_sync(kFullMask, ok);
+            if (okb) {   // one counter update per warp: the row's survivor list may be shared by many CTAs
+              const int leader = __ffs(okb) - 1;
+              int base = 0;
+              if (lane == leader) base = atomicAdd(&cnt[slot0 + r], __popc(okb));
+              base = __shfl_sync(kFullMask, base, leader);
+              const int pos = base + __popc(okb & ((1u << lane) - 1u));
+              if (ok && pos < K6B_LIST) {
+                surv_key[static_cast<size_t>(slot0 + r) * K6B_LIST + pos] = key;
+                surv_j[static_cast<size_t>(slot0 + r) * K6B_LIST + pos] = j;
+              }
             }
           }
         }
       }
+      __syncthreads();
     }
     // the last CTA to finish a batch selects its rows (no waiting: everybody else just leaves)
     __threadfence();
     __syncthreads();
-    if (S > 1) {
+    if (split && S > 1) {
       if (tid == 0) s_last = atomicAdd(&ticket[batch], 1) == S - 1;
       __syncthreads();
       if (!s_last) continue;
@@ -1036,6 +993,44 @@ exact_rows_text_kernel(const ScoreParams sp, const int* __restrict__ rows, int n
                           surv_j + slot * K6B_LIST, dense_keys + slot * n, dense, small_key, small_j,
                           static_cast<size_t>(orow), out);
     }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// postings: a stable radix sort of the entry numbers by column, then the column offsets and the
+// (show, value) pairs in sorted order.  Layout behind the K6 scratch (postings_layout): col_ptr,
+// row, val, and the sort's second value buffer and temporary storage; the sort's two key buffers
+// are the two halves of val, its first value buffer is row (both overwritten in postings_fill_kernel).
+// ---------------------------------------------------------------------------------------------
+__global__ void postings_init_kernel(const int* __restrict__ indices, int nnz, int* __restrict__ keys,
+                                     int* __restrict__ ids) {
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += gridDim.x * blockDim.x) {
+    keys[e] = indices[e];
+    ids[e] = e;
+  }
+}
+
+// col_ptr[c] = first sorted position with column >= c, for c in [0, V]
+__global__ void postings_offsets_kernel(const int* __restrict__ keys, int nnz, int vocab,
+                                        long long* __restrict__ col_ptr) {
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p <= nnz; p += gridDim.x * blockDim.x) {
+    const int c_hi = p < nnz ? keys[p] : vocab;
+    const int c_lo = p > 0 ? keys[p - 1] + 1 : 0;
+    for (int c = c_lo; c <= c_hi; ++c) col_ptr[c] = p;
+  }
+}
+
+__global__ void postings_fill_kernel(const int64_t* __restrict__ indptr, int n, const double* __restrict__ values,
+                                     const int* ids, int nnz, int* row, double* __restrict__ val) {
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < nnz; p += gridDim.x * blockDim.x) {
+    const int e = ids[p];   // ids may be `row` itself: read before the write below
+    int a = 0, b = n;       // the show whose entries hold e: last a with indptr[a] <= e
+    while (b - a > 1) {
+      const int mid = (a + b) >> 1;
+      if (indptr[mid] <= e) a = mid; else b = mid;
+    }
+    row[p] = a;
+    val[p] = values[e];
   }
 }
 
@@ -1130,12 +1125,67 @@ int k5_launch_listed(const ScoreParams& sp, const uint2* cand, const int* cand_c
 
 static int k6_cap_rows(int sm_count) { return sm_count * K6B_MAXB; }
 
-size_t k6_scratch_bytes(int n_shows, int sm_count) {
-  // no-text kernel: one CTA per SM, up to K6B_MAXB rows each: dense keys + survivor lists of
-  // K6B_LIST (key, column) entries per row; the text kernel lays the same bytes out per listed row
-  // behind its counters
+static size_t k6_align(size_t x) { return (x + 255) / 256 * 256; }
+
+// no-text kernel: one CTA per SM, up to K6B_MAXB rows each: dense keys + survivor lists of K6B_LIST
+// (key, column) entries per row; the text kernel lays the same bytes out per listed row behind its
+// counters
+static size_t k6_key_bytes(int n_shows, int sm_count) {
   return K6T_COUNTER_BYTES + static_cast<size_t>(k6_cap_rows(sm_count)) *
                                  (static_cast<size_t>(n_shows) * 8 + K6B_LIST * 12);
+}
+
+// byte offsets of the postings (and of the sort that builds them) behind the key scratch
+struct PostingsLayout {
+  size_t col_ptr, row, val, ids2, sort, sort_bytes, total;
+  int end_bit;
+};
+
+static PostingsLayout postings_layout(const tvbf_features& f, int sm_count) {
+  PostingsLayout L{};
+  const size_t nnz = static_cast<size_t>(f.text_nnz);
+  L.end_bit = 1;
+  while (L.end_bit < 31 && (1ll << L.end_bit) < f.vocab) ++L.end_bit;
+  L.col_ptr = k6_align(k6_key_bytes(f.n_shows, sm_count));
+  L.row = k6_align(L.col_ptr + (static_cast<size_t>(f.vocab) + 1) * 8);
+  L.val = k6_align(L.row + nnz * 4);
+  L.ids2 = k6_align(L.val + nnz * 8);
+  L.sort = k6_align(L.ids2 + nnz * 4);
+  L.sort_bytes = 0;
+  if (nnz > 0) {
+    cub::DoubleBuffer<int> keys(nullptr, nullptr), ids(nullptr, nullptr);
+    cub::DeviceRadixSort::SortPairs(nullptr, L.sort_bytes, keys, ids, static_cast<int>(nnz), 0, L.end_bit);
+  }
+  L.total = nnz > 0 ? k6_align(L.sort + L.sort_bytes) : L.col_ptr;
+  return L;
+}
+
+size_t k6_scratch_bytes(const tvbf_features& f, int sm_count) { return postings_layout(f, sm_count).total; }
+
+// the postings of the catalogue's text (Postings) in the scratch behind the keys
+static int build_postings(const tvbf_features& f, unsigned long long* key_scratch, int grid, cudaStream_t st,
+                          Postings* pt) {
+  *pt = Postings{nullptr, nullptr, nullptr};
+  const int nnz = static_cast<int>(f.text_nnz);
+  if (nnz == 0) return TVBF_OK;
+  const PostingsLayout L = postings_layout(f, grid);
+  uint8_t* base = reinterpret_cast<uint8_t*>(key_scratch);
+  int* row = reinterpret_cast<int*>(base + L.row);
+  double* val = reinterpret_cast<double*>(base + L.val);
+  cub::DoubleBuffer<int> keys(reinterpret_cast<int*>(val), reinterpret_cast<int*>(val) + nnz);
+  cub::DoubleBuffer<int> ids(row, reinterpret_cast<int*>(base + L.ids2));
+  const int blocks = std::min((nnz + 255) / 256, grid * 8);
+  postings_init_kernel<<<blocks, 256, 0, st>>>(f.text_indices, nnz, keys.Current(), ids.Current());
+  TVBF_LAUNCH_OK("postings_init_kernel");
+  size_t sort_bytes = L.sort_bytes;
+  TVBF_CUDA_OK(cub::DeviceRadixSort::SortPairs(base + L.sort, sort_bytes, keys, ids, nnz, 0, L.end_bit, st));
+  long long* col_ptr = reinterpret_cast<long long*>(base + L.col_ptr);
+  postings_offsets_kernel<<<blocks, 256, 0, st>>>(keys.Current(), nnz, f.vocab, col_ptr);
+  TVBF_LAUNCH_OK("postings_offsets_kernel");
+  postings_fill_kernel<<<blocks, 256, 0, st>>>(f.text_indptr, f.n_shows, f.text_values, ids.Current(), nnz, row, val);
+  TVBF_LAUNCH_OK("postings_fill_kernel");
+  *pt = Postings{col_ptr, row, val};
+  return TVBF_OK;
 }
 
 int k6_launch(const ScoreParams& sp, const int* rows, int n_listed, const int* count_ptr,
@@ -1145,9 +1195,8 @@ int k6_launch(const ScoreParams& sp, const int* rows, int n_listed, const int* c
     tvbf_set_error("exact rows: k=%d exceeds %d", sp.k, K6_MAXK);
     return TVBF_ERR_INVALID;
   }
-  const size_t mask_bytes = (static_cast<size_t>(sp.f.vocab) + 15) / 16 * 16;
   if (no_text) {
-    // rows known to have no text: no mask, no CSR
+    // rows known to have no text: no postings, no CSR
     const size_t smem = static_cast<size_t>(K6B_SMALL) * 12;
     TVBF_CUDA_OK(cudaFuncSetAttribute(exact_rows_notext_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       static_cast<int>(smem)));
@@ -1156,28 +1205,21 @@ int k6_launch(const ScoreParams& sp, const int* rows, int n_listed, const int* c
     TVBF_LAUNCH_OK("exact_rows_notext_kernel");
     return TVBF_OK;
   }
-  const size_t smem = mask_bytes + static_cast<size_t>(K6B_SMALL) * 12;
   if (k6_cap_rows(grid) > 8192) {   // counters and tickets: two int arrays of 8192 in K6T_COUNTER_BYTES
     tvbf_set_error("exact rows: grid of %d CTAs exceeds the counter area", grid);
     return TVBF_ERR_INVALID;
   }
-  if (smem <= 160 * 1024) {
-    TVBF_CUDA_OK(cudaFuncSetAttribute(exact_rows_text_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(smem)));
-    TVBF_CUDA_OK(cudaMemsetAsync(key_scratch, 0, K6T_COUNTER_BYTES, st));
-    exact_rows_text_kernel<<<grid, K6B_THREADS, smem, st>>>(sp, rows, n_listed, count_ptr, list_cap, floors,
-                                                            row_begin, rows_are_local,
-                                                            static_cast<int>(mask_bytes), key_scratch,
-                                                            k6_cap_rows(grid), out);
-    TVBF_LAUNCH_OK("exact_rows_text_kernel");
-    return TVBF_OK;
-  }
-  // vocabulary too wide for the shared-memory mask: one row per CTA pass
-  FeatureScorer sc{sp};
-  SelectParams sel{sp.f.n_shows, sp.k, sp.exclude_self, sp.min_similarity};
-  exact_rows_kernel<FeatureScorer><<<grid, K6_THREADS, 0, st>>>(
-      sc, sel, rows, n_listed, count_ptr, list_cap, row_begin, rows_are_local, key_scratch, out);
-  TVBF_LAUNCH_OK("exact_rows_kernel");
+  Postings pt;
+  int rc = build_postings(sp.f, key_scratch, grid, st, &pt);
+  if (rc != TVBF_OK) return rc;
+  const size_t smem = K6T_ACC_BYTES + static_cast<size_t>(K6B_SMALL) * 12;
+  TVBF_CUDA_OK(cudaFuncSetAttribute(exact_rows_text_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    static_cast<int>(smem)));
+  TVBF_CUDA_OK(cudaMemsetAsync(key_scratch, 0, K6T_COUNTER_BYTES, st));
+  exact_rows_text_kernel<<<grid, K6B_THREADS, smem, st>>>(sp, pt, rows, n_listed, count_ptr, list_cap, floors,
+                                                          row_begin, rows_are_local, key_scratch, k6_cap_rows(grid),
+                                                          out);
+  TVBF_LAUNCH_OK("exact_rows_text_kernel");
   return TVBF_OK;
 }
 

@@ -380,6 +380,7 @@ class HybridTopKEngine:
             f.text_scale_log2, f.vocab = TEXT_SCALE_LOG2, v
             f.operand = operand.data_ptr()
             f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_nnz = int(raw["values"].numel())
             f.col_side, f.meta_scale = col_side.data_ptr(), meta_scale.data_ptr()
             f.text_signed = int(st.text_signed)
             f.meta_kind = _lib.META_MEAN3 if st.metadata_mode == "mean3" else _lib.META_HSTACK
@@ -555,6 +556,7 @@ class HybridTopKEngine:
             f.text_scale_log2, f.vocab = TEXT_SCALE_LOG2, v
             f.operand = operand.data_ptr()
             f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_nnz = nnz
             f.col_side, f.meta_scale = col_side.data_ptr(), meta_scale.data_ptr()
             f.meta_kind = kind
             f.genre_mode, f.genre_dim = _lib.GROUP_PACKED, int(genre.shape[1])
@@ -833,6 +835,7 @@ class HybridTopKEngine:
             f.n_shows, f.n_pad = n, n_pad
             f.operand = operand.data_ptr()
             f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_nnz = nnz_old + nnz_new
             f.col_side, f.meta_scale = col_side.data_ptr(), meta_scale.data_ptr()
             f.genre_hi = None if genre_hi is None else genre_hi.data_ptr()
             f.text_signed = int(bool(c.text_signed) or bool(nc.text_signed))
@@ -857,8 +860,8 @@ class HybridTopKEngine:
                                   p_new["values"].data_ptr(), q, buf[n_old:].data_ptr(), col_side[n_old:].data_ptr(),
                                   None if genre_hi is None else genre_hi[n_old:].data_ptr(),
                                   meta_scale[n_old:].data_ptr())
-                for name in ("n_shows", "text_indptr", "text_indices", "text_values", "col_side", "meta_scale",
-                             "genre_hi"):
+                for name in ("n_shows", "text_indptr", "text_indices", "text_values", "text_nnz", "col_side",
+                             "meta_scale", "genre_hi"):
                     setattr(ff, name, getattr(f, name))
                 grown.fold = self._fold_owner = {**fc, "c": ff}
             grown.keep.append(new)          # the new rows' tensors stay alive while the grown catalogue uses them
@@ -1047,6 +1050,7 @@ class HybridTopKEngine:
                 values = torch.cat([p_old["values"][:nnz_old], p_new["values"][:nnz_new]])[pos]
             f = Features.from_buffer_copy(c)
             f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_nnz = nnz
             signed = bool(c.text_signed) or bool(nc.text_signed)
             f.text_signed = int(signed and nnz > 0 and bool((values < 0).any()))
             parts = {**p_old, "values": values, "nnz": nnz}
@@ -1067,7 +1071,7 @@ class HybridTopKEngine:
                                   None if p_new["genre_hi"] is None else p_new["genre_hi"].data_ptr(),
                                   p_new["meta_scale"].data_ptr())
                 buf.index_copy_(0, idx, rows_fold)
-                for name in ("text_indptr", "text_indices", "text_values"):
+                for name in ("text_indptr", "text_indices", "text_values", "text_nnz"):
                     setattr(ff, name, getattr(f, name))
                 upd.fold = self._fold_owner = {**fc, "c": ff}
         cat.operand = None                  # consumed: its buffers now belong to the updated catalogue
@@ -1200,6 +1204,7 @@ class HybridTopKEngine:
             f.n_shows, f.n_pad = m, n_pad
             f.operand = operand.data_ptr()
             f.text_indptr, f.text_indices, f.text_values = indptr.data_ptr(), indices.data_ptr(), values.data_ptr()
+            f.text_nnz = nnz
             f.text_signed = int(bool(c.text_signed) and nnz > 0 and bool((values < 0).any()))
             if genre_dense is not None:
                 f.genre_dense = genre_dense.data_ptr()
@@ -1221,7 +1226,7 @@ class HybridTopKEngine:
                 buf = compact(fc["operand"])
                 ff = Features.from_buffer_copy(fc["c"])
                 ff.n_shows, ff.n_pad, ff.operand = m, n_pad, buf.data_ptr()
-                for name in ("text_indptr", "text_indices", "text_values", "col_side", "meta_scale", "genre_hi"):
+                for name in ("text_indptr", "text_indices", "text_values", "text_nnz", "col_side", "meta_scale", "genre_hi"):
                     setattr(ff, name, getattr(f, name))
                 rem.fold = self._fold_owner = {**fc, "c": ff, "operand": buf}
         cat.operand = None                  # consumed: its buffers now belong to the compacted catalogue
