@@ -448,6 +448,44 @@ int tvbf_similarity_stats(const tvbf_features* f, const tvbf_params* p, void* ac
 int tvbf_score_pairs(const tvbf_features* f, const tvbf_params* p, const int32_t* pairs,
                      int32_t n_pairs, double* out4, void* stream);
 
+/* ---- every neighbour at or above a threshold (the loop populate_database.py:170-218 cut by
+ *      min_similarity alone): one variable-length row per show instead of a [N, k] table.  Two calls,
+ *      because the size of the result is known only after the sweep:
+ *        tvbf_neighbours_sweep   the tiles on/above the diagonal of the symmetric sweep; writes every
+ *                                pair {int32 i, int32 j}, i < j, whose tensor-core upper bound U
+ *                                (>= the exact hybrid) exceeds theta (the top-k sweep's initial
+ *                                threshold: min_similarity rounded to the nearest fp32, one fp32 step
+ *                                down; always below min_similarity) to pairs[0 .. capacity), in no
+ *                                particular order, and the number of such pairs to *n_candidates
+ *                                (DEVICE int64).  The count goes on past capacity (nothing is stored
+ *                                there): when it exceeds capacity, run the sweep again with at least
+ *                                that capacity.  pairs may be NULL when capacity is 0 (count only).  Every pair whose exact
+ *                                score is >= min_similarity is a candidate.
+ *        tvbf_neighbours_finish  n_candidates (HOST value, <= the sweep's capacity) pairs of the sweep
+ *                                scored in float64 exactly as tvbf_score_pairs and K5 score them
+ *                                (bit-identical), kept when hybrid >= min_similarity, emitted as (i, j)
+ *                                and (j, i), plus (i, i) when p->exclude_self == 0 and its score
+ *                                qualifies.  Row r is entries row_ptr[r] .. row_ptr[r + 1] of indices /
+ *                                hybrid / genre / text / metadata, ordered by (hybrid descending, column
+ *                                ascending) and cut to max_per_row entries (0: no cap); row_ptr has
+ *                                n_shows + 1 int64 entries and row_ptr[n_shows] is the number of entries
+ *                                written.  The outputs need room for 2 * n_candidates + n_shows entries.
+ *                                With max_per_row = k, row r equals row r of tvbf_hybrid_topk's table
+ *                                for the same p and k (indices, count and the four scores).
+ *      Workspace: tvbf_neighbours_workspace_bytes for the sweep's capacity, shared by both calls.
+ *      p supplies the weights, min_similarity and exclude_self; k, candidates, splits and the row range
+ *      are ignored.  Jobs are taken when tvbf_sym_eligible takes them for the whole catalogue with
+ *      exclude_self = 1 and without its k <= 100 condition, and min_similarity > 0; everything else
+ *      (min_similarity <= 0, float (folded) groups, negative weights, ...) is refused with
+ *      TVBF_ERR_INVALID and a message.  Neither call synchronises; the caller reads *n_candidates
+ *      back before it sizes the finish.  Single GPU. */
+size_t tvbf_neighbours_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int64_t capacity);
+int tvbf_neighbours_sweep(const tvbf_features* f, const tvbf_params* p, int32_t* pairs, int64_t capacity,
+                          int64_t* n_candidates, void* workspace, size_t workspace_bytes, void* stream);
+int tvbf_neighbours_finish(const tvbf_features* f, const tvbf_params* p, const int32_t* pairs, int64_t n_candidates,
+                           int32_t max_per_row, int64_t* row_ptr, int32_t* indices, double* hybrid, double* genre,
+                           double* text, double* metadata, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- diagnostics ---------------------------------------------------------------------------- */
 /* host-only (no device): the work items of one K1 launch for a catalogue of col_tiles 256-column
  * tiles and super_blocks 256-row super blocks dealt to `world` GPUs; out[6 * item + {0..5}] =

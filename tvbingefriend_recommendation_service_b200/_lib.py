@@ -144,6 +144,12 @@ SIGNATURES = {
     "tvbf_similarity_stats": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_void_p, c_size_t,
                                         c_void_p]),
     "tvbf_score_pairs": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int32, c_void_p, c_void_p]),
+    "tvbf_neighbours_workspace_bytes": (c_size_t, [C.POINTER(Features), C.POINTER(Params), c_int64]),
+    "tvbf_neighbours_sweep": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int64, c_void_p,
+                                        c_void_p, c_size_t, c_void_p]),
+    "tvbf_neighbours_finish": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_void_p, c_int64, c_int32,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_size_t, c_void_p]),
     "tvbf_debug_schedule": (c_int32, [c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32,
                                       C.POINTER(c_int32), c_int32]),
     "tvbf_append_plan_tiles": (C.c_int, [C.POINTER(Features), C.POINTER(Params), c_int32, C.POINTER(c_int64)]),

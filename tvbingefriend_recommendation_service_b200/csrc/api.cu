@@ -2088,6 +2088,111 @@ int tvbf_score_pairs(const tvbf_features* f, const tvbf_params* p, const int32_t
   return tvbf::score_pairs_launch(sp, pairs, n_pairs, out4, static_cast<cudaStream_t>(stream));
 }
 
+// ---- every pair above a threshold (tvbf_neighbours_*) ------------------------------------------
+// The sweep walks the tiles of the symmetric top-k sweep of the same job with kMode 11 of the candidate
+// kernel: no lists, no thresholds, no seed pass.  Every pair i < j whose upper bound U (which is >= its
+// exact hybrid) exceeds theta_init (an fp32 below min_similarity, fill_k1_params) is emitted, so every pair whose exact
+// score reaches min_similarity is among the candidates; the finish rescores them in float64.
+namespace {
+
+// the job as the symmetric top-k sweep would take it: k and the candidate knobs do not apply, the
+// diagonal is added by the finish
+int neighbours_plan(const tvbf_features* f, const tvbf_params* p, SymPlan* sp, tvbf_params* q) {
+  TVBF_REQUIRE(p != nullptr, "params is NULL");
+  TVBF_REQUIRE(p->min_similarity > 0.0,
+               "neighbour sweep: min_similarity must be > 0 (got %g); a threshold at or below 0 selects every pair",
+               p->min_similarity);
+  TVBF_REQUIRE(f->genre_mode != TVBF_GROUP_FOLDED && f->meta_mode != TVBF_GROUP_FOLDED,
+               "neighbour sweep: float (folded) genre / metadata groups are not supported, only packed ones");
+  TVBF_REQUIRE(p->genre_weight >= 0.0 && p->text_weight >= 0.0 && p->metadata_weight >= 0.0,
+               "neighbour sweep: the weights must be non-negative (got %g, %g, %g)", p->genre_weight,
+               p->text_weight, p->metadata_weight);
+  *q = *p;
+  q->k = 1;
+  q->exclude_self = 1;
+  q->candidates = 0;
+  q->force_exact = 0;
+  q->row_begin = 0;
+  q->row_end = f->n_shows;
+  const int rc = make_sym_plan(f, q, 0, 1, sp);
+  if (rc != TVBF_OK) {
+    char why[512];
+    snprintf(why, sizeof(why), "%s", g_last_error);
+    tvbf_set_error("neighbour sweep: the symmetric sweep does not take this job (%s)", why);
+  }
+  return rc;
+}
+
+int neighbours_sizes_ok(const tvbf_features* f, int64_t n_pairs) {
+  TVBF_REQUIRE(n_pairs >= 0 && 2 * n_pairs + f->n_shows <= INT32_MAX,
+               "neighbour finish: %lld candidate pairs are more than one call takes", static_cast<long long>(n_pairs));
+  return TVBF_OK;
+}
+
+}  // namespace
+
+size_t tvbf_neighbours_workspace_bytes(const tvbf_features* f, const tvbf_params* p, int64_t capacity) {
+  if (validate_features(f) != TVBF_OK || capacity < 0 || neighbours_sizes_ok(f, capacity) != TVBF_OK) return 0;
+  SymPlan sp;
+  tvbf_params q;
+  if (neighbours_plan(f, p, &sp, &q) != TVBF_OK) return 0;
+  const size_t finish = tvbf::neighbours_finish_bytes(f->n_shows, capacity, p->exclude_self);
+  return finish > 256 ? finish : 256;
+}
+
+int tvbf_neighbours_sweep(const tvbf_features* f, const tvbf_params* p, int32_t* pairs, int64_t capacity,
+                          int64_t* n_candidates, void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(n_candidates && workspace && capacity >= 0 && (pairs || capacity == 0),
+               "tvbf_neighbours_sweep: bad arguments");
+  SymPlan sp;
+  tvbf_params q;
+  rc = neighbours_plan(f, p, &sp, &q);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(workspace_bytes >= 256, "workspace too small: %zu < 256", workspace_bytes);
+  auto st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  tvbf::K1Params kp;
+  rc = fill_k1_params(f, &q, sp.pl, ws, &kp);
+  if (rc != TVBF_OK) return rc;
+  // nothing of the top-k sweep's lists is used
+  kp.scratch = kp.cand = kp.g_list = nullptr;
+  kp.cand_cnt = nullptr;
+  kp.cand_theta = nullptr;
+  kp.g_theta = kp.g_cnt = nullptr;
+  kp.progress = reinterpret_cast<unsigned int*>(ws);
+  kp.pairs = reinterpret_cast<int2*>(pairs);
+  kp.pair_count = reinterpret_cast<unsigned long long*>(n_candidates);
+  kp.pair_cap = capacity;
+  TVBF_CUDA_OK(cudaMemsetAsync(kp.progress, 0, 256, st));
+  TVBF_CUDA_OK(cudaMemsetAsync(n_candidates, 0, sizeof(int64_t), st));
+  return tvbf::k1_launch_pairs(f, kp, sp.pl.grid, st);
+}
+
+int tvbf_neighbours_finish(const tvbf_features* f, const tvbf_params* p, const int32_t* pairs, int64_t n_candidates,
+                           int32_t max_per_row, int64_t* row_ptr, int32_t* indices, double* hybrid, double* genre,
+                           double* text, double* metadata, void* workspace, size_t workspace_bytes, void* stream) {
+  TVBF_ENTER_CALL(stream);
+  int rc = validate_features(f);
+  if (rc != TVBF_OK) return rc;
+  TVBF_REQUIRE(row_ptr && indices && hybrid && genre && text && metadata && workspace && (pairs || n_candidates == 0),
+               "tvbf_neighbours_finish: NULL buffer");
+  TVBF_REQUIRE(max_per_row >= 0, "max_per_row must be >= 0 (0: no cap)");
+  rc = neighbours_sizes_ok(f, n_candidates);
+  if (rc != TVBF_OK) return rc;
+  SymPlan sp;
+  tvbf_params q;
+  rc = neighbours_plan(f, p, &sp, &q);
+  if (rc != TVBF_OK) return rc;
+  tvbf::ScoreParams scp = score_params(f, p);
+  scp.exclude_self = p->exclude_self ? 1 : 0;
+  const tvbf::NeighboursOut out{reinterpret_cast<long long*>(row_ptr), indices, hybrid, genre, text, metadata};
+  return tvbf::neighbours_finish_launch(scp, reinterpret_cast<const int2*>(pairs), n_candidates, max_per_row, out,
+                                        workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
 size_t tvbf_exact_workspace_bytes(const tvbf_features* f, int32_t n_rows_listed) {
   if (f == nullptr || n_rows_listed <= 0) return 0;
   int sms = 0;

@@ -355,6 +355,21 @@ __device__ __noinline__ void sym_ring_flush(const uint32_t* ring, int n, unsigne
   }
 }
 
+// Drain one epilogue warp's ring of pending pairs {row show, column show} into the global pair buffer
+// of the neighbour sweep: one 64-bit atomicAdd reserves the slots of the whole ring.  Slots at or past
+// cap are counted but not stored.  Not inlined, as sym_ring_flush.
+__device__ __noinline__ void pair_ring_flush(const uint32_t* ring, int n, unsigned long long* count, int2* pairs,
+                                             long long cap, int lane) {
+  unsigned long long base = 0ull;
+  if (lane == 0) base = atomicAdd(count, static_cast<unsigned long long>(n));
+  base = __shfl_sync(kFullMask, base, 0);
+  for (int i = lane; i < n; i += 32) {
+    const unsigned long long slot = base + static_cast<unsigned long long>(i);
+    if (slot < static_cast<unsigned long long>(cap))
+      __stcg(pairs + slot, make_int2(static_cast<int>(ring[i]), static_cast<int>(ring[RING + i])));
+  }
+}
+
 // u[e] for a run-time e without spilling the array to local memory: a select tree
 template <int GW>
 __device__ __forceinline__ float pick(const float (&u)[GW], int e) {
@@ -410,7 +425,10 @@ struct Pacer {
 // 9 repair sweep of a removal: the update sweep without the column side -- every score goes to the
 // gathered row's list only, and that list, its count and its threshold are indexed by the gathered row,
 // 10 refresh sweep: the update sweep over the gathered rows of the shows in G = S + A (p.upd_bits), where
-// only a row whose show is in S (p.upd_sbits: updated or appended) feeds the column side
+// only a row whose show is in S (p.upd_sbits: updated or appended) feeds the column side,
+// 11 neighbour sweep: the tiles of the symmetric top-k sweep, no lists and no thresholds -- every pair
+// i < j whose upper bound U exceeds theta_init (an fp32 below min_similarity) is appended to
+// p.pairs (pair_ring_flush)
 // kG2: multi-hot genres with 64 < G <= 128 -- the second word of every column's mask is staged beside
 // the column-side records (in the threshold slices a single-triple sweep leaves unused) and the
 // popcount runs over both words.
@@ -434,6 +452,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
   constexpr bool kUpdate = kMode == 7 || kRefresh;   // update sweep (or its refresh variant)
   constexpr bool kRepair = kMode == 9;   // repair sweep of a removal
   constexpr bool kGather = kMode == 7 || kMode == 8 || kRepair || kRefresh;   // rows are gathered rows
+  constexpr bool kPairs = kMode == 11;   // neighbour sweep: pairs above the threshold, no lists
   static_assert(!(kG2 && (kMulti || kStats)), "two-word genre masks: single-triple top-k sweeps only");
   static_assert(!(kFold && (kMulti || kStats || kDump || kG2)), "folded groups: single-triple top-k sweeps only");
   // Seed pass: hist[bin][row of the CTA] (32-bit counters; bank = row % 32, so the 32 lanes of a warp
@@ -527,14 +546,14 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
             if (elect_one()) {
               const uint32_t n_th = kMulti ? static_cast<uint32_t>(p.n_weights) : 1u;
               mbar_arrive_expect_tx(&col_full[b], (kFold ? 0u : COL_BYTES + MS_BYTES) +
-                                                      ((kSym && !kStats && !kRepair) ? n_th * MS_BYTES : 0u) +
+                                                      ((kSym && !kStats && !kRepair && !kPairs) ? n_th * MS_BYTES : 0u) +
                                                       (kG2 ? GH_BYTES : 0u));
               if (!kFold) bulk_load_1d(smem + L::OFF_COL + b * COL_BYTES, p.col_side + col0, COL_BYTES, &col_full[b]);
               if (kG2)   // threshold slices 1-2 of this buffer (slice 0 holds the thresholds)
                 bulk_load_1d(smem + L::OFF_TH + (b * kMaxSweep + 1) * MS_BYTES, p.genre_hi + col0, GH_BYTES,
                              &col_full[b]);
               if (!kFold) bulk_load_1d(smem + L::OFF_MS + b * MS_BYTES, p.meta_scale + col0, MS_BYTES, &col_full[b]);
-              if (kSym && !kStats && !kRepair)  // snapshot of the column shows' thresholds (stale = lower = conservative)
+              if (kSym && !kStats && !kRepair && !kPairs)  // snapshot of the column shows' thresholds (stale = lower = conservative)
                 for (uint32_t w = 0; w < n_th; ++w)
                   bulk_load_1d(smem + L::OFF_TH + (b * kMaxSweep + w) * MS_BYTES,
                                p.g_theta + static_cast<size_t>(w) * (kMulti ? p.n_pad : 0) + col0, MS_BYTES,
@@ -708,7 +727,8 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
       // loses one.
       auto ring_flush = [&]() {
         __syncwarp();
-        sym_ring_flush(ring, ring_n, p.g_cnt, p.g_list, p.g_theta, sym_cap, p.kp, p.refresh_period, lane);
+        if constexpr (kPairs) pair_ring_flush(ring, ring_n, p.pair_count, p.pairs, p.pair_cap, lane);
+        else sym_ring_flush(ring, ring_n, p.g_cnt, p.g_list, p.g_theta, sym_cap, p.kp, p.refresh_period, lane);
         ring_n = 0;
         __syncwarp();
       };
@@ -735,6 +755,27 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
           ring_n += __popc(m);
         }
       };
+      // neighbour sweep: bit e of hits = U of column colbase + e passed; only the pairs row < column
+      // < n_shows are kept (the diagonal tile holds both orders of its pairs and the show itself)
+      auto push_pairs = [&](uint32_t hits, int colbase) {
+        if (!__any_sync(kFullMask, hits != 0u)) return;   // the usual case: one vote per group
+        const int lo = row + 1 - colbase, hi = p.n_shows - colbase;   // bits [lo, hi) are real columns > row
+        if (lo > 0) hits = lo >= GW ? 0u : hits & ~((1u << lo) - 1u);
+        if (hi < GW) hits = hi <= 0 ? 0u : hits & ((1u << hi) - 1u);
+        while (__any_sync(kFullMask, hits != 0u)) {
+          if (ring_n > RING - 32) ring_flush();
+          const bool act = hits != 0u;
+          const int col = colbase + (act ? __ffs(hits) - 1 : 0);
+          hits &= hits - 1u;
+          const unsigned m = __ballot_sync(kFullMask, act);
+          const int slot = ring_n + __popc(m & ((1u << lane) - 1u));
+          if (act) {
+            ring[slot] = static_cast<uint32_t>(row);
+            ring[RING + slot] = static_cast<uint32_t>(col);
+          }
+          ring_n += __popc(m);
+        }
+      };
 
       const int tile_beg = kDump ? c.tile0 : c.real0, tile_end = kDump ? c.tile1 : c.real1;
       for (int jt = tile_beg; jt < tile_end; jt += p.tile_stride, ++it) {
@@ -743,7 +784,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
         const int col0 = kDump ? p.dump_col0 : jt * BN;
         if (kMulti) {
           load_thw();
-        } else if (kSym && !kStats) {
+        } else if (kSym && !kStats && !kPairs) {
           // current shared threshold of this thread's show (raised by any CTA working on it)
           unsigned int tb = 0x7f800000u;
           if (row_valid)
@@ -873,7 +914,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #pragma unroll
               for (int e4 = 0; e4 < GW / 4; ++e4) {
                 float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (kSym) t4 = reinterpret_cast<const float4*>(sth + cbase + h * GW)[e4];
+                if (kSym && !kPairs) t4 = reinterpret_cast<const float4*>(sth + cbase + h * GW)[e4];
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
                   const int e = e4 * 4 + q;
@@ -890,13 +931,15 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
                   }
                   u[e] = ue;
                   hit_r |= ue > theta ? (1u << e) : 0u;
-                  if (kSym) {
+                  if (kSym && !kPairs) {
                     const float tc = q == 0 ? t4.x : (q == 1 ? t4.y : (q == 2 ? t4.z : t4.w));
                     hit_c |= ue > tc ? (1u << e) : 0u;   // padded columns carry threshold +inf
                   }
                 }
               }
-              if (kSym) {
+              if constexpr (kPairs) {
+                push_pairs(hit_r, col0 + cbase + h * GW);
+              } else if (kSym) {
                 if (!do_col) hit_c = 0u;
                 if constexpr (kAppend) {
                   // a pair of two old shows is in the previous table already (or ranks below all of it):
@@ -986,7 +1029,7 @@ hybrid_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
               ring_flush();
               if (kMulti) {
                 load_thw();
-              } else if (row_valid) {
+              } else if (!kPairs && row_valid) {
                 unsigned int tb;
                 asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(tb) : "l"(p.g_theta + lrow) : "memory");
                 theta = __uint_as_float(tb);
@@ -1885,6 +1928,26 @@ int k1_launch(const tvbf_features* f, const K1Params& kp, int entries_per_lane, 
   }
   tvbf_set_error("unsupported candidate capacity (entries per lane %d)", entries_per_lane);
   return TVBF_ERR_INVALID;
+}
+
+// the same operands, tiles and epilogue width as the symmetric top-k sweep; no lists to clear, no seed
+int k1_launch_pairs(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st) {
+  // a NULL pair buffer is fine at capacity 0: the kernel stores no slot >= pair_cap (count only)
+  if (!kp.sym || (kp.pairs == nullptr && kp.pair_cap > 0) || kp.pair_count == nullptr || kp.pair_cap < 0) {
+    tvbf_set_error("neighbour sweep: bad parameters");
+    return TVBF_ERR_INVALID;
+  }
+  K1Params sweep = kp;
+  sweep.tile_stride = 1;
+  if (kp.wide_epilogue) {
+    if (sweep.stages > Smem<2, true>::STAGES) sweep.stages = Smem<2, true>::STAGES;
+    if (kp.fold) return launch_k1<4, false, 2, 11, true, false, true>(f, sweep, grid, st);
+    return kp.genre_hi ? launch_k1<4, false, 2, 11, true, true>(f, sweep, grid, st)
+                       : launch_k1<4, false, 2, 11, true>(f, sweep, grid, st);
+  }
+  if (kp.fold) return launch_k1<4, false, 2, 11, false, false, true>(f, sweep, grid, st);
+  return kp.genre_hi ? launch_k1<4, false, 2, 11, false, true>(f, sweep, grid, st)
+                     : launch_k1<4, false, 2, 11>(f, sweep, grid, st);
 }
 
 // histogram seed pass of an append: over the super blocks that hold new shows (from append_b0 on; the old

@@ -132,6 +132,12 @@ struct K1Params {
   // refresh sweep (kMode 10, tvbf_refresh_topk): upd_bits marks G (every gathered show), upd_sbits the
   // shows of S (updated or appended); only a gathered row whose show is in S feeds the column side
   const unsigned int* upd_sbits;
+  // neighbour sweep (kMode 11, tvbf_neighbours_sweep): every pair i < j with U > theta_init goes to
+  // pairs[slot] for a slot reserved on *pair_count; the count goes on past pair_cap (nothing is stored
+  // there), so that it is the size a complete run needs
+  int2* pairs;
+  unsigned long long* pair_count;
+  long long pair_cap;
 };
 
 // The previous table of an update and where its rows go (list 1 of the two-list candidate table, as
@@ -248,6 +254,17 @@ int k1_launch_remove(const tvbf_features* f, const tvbf_features* g, const K1Par
 int k1_launch_refresh(const tvbf_features* f, const tvbf_features* g, const K1Params& kp, int grid,
                       const RefreshPrev& prev, cudaStream_t st);
 int k4s_launch(const K1Params& kp, int n_rows, cudaStream_t st);
+// the neighbour sweep (kMode 11) over the tiles on/above the diagonal; kp.pair_count is zeroed by the caller
+int k1_launch_pairs(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
+// float64 finish of a neighbour sweep: score, filter, both directions, per-row order and cap (rescore.cu)
+struct NeighboursOut {
+  long long* row_ptr;   // [n_shows + 1]
+  int* indices;
+  double *hybrid, *genre, *text, *metadata;
+};
+size_t neighbours_finish_bytes(int n_shows, long long n_pairs, int exclude_self);
+int neighbours_finish_launch(const ScoreParams& sp, const int2* pairs, long long n_pairs, int max_per_row,
+                             const NeighboursOut& out, void* ws, size_t ws_bytes, cudaStream_t st);
 int k1_launch_stats(const tvbf_features* f, const K1Params& kp, int grid, cudaStream_t st);
 int score_pairs_launch(const ScoreParams& sp, const int* pairs, int n_pairs, double* out, cudaStream_t st);
 // exact row kernels' scratch: survivor lists, dense keys, and the column-major copy of the text

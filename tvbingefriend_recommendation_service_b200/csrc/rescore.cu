@@ -16,6 +16,7 @@
 #include <algorithm>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include "internal.cuh"
 
@@ -1244,6 +1245,213 @@ int k6_launch_matrix(const double* h, const double* g, const double* t, const do
   exact_rows_kernel<MatrixScorer><<<grid, K6_THREADS, 0, st>>>(sc, sel, rows, n_listed, nullptr, 0, 0,
                                                                0, key_scratch, out);
   TVBF_LAUNCH_OK("exact_rows_kernel<matrix>");
+  return TVBF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Finish of a neighbour sweep (tvbf_neighbours_finish): the candidate pairs i < j of the sweep are
+// scored in float64 by score_pair (the scorer of K5 and tvbf_score_pairs), kept when hybrid >=
+// min_similarity, and emitted in both directions -- plus (i, i) when the job keeps the show itself.
+// Directed entry e < 2n is pair e / 2 read as (i, j) (even e) or (j, i) (odd e); entry 2n + i is
+// (i, i).  Three stable radix passes order the entries by (row, hybrid descending, column): column
+// first, then the hybrid key, then the row (a dropped entry carries row n_shows and sorts last).  The
+// key is unique per entry, so the output does not depend on the order in which the sweep emitted.
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+struct NbLayout {
+  size_t sc, cnt, start, capcnt, perm0, perm1, key0, key1, temp, temp_bytes, total;
+  int m;            // directed entries
+  int row_bits;     // radix bits of a row / column key (values 0 .. n_shows)
+};
+
+__host__ __device__ __forceinline__ size_t nb_align(size_t v) { return (v + 255) / 256 * 256; }
+
+NbLayout nb_layout(int n_shows, long long n_pairs, int exclude_self) {
+  NbLayout L{};
+  const long long m = 2 * n_pairs + (exclude_self ? 0 : n_shows);
+  L.m = static_cast<int>(m);
+  L.row_bits = 1;
+  while (L.row_bits < 31 && (1ll << L.row_bits) <= n_shows) ++L.row_bits;
+  const size_t scored = static_cast<size_t>(n_pairs) + (exclude_self ? 0 : n_shows);
+  size_t off = 0;
+  L.sc = off;     off = nb_align(off + scored * 4 * sizeof(double));
+  L.cnt = off;    off = nb_align(off + (static_cast<size_t>(n_shows) + 1) * 8);
+  L.start = off;  off = nb_align(off + (static_cast<size_t>(n_shows) + 1) * 8);
+  L.capcnt = off; off = nb_align(off + (static_cast<size_t>(n_shows) + 1) * 8);
+  L.perm0 = off;  off = nb_align(off + static_cast<size_t>(m) * 4);
+  L.perm1 = off;  off = nb_align(off + static_cast<size_t>(m) * 4);
+  L.key0 = off;   off = nb_align(off + static_cast<size_t>(m) * 8);   // 64-bit keys; the 32-bit passes alias them
+  L.key1 = off;   off = nb_align(off + static_cast<size_t>(m) * 8);
+  size_t b32 = 0, b64 = 0, bscan = 0;
+  if (m > 0) {
+    cub::DoubleBuffer<unsigned int> k32(nullptr, nullptr);
+    cub::DoubleBuffer<unsigned long long> k64(nullptr, nullptr);
+    cub::DoubleBuffer<int> v(nullptr, nullptr);
+    cub::DeviceRadixSort::SortPairs(nullptr, b32, k32, v, L.m, 0, L.row_bits);
+    cub::DeviceRadixSort::SortPairs(nullptr, b64, k64, v, L.m, 0, 64);
+  }
+  cub::DeviceScan::ExclusiveSum(nullptr, bscan, static_cast<long long*>(nullptr), static_cast<long long*>(nullptr),
+                                n_shows + 1);
+  L.temp_bytes = std::max(std::max(b32, b64), bscan);
+  L.temp = off;   off = nb_align(off + L.temp_bytes);
+  L.total = off;
+  return L;
+}
+
+struct NbEntry {
+  int row, col, t;   // t: scored pair (candidate t, or n_pairs + i for (i, i))
+};
+
+__device__ __forceinline__ NbEntry nb_entry(const int2* pairs, long long n_pairs, int e) {
+  if (e < 2 * n_pairs) {
+    const int2 q = pairs[e >> 1];
+    return (e & 1) ? NbEntry{q.y, q.x, e >> 1} : NbEntry{q.x, q.y, e >> 1};
+  }
+  const int i = static_cast<int>(e - 2 * n_pairs);
+  return NbEntry{i, i, static_cast<int>(n_pairs) + i};
+}
+
+__global__ void nb_score_kernel(const ScoreParams sp, const int2* __restrict__ pairs, long long n_pairs,
+                                int n_scored, double* __restrict__ sc) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_scored) return;
+  int i, j;
+  if (t < n_pairs) {
+    const int2 q = pairs[t];
+    i = q.x;
+    j = q.y;
+  } else {
+    i = j = static_cast<int>(t - n_pairs);
+  }
+  const Scores s = score_pair(sp, i, j);
+  sc[4 * static_cast<size_t>(t) + 0] = s.h;
+  sc[4 * static_cast<size_t>(t) + 1] = s.g;
+  sc[4 * static_cast<size_t>(t) + 2] = s.t;
+  sc[4 * static_cast<size_t>(t) + 3] = s.m;
+}
+
+// pass 1 keys (column) and the kept entries per row
+__global__ void nb_col_keys_kernel(const int2* __restrict__ pairs, long long n_pairs, int m, const double* __restrict__ sc,
+                                   double min_similarity, unsigned int* __restrict__ key, int* __restrict__ perm,
+                                   unsigned long long* __restrict__ cnt) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= m) return;
+  const NbEntry en = nb_entry(pairs, n_pairs, e);
+  key[e] = static_cast<unsigned int>(en.col);
+  perm[e] = e;
+  if (sc[4 * static_cast<size_t>(en.t)] >= min_similarity) atomicAdd(cnt + en.row, 1ull);
+}
+
+// pass 2 keys: hybrid descending
+__global__ void nb_score_keys_kernel(const int* __restrict__ perm, int m, const int2* __restrict__ pairs, long long n_pairs,
+                                     const double* __restrict__ sc, unsigned long long* __restrict__ key) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= m) return;
+  const NbEntry en = nb_entry(pairs, n_pairs, perm[q]);
+  key[q] = ~f64_orderable(sc[4 * static_cast<size_t>(en.t)]);
+}
+
+// pass 3 keys: row, n_shows for a dropped entry
+__global__ void nb_row_keys_kernel(const int* __restrict__ perm, int m, const int2* __restrict__ pairs, long long n_pairs,
+                                   const double* __restrict__ sc, double min_similarity, int n_shows,
+                                   unsigned int* __restrict__ key) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= m) return;
+  const NbEntry en = nb_entry(pairs, n_pairs, perm[q]);
+  key[q] = static_cast<unsigned int>(sc[4 * static_cast<size_t>(en.t)] >= min_similarity ? en.row : n_shows);
+}
+
+__global__ void nb_cap_kernel(const unsigned long long* __restrict__ cnt, int n_shows, int max_per_row,
+                              unsigned long long* __restrict__ capcnt) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r > n_shows) return;
+  unsigned long long c = r < n_shows ? cnt[r] : 0ull;
+  if (max_per_row > 0 && c > static_cast<unsigned long long>(max_per_row)) c = static_cast<unsigned long long>(max_per_row);
+  capcnt[r] = c;
+}
+
+__global__ void nb_write_kernel(const unsigned int* __restrict__ rows, const int* __restrict__ perm, int m,
+                                const int2* __restrict__ pairs, long long n_pairs, const double* __restrict__ sc,
+                                const long long* __restrict__ start, int n_shows, NeighboursOut out) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= m) return;
+  const int r = static_cast<int>(rows[q]);
+  if (r >= n_shows) return;
+  const long long rank = q - start[r];
+  if (rank >= out.row_ptr[r + 1] - out.row_ptr[r]) return;
+  const long long o = out.row_ptr[r] + rank;
+  const NbEntry en = nb_entry(pairs, n_pairs, perm[q]);
+  const double* s = sc + 4 * static_cast<size_t>(en.t);
+  out.indices[o] = en.col;
+  out.hybrid[o] = s[0];
+  out.genre[o] = s[1];
+  out.text[o] = s[2];
+  out.metadata[o] = s[3];
+}
+
+}  // namespace
+
+size_t neighbours_finish_bytes(int n_shows, long long n_pairs, int exclude_self) {
+  return nb_layout(n_shows, n_pairs, exclude_self).total;
+}
+
+int neighbours_finish_launch(const ScoreParams& sp, const int2* pairs, long long n_pairs, int max_per_row,
+                             const NeighboursOut& out, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const int n = sp.f.n_shows;
+  const NbLayout L = nb_layout(n, n_pairs, sp.exclude_self);
+  if (ws_bytes < L.total) {
+    tvbf_set_error("workspace too small: %zu < %zu", ws_bytes, L.total);
+    return TVBF_ERR_WORKSPACE;
+  }
+  uint8_t* base = static_cast<uint8_t*>(ws);
+  double* sc = reinterpret_cast<double*>(base + L.sc);
+  auto* cnt = reinterpret_cast<unsigned long long*>(base + L.cnt);
+  auto* start = reinterpret_cast<long long*>(base + L.start);
+  auto* capcnt = reinterpret_cast<unsigned long long*>(base + L.capcnt);
+  int* perm0 = reinterpret_cast<int*>(base + L.perm0);
+  int* perm1 = reinterpret_cast<int*>(base + L.perm1);
+  void* key0 = base + L.key0;
+  void* key1 = base + L.key1;
+  void* temp = base + L.temp;
+  const int m = L.m;
+  const int n_scored = static_cast<int>(n_pairs) + (sp.exclude_self ? 0 : n);
+  TVBF_CUDA_OK(cudaMemsetAsync(cnt, 0, (static_cast<size_t>(n) + 1) * 8, st));
+  if (m > 0) {
+    if (n_scored > 0) {
+      nb_score_kernel<<<(n_scored + 127) / 128, 128, 0, st>>>(sp, pairs, n_pairs, n_scored, sc);
+      TVBF_LAUNCH_OK("nb_score_kernel");
+    }
+    const unsigned blocks = static_cast<unsigned>((m + 255) / 256);
+    cub::DoubleBuffer<int> v(perm0, perm1);
+    cub::DoubleBuffer<unsigned int> k32(static_cast<unsigned int*>(key0), static_cast<unsigned int*>(key1));
+    nb_col_keys_kernel<<<blocks, 256, 0, st>>>(pairs, n_pairs, m, sc, sp.min_similarity, k32.Current(), v.Current(), cnt);
+    TVBF_LAUNCH_OK("nb_col_keys_kernel");
+    size_t tb = L.temp_bytes;
+    TVBF_CUDA_OK(cub::DeviceRadixSort::SortPairs(temp, tb, k32, v, m, 0, L.row_bits, st));
+    cub::DoubleBuffer<unsigned long long> k64(static_cast<unsigned long long*>(key0),
+                                              static_cast<unsigned long long*>(key1));
+    nb_score_keys_kernel<<<blocks, 256, 0, st>>>(v.Current(), m, pairs, n_pairs, sc, k64.Current());
+    TVBF_LAUNCH_OK("nb_score_keys_kernel");
+    tb = L.temp_bytes;
+    TVBF_CUDA_OK(cub::DeviceRadixSort::SortPairs(temp, tb, k64, v, m, 0, 64, st));
+    k32 = cub::DoubleBuffer<unsigned int>(static_cast<unsigned int*>(key0), static_cast<unsigned int*>(key1));
+    nb_row_keys_kernel<<<blocks, 256, 0, st>>>(v.Current(), m, pairs, n_pairs, sc, sp.min_similarity, n, k32.Current());
+    TVBF_LAUNCH_OK("nb_row_keys_kernel");
+    tb = L.temp_bytes;
+    TVBF_CUDA_OK(cub::DeviceRadixSort::SortPairs(temp, tb, k32, v, m, 0, L.row_bits, st));
+    // rows of the sorted entries: k32.Current(); their first position per row: start
+    size_t sb = L.temp_bytes;
+    TVBF_CUDA_OK(cub::DeviceScan::ExclusiveSum(temp, sb, reinterpret_cast<long long*>(cnt), start, n + 1, st));
+    nb_cap_kernel<<<(n + 256) / 256, 256, 0, st>>>(cnt, n, max_per_row, capcnt);
+    TVBF_LAUNCH_OK("nb_cap_kernel");
+    sb = L.temp_bytes;
+    TVBF_CUDA_OK(cub::DeviceScan::ExclusiveSum(temp, sb, reinterpret_cast<long long*>(capcnt), out.row_ptr, n + 1, st));
+    nb_write_kernel<<<blocks, 256, 0, st>>>(k32.Current(), v.Current(), m, pairs, n_pairs, sc, start, n, out);
+    TVBF_LAUNCH_OK("nb_write_kernel");
+  } else {
+    TVBF_CUDA_OK(cudaMemsetAsync(out.row_ptr, 0, (static_cast<size_t>(n) + 1) * 8, st));
+  }
   return TVBF_OK;
 }
 

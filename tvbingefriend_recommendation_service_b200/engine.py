@@ -218,6 +218,60 @@ class TopK:
                 "text_score": self.text[mask], "metadata_score": self.metadata[mask]}
 
 
+@dataclass
+class NeighbourTable:
+    """Every neighbour at or above ``min_similarity`` of source rows [row_begin, row_begin + R): row r is
+    entries ``row_ptr[r] .. row_ptr[r + 1]``, ordered by (score descending, column ascending) -- the
+    record stream of scripts/populate_database.py:211-217 cut by the threshold alone (or also by
+    ``max_per_row``)."""
+
+    row_ptr: np.ndarray      # int64 [R + 1], row_ptr[0] == 0
+    indices: np.ndarray      # int32 [row_ptr[R]] (column = position in show_ids)
+    hybrid: np.ndarray       # float64 [row_ptr[R]] similarity_score
+    genre: np.ndarray
+    text: np.ndarray
+    metadata: np.ndarray
+    candidate_pairs: int = 0   # pairs i < j the tensor-core sweep passed to the float64 finish
+    row_begin: int = 0
+    flagged_rows: int = 0      # always 0: the threshold job has no certificate to fail
+
+    @property
+    def counts(self) -> np.ndarray:
+        return np.diff(self.row_ptr).astype(np.int32)
+
+    def slice(self, begin: int, end: int) -> "NeighbourTable":
+        """Rows [begin, end) of this table (positions within the table); the arrays are views."""
+        b, e = int(self.row_ptr[begin]), int(self.row_ptr[end])
+        return NeighbourTable(self.row_ptr[begin:end + 1] - b, self.indices[b:e], self.hybrid[b:e], self.genre[b:e],
+                              self.text[b:e], self.metadata[b:e], candidate_pairs=self.candidate_pairs,
+                              row_begin=self.row_begin + begin)
+
+    def to_dict(self, show_ids, id_key: str = "similar_show_id") -> dict:
+        """``all_similarities`` as the hot loop builds it, in the shape of ``TopK.to_dict``: shows
+        without a qualifying neighbour are omitted."""
+        ids = TopK._ids(show_ids)
+        sim = ids[self.indices].tolist()
+        hyb, gen, txt, met = self.hybrid.tolist(), self.genre.tolist(), self.text.tolist(), self.metadata.tolist()
+        ptr = self.row_ptr.tolist()
+        own = ids[self.row_begin:self.row_begin + len(ptr) - 1].tolist()
+        out = {}
+        for r in range(len(ptr) - 1):
+            b, e = ptr[r], ptr[r + 1]
+            if b == e:
+                continue
+            out[own[r]] = [{id_key: sim[q], "similarity_score": hyb[q], "genre_score": gen[q], "text_score": txt[q],
+                            "metadata_score": met[q]} for q in range(b, e)]
+        return out
+
+    def records(self, show_ids) -> dict:
+        """Flat columnar records (one per pair, in table order), as ``TopK.records``."""
+        ids = TopK._ids(show_ids)
+        rows = np.repeat(np.arange(len(self.row_ptr) - 1), np.diff(self.row_ptr))
+        return {"show_id": ids[self.row_begin + rows], "similar_show_id": ids[self.indices],
+                "similarity_score": self.hybrid, "genre_score": self.genre, "text_score": self.text,
+                "metadata_score": self.metadata}
+
+
 class HybridTopKEngine:
     """One engine per process / GPU.  It caches a device workspace and pinned host buffers, so it
     must not be shared between threads that run jobs concurrently (the reference's callers are
@@ -1495,6 +1549,95 @@ class HybridTopKEngine:
         device: ``ingest``)."""
         cat = self.ingest(features, metadata_mode, weights)
         return self.to_host(self.top_k_device(cat, weights, k, min_similarity, exclude_self, **kw))
+
+    # ------------------------------------------------------------------------------------ threshold
+    def neighbours_device(self, cat: DeviceCatalogue, weights=(0.4, 0.5, 0.1), min_similarity: float = 0.1,
+                          exclude_self: bool = True, max_per_row: int = 0, capacity: int | None = None,
+                          max_pairs: int | None = None) -> dict:
+        """Every pair with hybrid >= ``min_similarity``, one row per show (``tvbf_neighbours_*``):
+        the tensor-core sweep emits the candidate pairs (a superset, by the upper bound), the finish
+        rescores them in float64 and orders each row.  The sweep writes into ``capacity`` pair slots
+        (default 64 N: 8 bytes per pair, 51 MB at 100 000 shows); when it finds more candidates it runs
+        once more with room for all of them (one synchronisation per sweep reads the count).
+        ``max_pairs`` bounds the output: a ValueError is raised before anything larger than
+        ``max_pairs`` entries (2 candidates + N) is allocated.  It also bounds the default pair buffer
+        to the (max_pairs - N) / 2 candidates such an output can take; an explicit ``capacity`` is
+        used as given.
+        ``max_per_row`` > 0 keeps the first entries of every row.  Returns device tensors ``row_ptr``
+        (int64 [N + 1]), ``indices``, ``hybrid``, ``genre``, ``text``, ``metadata`` and the count
+        ``candidate_pairs``."""
+        gw, tw, mw = (float(w) for w in weights)
+        n = cat.n_shows
+        p = self._params(cat, weights, 1, min_similarity, exclude_self)
+        lib, dev = self.lib, self.device
+        cap = 64 * n if capacity is None else int(capacity)
+        if capacity is None and max_pairs is not None:
+            cap = min(cap, max(0, (int(max_pairs) - n) // 2))   # more candidates raise anyway
+        if cap < 0:
+            raise ValueError(f"capacity must be >= 0, got {cap}")
+        with torch.cuda.device(dev):
+            if lib.tvbf_neighbours_workspace_bytes(C.byref(cat.c), C.byref(p), 0) == 0:
+                check(-1, "tvbf_neighbours_workspace_bytes")
+            feats = self._folded(cat, gw, tw, mw, 1)
+            if feats is None:
+                feats = cat.c
+            count = torch.zeros((1,), dtype=torch.int64, device=dev)
+
+            def workspace(n_pairs: int) -> torch.Tensor:
+                # the sweep itself needs the workspace of 0 pairs; the finish that of the pairs it takes
+                nbytes = lib.tvbf_neighbours_workspace_bytes(C.byref(feats), C.byref(p), n_pairs)
+                if nbytes == 0:
+                    check(-1, "tvbf_neighbours_workspace_bytes")
+                return self._workspace(nbytes)
+
+            def sweep(cap: int):
+                ws = workspace(0)
+                pairs = torch.empty((max(cap, 1), 2), dtype=torch.int32, device=dev)
+                check(lib.tvbf_neighbours_sweep(C.byref(feats), C.byref(p), pairs.data_ptr(), cap, count.data_ptr(),
+                                                ws.data_ptr(), ws.numel(), self._stream()), "tvbf_neighbours_sweep")
+                return pairs, int(count.item())
+
+            def guard(n_cand: int) -> None:
+                if max_pairs is not None and 2 * n_cand + n > int(max_pairs):
+                    raise ValueError(f"the sweep found {n_cand} candidate pairs: the output needs room for "
+                                     f"{2 * n_cand + n} entries, more than max_pairs={int(max_pairs)}")
+
+            pairs, n_cand = sweep(cap)
+            while n_cand > cap:
+                guard(n_cand)
+                cap = n_cand
+                pairs = None
+                pairs, n_cand = sweep(cap)
+            guard(n_cand)
+            ws = workspace(n_cand)
+            m = 2 * n_cand + n
+            out = {"row_ptr": torch.empty((n + 1,), dtype=torch.int64, device=dev),
+                   "indices": torch.empty((m,), dtype=torch.int32, device=dev)}
+            for name in ("hybrid", "genre", "text", "metadata"):
+                out[name] = torch.empty((m,), dtype=torch.float64, device=dev)
+            check(lib.tvbf_neighbours_finish(C.byref(feats), C.byref(p), pairs.data_ptr(), n_cand, int(max_per_row),
+                                             *(out[k].data_ptr() for k in ("row_ptr", "indices", "hybrid", "genre",
+                                                                             "text", "metadata")),
+                                             ws.data_ptr(), ws.numel(), self._stream()), "tvbf_neighbours_finish")
+            nnz = int(out["row_ptr"][-1].item())
+        for name in ("indices", "hybrid", "genre", "text", "metadata"):
+            out[name] = out[name][:nnz]
+        out["candidate_pairs"] = n_cand
+        return out
+
+    @staticmethod
+    def neighbours_to_host(t: dict) -> NeighbourTable:
+        """D2H of a ``neighbours_device`` result (synchronises)."""
+        host = {k: t[k].cpu().numpy() for k in ("row_ptr", "indices", "hybrid", "genre", "text", "metadata")}
+        return NeighbourTable(**host, candidate_pairs=int(t["candidate_pairs"]))
+
+    def compute_neighbours(self, features: dict, weights=(0.4, 0.5, 0.1), min_similarity: float = 0.1,
+                           metadata_mode: str = "mean3", exclude_self: bool = True, max_per_row: int = 0,
+                           **kw) -> NeighbourTable:
+        """features dict -> every neighbour at or above ``min_similarity`` of every show, on this GPU."""
+        cat = self.ingest(features, metadata_mode, weights)
+        return self.neighbours_to_host(self.neighbours_device(cat, weights, min_similarity, exclude_self,
+                                                              max_per_row, **kw))
 
     # ------------------------------------------------------------------------------------ several GPUs
     def _params(self, cat: DeviceCatalogue, weights, k, min_similarity, exclude_self=True, row_begin=0,

@@ -13,7 +13,7 @@ import logging
 import numpy as np
 import torch
 
-from ..engine import HybridTopKEngine, TopK, default_engine
+from ..engine import HybridTopKEngine, NeighbourTable, TopK, default_engine
 
 logger = logging.getLogger(__name__)
 
@@ -161,6 +161,18 @@ class SimilarityComputer:
                                            exclude_self, list(device_ids), **kw)
         eng = self.engine if device_ids is None else HybridTopKEngine(device_ids[0])
         return eng.compute_top_k(features, weights, k, min_similarity, metadata_mode, exclude_self, **kw)
+
+    def compute_neighbours(self, features: dict, min_similarity: float = 0.1, max_per_row: int | None = None,
+                           metadata_mode: str = "mean3", normalize_weights: bool = False, **kw) -> NeighbourTable:
+        """features -> every neighbour with score >= ``min_similarity`` of every show (the production
+        loop, scripts/populate_database.py:170-218, with no ``top_n`` cut), one variable-length row per
+        show ordered by (score descending, column index ascending).  ``max_per_row`` also cuts each row
+        to that many entries: the rows then equal ``compute_top_k(k=max_per_row)``'s.  Needs
+        ``min_similarity > 0``, packed genre / metadata features and non-negative weights."""
+        weights = self._normalized_weights() if normalize_weights else \
+            (self.genre_weight, self.text_weight, self.metadata_weight)
+        return self.engine.compute_neighbours(features, weights, min_similarity, metadata_mode,
+                                              max_per_row=int(max_per_row or 0), **kw)
 
     def extend_top_k(self, features: dict, previous: TopK, k: int = 20, min_similarity: float = 0.1,
                      exclude_self: bool = True, metadata_mode: str = "mean3",

@@ -25,8 +25,10 @@ BATCH_SIZE = 5000  # reference :166
 
 
 def compute_and_store_similarities(input_dir: Path, genre_weight: float = 0.4, text_weight: float = 0.5,
-                                   metadata_weight: float = 0.1, top_n_per_show: int = 20,
+                                   metadata_weight: float = 0.1, top_n_per_show: int | None = 20,
                                    min_similarity: float = 0.1, sink=None, device_ids=None) -> dict:
+    """``top_n_per_show=None`` stores every neighbour at or above ``min_similarity`` (no top-n cut): the
+    threshold job of ``SimilarityComputer.compute_neighbours``, single GPU."""
     input_dir = Path(input_dir)
     logger.info("COMPUTING AND STORING SIMILARITIES")
     logger.info(f"Genre weight: {genre_weight}  Text weight: {text_weight}  Metadata weight: {metadata_weight}")
@@ -37,9 +39,15 @@ def compute_and_store_similarities(input_dir: Path, genre_weight: float = 0.4, t
     computer = SimilarityComputer(genre_weight=genre_weight, text_weight=text_weight,
                                   metadata_weight=metadata_weight)
     # production conventions (reference :184-192): mean of three metadata cosines, raw weights
-    top = computer.compute_top_k(features, k=top_n_per_show, min_similarity=min_similarity,
-                                 exclude_self=True, metadata_mode="mean3", normalize_weights=False,
-                                 device_ids=device_ids)
+    if top_n_per_show is None:
+        if device_ids is not None and len(device_ids) > 1:
+            raise ValueError("every neighbour above the threshold (top_n_per_show=None) runs on one GPU")
+        top = computer.compute_neighbours(features, min_similarity=min_similarity, metadata_mode="mean3",
+                                          normalize_weights=False)
+    else:
+        top = computer.compute_top_k(features, k=top_n_per_show, min_similarity=min_similarity,
+                                     exclude_self=True, metadata_mode="mean3", normalize_weights=False,
+                                     device_ids=device_ids)
     sink = sink if sink is not None else InMemorySimilaritySink()
     total_records_stored = store_similarity_batches(top, show_ids, sink)
     return finish_stats(sink, total_records_stored, top.flagged_rows, top_n_per_show, min_similarity)
@@ -48,7 +56,8 @@ def compute_and_store_similarities(input_dir: Path, genre_weight: float = 0.4, t
 def store_similarity_batches(top, show_ids, sink) -> int:
     """The storage half of the reference loop: delete-all up front (reference :156-162), then one
     ``bulk_store_all_similarities(batch, clear_existing=False)`` per 5000 shows (:223-234).  A sink
-    with ``bulk_store_records`` gets the columnar batch instead of 5000 x k dicts."""
+    with ``bulk_store_records`` gets the columnar batch instead of 5000 x k dicts.  ``top`` is a
+    ``TopK`` or a ``NeighbourTable`` (both slice into the same record shape)."""
     ids = np.asarray(list(show_ids))
     n = len(ids)
     columnar = getattr(sink, "bulk_store_records", None)
@@ -119,6 +128,8 @@ def main(argv=None, sink=None):
     parser.add_argument("--input-dir", type=str, default="data/processed")
     parser.add_argument("--top-n", type=int, default=20)
     parser.add_argument("--min-similarity", type=float, default=0.1)
+    parser.add_argument("--all-above-threshold", action="store_true",
+                        help="Store every neighbour with score >= --min-similarity (no --top-n cut)")
     parser.add_argument("--skip-metadata", action="store_true", help="Skip metadata sync (only compute similarities)")
     parser.add_argument("--skip-test", action="store_true", help="Skip recommendation testing")
     parser.add_argument("--genre-weight", type=float, default=0.4)
@@ -140,7 +151,8 @@ def main(argv=None, sink=None):
         else:
             logger.info("\n⊘ Skipping metadata sync")
         stats = compute_and_store_similarities(input_dir, args.genre_weight, args.text_weight, args.metadata_weight,
-                                               args.top_n, args.min_similarity, sink=sink)
+                                               None if args.all_above_threshold else args.top_n,
+                                               args.min_similarity, sink=sink)
         if not args.skip_test:
             verify_recommendations(service, input_dir / "shows_metadata.csv", num_tests=3)
         else:
