@@ -234,7 +234,28 @@ def _sharded(eng, cat, w, k, ms, world, tuning):
                   ("indices", "counts", "hybrid", "genre", "text", "metadata")))
 
 
-def test_random_job_sequence_on_one_engine(engine, fresh):
+def _assert_same_stats(got, exp, what):
+    for name, d in exp.items():
+        for q, x in d.items():
+            if isinstance(x, float):
+                assert np.isclose(got[name][q], x, rtol=1e-9, atol=1e-12), (what, name, q)
+            else:
+                assert got[name][q] == x, (what, name, q)
+
+
+def _assert_stats_refuse_signed(eng, cat, what):
+    from tvbingefriend_recommendation_service_b200._lib import TvbfError
+
+    assert cat.c.text_signed, what
+    with pytest.raises(TvbfError, match="signed text"):
+        eng.similarity_stats(cat, W)
+
+
+def test_random_job_sequence_on_one_engine_refusing_signed_stats(engine, fresh):
+    """30 seeded jobs of every entry point through one engine, each compared with a fresh engine and
+    the oracle.  A statistics job on the signed-text catalogue of the pool must be refused
+    (``TvbfError``: the streaming statistics take non-negative text only); the refusal is also
+    checked after the sequence, whether or not the draw reached such a job."""
     from tvbingefriend_recommendation_service_b200._lib import TvbfError
     from tvbingefriend_recommendation_service_b200.synthetic import WEIGHT_SWEEP
 
@@ -320,14 +341,25 @@ def test_random_job_sequence_on_one_engine(engine, fresh):
                 got.row_begin = b
                 assert_topk_matches(got, f, spread_rows(b, e, 3), W, k, MS)
             else:
-                got = engine.similarity_stats(cat, W)
-                exp = fresh.similarity_stats(ref, W)
-                for name, d in exp.items():
-                    for q, x in d.items():
-                        if isinstance(x, float):
-                            assert np.isclose(got[name][q], x, rtol=1e-9, atol=1e-12), (log[-1], name, q)
-                        else:
-                            assert got[name][q] == x, (log[-1], name, q)
+                if POOL[key][4]:
+                    # signed text: the streaming statistics refuse it, on a recycled catalogue as well
+                    _assert_stats_refuse_signed(engine, cat, log[-1])
+                    log.append("  refused (signed text)")
+                    continue
+                _assert_same_stats(engine.similarity_stats(cat, W), fresh.similarity_stats(ref, W), log[-1])
+        # whether the seeded draw reaches a stats job on the signed catalogue or not: it is refused
+        # through the long-lived engine, and the engine still computes statistics afterwards
+        signed = next(i for i, entry in enumerate(POOL) if entry[4])
+        cat = live.get(signed)
+        if cat is None:
+            feats.setdefault(signed, catalogue(*POOL[signed][:3], seed=100 + signed, genres=POOL[signed][3],
+                                               signed=True))
+            cat = upload(engine, feats[signed], "ingest")
+        log.append(f"after the sequence: stats on signed catalogue {signed}")
+        _assert_stats_refuse_signed(engine, cat, log[-1])
+        f = catalogue(300, 200, seed=7)
+        _assert_same_stats(engine.similarity_stats(engine.ingest(f), W),
+                           fresh.similarity_stats(upload(fresh, f, "upload"), W), log[-1])
     except Exception as e:
         raise AssertionError("job log (seeded, replayable):\n" + "\n".join(log)) from e
     finally:

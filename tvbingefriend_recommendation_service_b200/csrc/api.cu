@@ -2021,6 +2021,10 @@ int tvbf_similarity_stats(const tvbf_features* f, const tvbf_params* p, void* ac
                "streaming statistics need binary genre (at most 64 columns) / one-hot metadata features");
   TVBF_REQUIRE(!f->bits_folded, "streaming statistics need the plain text operand (bits_folded is set)");
   TVBF_REQUIRE(f->text_cols == 0, "streaming statistics need the plain text operand (text_cols is set)");
+  // the epilogue's extrema (atomicMin / atomicMax on raw float bits) and histograms (bins of [0, hi))
+  // hold for non-negative elements only
+  TVBF_REQUIRE(!f->text_signed,
+               "streaming statistics need non-negative text: signed text (negative values) is not supported");
   TVBF_REQUIRE(p->genre_weight >= 0.0 && p->text_weight >= 0.0 && p->metadata_weight >= 0.0,
                "streaming statistics need non-negative weights");
   tvbf_params q = *p;

@@ -369,7 +369,11 @@ struct MatrixScorer {
   __device__ __forceinline__ Scores operator()(int i, int j) const {
     const size_t e = static_cast<size_t>(i) * n + j;
     Scores s;
-    s.h = h[e]; s.g = g[e]; s.t = t[e]; s.m = m[e];
+    // -0.0 and +0.0 are one score: the order-preserving keys would rank +0.0 first whatever the
+    // columns, so a hybrid zero is read as +0.0 and the tie falls to the lower column
+    const double hv = h[e];
+    s.h = hv == 0.0 ? 0.0 : hv;
+    s.g = g[e]; s.t = t[e]; s.m = m[e];
     return s;
   }
 };

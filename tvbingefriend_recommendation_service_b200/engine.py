@@ -1845,6 +1845,8 @@ class HybridTopKEngine:
                     m.sum_duplicates()
                     m.sort_indices()
                 n, d = m.shape
+                if m.nnz == 0:       # every row is zero: so is every cosine (and there is nothing to upload)
+                    return torch.zeros((n, n), dtype=torch.float64, device=dev)
                 indptr = torch.from_numpy(m.indptr.astype(np.int64)).to(dev)
                 indices = torch.from_numpy(m.indices.astype(np.int32)).to(dev)
                 raw = torch.from_numpy(np.ascontiguousarray(m.data, dtype=np.float64)).to(dev)
@@ -1908,12 +1910,29 @@ class HybridTopKEngine:
         matrices (``tvbf_text_moments``: column sums, [64, V], [32, V] and, memory permitting, the
         [V, V] vocabulary Gram matrix) and the hybrid's moments are assembled from them, so mean and
         std agree with the reference's float64 to ~1e-9 (genre / metadata elements are fp32 values
-        summed in float64: ~1e-8).  min / max: exact zeros and exactly rescored maxima; otherwise the
-        fp32 / fp16 element value.  median to one histogram bin (``median_resolution``)."""
+        summed in float64: ~1e-8); std has an absolute floor of ~2^-26 sqrt(rms^2 + 2 / (N - 1)), where
+        the one-pass variance cancels (nearly equal elements, tiny N).  min: an exact 0.0 when some element is zero, otherwise the fp32
+        element value.  median to one histogram bin (``median_resolution``).
+
+        The text and hybrid max are the float64 maxima, bit-identical to ``tvbf_score_pairs`` of the
+        pair that attains them.  The sweep keeps the pair with the largest fp16 / fp32 element value
+        of every epilogue warp; many pairs can share that value, so the true maximum need not be among
+        them.  Their best exact score tau is a score some pair attains, hence a lower bound of the
+        maximum.  An exact top-1 job at ``min_similarity = tau`` (``top_k_device``: certified, its
+        scores those of ``tvbf_score_pairs``) then finds every row's best neighbour scoring >= tau;
+        the largest of those is the maximum over all pairs, in O(N) memory however many pairs tie.
+        Text runs with weights (0, 1, 0), the hybrid with ``weights``; tau <= 0 means the maximum is
+        0 and needs no job.  genre / metadata max: the fp32 element value.
+
+        Needs N >= 2 (ValueError: the upper triangle is empty) and non-negative text: signed text
+        (embeddings) raises ``TvbfError``; the N x N path (``matrix_stats``) takes it."""
         gw, tw, mw = (float(w) for w in weights)
+        n = cat.n_shows
+        if n < 2:
+            raise ValueError(f"similarity statistics need at least 2 shows: the upper triangle of {n} x {n} "
+                             "is empty")
         p = self._params(cat, (gw, tw, mw), 20, 0.5)
         lib, dev = self.lib, self.device
-        n = cat.n_shows
         with torch.cuda.device(dev):
             nbytes = int(lib.tvbf_stats_accum_bytes())
             assert nbytes == self._STATS_DTYPE.itemsize, (nbytes, self._STATS_DTYPE.itemsize)
@@ -1934,7 +1953,13 @@ class HybridTopKEngine:
                 check(lib.tvbf_score_pairs(C.byref(cat.c), C.byref(p), pd.data_ptr(), pk.shape[0], out4.data_ptr(),
                                            self._stream()), "tvbf_score_pairs")
                 o = out4.cpu().numpy()
-                exact_max = {"text_similarity": float(o[:, 2].max()), "hybrid_similarity": float(o[:, 0].max())}
+                for name, w, col in (("text_similarity", (0.0, 1.0, 0.0), 2), ("hybrid_similarity", (gw, tw, mw), 0)):
+                    tau = float(o[:, col].max())
+                    if tau > 0.0:
+                        top = self.to_host(self.top_k_device(cat, w, 1, tau))
+                        best = getattr(top, "text" if col == 2 else "hybrid")[top.counts > 0, 0]
+                        tau = float(best.max(initial=tau))
+                    exact_max[name] = tau
             moments = None
             if exact_moments:
                 v = int(cat.c.vocab)

@@ -136,8 +136,13 @@ class SimilarityComputer:
         """The four ``get_similarity_statistics`` results of scripts/compute_similarities.py:119-131
         for catalogues whose N x N matrices cannot exist: one streaming tensor-core sweep (defaults =
         this class' conventions: hstack metadata, normalised weights).  mean / std / min / max as
-        the reference's, median to ``median_resolution``.  Needs binary genre and one-hot metadata
-        features."""
+        the reference's, median to ``median_resolution``.  Needs at least 2 shows (ValueError),
+        binary genre and one-hot metadata features and non-negative text: signed text raises
+        ``TvbfError`` (``get_similarity_statistics`` on the N x N matrices takes it)."""
+        n = int(features["genre_features"].shape[0])
+        if n < 2:
+            raise ValueError(f"similarity statistics need at least 2 shows: the upper triangle of {n} x {n} "
+                             "is empty")
         weights = self._normalized_weights() if normalize_weights else \
             (self.genre_weight, self.text_weight, self.metadata_weight)
         cat = self.engine.ingest(features, metadata_mode, weights)

@@ -10,6 +10,7 @@ from pathlib import Path
 
 import numpy as np
 
+from .._lib import TvbfError
 from ..ml.similarity_computer import SimilarityComputer
 
 logger = logging.getLogger(__name__)
@@ -75,7 +76,14 @@ def compute_similarities(features: dict, genre_weight: float = 0.4, text_weight:
     else:
         logger.info(f"⊘ {n_shows} shows: 4 N x N float64 matrices = {32 * n_shows * n_shows / 1e9:.1f} GB do not fit; "
                     "computing their statistics with the streaming sweep")
-        all_stats = computer.compute_similarity_statistics(features)
+        try:
+            all_stats = computer.compute_similarity_statistics(features)
+        except TvbfError as e:
+            if "signed text" not in str(e):
+                raise
+            raise ValueError(f"the streaming statistics do not take text features with negative values ({e}); "
+                             "the N x N matrices do: raise --max-matrix-bytes (32 * N^2 bytes are needed, "
+                             f"{32 * n_shows * n_shows} here)") from e
         similarities = {name: None for name in SIM_NAMES}
         similarities["statistics"] = all_stats
     for sim_name in SIM_NAMES:
