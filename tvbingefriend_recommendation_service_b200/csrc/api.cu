@@ -359,10 +359,15 @@ int fill_k1_params(const tvbf_features* f, const tvbf_params* p, const Plan& pl,
     kp.wait_ns = env_wait >= 0 ? env_wait : 64;
   }
   // 16 epilogue warps when the tile's MMAs (~0.27 us per 64-wide k-block) cannot hide the epilogue
-  // (~30 us per tile with 8 warps); bits 28-29 of tuning: 0 auto, 1 off, 2 on
+  // (~30 us per tile with 8 warps); bits 28-29 of tuning: 0 auto, 1 off, 2 on.
+  // A folded operand costs one FMA and two compares per element, so 8 warps keep up with far shorter
+  // tiles, and their kernel keeps a sixth ring stage.  Measured on one B200 (1000 W): C3 after merging
+  // (K_pad 4 096, 64 k-blocks) 8 warps 22.2-22.3 ms against 16 warps 23.0-23.2 ms for the candidate
+  // pass; P80k (K_pad 576, 9 k-blocks) needs 16.  The cut at 32 k-blocks lies between the two.
   {
     const int wide_req = (p->tuning >> 28) & 0x3;
-    kp.wide_epilogue = (wide_req == 2 || (wide_req == 0 && f->k_pad / 64 <= 96)) && pl.kp <= 64 ? 1 : 0;
+    const int wide_max_kb = f->bits_folded ? 32 : 96;
+    kp.wide_epilogue = (wide_req == 2 || (wide_req == 0 && f->k_pad / 64 <= wide_max_kb)) && pl.kp <= 64 ? 1 : 0;
   }
   kp.progress = reinterpret_cast<unsigned int*>(ws + pl.off_count);
   kp.kp = pl.kp;
